@@ -25,6 +25,8 @@ One JSON line on rank 0:
 `--impl reference` times that CPU port alone (the Scala reference cannot run here: no JVM; its loops as written are infeasible beyond
 configs[0]/[1] — SURVEY.md §8d) on rank 0 with every host thread the process may use and prints the same line with "impl": "reference".
 `--workload c1|c2` add the as-written sequential and `.par` CPU legs; `--workload ksplit` is BASELINE configs[4] (K-split item-item sweep).
+`--dump-outputs DIR` writes the UBM and IBM top-500 lists that the last timed step computed for a fixed, seeded sample of rank 0's test
+users to DIR/*.npy (float64), so that two builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -45,6 +47,8 @@ sys.path.insert(0, str(ROOT))
 K_TOP = 500
 N_TEST_USERS = 110000          # BASELINE configs[3]
 METRIC = "scored (test-user, song) pairs/sec, UBM+IBM with top-500"
+DUMP_USERS = 2048              # --dump-outputs: 2 models x (song, score) x 2048 x 500 float64 = 33 MB, under the 64 MB a dump may take
+DUMP_SEED = 0
 
 
 def log(*a):
@@ -282,7 +286,14 @@ def main():
     ap.add_argument("--ksplit-mode", default="auto", choices=["auto", "fused", "nccl"])
     ap.add_argument("--ksplit-panel", type=int, default=4096)
     ap.add_argument("--ksplit-verify", action="store_true", help="check every row of every panel against the oracle (small S only)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help=f"write the top-{K_TOP} lists of UBM and IBM (song, score, len) that the last timed step computed for {DUMP_USERS} test users "
+                         f"of rank 0 (seeded sample, ids in users.npy) as DIR/<model>_<array>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "ksplit"):
+        ap.error("--dump-outputs covers the GPU scoring path (--impl ours, workloads msd and c1-c3)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -363,20 +374,31 @@ def main():
             joined[model] = (block, block[:n_mine * k * 4].view(torch.int32).view(n_mine, k), block[song_b:song_b + score_b].view(torch.float64).view(n_mine, k),
                              block[song_b + score_b:song_b + score_b + n_mine * 4].view(torch.int32))
 
-    def score_model(model):
-        """One model for this rank's part of the job, result left on the device."""
+    # --dump-outputs: the sampled rows of rank 0's lists are copied aside right after each model, on the library stream, because the next
+    # model's mr_topk_device reuses the result block
+    dump_rows = None
+    if args.dump_outputs and rank == 0:
+        pick = np.random.default_rng(DUMP_SEED).choice(n_mine, min(n_mine, DUMP_USERS), replace=False)
+        dump_rows = torch.from_numpy(np.sort(pick)).cuda()
+    dumped = {}
+
+    def score_model(model, keep=None):
+        """One model for this rank's part of the job, result left on the device; `keep` receives the dump rows of its lists."""
         check(lib.mr_topk_device(h, model, 0.0, 0, k))
         if by_songs:      # exchange step of the song partitioning: all-to-all of the ranked lists, then the join (mr_topk_merge), in stream order
             with torch.cuda.stream(stream):
                 parts = exchange_song_partitions(*mr.topk_device_tensors(k), ds.U, world, rank)
             mr.mergeTopK(*parts, *joined[model][1:])
+        if keep is not None:
+            with torch.cuda.stream(stream):
+                keep[model] = [t.index_select(0, dump_rows) for t in (joined[model][1:] if by_songs else mr.topk_device_tensors(k))]
 
-    def step_device(rebuild=True):
+    def step_device(rebuild=True, keep=None):
         if rebuild and item_space:
             check(lib.mr_invalidate_prepared(h))
             check(lib.mr_prepare(h))
-        score_model(_lib.MR_UBM)
-        score_model(_lib.MR_IBM)
+        score_model(_lib.MR_UBM, keep)
+        score_model(_lib.MR_IBM, keep)
 
     def barrier():
         torch.cuda.synchronize()
@@ -384,12 +406,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, n):
+    def timed(fn, n, last=None):
+        """n steps between two events on the library stream; the n-th step is `last` where one is given."""
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         ev0.record(stream)
-        for _ in range(n):
-            fn()
+        for i in range(n):
+            (last if last is not None and i == n - 1 else fn)()
         ev1.record(stream)
         ev1.synchronize()
         barrier()
@@ -401,8 +424,17 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     l0 = mr.info()["launches"]
-    dev_ms = timed(step_device, args.steps)
+    dev_ms = timed(step_device, args.steps, last=(lambda: step_device(keep=dumped)) if dump_rows is not None else None)
     launches = mr.info()["launches"] - l0
+    if dump_rows is not None:       # timed() ends in a device synchronise
+        dump_dir = Path(args.dump_outputs)
+        dump_dir.mkdir(parents=True, exist_ok=True)
+        arrays = {"users": my_u0 + dump_rows.cpu().numpy()}
+        for model, name in ((_lib.MR_UBM, "ubm"), (_lib.MR_IBM, "ibm")):
+            arrays.update({f"{name}_{part}": t.cpu().numpy() for part, t in zip(("song", "score", "len"), dumped[model])})
+        for name, a in arrays.items():
+            np.save(dump_dir / f"{name}.npy", a.astype(np.float64))
+        log(f"[rank {rank}] top-{k} lists of {len(arrays['users'])} sampled users written to {dump_dir}")
     # secondary: steady state of a service that keeps the head rows of its train set (no precompute in the step)
     steady_ms = timed(lambda: step_device(rebuild=False), args.steps)
 

@@ -17,6 +17,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -32,9 +33,14 @@ UBM, IBM = 0, 1
 
 
 def build(force: bool = False) -> Path:
-    """Compile mr_oracle.c → oracle/_build/libmroracle.so (gcc, OpenMP, no FMA contraction)."""
-    _BUILD.mkdir(exist_ok=True)
+    """Compile mr_oracle.c → oracle/_build/libmroracle.so (gcc, OpenMP, no FMA contraction).  A tree that cannot be written (a
+    read-only checkout running bench.py) gets the library in a temporary directory instead."""
+    global _SO
     if force or not _SO.exists() or _SO.stat().st_mtime < _SRC.stat().st_mtime:
+        if os.access(_BUILD if _BUILD.exists() else _HERE, os.W_OK):
+            _BUILD.mkdir(exist_ok=True)
+        else:
+            _SO = Path(tempfile.mkdtemp(prefix="mroracle-")) / _SO.name
         cmd = ["gcc", "-O2", "-std=c11", "-fopenmp", "-ffp-contract=off", "-fvisibility=hidden", "-shared", "-fPIC",
                str(_SRC), "-o", str(_SO), "-lm"]
         subprocess.run(cmd, check=True)

@@ -165,6 +165,33 @@ int mr_blend_dense(mr_handle* h, int kind, double param, uint64_t seed, const do
 int mr_evaluate_dense(mr_handle* h, const double* scores_UxS, int n_users, int n_songs, const int64_t* lab_rowptr, const int32_t* lab_col,
                       int n_thresholds, double* out_map);
 
+/* evaluateModel(model) (MR:521-639) for models too large to materialise: the same metric, streamed over the batches of the scoring
+ * pipeline, with the same bits as mr_evaluate_dense on the materialised model.  It decomposes into integers that add exactly over batches,
+ * user shards and song windows (DESIGN.md §4.5): per label song c and threshold t, pred_t(c) = test users whose normalised score for c
+ * exceeds TH[t] (MR:541-553), tp_t(c) = the same among the users labelled with c, nlab(c) = users labelled with c; only the global min /
+ * max (MR:524-529) must be known first.  A distributed caller runs range -> all-reduce(min, max) -> counts -> all-reduce(sum) -> finish
+ * (INTEGRATION.md).  model / param / seed as in mr_topk; the LC alpha must be in [0, 1] (MR_ERR_PARAM_RANGE), as for getTopK.
+ *
+ * Range pass: min and max over the pairs this handle scores (its shard, its song window) that the model emits (listened pairs are not
+ * emitted, MR:109); +inf / -inf when it emits none. */
+int mr_eval_range(mr_handle* h, int model, double param, uint64_t seed, double* out_min, double* out_max);
+/* Count pass, with the global mn / mx.  lab_rowptr [U + 1] / lab_col: the labels of the CURRENT shard's test users, rows ascending and
+ * unique (song ids >= n_songs are label-only songs).  new_songs [n_new]: the distinct label songs of ALL test users (newSongs, MR:72, 79),
+ * strictly ascending, containing every label song of this shard (MR_ERR_BAD_ARG naming the first one missing).  Outputs, row c for
+ * new_songs[c]: out_pred / out_tp [n_new][n_thresholds], out_nlab [n_new].  A label entry (u, c) is counted by the handle whose shard holds
+ * u and whose song window holds c, a label-only song by none (its AP is 0 whatever its counts), so the sums over any partitioning of
+ * users and songs are the counts of the whole model.  n_thresholds = 10 (MR:590) or 11 (DIST:395).  On a single-batch item-space shard
+ * the count pass reuses the score panels of an mr_eval_range of the same (model, param, seed) just before it: one scoring pass, not two. */
+int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double mn, double mx, int n_thresholds,
+                   const int64_t* lab_rowptr, const int32_t* lab_col, const int32_t* new_songs, int n_new,
+                   int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab);
+/* Host only (no handle, no GPU): precision tp / pred and recall tp / nlab per threshold (MR:561-579), the per-song AP (MR:600-610,
+ * out_ap [n_new], may be NULL) and the mean over the n_new songs (MR:626), in the operation order of mr_evaluate_dense. */
+int mr_eval_finish(const int64_t* pred, const int64_t* tp, const int64_t* nlab, int n_new, int n_thresholds, double* out_ap, double* out_map);
+/* Host only: out[t] = the least double x with RN(RN(x - mn) / RN(mx - mn)) > TH[t], TH = 0.0, 0.1, ..., 1.0, or +inf when no x in
+ * [mn, mx] qualifies (always when mx - mn is not > 0).  The count pass predicts a pair at t iff its score >= out[t]. */
+int mr_eval_cutoffs(double mn, double mx, int n_thresholds, double* out);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.

@@ -22,7 +22,8 @@ TIMING_NAMES = ["expand", "count", "agg_ubm", "agg_ibm", "topk", "other", "preco
 SYMBOLS = ["mr_create", "mr_destroy", "mr_last_error", "mr_load", "mr_set_test_users", "mr_prepare", "mr_prepare_async", "mr_counts_ubm", "mr_counts_ibm", "mr_gram_rows_device", "mr_gram_rows_scatter", "mr_peer_alloc", "mr_peer_open", "mr_peer_close",
            "mr_similarity_ubm", "mr_similarity_ibm", "mr_score_dense", "mr_blend_dense", "mr_evaluate_dense", "mr_topk", "mr_topk_device",
            "mr_topk_fetch", "mr_topk_device_ptrs", "mr_set_option", "mr_invalidate_prepared", "mr_score_users", "mr_score_songs", "mr_map_at_k", "mr_write_model", "mr_format_double", "mr_topk_packed", "mr_topk_merge", "mr_gram_rows_scatter_async", "mr_peer_signal", "mr_peer_wait", "mr_sync", "mr_get_timing", "mr_reset_timing", "mr_set_profile", "mr_get_info", "mr_stream",
-           "mr_ingest_tsv", "mr_ingest_error", "mr_ingest_dims", "mr_ingest_get", "mr_ingest_free"]
+           "mr_ingest_tsv", "mr_ingest_error", "mr_ingest_dims", "mr_ingest_get", "mr_ingest_free",
+           "mr_eval_range", "mr_eval_counts", "mr_eval_finish", "mr_eval_cutoffs"]
 
 _lib = None
 
@@ -96,5 +97,9 @@ def load():
     lib.mr_ingest_get.argtypes = [vp, i32, C.POINTER(vp), C.POINTER(i64)]
     lib.mr_ingest_free.argtypes = [vp]
     lib.mr_ingest_free.restype = None
+    lib.mr_eval_range.argtypes = [vp, i32, dbl, u64, C.POINTER(dbl), C.POINTER(dbl)]
+    lib.mr_eval_counts.argtypes = [vp, i32, dbl, u64, dbl, dbl, i32, vp, vp, vp, i32, vp, vp, vp]
+    lib.mr_eval_finish.argtypes = [vp, vp, vp, i32, i32, vp, C.POINTER(dbl)]
+    lib.mr_eval_cutoffs.argtypes = [dbl, dbl, i32, vp]
     _lib = lib
     return lib

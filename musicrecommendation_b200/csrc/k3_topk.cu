@@ -13,17 +13,6 @@
 
 namespace mr {
 
-__device__ __forceinline__ double blend_score(int model, long long su, long long si, double rsu, double rds, double alpha,
-                                              double oma, bool pick_ibm) {
-  switch (model) {
-    case MODEL_UBM: return __dmul_rn(__ll2double_rn(su), rsu);
-    case MODEL_IBM: return __dmul_rn(__ll2double_rn(si), rds);
-    case MODEL_LC:
-      return __dadd_rn(__dmul_rn(__dmul_rn(__ll2double_rn(su), rsu), alpha), __dmul_rn(__dmul_rn(__ll2double_rn(si), rds), oma));
-    default: return pick_ibm ? __dmul_rn(__ll2double_rn(si), rds) : __dmul_rn(__ll2double_rn(su), rsu);
-  }
-}
-
 // ---------------------------------------------------------------- listened-pair sentinel (getModel's filter, MR:109)
 // te_end[u] = end of the row's scored columns: te_ptr[u + 1], or — with a song window — the end of the in-window prefix of the row
 __global__ void mask_listened_kernel(const long long* __restrict__ te_ptr, const long long* __restrict__ te_end, const int* __restrict__ te_col,

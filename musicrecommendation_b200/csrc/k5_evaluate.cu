@@ -104,6 +104,175 @@ int launch_evaluate(const double* scores, int n_users, int n_songs, const long l
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
+// The same metric streamed over the batches of the scoring pipeline (DESIGN.md §4.5), for models too large to materialise.  Per label
+// song c and threshold t it needs only integers: pred_t(c) = #users whose normalised score for c exceeds TH[t], tp_t(c) = the same over
+// the users labelled with c, nlab(c) = #users labelled with c; they add exactly over batches, user shards and song windows.  The
+// normalisation f(x) = RN(RN(x - mn) / RN(mx - mn)) is monotone in x, so f(x) > TH[t] <=> x >= c_t with host-computed cutoffs
+// (mr_eval_cutoffs): the kernels compare bit patterns of non-negative doubles and never divide.  A pair's bucket is the number of
+// cutoffs <= its score (it is predicted at exactly the thresholds t < bucket); counts are kept per bucket, the host sums them up.
+// ---------------------------------------------------------------------------------------------------------------------
+constexpr int kEvalThreads = 256;
+constexpr int kEvalTile = 4 * kEvalThreads;   // songs per CTA column tile: 4 consecutive songs per thread (two 16-byte loads per panel)
+constexpr int kEvalRows = 512;                // at most this many panel rows per eval_count_kernel CTA: its histogram is flushed once per CTA
+
+// Score bit patterns of the songs s .. s+3 of one panel row; ok = emitted (not listened, inside the row), exactly as scan_row (k3_topk.cu)
+__device__ __forceinline__ void eval_quad(const BlendParams& bp, const long long* ru, const long long* ri, const uint64_t* rsel, int s,
+                                          int n_songs, double rsu, const double (&rd)[4], unsigned long long (&kb)[4], bool (&ok)[4]) {
+  long long a[4] = {-1, -1, -1, -1}, b[4] = {-1, -1, -1, -1};
+  if (bp.model != MODEL_IBM) {
+    const longlong2 x = *reinterpret_cast<const longlong2*>(ru + s), y = *reinterpret_cast<const longlong2*>(ru + s + 2);
+    a[0] = x.x; a[1] = x.y; a[2] = y.x; a[3] = y.y;
+  }
+  if (bp.model != MODEL_UBM) {
+    const longlong2 x = *reinterpret_cast<const longlong2*>(ri + s), y = *reinterpret_cast<const longlong2*>(ri + s + 2);
+    b[0] = x.x; b[1] = x.y; b[2] = y.x; b[3] = y.y;
+  }
+  const uint64_t selw = bp.model >= MODEL_AGG ? rsel[s >> 6] >> (s & 63) : 0;
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    ok[t] = s + t < n_songs && (bp.model == MODEL_IBM || a[t] >= 0) && (bp.model == MODEL_UBM || b[t] >= 0);
+    kb[t] = ok[t] ? static_cast<unsigned long long>(__double_as_longlong(
+                        blend_score(bp.model, a[t], b[t], rsu, rd[t], bp.alpha, bp.one_minus_alpha, (selw >> t) & 1ULL)))
+                  : 0ULL;
+  }
+}
+
+__device__ __forceinline__ void eval_rsd4(const BlendParams& bp, const double* rsd, int s, int n_songs, double (&rd)[4]) {
+#pragma unroll
+  for (int t = 0; t < 4; ++t) rd[t] = (bp.model != MODEL_UBM && s + t < n_songs) ? rsd[s + t] : 0.0;
+}
+
+__device__ __forceinline__ int eval_bucket(const EvalCounts& ec, unsigned long long kb) {
+  int bk = 0;
+#pragma unroll
+  for (int t = 0; t < 11; ++t) bk += (t < ec.n_thresholds && kb >= ec.cut[t]) ? 1 : 0;
+  return bk;
+}
+
+// min / max of the emitted scores of a slice: warp shuffles, one pair of atomics per warp that saw an emitted pair
+__global__ void __launch_bounds__(kEvalThreads)
+eval_range_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+                  const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_songs, const double* __restrict__ rsa,
+                  const double* __restrict__ rsd, unsigned long long* __restrict__ mm) {
+  const int b = blockIdx.y;
+  const double rsu = rsa[u0 + b];
+  const long long* ru = sint_u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
+  const long long* ri = sint_i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
+  const uint64_t* rsel = sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
+  unsigned long long lo = ~0ULL, hi = 0ULL;
+  for (int s = 4 * (blockIdx.x * kEvalThreads + static_cast<int>(threadIdx.x)); s < n_songs; s += 4 * kEvalThreads * gridDim.x) {
+    double rd[4]; unsigned long long kb[4]; bool ok[4];
+    eval_rsd4(bp, rsd, s, n_songs, rd);
+    eval_quad(bp, ru, ri, rsel, s, n_songs, rsu, rd, kb, ok);
+#pragma unroll
+    for (int t = 0; t < 4; ++t)
+      if (ok[t]) { lo = kb[t] < lo ? kb[t] : lo; hi = kb[t] > hi ? kb[t] : hi; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const unsigned long long a = __shfl_xor_sync(0xffffffffu, lo, o), c = __shfl_xor_sync(0xffffffffu, hi, o);
+    lo = a < lo ? a : lo; hi = c > hi ? c : hi;
+  }
+  if ((threadIdx.x & 31) == 0 && lo != ~0ULL) { atomicMin(mm, lo); atomicMax(mm + 1, hi); }
+}
+
+// Prediction counts of the label songs.  A CTA owns a tile of 1024 songs (4 per thread) over `rows` panel rows (<= 512: the flush, one
+// global atomic per non-zero (song, bucket) per CTA, is paid once per up to 512 rows); each thread counts its own
+// songs' buckets in a private slice of the shared histogram (no shared atomics), then flushes the non-zero entries with global atomics.
+// Threads whose 4 songs are no label song read nothing: the kernel moves only the panel sectors of label songs.
+__global__ void __launch_bounds__(kEvalThreads)
+eval_count_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+                  const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_users, int n_songs, const double* __restrict__ rsa,
+                  const double* __restrict__ rsd, int rows, EvalCounts ec) {
+  __shared__ unsigned int hist[11 * 4 * kEvalThreads];   // [bucket - 1][song of the thread][thread]
+  const int tid = threadIdx.x;
+  const int s = blockIdx.x * kEvalTile + 4 * tid;
+  int li[4];
+  bool any = false;
+#pragma unroll
+  for (int t = 0; t < 4; ++t) { li[t] = s + t < n_songs ? ec.colmap[s + t] : -1; any = any || li[t] >= 0; }
+  if (!any) return;
+  const int nh = 4 * ec.n_thresholds;
+  for (int i = 0; i < nh; ++i) hist[i * kEvalThreads + tid] = 0;
+  double rd[4];
+  eval_rsd4(bp, rsd, s, n_songs, rd);
+  const int r0 = blockIdx.y * rows, r1 = min(n_users, r0 + rows);
+#pragma unroll 4
+  for (int b = r0; b < r1; ++b) {
+    const long long* ru = sint_u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
+    const long long* ri = sint_i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
+    const uint64_t* rsel = sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
+    unsigned long long kb[4]; bool ok[4];
+    eval_quad(bp, ru, ri, rsel, s, n_songs, bp.model == MODEL_IBM ? 0.0 : rsa[u0 + b], rd, kb, ok);
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const int bk = (ok[t] && li[t] >= 0) ? eval_bucket(ec, kb[t]) : 0;
+      if (bk) hist[((bk - 1) * 4 + t) * kEvalThreads + tid] += 1;
+    }
+  }
+  for (int k = 0; k < ec.n_thresholds; ++k)
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      const unsigned int v = hist[(k * 4 + t) * kEvalThreads + tid];
+      if (v) atomicAdd(ec.pred_b + static_cast<long long>(li[t]) * ec.n_thresholds + k, static_cast<unsigned long long>(v));
+    }
+}
+
+// One warp per test user of the slice: its label songs inside the scored columns add to nlab, and to tp in the bucket of their score
+__global__ void __launch_bounds__(128)
+eval_label_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+                  const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_users, int n_songs, const double* __restrict__ rsa,
+                  const double* __restrict__ rsd, EvalCounts ec) {
+  const int lane = threadIdx.x & 31;
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (b >= n_users) return;
+  const int u = u0 + b;
+  for (long long e = ec.lab_ptr[u] + lane; e < ec.lab_ptr[u + 1]; e += 32) {
+    const int c = ec.lab_col[e] - ec.col_lo;
+    if (c < 0 || c >= n_songs) continue;                  // another song window's label, or a label-only song (id >= S)
+    const int li = ec.colmap[c];
+    if (li < 0) continue;                                  // cannot happen: mr_eval_counts checks new_songs covers every label
+    atomicAdd(ec.nlab + li, 1ULL);
+    const long long o = static_cast<long long>(b) * spitch + c;
+    const long long a = bp.model != MODEL_IBM ? sint_u[o] : 0, x = bp.model != MODEL_UBM ? sint_i[o] : 0;
+    if (a < 0 || x < 0) continue;                          // listened: not emitted, a false negative at every threshold
+    const bool pick = bp.model >= MODEL_AGG && ((sel[static_cast<long long>(b) * sel_pitch_words + (c >> 6)] >> (c & 63)) & 1ULL);
+    const unsigned long long kb = static_cast<unsigned long long>(__double_as_longlong(
+        blend_score(bp.model, a, x, rsa[u], bp.model != MODEL_UBM ? rsd[c] : 0.0, bp.alpha, bp.one_minus_alpha, pick)));
+    const int bk = eval_bucket(ec, kb);
+    if (bk) atomicAdd(ec.tp_b + static_cast<long long>(li) * ec.n_thresholds + (bk - 1), 1ULL);
+  }
+}
+
+int launch_eval_range(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+                      long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
+                      unsigned long long* mm, cudaStream_t st) {
+  if (n_songs <= 0) return 0;
+  for (int r0 = 0; r0 < n_users; r0 += 32768) {   // grid.y limit
+    const int n = min(32768, n_users - r0);
+    const long long off = static_cast<long long>(r0) * spitch;
+    const int tiles = (n_songs + kEvalTile - 1) / kEvalTile;
+    const int gx = max(1, min(tiles, (2048 + n - 1) / n));   // >= ~2048 CTAs per launch, each sweeping a long stretch of its row
+    eval_range_kernel<<<dim3(gx, n), kEvalThreads, 0, st>>>(bp, sint_u ? sint_u + off : nullptr, sint_i ? sint_i + off : nullptr, spitch,
+                                                            sel ? sel + static_cast<long long>(r0) * sel_pitch_words : nullptr, sel_pitch_words,
+                                                            u0 + r0, n_songs, rsa, rsd, mm);
+  }
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+int launch_eval_count(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+                      long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
+                      const EvalCounts& ec, cudaStream_t st) {
+  if (n_users <= 0 || n_songs <= 0) return 0;
+  if (ec.n_thresholds < 1 || ec.n_thresholds > 11) return -2;
+  const int chunks = (n_users + kEvalRows - 1) / kEvalRows, rows = (n_users + chunks - 1) / chunks;   // equal row chunks
+  const dim3 grid((n_songs + kEvalTile - 1) / kEvalTile, chunks);
+  eval_count_kernel<<<grid, kEvalThreads, 0, st>>>(bp, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, rows, ec);
+  eval_label_kernel<<<(n_users + 3) / 4, 128, 0, st>>>(bp, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, ec);
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
 // mAP@k of the ranked lists (north_star's "mAP@500"; the reference has no ranking, so this is the Million Song Dataset Challenge
 // definition, stated in include/mrscore.h at mr_map_at_k):  AP@k(u) = (sum_i [r_i in L_u] * hits_i / i) / min(|L_u|, k).
 // One warp per test user: the lanes test 32 ranks at a time against the user's ascending label row (binary search), lane 0 adds the

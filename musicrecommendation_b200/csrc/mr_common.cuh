@@ -4,6 +4,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "mr_kernels.h"
+
 namespace mr {
 
 // Fixed-point scales of the canonical arithmetic (see DESIGN.md §3): q(deg) = rint(scale / sqrt(deg)).
@@ -16,6 +18,19 @@ constexpr double kQInvUbm = 1.0 / 16777216.0;
 constexpr double kQScaleIbm = 67108864.0;         // 2^26
 constexpr double kQInvIbm = 1.0 / 67108864.0;
 constexpr long long kListened = -1;               // sentinel written into Sint at listened (u, s) pairs
+
+// fp64 score of one (user, song) pair from its Sint numerators (DESIGN.md §3), shared by the top-k select and the evaluator:
+// ubm = (double)Sint_u * rsa[u], ibm = (double)Sint_i * rsd[s], blends as in k3_topk.cu's header
+__device__ __forceinline__ double blend_score(int model, long long su, long long si, double rsu, double rds, double alpha,
+                                              double oma, bool pick_ibm) {
+  switch (model) {
+    case MODEL_UBM: return __dmul_rn(__ll2double_rn(su), rsu);
+    case MODEL_IBM: return __dmul_rn(__ll2double_rn(si), rds);
+    case MODEL_LC:
+      return __dadd_rn(__dmul_rn(__dmul_rn(__ll2double_rn(su), rsu), alpha), __dmul_rn(__dmul_rn(__ll2double_rn(si), rds), oma));
+    default: return pick_ibm ? __dmul_rn(__ll2double_rn(si), rds) : __dmul_rn(__ll2double_rn(su), rsu);
+  }
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));

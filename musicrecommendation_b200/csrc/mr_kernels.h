@@ -134,6 +134,26 @@ int launch_blend_arrays(const BlendParams& bp, const double* ubm, const double* 
 int launch_evaluate(const double* scores, int n_users, int n_songs, const long long* lab_ptr, const int* lab_col, const int* new_songs,
                     int n_new, int n_thresholds, unsigned long long* minmax, double* ap_out, int num_sms, cudaStream_t st);
 
+// Streamed evaluateModel (DESIGN.md §4.5): per slice of a batch's score panels (masked, select bits built), either the min / max of
+// the emitted scores (bit patterns, mm[0] / mm[1]) or the confusion counts of the label songs by threshold bucket.
+int launch_eval_range(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+                      long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
+                      unsigned long long* mm, cudaStream_t st);
+struct EvalCounts {
+  unsigned long long cut[11];    // bit patterns of the cutoffs c_t (non-negative doubles or +inf): predicted at t <=> score >= c_t
+  int n_thresholds;
+  const int* colmap;             // [n_songs] scored column -> label-song index, -1 for columns that are no label song
+  unsigned long long* pred_b;    // [n_new][n_thresholds] emitted pairs whose bucket (number of cutoffs <= score) is b + 1
+  unsigned long long* tp_b;      // [n_new][n_thresholds] the same, restricted to labelled pairs
+  unsigned long long* nlab;      // [n_new] labelled pairs of the scored columns
+  const long long* lab_ptr;      // [U + 1] label CSR of the shard (global song ids)
+  const int* lab_col;
+  int col_lo;                    // first song of the scored columns (song window); column = song - col_lo
+};
+int launch_eval_count(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+                      long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
+                      const EvalCounts& ec, cudaStream_t st);
+
 int launch_map_at_k(const int* top_song, const int* top_len, int n_users, int k, const long long* lab_ptr, const int* lab_col,
                     double* ap_out, cudaStream_t st);
 

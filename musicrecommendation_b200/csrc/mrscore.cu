@@ -20,6 +20,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <string>
 #include <queue>
 #include <mutex>
@@ -97,7 +98,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard and its results: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -111,6 +112,12 @@ struct mr_handle {
   double* d_dense = nullptr; int32_t* d_cnt = nullptr; float* d_simf = nullptr;
   // results
   int *d_out_song = nullptr, *d_out_len = nullptr; double* d_out_score = nullptr; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;
+  // streamed evaluation (mr_eval_range / mr_eval_counts).  gen counts the calls that may rewrite the score panels; after a range pass
+  // over a single-batch item-space shard the panels still hold the masked numerators of (eval_model, eval_param, eval_seed), and a
+  // count pass of the same model at the same gen reuses them instead of scoring again.
+  unsigned long long gen = 0, eval_gen = ~0ULL; int eval_model = -1; double eval_param = 0; uint64_t eval_seed = 0;
+  unsigned long long* d_eval_mm = nullptr;   // [2] min / max bit patterns of the range pass
+  EvalCounts ec{};                           // device state of the count pass
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -682,16 +689,31 @@ int plan_item_batches(mr_handle* h, const std::vector<long long>& hu_ptr) {
   }
 }
 
-enum RunMode { RUN_TOPK, RUN_DENSE, RUN_COUNTS_UBM, RUN_SIM_UBM };
+// RUN_EVAL_RANGE / RUN_EVAL_COUNT: the streamed evaluateModel passes (DESIGN.md §4.5) in place of the top-k select of each slice;
+// host_out is null / points to a bool "the panels already hold this model's masked numerators" (resident reuse, mr_eval_counts).
+enum RunMode { RUN_TOPK, RUN_DENSE, RUN_COUNTS_UBM, RUN_SIM_UBM, RUN_EVAL_RANGE, RUN_EVAL_COUNT };
 struct TopkHostOut { int32_t* song; double* score; int32_t* len; };   // RUN_TOPK: caller buffers the finished slices are copied into
 // RUN_DENSE: where the fp64 rows go.  ALL: out[u][s] for every test user (mr_score_dense).  USERS: out[i][s] for the listed users
 // (DIST getRanks1 granularity).  SONGS: d_out[i][u] for the listed songs, gathered on the device (DIST getRanks2 granularity).
 struct DenseOut { enum Kind { ALL, USERS, SONGS } kind; double* out; const int32_t* ids; int n_ids; const int* d_ids; double* d_out; };
 
+int eval_slice(mr_handle* h, RunMode mode, const BlendParams& bp, const long long* su, const long long* si, const uint64_t* sel, int u0, int n,
+               cudaStream_t st) {
+  if (mode == RUN_EVAL_RANGE)
+    MR_LAUNCH(h, launch_eval_range(bp, su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->d_eval_mm, st));
+  else
+    MR_LAUNCH(h, launch_eval_count(bp, su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->ec, st));
+  return MR_OK;
+}
+
 int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode mode, void* host_out) {
   const bool need_ubm = model != MODEL_IBM;
   const bool need_ibm = model != MODEL_UBM && mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM;
-  const bool item_space = h->space == MR_SPACE_ITEM && (mode == RUN_TOPK || mode == RUN_DENSE);
+  const bool eval = mode == RUN_EVAL_RANGE || mode == RUN_EVAL_COUNT;
+  const bool ranked = mode == RUN_TOPK || eval;      // per-slice consumers of the masked panels: top-k select or evaluation
+  const bool item_space = h->space == MR_SPACE_ITEM && (mode == RUN_DENSE || ranked);
+  const bool reuse = mode == RUN_EVAL_COUNT && *static_cast<const bool*>(host_out);   // skip head pass, tail scatter, mask and select
+  if (!reuse) ++h->gen;
   if (item_space) { int rc = ensure_head_rows(h); if (rc) return rc; }
   const int batch = item_space ? h->batch_rows : kUserBatch;
   // Batch pipeline (item-space top-k of a pure model over >= 2 batches; not under MR_PROFILE, whose phase timers serialise the
@@ -702,13 +724,13 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
   // What it buys is the kernel boundaries (the next kernel's CTAs start while the previous grid drains): 727 -> 701 ms for the two
   // models of the one-GPU job.  Making the kernels truly share the SMs was measured and is WORSE (profiles/r02_summary.md §8): the head
   // pass lives on every resident CTA working on the same song tile out of L2, and a select streaming 48 GB through L2 beside it breaks that.
-  const bool pipelined = item_space && mode == RUN_TOPK && (model == MODEL_UBM || model == MODEL_IBM) && !(h->flags & MR_PROFILE) &&
+  const bool pipelined = item_space && ranked && (model == MODEL_UBM || model == MODEL_IBM) && !(h->flags & MR_PROFILE) &&
                          h->U > batch && !getenv("MRSCORE_NO_PIPELINE");
   // Every other item-space top-k (one batch, e.g. a GPU's share of a song-partitioned job, or a blend) puts consecutive slices on two
   // alternating streams instead: same idea, the boundaries between the slices' kernels (107.6 -> 105.1 ms for both models of a 1/8 song
   // partition; next to the batch pipeline it adds nothing).  The two streams' kernels have different shared-memory carve-outs and never
   // share an SM; asking for matched carve-outs makes them do so and is slower (profiles/r02_summary.md §8).
-  const bool alternating = item_space && mode == RUN_TOPK && !pipelined && !(h->flags & MR_PROFILE) && !getenv("MRSCORE_NO_PIPELINE");
+  const bool alternating = item_space && ranked && !pipelined && !(h->flags & MR_PROFILE) && !getenv("MRSCORE_NO_PIPELINE");
   const bool streamed = pipelined || alternating;   // the slices run off the library stream and are joined back into it
   cudaStream_t const hs = h->stream;
   cudaStream_t const sl[2] = {streamed ? h->slice_stream : h->stream, alternating ? h->slice_stream2 : (streamed ? h->slice_stream : h->stream)};
@@ -721,7 +743,7 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       long long* const panel = par ? h->d_sint_i : h->d_sint_u;
       long long* const pu = pipelined ? (model == MODEL_UBM ? panel : nullptr) : h->d_sint_u;
       long long* const pi = pipelined ? (model == MODEL_IBM ? panel : nullptr) : h->d_sint_i;
-      {
+      if (!reuse) {
         PhaseTimer t(h, MR_T_HEAD_ROWSUM);
         const int bi = b0 / batch;
         const int4* grp = h->d_grp_hdr + static_cast<long long>(bi) * h->n_groups;
@@ -741,11 +763,11 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
         if (h->n_ex > 0)
           MR_LAUNCH(h, launch_head_fixup(models, h->d_hu_ptr, h->d_hu_row, h->d_hu_song, h->d_hu_q, b0, nb, h->d_ex_ptr, h->d_ex_song, h->d_ex_g,
                                          h->d_ex_gq, pu, pi, h->spitch, hs));
-        if (streamed) {
-          MR_CUDA(h, cudaEventRecord(h->ev_head[par], hs));
-          MR_CUDA(h, cudaStreamWaitEvent(sl[0], h->ev_head[par], 0));
-          if (alternating) MR_CUDA(h, cudaStreamWaitEvent(sl[1], h->ev_head[par], 0));
-        }
+      }
+      if (streamed) {
+        MR_CUDA(h, cudaEventRecord(h->ev_head[par], hs));
+        MR_CUDA(h, cudaStreamWaitEvent(sl[0], h->ev_head[par], 0));
+        if (alternating) MR_CUDA(h, cudaStreamWaitEvent(sl[1], h->ev_head[par], 0));
       }
       // per slice of users so that the atomics of one launch stay within a few GB of the Sint panels (measured optimum: 300-600 users);
       // in top-k mode the slice is masked and selected right away, and its rows of the result go to the caller's buffers on the copy
@@ -761,20 +783,27 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       for (int s0 = 0; s0 < nb; s0 += tail_sub) {
         const int sn = std::min(tail_sub, nb - s0);
         cudaStream_t const ts = sl[(s0 / tail_sub) & 1];
-        {
+        if (!reuse) {
           PhaseTimer t(h, MR_T_TAIL_SCATTER);
           const long long e0 = h->h_tu_ptr[b0 + s0], e1 = h->h_tu_ptr[b0 + s0 + sn];
           MR_LAUNCH(h, launch_tail_scatter(models, h->d_tu_user, h->d_tu_song, h->d_tu_lptr, e0, e1, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr,
                                            h->d_tr_end, h->d_tr_col, h->d_qv, h->d_qd, b0, pu, pi, h->spitch, h->h_tu_lptr[e1] - h->h_tu_lptr[e0], tail_lanes, ts));
         }
-        if (mode != RUN_TOPK) continue;
-        PhaseTimer t(h, MR_T_TOPK);
+        if (mode == RUN_DENSE) continue;
+        PhaseTimer t(h, eval ? MR_T_OTHER : MR_T_TOPK);
         long long* su = need_ubm ? pu + static_cast<long long>(s0) * h->spitch : nullptr;
         long long* si = need_ibm ? pi + static_cast<long long>(s0) * h->spitch : nullptr;
         uint64_t* sel = sel_needed ? h->d_sel + static_cast<long long>(s0) * h->sel_pitch : nullptr;
         const int u0 = b0 + s0;
-        MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
-        if (sel_needed) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, sn, h->n_cols, sel, h->sel_pitch, ts));
+        if (!reuse) {
+          MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
+          if (sel_needed) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, sn, h->n_cols, sel, h->sel_pitch, ts));
+        }
+        if (eval) {
+          const int rc = eval_slice(h, mode, bp, su, si, sel, u0, sn, ts);
+          if (rc) return rc;
+          continue;
+        }
         MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, su, si, h->spitch, sel, h->sel_pitch, u0, sn, h->n_cols, h->d_rsa, h->d_rsd, k, h->d_out_song,
                                  h->d_out_score, h->d_out_len, ts));
         if (ho) {
@@ -797,7 +826,7 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
           if (pipelined) MR_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_done[par ^ 1], 0));
         }
       }
-      if (mode == RUN_TOPK) continue;   // the batch is finished; RUN_DENSE continues below on the whole batch
+      if (mode != RUN_DENSE) continue;   // the batch is finished; RUN_DENSE continues below on the whole batch
     } else if (need_ubm) {
       int rc = count_ubm_batch(h, b0, nb);
       if (rc) return rc;
@@ -849,7 +878,7 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       MR_LAUNCH(h, launch_aggregate_ibm(h->d_te_ptr, h->d_te_col, h->d_te_grow, h->d_qd, b0, nb, h->d_g, h->ldg, h->S, h->d_sint_i,
                                         h->spitch, h->stream));
     }
-    PhaseTimer t(h, MR_T_TOPK);
+    PhaseTimer t(h, eval ? MR_T_OTHER : MR_T_TOPK);
     MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, need_ubm ? h->d_sint_u : nullptr,
                                       need_ibm ? h->d_sint_i : nullptr, h->spitch, h->stream));
     if (mode == RUN_DENSE) {
@@ -876,6 +905,12 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
     } else {
       if (model == MODEL_AGG || model == MODEL_STOCH)
         MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, b0, nb, h->n_cols, h->d_sel, h->sel_pitch, h->stream));
+      if (eval) {
+        const int rc = eval_slice(h, mode, bp, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr,
+                                  (model == MODEL_AGG || model == MODEL_STOCH) ? h->d_sel : nullptr, b0, nb, h->stream);
+        if (rc) return rc;
+        continue;
+      }
       MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr, h->spitch,
                                (model == MODEL_AGG || model == MODEL_STOCH) ? h->d_sel : nullptr, h->sel_pitch, b0, nb, h->n_cols, h->d_rsa,
                                h->d_rsd, k, h->d_out_song, h->d_out_score, h->d_out_len, h->stream));
@@ -998,6 +1033,7 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
             const int32_t* deg_song_all) {
   if (!h || !h->stream) return MR_ERR_STATE;
   if (h->loaded) return fail(h, MR_ERR_STATE, "mr_load called twice on one handle");
+  ++h->gen;
   if (n_train <= 0 || n_songs <= 0 || n_test < 0 || !deg_train || !deg_song_all) return fail(h, MR_ERR_BAD_ARG, "bad sizes / null degree arrays");
   int rc = check_csr(h, "train", n_train, n_songs, tr_rowptr, tr_col);
   if (rc) return rc;
@@ -1200,7 +1236,7 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   MR_CUDA(h, cudaSetDevice(h->device));
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   lap("check_csr + sync");
-  h->have_test = false; h->have_topk = false; h->out_k = 0;
+  h->have_test = false; h->have_topk = false; h->out_k = 0; ++h->gen;
   const int U = n_test; const long long nnz = te_rowptr[U];
   h->U = U; h->nnz_te = nnz;
   h->h_te_ptr.assign(te_rowptr, te_rowptr + U + 1);
@@ -1614,6 +1650,7 @@ int mr_map_at_k(mr_handle* h, int k, const int32_t* top_song, const int32_t* top
 
 int mr_set_option(mr_handle* h, int option, int64_t value) {
   if (!h) return MR_ERR_STATE;
+  ++h->gen;
   switch (option) {
     case MR_OPT_HEAD_MIN_DEG:
       if (h->loaded) return fail(h, MR_ERR_STATE, "MR_OPT_HEAD_MIN_DEG must be set before mr_load (it selects the head songs)");
@@ -1641,7 +1678,7 @@ int mr_invalidate_prepared(mr_handle* h) {
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_invalidate_prepared: %s", cudaGetErrorString(e));
   if (h->head_pending) { cudaEventSynchronize(h->ev_pre); h->head_pending = false; }   // a build in flight is abandoned once it has drained
-  h->head_ready = false; h->n_ex = 0;
+  h->head_ready = false; h->n_ex = 0; ++h->gen;
   return MR_OK;
 }
 
@@ -1708,6 +1745,167 @@ int mr_evaluate_dense(mr_handle* h, const double* scores_UxS, int n_users, int n
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_evaluate_dense: %s", cudaGetErrorString(e));
   double total = 0.0;
   for (int c = 0; c < n_new; ++c) total += ap[c];                              // foldLeft(0.0)(_+_), MR:626
+  *out_map = total / n_new;
+  return MR_OK;
+}
+
+// ---- streamed evaluateModel (MR:521-639; DESIGN.md §4.5)
+namespace {
+const double kEvalTh[11] = {0.0, 0.1, 0.2, 0.3, 0.4, 0.5, 0.6, 0.7, 0.8, 0.9, 1.0};   // the TH literals of eval_ap_kernel
+
+// doubles -> unsigned integers in the same order (negative values included), and back
+inline unsigned long long ord_key(double x) { unsigned long long b; memcpy(&b, &x, 8); return (b >> 63) ? ~b : b | (1ULL << 63); }
+inline double from_key(unsigned long long k) { const unsigned long long b = (k >> 63) ? k & ~(1ULL << 63) : ~k; double x; memcpy(&x, &b, 8); return x; }
+
+// c_t = the least double x in [mn, mx] with RN(RN(x - mn) / RN(mx - mn)) > TH[t], +inf when there is none.  The normalisation is
+// monotone non-decreasing in x (RN subtraction, RN division by a positive number), so a bisection over the ordered bit patterns finds it.
+void eval_cutoffs(double mn, double mx, int n_thresholds, double* out) {
+  const double range = mx - mn;
+  auto f = [&](double x) { return (x - mn) / range; };
+  for (int t = 0; t < n_thresholds; ++t) {
+    out[t] = std::numeric_limits<double>::infinity();
+    if (!(range > 0) || !(f(mx) > kEvalTh[t])) continue;
+    unsigned long long lo = ord_key(mn), hi = ord_key(mx);
+    while (lo < hi) {
+      const unsigned long long mid = lo + (hi - lo) / 2;
+      if (f(from_key(mid)) > kEvalTh[t]) hi = mid; else lo = mid + 1;
+    }
+    out[t] = from_key(hi);
+  }
+}
+
+void join_slice_streams(mr_handle* h) {   // an eval call that fails inside the streamed region leaves no work behind h->stream's back
+  for (cudaStream_t s : {h->slice_stream, h->slice_stream2})
+    if (s && cudaEventRecord(h->ev_join, s) == cudaSuccess) cudaStreamWaitEvent(h->stream, h->ev_join, 0);
+}
+
+int eval_params(mr_handle* h, int model, double param, uint64_t seed, BlendParams* bp) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  // min / max are taken on the bit patterns of non-negative scores, as in getTopK (documented deviation, DESIGN.md §3)
+  if (model == MR_LC && !(param >= 0 && param <= 1))
+    return fail(h, MR_ERR_PARAM_RANGE, "evaluation: alpha of the linear combination must be between 0 and 1");
+  if ((rc = make_blend_params(h, model, param, seed, h->n_pairs_total, bp))) return rc;
+  bp->pair_base = h->d_pair_base;
+  bp->stats = nullptr;
+  if (model != MR_UBM && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
+  return MR_OK;
+}
+}  // namespace
+
+int mr_eval_cutoffs(double mn, double mx, int n_thresholds, double* out) {
+  if (!out || (n_thresholds != 10 && n_thresholds != 11)) return MR_ERR_BAD_ARG;
+  eval_cutoffs(mn, mx, n_thresholds, out);
+  return MR_OK;
+}
+
+int mr_eval_range(mr_handle* h, int model, double param, uint64_t seed, double* out_min, double* out_max) {
+  if (!h) return MR_ERR_STATE;
+  if (!out_min || !out_max) return fail(h, MR_ERR_BAD_ARG, "null output");
+  BlendParams bp;
+  int rc = eval_params(h, model, param, seed, &bp);
+  if (rc) return rc;
+  if ((rc = slot_alloc(h, mr_handle::SL_EVAL_MM, &h->d_eval_mm, 2))) return rc;
+  const unsigned long long init[2] = {~0ULL, 0ULL};
+  MR_CUDA(h, cudaMemcpyAsync(h->d_eval_mm, init, sizeof init, cudaMemcpyHostToDevice, h->stream));
+  if ((rc = run_batches(h, model, bp, 0, RUN_EVAL_RANGE, nullptr))) { join_slice_streams(h); return rc; }
+  unsigned long long mm[2];
+  MR_CUDA(h, cudaMemcpyAsync(mm, h->d_eval_mm, sizeof mm, cudaMemcpyDeviceToHost, h->stream));
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->eval_gen = h->gen; h->eval_model = model; h->eval_param = param; h->eval_seed = seed;
+  if (mm[0] == ~0ULL) {   // no emitted pair
+    *out_min = std::numeric_limits<double>::infinity(); *out_max = -std::numeric_limits<double>::infinity();
+  } else {
+    memcpy(out_min, &mm[0], 8); memcpy(out_max, &mm[1], 8);
+  }
+  return MR_OK;
+}
+
+int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double mn, double mx, int n_thresholds, const int64_t* lab_rowptr,
+                   const int32_t* lab_col, const int32_t* new_songs, int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab) {
+  if (!h) return MR_ERR_STATE;
+  if (n_thresholds != 10 && n_thresholds != 11) return fail(h, MR_ERR_BAD_ARG, "n_thresholds must be 10 (MR:590) or 11 (DIST:395)");
+  if (!lab_rowptr || !new_songs || n_new <= 0 || !out_pred || !out_tp || !out_nlab) return fail(h, MR_ERR_BAD_ARG, "null / empty arguments");
+  BlendParams bp;
+  int rc = eval_params(h, model, param, seed, &bp);
+  if (rc) return rc;
+  const int U = h->U;
+  const long long n_lab = lab_rowptr[U];
+  if (lab_rowptr[0] != 0 || n_lab < 0 || (n_lab > 0 && !lab_col)) return fail(h, MR_ERR_BAD_ARG, "bad label CSR");
+  for (int u = 0; u < U; ++u) {
+    if (lab_rowptr[u + 1] < lab_rowptr[u]) return fail(h, MR_ERR_BAD_ARG, "label rowptr not monotone at row %d", u);
+    for (long long i = lab_rowptr[u]; i < lab_rowptr[u + 1]; ++i)
+      if (lab_col[i] < 0 || (i > lab_rowptr[u] && lab_col[i] <= lab_col[i - 1])) return fail(h, MR_ERR_BAD_ARG, "label row %d not ascending/unique", u);
+  }
+  if (new_songs[0] < 0) return fail(h, MR_ERR_BAD_ARG, "new_songs: negative song id");
+  for (int i = 1; i < n_new; ++i)
+    if (new_songs[i] <= new_songs[i - 1]) return fail(h, MR_ERR_BAD_ARG, "new_songs not strictly ascending at %d", i);
+  for (long long i = 0; i < n_lab; ++i)
+    if (!std::binary_search(new_songs, new_songs + n_new, lab_col[i]))
+      return fail(h, MR_ERR_BAD_ARG, "new_songs lacks label song %d", lab_col[i]);
+  if (mx - mn > 0 && !(mn >= 0)) return fail(h, MR_ERR_BAD_ARG, "mn must be >= 0 (scores are non-negative)");
+  double cut[11];
+  eval_cutoffs(mn, mx, n_thresholds, cut);
+  EvalCounts& ec = h->ec;
+  ec = EvalCounts{};
+  for (int t = 0; t < n_thresholds; ++t) memcpy(&ec.cut[t], &cut[t], 8);
+  ec.n_thresholds = n_thresholds; ec.col_lo = h->win_lo;
+  std::vector<int> colmap(h->n_cols, -1);   // scored column -> label-song index
+  for (int i = 0; i < n_new; ++i)
+    if (new_songs[i] >= h->win_lo && new_songs[i] < h->win_lo + h->n_cols) colmap[new_songs[i] - h->win_lo] = i;
+  const size_t per = static_cast<size_t>(n_new) * n_thresholds, n_cnt = 2 * per + n_new;
+  int* d_colmap = nullptr; long long* d_lp = nullptr; int* d_lc = nullptr; unsigned long long* d_cnt = nullptr;
+  if ((rc = slot_upload(h, mr_handle::SL_EVAL_COLMAP, &d_colmap, colmap.data(), colmap.size())) ||
+      (rc = slot_upload(h, mr_handle::SL_LAB_PTR, &d_lp, reinterpret_cast<const long long*>(lab_rowptr), static_cast<size_t>(U) + 1)) ||
+      (rc = slot_upload(h, mr_handle::SL_LAB_COL, &d_lc, lab_col, static_cast<size_t>(n_lab))) ||
+      (rc = slot_alloc(h, mr_handle::SL_EVAL_CNT, &d_cnt, n_cnt)))
+    return rc;
+  MR_CUDA(h, cudaMemsetAsync(d_cnt, 0, n_cnt * sizeof(unsigned long long), h->stream));
+  ec.colmap = d_colmap; ec.lab_ptr = d_lp; ec.lab_col = d_lc; ec.pred_b = d_cnt; ec.tp_b = d_cnt + per; ec.nlab = d_cnt + 2 * per;
+  // resident reuse: a single-batch item-space shard whose panels the range pass of the same model has just filled
+  bool reuse = h->space == MR_SPACE_ITEM && h->U <= h->batch_rows && h->eval_gen == h->gen && h->eval_model == model &&
+               memcmp(&h->eval_param, &param, sizeof param) == 0 && h->eval_seed == seed;
+  if ((rc = run_batches(h, model, bp, 0, RUN_EVAL_COUNT, &reuse))) { join_slice_streams(h); return rc; }
+  std::vector<unsigned long long> cnt(n_cnt);
+  MR_CUDA(h, cudaMemcpyAsync(cnt.data(), d_cnt, n_cnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  for (int c = 0; c < n_new; ++c) {   // bucket counts -> counts per threshold: predicted at t <=> bucket > t
+    long long p = 0, q = 0;
+    for (int t = n_thresholds - 1; t >= 0; --t) {
+      const size_t i = static_cast<size_t>(c) * n_thresholds + t;
+      p += static_cast<long long>(cnt[i]); q += static_cast<long long>(cnt[per + i]);
+      out_pred[i] = p; out_tp[i] = q;
+    }
+    out_nlab[c] = static_cast<long long>(cnt[2 * per + c]);
+  }
+  return MR_OK;
+}
+
+// fp64 in exactly the operation order of eval_ap_kernel and mr_evaluate_dense; no contraction into FMAs
+__attribute__((optimize("fp-contract=off")))
+int mr_eval_finish(const int64_t* pred, const int64_t* tp, const int64_t* nlab, int n_new, int n_thresholds, double* out_ap, double* out_map) {
+  if (!pred || !tp || !nlab || !out_map || n_new <= 0 || (n_thresholds != 10 && n_thresholds != 11)) return MR_ERR_BAD_ARG;
+  double total = 0.0;
+  for (int c = 0; c < n_new; ++c) {
+    double prec[11], rec[11];
+    const long long l = nlab[c];
+    for (int t = 0; t < n_thresholds; ++t) {
+      const long long p = pred[static_cast<size_t>(c) * n_thresholds + t], x = tp[static_cast<size_t>(c) * n_thresholds + t];
+      if (x < 0 || x > p || x > l) return MR_ERR_BAD_ARG;                                     // not counts of one partitioning
+      prec[t] = p > 0 ? static_cast<double>(x) / static_cast<double>(p) : 0.0;               // tp / (tp + fp), MR:561-566
+      rec[t] = l > 0 ? static_cast<double>(x) / static_cast<double>(l) : 0.0;                // tp / (tp + fn), MR:574-579
+    }
+    double ap = 0.0;
+    for (int t = 0; t < n_thresholds; ++t) {
+      double term;
+      if (t == n_thresholds - 1) term = 0.0;
+      else if (t == n_thresholds - 2) term = (rec[t] - 0.0) * prec[t];
+      else term = (rec[t] - rec[t + 1]) * prec[t];
+      ap = ap + term;
+    }
+    if (out_ap) out_ap[c] = ap;
+    total += ap;                                                                              // foldLeft(0.0)(_+_), MR:626
+  }
   *out_map = total / n_new;
   return MR_OK;
 }

@@ -138,6 +138,58 @@ def exchange_song_partitions(song, score, length, n_users_total: int, world: int
     return tuple(outs)
 
 
+def _collective_device(group):
+    import torch
+    import torch.distributed as dist
+    return torch.device("cuda", torch.cuda.current_device()) if dist.get_backend(group) == "nccl" else torch.device("cpu")
+
+
+def global_label_songs(lab_col, group=None) -> np.ndarray:
+    """newSongs of the whole test set (MR:72, 79) when each rank holds only its own users' labels: all-gather of the ranks' distinct
+    label songs, ascending int32."""
+    import torch
+    import torch.distributed as dist
+    dev = _collective_device(group)
+    mine = torch.from_numpy(np.unique(np.asarray(lab_col, np.int64))).to(dev)
+    world = dist.get_world_size(group)
+    n = torch.tensor([mine.numel()], dtype=torch.int64, device=dev)
+    sizes = [torch.zeros_like(n) for _ in range(world)]
+    dist.all_gather(sizes, n, group=group)
+    sizes = [int(x.item()) for x in sizes]
+    pad = torch.full((max(sizes),), -1, dtype=torch.int64, device=dev)
+    pad[:mine.numel()] = mine
+    parts = [torch.empty_like(pad) for _ in range(world)]
+    dist.all_gather(parts, pad, group=group)
+    allv = torch.cat([p[:k] for p, k in zip(parts, sizes)]).cpu().numpy()
+    return np.unique(allv).astype(np.int32)
+
+
+def evaluate_reference_map(mr, model: int, param: float = 0.5, seed: int = 0, n_thresholds: int = 10, new_songs=None, group=None,
+                           labels: Dataset | None = None) -> float:
+    """evaluateModel (MR:521-639) of a model whose parts are scored by the ranks of a job (user shards, song windows, or both), with
+    the same bits as on the materialised whole model: every rank's handle gives the min / max of its part, one all-reduce makes them
+    global, every rank counts its part's label pairs under the global normalisation, one all-reduce sums the integer counts, and every
+    rank finishes the mAP.  new_songs: the distinct label songs of ALL test users (default: global_label_songs of this rank's labels).
+    CUDA tensors under NCCL, CPU tensors under gloo."""
+    import torch
+    import torch.distributed as dist
+    from .recommender import eval_finish
+    dev = _collective_device(group)
+    lab = labels if labels is not None else mr.ds
+    if new_songs is None:
+        new_songs = global_label_songs(lab.lab_col, group)
+    mn, mx = mr.eval_range(model, param, seed)
+    r = torch.tensor([mn, -mx], dtype=torch.float64, device=dev)      # min of (mn, -mx): the global min and max in one collective
+    dist.all_reduce(r, op=dist.ReduceOp.MIN, group=group)
+    mn, mx = float(r[0].item()), -float(r[1].item())
+    pred, tp, nlab = mr.eval_counts(model, mn, mx, new_songs, param, seed, n_thresholds, lab)
+    c = torch.from_numpy(np.concatenate([pred.ravel(), tp.ravel(), nlab])).to(dev)
+    dist.all_reduce(c, group=group)
+    c = c.cpu().numpy()
+    n, k = len(nlab), n_thresholds
+    return eval_finish(c[:n * k].reshape(n, k), c[n * k:2 * n * k].reshape(n, k), c[2 * n * k:], n_thresholds)
+
+
 def split_train_users(ds: Dataset, rank: int, world: int) -> Dataset:
     """K-split of the item-item Gram (BASELINE configs[4]): rank r keeps the train users of its contiguous range, every song.
     deg_song stays global — the cosine denominators count all listeners (MR:237)."""

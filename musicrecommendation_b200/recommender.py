@@ -197,6 +197,7 @@ class MusicRecommender:
         if item_batch:
             self._check(self._lib.mr_set_option(self._h, _lib.MR_OPT_ITEM_BATCH, int(item_batch)))
         self.song_window = (0, ds.S) if song_window is None else (int(song_window[0]), int(song_window[1]))
+        self._whole_test_set = True      # the test users are the whole test set (not a shard of it): evaluateOnDevice is the model's mAP
         if song_window is not None:
             self._check(self._lib.mr_set_option(self._h, _lib.MR_OPT_SONG_WINDOW_LO, self.song_window[0]))
             self._check(self._lib.mr_set_option(self._h, _lib.MR_OPT_SONG_WINDOW_HI, self.song_window[1]))
@@ -247,6 +248,7 @@ class MusicRecommender:
         self._check(self._lib.mr_set_test_users(self._h, ds_shard.U, _p(a["te_ptr"]), _p(a["te_col"]), _p(a["deg_te"]),
                                                 pair_index_base, n_pairs_total))
         self.ds = ds_shard
+        self._whole_test_set = pair_index_base == 0 and n_pairs_total == 0   # the ABI's "this shard is the whole test set"
 
     def _model(self, kind: int, name: str) -> Model:
         lo, hi = self.song_window
@@ -480,6 +482,48 @@ class MusicRecommender:
         self._check(self._lib.mr_evaluate_dense(self._h, _p(sc), sc.shape[0], sc.shape[1], _p(lp), _p(lc), n_thresholds, C.byref(out)))
         return float(out.value)
 
+    # ---- the same metric streamed over the scoring batches: no materialised model (include/mrscore.h mr_eval_*, DESIGN.md §4.5)
+    def eval_range(self, model: int = _lib.MR_UBM, param: float = 0.5, seed: int = 0) -> tuple[float, float]:
+        """(min, max) of the scores this handle's shard and song window emit (MR:524-529); (inf, -inf) when it emits none."""
+        mn, mx = C.c_double(), C.c_double()
+        self._check(self._lib.mr_eval_range(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), C.byref(mn), C.byref(mx)))
+        return float(mn.value), float(mx.value)
+
+    def eval_counts(self, model: int, mn: float, mx: float, new_songs, param: float = 0.5, seed: int = 0, n_thresholds: int = 10,
+                    labels: Dataset | None = None):
+        """Confusion counts of this handle's part of the model under the global (mn, mx): (pred [n_new, n_thr], tp [n_new, n_thr],
+        nlab [n_new]) int64, row c for new_songs[c] (all test users' distinct label songs, ascending).  labels: the data set whose
+        label rows belong to the current shard's users (default: the handle's)."""
+        lab = labels if labels is not None else self.ds
+        lp = np.ascontiguousarray(lab.lab_ptr, np.int64)
+        lc = np.ascontiguousarray(lab.lab_col, np.int32)
+        if len(lp) != self.ds.U + 1 or len(lc) < (lp[-1] if len(lp) else 0):   # mr_eval_counts reads U + 1 row offsets
+            raise ValueError(f"labels must hold {self.ds.U} label rows (the current shard's users), got {len(lp) - 1}")
+        ns = np.ascontiguousarray(new_songs, np.int32)
+        pred = np.zeros((len(ns), n_thresholds), np.int64)
+        tp = np.zeros((len(ns), n_thresholds), np.int64)
+        nlab = np.zeros(len(ns), np.int64)
+        self._check(self._lib.mr_eval_counts(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), float(mn), float(mx), n_thresholds,
+                                             _p(lp), _p(lc), _p(ns), len(ns), _p(pred), _p(tp), _p(nlab)))
+        return pred, tp, nlab
+
+    def evaluateOnDevice(self, model: int = _lib.MR_UBM, param: float = 0.5, seed: int = 0, n_thresholds: int = 10,
+                         labels: Dataset | None = None) -> float:
+        """evaluateModel (MR:521-639) of the model this handle scores, without materialising it: range pass, count pass, finish.
+        Same bits as evaluateModel(getXxxModel()) on shapes where that fits.  The handle must hold the whole model: no song window, and
+        test users that are the whole test set (ValueError otherwise); a partitioned job combines its handles' parts with
+        distributed.evaluate_reference_map."""
+        if self.song_window != (0, self.ds.S):
+            raise ValueError("evaluateOnDevice needs the whole model: this handle scores a song window (use distributed.evaluate_reference_map)")
+        if not self._whole_test_set:
+            raise ValueError("evaluateOnDevice needs the whole model: this handle holds a shard of the test users (set_test_users with a "
+                             "pair index base / total); use distributed.evaluate_reference_map")
+        lab = labels if labels is not None else self.ds
+        mn, mx = self.eval_range(model, param, seed)
+        new_songs = np.unique(np.asarray(lab.lab_col, np.int32))
+        pred, tp, nlab = self.eval_counts(model, mn, mx, new_songs, param, seed, n_thresholds, lab)
+        return eval_finish(pred, tp, nlab, n_thresholds)
+
 
 def _string_table(names, n):
     """id -> string list as (uint8 chars, int64 offsets [n+1]); ints stand in for missing tables."""
@@ -524,6 +568,63 @@ def import_model_file(path: str):
             rows.append((parts[0], parts[1], float(parts[2])))
     rows.sort(key=lambda r: (r[0], r[1], -r[2]))
     return rows
+
+
+def eval_finish(pred, tp, nlab, n_thresholds: int = 10, per_song: bool = False):
+    """mr_eval_finish (host code, no GPU): the mAP of summed confusion counts, bit for bit as mr_evaluate_dense; per_song=True also
+    returns the per-label-song AP."""
+    pred = np.ascontiguousarray(pred, np.int64)
+    tp = np.ascontiguousarray(tp, np.int64)
+    nlab = np.ascontiguousarray(nlab, np.int64)
+    n_new = len(nlab)
+    if pred.shape != (n_new, n_thresholds) or tp.shape != (n_new, n_thresholds):
+        raise ValueError("pred / tp must be [n_new, n_thresholds]")
+    ap = np.zeros(n_new, np.float64)
+    out = C.c_double(0.0)
+    rc = _lib.load().mr_eval_finish(_p(pred), _p(tp), _p(nlab), n_new, n_thresholds, _p(ap), C.byref(out))
+    if rc != _lib.MR_OK:
+        raise _lib.MrError(rc, "mr_eval_finish: bad counts or sizes")
+    return (float(out.value), ap) if per_song else float(out.value)
+
+
+def eval_cutoffs(mn: float, mx: float, n_thresholds: int = 10) -> np.ndarray:
+    """mr_eval_cutoffs: per threshold the least score the count pass predicts (+inf: none)."""
+    out = np.zeros(n_thresholds, np.float64)
+    rc = _lib.load().mr_eval_cutoffs(float(mn), float(mx), n_thresholds, _p(out))
+    if rc != _lib.MR_OK:
+        raise _lib.MrError(rc, "mr_eval_cutoffs: n_thresholds must be 10 or 11")
+    return out
+
+
+def eval_counts_host(scores: np.ndarray, ds: Dataset, lo: int, mn: float, mx: float, n_thresholds: int, new_songs):
+    """numpy mirror of mr_eval_counts over a dense block of a model: scores [U, W] are the songs [lo, lo + W) of ds's test users (NaN =
+    not emitted), normalised with the given global (mn, mx) as MR:529 does; labels of ds outside those songs are not counted (the
+    ownership rule).  Returns (pred, tp, nlab) like MusicRecommender.eval_counts."""
+    scores = np.asarray(scores, np.float64)
+    U, W = scores.shape
+    new_songs = np.asarray(new_songs, np.int64)
+    th = [0.0, 0.1, 0.2, 0.3, 0.4, 0.5, 0.6, 0.7, 0.8, 0.9, 1.0][:n_thresholds]
+    pred = np.zeros((len(new_songs), n_thresholds), np.int64)
+    tp = np.zeros((len(new_songs), n_thresholds), np.int64)
+    nlab = np.zeros(len(new_songs), np.int64)
+    idx = np.flatnonzero((new_songs >= lo) & (new_songs < lo + W))
+    if len(idx) == 0:
+        return pred, tp, nlab
+    rows = np.repeat(np.arange(U), np.diff(ds.lab_ptr))
+    cols = np.asarray(ds.lab_col, np.int64)
+    keep = (cols >= lo) & (cols < lo + W)
+    pos = np.searchsorted(new_songs[idx], cols[keep])
+    lab = np.zeros((U, len(idx)), bool)
+    lab[rows[keep], pos] = True
+    with np.errstate(invalid="ignore", divide="ignore"):
+        norm = (scores[:, new_songs[idx] - lo] - mn) / (mx - mn)
+    for t, thr in enumerate(th):
+        with np.errstate(invalid="ignore"):
+            p = norm > thr                              # NaN compares false (not emitted, max == min)
+        pred[idx, t] = p.sum(0)
+        tp[idx, t] = (p & lab).sum(0)
+    nlab[idx] = lab.sum(0)
+    return pred, tp, nlab
 
 
 def evaluate_map(scores: np.ndarray, ds: Dataset, n_thresholds: int = 10) -> float:

@@ -192,6 +192,33 @@ int mr_eval_finish(const int64_t* pred, const int64_t* tp, const int64_t* nlab, 
  * [mn, mx] qualifies (always when mx - mn is not > 0).  The count pass predicts a pair at t iff its score >= out[t]. */
 int mr_eval_cutoffs(double mn, double mx, int n_thresholds, double* out);
 
+/* ---- model sets: several models from one scoring of the shard (DESIGN.md §4.6) ------------------------------------------------------
+ * A model set is 1..16 entries (models[i], params[i], seeds[i]), each with the meaning it has in mr_topk; duplicates are allowed (a
+ * parameter sweep is a set).  The calls score the shard and song window once per batch (one head pass per panel the set needs, one tail
+ * scatter, one listened mask) and run every entry's consumer on the masked panels; entry i's outputs have exactly the bits of the
+ * single-model call for entry i.  Every entry is checked before any GPU work: an LC alpha or an AGG / STOCH parameter outside [0, 1] or NaN
+ * is MR_ERR_PARAM_RANGE, an unknown selector MR_ERR_BAD_ARG, and the message names the first bad entry ("entry i: ...").  The ownership
+ * rule and the partition sums of the single-model calls hold per entry.  A set call leaves the single-model results (mr_topk_fetch,
+ * mr_topk_device_ptrs, mr_map_at_k with NULL lists) untouched.
+ *
+ * getTopK for every entry: out_song[i] / out_score[i] / out_len[i] as mr_topk's for entry i (host arrays). */
+int mr_topk_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k,
+                  int32_t* const* out_song, double* const* out_score, int32_t* const* out_len);
+/* The same with the results kept in HBM, n_models x U x k x 12 bytes in a grow-only block of their own.  It must fit in the device memory
+ * the batch plan leaves free (MR_ERR_OOM stating the bytes otherwise; the plan is not changed for it).  mr_topk_multi_ptrs gives entry i's
+ * device arrays (int32 [U,k], double [U,k], int32 [U]), valid until the next set call or mr_set_test_users. */
+int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k);
+int mr_topk_multi_ptrs(mr_handle* h, int i, int k, void** song, void** score, void** len);
+/* Streamed evaluateModel for a set: out_min / out_max [n_models] as mr_eval_range's per entry; then the counts under per-entry global
+ * (mn[i], mx[i]): out_pred / out_tp [n_models][n_new][n_thresholds], out_nlab [n_new] (label counts do not depend on the model).  Labels
+ * and new_songs are checked as in mr_eval_counts, once per call.  On a single-batch item-space shard, mr_eval_counts_multi right after
+ * mr_eval_range_multi of the same set reuses the score panels. */
+int mr_eval_range_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds,
+                        double* out_min, double* out_max);
+int mr_eval_counts_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds,
+                         const double* mn, const double* mx, int n_thresholds, const int64_t* lab_rowptr, const int32_t* lab_col,
+                         const int32_t* new_songs, int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -264,7 +291,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  test users per batch, head_rowsum work groups per batch, users split over groups,
                                                                  scored columns (= songs of the window), first song of the window,
                                                                  top-k select since mr_load: rows its sampled fast path handed to the exact path, short rows
-                                                                 (exact path by design), degenerate rows (radix select)] */
+                                                                 (exact path by design), degenerate rows (radix select),
+                                                                 scoring passes since mr_load (batches whose score panels were built)] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

@@ -136,6 +136,30 @@ int launch_select_bits(const BlendParams& bp, const long long* te_ptr, const int
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
+// AGG's select bits as one column per user.  In select_bits_kernel the index of an unlistened column s is pair_base[u] + f(s) with
+// f(s) = s - (listened songs < s), and the bit is idx < agg_threshold, i.e. f(s) < m = agg_threshold - pair_base[u].  f grows by one
+// per unlistened column, so the unlistened columns with bit 1 are exactly those below split[u] = m + #{j : row[j] - j < m} (row[j] - j is
+// non-decreasing along the ascending row, so that count is a binary search), clamped to [0, n_songs].
+__global__ void agg_split_kernel(BlendParams bp, const long long* __restrict__ te_ptr, const int* __restrict__ te_col, int n_users,
+                                 int n_songs, int* __restrict__ split) {
+  const int u = blockIdx.x * blockDim.x + threadIdx.x;
+  if (u >= n_users) return;
+  const long long m = bp.agg_threshold - bp.pair_base[u];
+  if (m <= 0) { split[u] = 0; return; }
+  if (m >= n_songs) { split[u] = n_songs; return; }
+  const long long beg = te_ptr[u];
+  const int* row = te_col + beg;
+  int lo = 0, hi = static_cast<int>(bp.te_end[u] - beg);
+  while (lo < hi) { const int j = (lo + hi) >> 1; if (row[j] - j < m) lo = j + 1; else hi = j; }
+  split[u] = static_cast<int>(m + lo < n_songs ? m + lo : n_songs);
+}
+
+int launch_agg_split(const BlendParams& bp, const long long* te_ptr, const int* te_col, int n_users, int n_songs, int* split, cudaStream_t st) {
+  if (n_users <= 0) return 0;
+  agg_split_kernel<<<(n_users + 255) / 256, 256, 0, st>>>(bp, te_ptr, te_col, n_users, n_songs, split);
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
 // ---------------------------------------------------------------- top-k select
 // One CTA per test user.  Keys are the composite (score bits : 64, ~song : 32), so "larger key" == "better" with ties broken by
 // the smaller song id; scores are >= 0, so their IEEE bit patterns order like unsigned integers.

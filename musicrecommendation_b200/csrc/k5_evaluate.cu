@@ -111,118 +111,165 @@ int launch_evaluate(const double* scores, int n_users, int n_songs, const long l
 // (mr_eval_cutoffs): the kernels compare bit patterns of non-negative doubles and never divide.  A pair's bucket is the number of
 // cutoffs <= its score (it is predicted at exactly the thresholds t < bucket); counts are kept per bucket, the host sums them up.
 // ---------------------------------------------------------------------------------------------------------------------
+// A launch serves a group of models (EvalGroup, DESIGN.md §4.6): the panel words, the select word and the label entries are read once and
+// every model of the group scores them.  AGG needs no select plane here: its pick is "column < split[u]" (launch_agg_split).
 constexpr int kEvalThreads = 256;
 constexpr int kEvalTile = 4 * kEvalThreads;   // songs per CTA column tile: 4 consecutive songs per thread (two 16-byte loads per panel)
-constexpr int kEvalRows = 512;                // at most this many panel rows per eval_count_kernel CTA: its histogram is flushed once per CTA
+constexpr int kEvalRows = 512;                // at most this many panel rows per eval_count_kernel CTA: its u16 histogram cannot wrap
 
-// Score bit patterns of the songs s .. s+3 of one panel row; ok = emitted (not listened, inside the row), exactly as scan_row (k3_topk.cu)
-__device__ __forceinline__ void eval_quad(const BlendParams& bp, const long long* ru, const long long* ri, const uint64_t* rsel, int s,
-                                          int n_songs, double rsu, const double (&rd)[4], unsigned long long (&kb)[4], bool (&ok)[4]) {
-  long long a[4] = {-1, -1, -1, -1}, b[4] = {-1, -1, -1, -1};
-  if (bp.model != MODEL_IBM) {
+struct GroupNeeds { bool u, i, sel; };        // which panels / the select plane the group's models read
+__device__ __forceinline__ GroupNeeds group_needs(const EvalGroup& g) {
+  GroupNeeds r{false, false, false};
+#pragma unroll
+  for (int m = 0; m < kEvalGroupMax; ++m)
+    if (m < g.n) { r.u = r.u || g.model[m] != MODEL_IBM; r.i = r.i || g.model[m] != MODEL_UBM; r.sel = r.sel || g.model[m] == MODEL_STOCH; }
+  return r;
+}
+
+// Numerators of the songs s .. s+3 of one panel row; ok = emitted (not listened, inside the row), exactly as scan_row (k3_topk.cu).
+// Both panels of a set carry the same listened mask, so whichever one is read decides.
+__device__ __forceinline__ void eval_load4(const GroupNeeds& nd, const long long* ru, const long long* ri, int s, int n_songs,
+                                           long long (&a)[4], long long (&b)[4], bool (&ok)[4]) {
+#pragma unroll
+  for (int t = 0; t < 4; ++t) { a[t] = 0; b[t] = 0; }
+  if (nd.u) {
     const longlong2 x = *reinterpret_cast<const longlong2*>(ru + s), y = *reinterpret_cast<const longlong2*>(ru + s + 2);
     a[0] = x.x; a[1] = x.y; a[2] = y.x; a[3] = y.y;
   }
-  if (bp.model != MODEL_UBM) {
+  if (nd.i) {
     const longlong2 x = *reinterpret_cast<const longlong2*>(ri + s), y = *reinterpret_cast<const longlong2*>(ri + s + 2);
     b[0] = x.x; b[1] = x.y; b[2] = y.x; b[3] = y.y;
   }
-  const uint64_t selw = bp.model >= MODEL_AGG ? rsel[s >> 6] >> (s & 63) : 0;
 #pragma unroll
-  for (int t = 0; t < 4; ++t) {
-    ok[t] = s + t < n_songs && (bp.model == MODEL_IBM || a[t] >= 0) && (bp.model == MODEL_UBM || b[t] >= 0);
-    kb[t] = ok[t] ? static_cast<unsigned long long>(__double_as_longlong(
-                        blend_score(bp.model, a[t], b[t], rsu, rd[t], bp.alpha, bp.one_minus_alpha, (selw >> t) & 1ULL)))
-                  : 0ULL;
-  }
+  for (int t = 0; t < 4; ++t) ok[t] = s + t < n_songs && a[t] >= 0 && b[t] >= 0;
 }
 
-__device__ __forceinline__ void eval_rsd4(const BlendParams& bp, const double* rsd, int s, int n_songs, double (&rd)[4]) {
-#pragma unroll
-  for (int t = 0; t < 4; ++t) rd[t] = (bp.model != MODEL_UBM && s + t < n_songs) ? rsd[s + t] : 0.0;
+// score bits of model m at column c; selbit = the STOCH plane's bit of c, split = the AGG split column of this row
+__device__ __forceinline__ unsigned long long eval_key(const EvalGroup& g, int m, long long a, long long b, double rsu, double rd, int c,
+                                                       bool selbit, int split) {
+  const int model = g.model[m];
+  const bool pick = model == MODEL_STOCH ? selbit : (model == MODEL_AGG && c < split);
+  return static_cast<unsigned long long>(__double_as_longlong(blend_score(model, a, b, rsu, rd, g.alpha[m], g.oma[m], pick)));
 }
 
-__device__ __forceinline__ int eval_bucket(const EvalCounts& ec, unsigned long long kb) {
+__device__ __forceinline__ void eval_rsd4(bool need_i, const double* rsd, int s, int n_songs, double (&rd)[4]) {
+#pragma unroll
+  for (int t = 0; t < 4; ++t) rd[t] = (need_i && s + t < n_songs) ? rsd[s + t] : 0.0;
+}
+
+__device__ __forceinline__ int eval_bucket(const EvalGroup& g, int m, int n_thresholds, unsigned long long kb) {
   int bk = 0;
 #pragma unroll
-  for (int t = 0; t < 11; ++t) bk += (t < ec.n_thresholds && kb >= ec.cut[t]) ? 1 : 0;
+  for (int t = 0; t < 11; ++t) bk += (t < n_thresholds && kb >= g.cut[m][t]) ? 1 : 0;
   return bk;
 }
 
-// min / max of the emitted scores of a slice: warp shuffles, one pair of atomics per warp that saw an emitted pair
+// min / max of each model's emitted scores of a slice: warp shuffles, one pair of atomics per model and warp that saw an emitted pair
 __global__ void __launch_bounds__(kEvalThreads)
-eval_range_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+eval_range_kernel(EvalGroup g, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
                   const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_songs, const double* __restrict__ rsa,
                   const double* __restrict__ rsd, unsigned long long* __restrict__ mm) {
+  const GroupNeeds nd = group_needs(g);
   const int b = blockIdx.y;
-  const double rsu = rsa[u0 + b];
-  const long long* ru = sint_u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
-  const long long* ri = sint_i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
-  const uint64_t* rsel = sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
-  unsigned long long lo = ~0ULL, hi = 0ULL;
+  const double rsu = nd.u ? rsa[u0 + b] : 0.0;
+  const long long* ru = nd.u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
+  const long long* ri = nd.i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
+  const uint64_t* rsel = nd.sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
+  int split[kEvalGroupMax];
+  unsigned long long lo[kEvalGroupMax], hi[kEvalGroupMax];
+#pragma unroll
+  for (int m = 0; m < kEvalGroupMax; ++m) {
+    split[m] = (m < g.n && g.model[m] == MODEL_AGG) ? g.split[m][u0 + b] : 0;
+    lo[m] = ~0ULL; hi[m] = 0ULL;
+  }
   for (int s = 4 * (blockIdx.x * kEvalThreads + static_cast<int>(threadIdx.x)); s < n_songs; s += 4 * kEvalThreads * gridDim.x) {
-    double rd[4]; unsigned long long kb[4]; bool ok[4];
-    eval_rsd4(bp, rsd, s, n_songs, rd);
-    eval_quad(bp, ru, ri, rsel, s, n_songs, rsu, rd, kb, ok);
+    double rd[4]; long long a[4], x[4]; bool ok[4];
+    eval_rsd4(nd.i, rsd, s, n_songs, rd);
+    eval_load4(nd, ru, ri, s, n_songs, a, x, ok);
+    const uint64_t selw = nd.sel ? rsel[s >> 6] >> (s & 63) : 0;
 #pragma unroll
-    for (int t = 0; t < 4; ++t)
-      if (ok[t]) { lo = kb[t] < lo ? kb[t] : lo; hi = kb[t] > hi ? kb[t] : hi; }
+    for (int t = 0; t < 4; ++t) {
+      if (!ok[t]) continue;
+#pragma unroll
+      for (int m = 0; m < kEvalGroupMax; ++m) {
+        if (m >= g.n) break;
+        const unsigned long long kb = eval_key(g, m, a[t], x[t], rsu, rd[t], s + t, (selw >> t) & 1ULL, split[m]);
+        lo[m] = kb < lo[m] ? kb : lo[m]; hi[m] = kb > hi[m] ? kb : hi[m];
+      }
+    }
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const unsigned long long a = __shfl_xor_sync(0xffffffffu, lo, o), c = __shfl_xor_sync(0xffffffffu, hi, o);
-    lo = a < lo ? a : lo; hi = c > hi ? c : hi;
+  for (int m = 0; m < kEvalGroupMax; ++m) {
+    if (m >= g.n) break;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long p = __shfl_xor_sync(0xffffffffu, lo[m], o), q = __shfl_xor_sync(0xffffffffu, hi[m], o);
+      lo[m] = p < lo[m] ? p : lo[m]; hi[m] = q > hi[m] ? q : hi[m];
+    }
+    if ((threadIdx.x & 31) == 0 && lo[m] != ~0ULL) { atomicMin(mm + 2 * g.out[m], lo[m]); atomicMax(mm + 2 * g.out[m] + 1, hi[m]); }
   }
-  if ((threadIdx.x & 31) == 0 && lo != ~0ULL) { atomicMin(mm, lo); atomicMax(mm + 1, hi); }
 }
 
 // Prediction counts of the label songs.  A CTA owns a tile of 1024 songs (4 per thread) over `rows` panel rows (<= 512: the flush, one
-// global atomic per non-zero (song, bucket) per CTA, is paid once per up to 512 rows); each thread counts its own
-// songs' buckets in a private slice of the shared histogram (no shared atomics), then flushes the non-zero entries with global atomics.
-// Threads whose 4 songs are no label song read nothing: the kernel moves only the panel sectors of label songs.
+// global atomic per non-zero (model, song, bucket) per CTA, is paid once per up to 512 rows, and a u16 counter cannot wrap); each thread
+// counts its own songs' buckets in a private slice of the shared histogram (no shared atomics), then flushes the non-zero entries with
+// global atomics.  Threads whose 4 songs are no label song read nothing: the kernel moves only the panel sectors of label songs.
 __global__ void __launch_bounds__(kEvalThreads)
-eval_count_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+eval_count_kernel(EvalGroup g, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
                   const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_users, int n_songs, const double* __restrict__ rsa,
                   const double* __restrict__ rsd, int rows, EvalCounts ec) {
-  __shared__ unsigned int hist[11 * 4 * kEvalThreads];   // [bucket - 1][song of the thread][thread]
+  extern __shared__ unsigned short hist[];   // [model][bucket - 1][song of the thread][thread]
+  const GroupNeeds nd = group_needs(g);
   const int tid = threadIdx.x;
   const int s = blockIdx.x * kEvalTile + 4 * tid;
+  const int nth = ec.n_thresholds;
   int li[4];
   bool any = false;
 #pragma unroll
   for (int t = 0; t < 4; ++t) { li[t] = s + t < n_songs ? ec.colmap[s + t] : -1; any = any || li[t] >= 0; }
   if (!any) return;
-  const int nh = 4 * ec.n_thresholds;
+  const int nh = g.n * nth * 4;
   for (int i = 0; i < nh; ++i) hist[i * kEvalThreads + tid] = 0;
   double rd[4];
-  eval_rsd4(bp, rsd, s, n_songs, rd);
+  eval_rsd4(nd.i, rsd, s, n_songs, rd);
   const int r0 = blockIdx.y * rows, r1 = min(n_users, r0 + rows);
-#pragma unroll 4
+#pragma unroll 2
   for (int b = r0; b < r1; ++b) {
-    const long long* ru = sint_u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
-    const long long* ri = sint_i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
-    const uint64_t* rsel = sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
-    unsigned long long kb[4]; bool ok[4];
-    eval_quad(bp, ru, ri, rsel, s, n_songs, bp.model == MODEL_IBM ? 0.0 : rsa[u0 + b], rd, kb, ok);
+    const long long* ru = nd.u ? sint_u + static_cast<long long>(b) * spitch : nullptr;
+    const long long* ri = nd.i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
+    long long a[4], x[4]; bool ok[4];
+    eval_load4(nd, ru, ri, s, n_songs, a, x, ok);
+    const uint64_t selw = nd.sel ? sel[static_cast<long long>(b) * sel_pitch_words + (s >> 6)] >> (s & 63) : 0;
+    const double rsu = nd.u ? rsa[u0 + b] : 0.0;
 #pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const int bk = (ok[t] && li[t] >= 0) ? eval_bucket(ec, kb[t]) : 0;
-      if (bk) hist[((bk - 1) * 4 + t) * kEvalThreads + tid] += 1;
+    for (int m = 0; m < kEvalGroupMax; ++m) {
+      if (m >= g.n) break;
+      const int split = g.model[m] == MODEL_AGG ? g.split[m][u0 + b] : 0;
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        const int bk = (ok[t] && li[t] >= 0) ? eval_bucket(g, m, nth, eval_key(g, m, a[t], x[t], rsu, rd[t], s + t, (selw >> t) & 1ULL, split)) : 0;
+        if (bk) hist[(((m * nth) + bk - 1) * 4 + t) * kEvalThreads + tid] += 1;
+      }
     }
   }
-  for (int k = 0; k < ec.n_thresholds; ++k)
+  for (int m = 0; m < g.n; ++m) {
+    unsigned long long* pred = ec.pred_b + g.out[m] * ec.model_stride;
+    for (int k = 0; k < nth; ++k)
 #pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const unsigned int v = hist[(k * 4 + t) * kEvalThreads + tid];
-      if (v) atomicAdd(ec.pred_b + static_cast<long long>(li[t]) * ec.n_thresholds + k, static_cast<unsigned long long>(v));
-    }
+      for (int t = 0; t < 4; ++t) {
+        const unsigned int v = hist[(((m * nth) + k) * 4 + t) * kEvalThreads + tid];
+        if (v) atomicAdd(pred + static_cast<long long>(li[t]) * nth + k, static_cast<unsigned long long>(v));
+      }
+  }
 }
 
-// One warp per test user of the slice: its label songs inside the scored columns add to nlab, and to tp in the bucket of their score
+// One warp per test user of the slice: its label songs inside the scored columns add to nlab, and to each model's tp in the bucket of
+// that model's score
 __global__ void __launch_bounds__(128)
-eval_label_kernel(BlendParams bp, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
+eval_label_kernel(EvalGroup g, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
                   const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_users, int n_songs, const double* __restrict__ rsa,
                   const double* __restrict__ rsd, EvalCounts ec) {
+  const GroupNeeds nd = group_needs(g);
   const int lane = threadIdx.x & 31;
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (b >= n_users) return;
@@ -232,43 +279,51 @@ eval_label_kernel(BlendParams bp, const long long* __restrict__ sint_u, const lo
     if (c < 0 || c >= n_songs) continue;                  // another song window's label, or a label-only song (id >= S)
     const int li = ec.colmap[c];
     if (li < 0) continue;                                  // cannot happen: mr_eval_counts checks new_songs covers every label
-    atomicAdd(ec.nlab + li, 1ULL);
+    if (ec.nlab) atomicAdd(ec.nlab + li, 1ULL);
     const long long o = static_cast<long long>(b) * spitch + c;
-    const long long a = bp.model != MODEL_IBM ? sint_u[o] : 0, x = bp.model != MODEL_UBM ? sint_i[o] : 0;
+    const long long a = nd.u ? sint_u[o] : 0, x = nd.i ? sint_i[o] : 0;
     if (a < 0 || x < 0) continue;                          // listened: not emitted, a false negative at every threshold
-    const bool pick = bp.model >= MODEL_AGG && ((sel[static_cast<long long>(b) * sel_pitch_words + (c >> 6)] >> (c & 63)) & 1ULL);
-    const unsigned long long kb = static_cast<unsigned long long>(__double_as_longlong(
-        blend_score(bp.model, a, x, rsa[u], bp.model != MODEL_UBM ? rsd[c] : 0.0, bp.alpha, bp.one_minus_alpha, pick)));
-    const int bk = eval_bucket(ec, kb);
-    if (bk) atomicAdd(ec.tp_b + static_cast<long long>(li) * ec.n_thresholds + (bk - 1), 1ULL);
+    const bool selbit = nd.sel && ((sel[static_cast<long long>(b) * sel_pitch_words + (c >> 6)] >> (c & 63)) & 1ULL);
+    const double rsu = nd.u ? rsa[u] : 0.0, rd = nd.i ? rsd[c] : 0.0;
+#pragma unroll
+    for (int m = 0; m < kEvalGroupMax; ++m) {
+      if (m >= g.n) break;
+      const int split = g.model[m] == MODEL_AGG ? g.split[m][u] : 0;
+      const int bk = eval_bucket(g, m, ec.n_thresholds, eval_key(g, m, a, x, rsu, rd, c, selbit, split));
+      if (bk) atomicAdd(ec.tp_b + g.out[m] * ec.model_stride + static_cast<long long>(li) * ec.n_thresholds + (bk - 1), 1ULL);
+    }
   }
 }
 
-int launch_eval_range(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+int launch_eval_range(const EvalGroup& g, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
                       long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
                       unsigned long long* mm, cudaStream_t st) {
   if (n_songs <= 0) return 0;
+  if (g.n < 1 || g.n > kEvalGroupMax) return -2;
   for (int r0 = 0; r0 < n_users; r0 += 32768) {   // grid.y limit
     const int n = min(32768, n_users - r0);
     const long long off = static_cast<long long>(r0) * spitch;
     const int tiles = (n_songs + kEvalTile - 1) / kEvalTile;
     const int gx = max(1, min(tiles, (2048 + n - 1) / n));   // >= ~2048 CTAs per launch, each sweeping a long stretch of its row
-    eval_range_kernel<<<dim3(gx, n), kEvalThreads, 0, st>>>(bp, sint_u ? sint_u + off : nullptr, sint_i ? sint_i + off : nullptr, spitch,
+    eval_range_kernel<<<dim3(gx, n), kEvalThreads, 0, st>>>(g, sint_u ? sint_u + off : nullptr, sint_i ? sint_i + off : nullptr, spitch,
                                                             sel ? sel + static_cast<long long>(r0) * sel_pitch_words : nullptr, sel_pitch_words,
                                                             u0 + r0, n_songs, rsa, rsd, mm);
   }
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
-int launch_eval_count(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+int launch_eval_count(const EvalGroup& g, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
                       long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
                       const EvalCounts& ec, cudaStream_t st) {
   if (n_users <= 0 || n_songs <= 0) return 0;
-  if (ec.n_thresholds < 1 || ec.n_thresholds > 11) return -2;
+  if (ec.n_thresholds < 1 || ec.n_thresholds > 11 || g.n < 1 || g.n > kEvalGroupMax) return -2;
+  const size_t smem = static_cast<size_t>(g.n) * ec.n_thresholds * 4 * kEvalThreads * sizeof(unsigned short);
+  // per call, not once per process: the attribute belongs to the current device, and a process may drive several
+  if (smem > 48 * 1024 && cudaFuncSetAttribute(eval_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)) != cudaSuccess) return -1;
   const int chunks = (n_users + kEvalRows - 1) / kEvalRows, rows = (n_users + chunks - 1) / chunks;   // equal row chunks
   const dim3 grid((n_songs + kEvalTile - 1) / kEvalTile, chunks);
-  eval_count_kernel<<<grid, kEvalThreads, 0, st>>>(bp, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, rows, ec);
-  eval_label_kernel<<<(n_users + 3) / 4, 128, 0, st>>>(bp, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, ec);
+  eval_count_kernel<<<grid, kEvalThreads, smem, st>>>(g, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, rows, ec);
+  eval_label_kernel<<<(n_users + 3) / 4, 128, 0, st>>>(g, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_users, n_songs, rsa, rsd, ec);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

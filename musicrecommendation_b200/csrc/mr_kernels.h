@@ -134,25 +134,39 @@ int launch_blend_arrays(const BlendParams& bp, const double* ubm, const double* 
 int launch_evaluate(const double* scores, int n_users, int n_songs, const long long* lab_ptr, const int* lab_col, const int* new_songs,
                     int n_new, int n_thresholds, unsigned long long* minmax, double* ap_out, int num_sms, cudaStream_t st);
 
-// Streamed evaluateModel (DESIGN.md §4.5): per slice of a batch's score panels (masked, select bits built), either the min / max of
-// the emitted scores (bit patterns, mm[0] / mm[1]) or the confusion counts of the label songs by threshold bucket.
-int launch_eval_range(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+// Streamed evaluateModel (DESIGN.md §4.5, §4.6): per slice of a batch's score panels (masked; the STOCH select plane built), the consumers
+// of a GROUP of models in one launch, reading each panel sector, select word and label entry once: either the min / max of each model's
+// emitted scores (bit patterns, mm[2 * out] / mm[2 * out + 1]) or each model's confusion counts of the label songs by threshold bucket.
+// kEvalGroupMax: eval_count_kernel keeps 4 songs x n_thresholds u16 counters per thread and model (22 KB per model at 11 thresholds);
+// five models take 110 KB, two CTAs per SM (sm_100a: 228 KB of shared memory per SM), so the five models of main.scala take one launch.
+constexpr int kEvalGroupMax = 5;
+struct EvalGroup {
+  int n;                                        // models in the group, 1..kEvalGroupMax; at most one MODEL_STOCH (it reads the select plane)
+  int model[kEvalGroupMax];
+  double alpha[kEvalGroupMax], oma[kEvalGroupMax];   // LC
+  const int* split[kEvalGroupMax];              // AGG: [U] per test user of the shard, the first column whose pair index reaches (pct * N).toInt
+  int out[kEvalGroupMax];                       // index of the model in its set: min / max pair mm[2 * out], count block pred_b + out * model_stride
+  unsigned long long cut[kEvalGroupMax][11];    // count pass: bit patterns of the model's cutoffs c_t (predicted at t <=> score >= c_t)
+};
+int launch_eval_range(const EvalGroup& g, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
                       long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
                       unsigned long long* mm, cudaStream_t st);
 struct EvalCounts {
-  unsigned long long cut[11];    // bit patterns of the cutoffs c_t (non-negative doubles or +inf): predicted at t <=> score >= c_t
   int n_thresholds;
   const int* colmap;             // [n_songs] scored column -> label-song index, -1 for columns that are no label song
-  unsigned long long* pred_b;    // [n_new][n_thresholds] emitted pairs whose bucket (number of cutoffs <= score) is b + 1
+  unsigned long long* pred_b;    // [n_new][n_thresholds] emitted pairs whose bucket (number of cutoffs <= score) is b + 1 (model 0 of the set)
   unsigned long long* tp_b;      // [n_new][n_thresholds] the same, restricted to labelled pairs
-  unsigned long long* nlab;      // [n_new] labelled pairs of the scored columns
+  long long model_stride;        // elements from one model's pred_b / tp_b block to the next model's
+  unsigned long long* nlab;      // [n_new] labelled pairs of the scored columns (counted by the launch that gets it non-null)
   const long long* lab_ptr;      // [U + 1] label CSR of the shard (global song ids)
   const int* lab_col;
   int col_lo;                    // first song of the scored columns (song window); column = song - col_lo
 };
-int launch_eval_count(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+int launch_eval_count(const EvalGroup& g, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
                       long long sel_pitch_words, int u0, int n_users, int n_songs, const double* rsa, const double* rsd,
                       const EvalCounts& ec, cudaStream_t st);
+// AGG's pick as one split column per test user (k3_topk.cu): split[u] for u in [0, n_users) of the shard
+int launch_agg_split(const BlendParams& bp, const long long* te_ptr, const int* te_col, int n_users, int n_songs, int* split, cudaStream_t st);
 
 int launch_map_at_k(const int* top_song, const int* top_len, int n_users, int k, const long long* lab_ptr, const int* lab_col,
                     double* ap_out, cudaStream_t st);

@@ -37,6 +37,7 @@ constexpr int kMaxDegUbm = 112589;      // (2e-5 * 2^24)^2 = 112 589.99
 constexpr int kPreStreams = 4;          // streams of the in-place head-row build (start_head_rows): 113.8 / 82.9 / 75.8 / 73.4 ms with 1 / 2 / 3 / 4
 constexpr int kPreExtraStreams = 3;     // at most 1 + 3 (MRSCORE_PRE_STREAMS)
 constexpr int kMaxDegIbm = 1801439;     // (2e-5 * 2^26)^2 = 1 801 439.85
+constexpr size_t kCallerReserve = 6ULL << 30;   // HBM the item-space batch plan leaves for the caller's context and small workspaces
 
 }  // namespace
 
@@ -98,7 +99,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard and its results: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -112,10 +113,13 @@ struct mr_handle {
   double* d_dense = nullptr; int32_t* d_cnt = nullptr; float* d_simf = nullptr;
   // results
   int *d_out_song = nullptr, *d_out_len = nullptr; double* d_out_score = nullptr; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;
-  // streamed evaluation (mr_eval_range / mr_eval_counts).  gen counts the calls that may rewrite the score panels; after a range pass
-  // over a single-batch item-space shard the panels still hold the masked numerators of (eval_model, eval_param, eval_seed), and a
-  // count pass of the same model at the same gen reuses them instead of scoring again.
-  unsigned long long gen = 0, eval_gen = ~0ULL; int eval_model = -1; double eval_param = 0; uint64_t eval_seed = 0;
+  // results of the last mr_topk_multi_device: entry i's block starts at multi_stride * i in the SL_MULTI_OUT slot (song | score | len)
+  int multi_n = 0, multi_k = 0; size_t multi_stride = 0;
+  long long passes = 0;   // scoring passes since mr_load: batches whose score panels were built
+  // streamed evaluation (mr_eval_range* / mr_eval_counts*).  gen counts the calls that may rewrite the score panels; after a range pass
+  // over a single-batch item-space shard the panels still hold the masked numerators of the model set (eval_n entries of eval_models,
+  // eval_params, eval_seeds), and a count pass of the same set at the same gen reuses them instead of scoring again.
+  unsigned long long gen = 0, eval_gen = ~0ULL; int eval_n = 0; int eval_models[16] = {}; double eval_params[16] = {}; uint64_t eval_seeds[16] = {};
   unsigned long long* d_eval_mm = nullptr;   // [2] min / max bit patterns of the range pass
   EvalCounts ec{};                           // device state of the count pass
   // profiling
@@ -578,7 +582,7 @@ int plan_item_batches_once(mr_handle* h, const std::vector<long long>& hu_ptr, i
     MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
     const size_t per_row = static_cast<size_t>(h->spitch) * 16 + static_cast<size_t>(h->sel_pitch) * 8;
     size_t avail = free_b + h->slot_cap[mr_handle::SL_SINT_U] + h->slot_cap[mr_handle::SL_SINT_I] + h->slot_cap[mr_handle::SL_SEL];
-    size_t reserve = 6ULL << 30;   // left for the caller's context (torch, NCCL buffers, gathered top-k blocks) and small workspaces
+    size_t reserve = kCallerReserve;   // left for the caller's context (torch, NCCL buffers, gathered top-k blocks) and small workspaces
     if (!h->head_ready && h->head_rows_cap == 0) reserve += static_cast<size_t>(std::max(h->n_head, 1)) * h->spitch * 6 + (1ULL << 30);   // head rows + staging come later
     long long max_rows = avail > reserve ? static_cast<long long>((avail - reserve) / per_row) : 0;
     max_rows = std::max<long long>(max_rows, kUserBatch);
@@ -690,25 +694,63 @@ int plan_item_batches(mr_handle* h, const std::vector<long long>& hu_ptr) {
 }
 
 // RUN_EVAL_RANGE / RUN_EVAL_COUNT: the streamed evaluateModel passes (DESIGN.md §4.5) in place of the top-k select of each slice;
-// host_out is null / points to a bool "the panels already hold this model's masked numerators" (resident reuse, mr_eval_counts).
+// host_out is null / points to a bool "the panels already hold this set's masked numerators" (resident reuse, mr_eval_counts*).
 enum RunMode { RUN_TOPK, RUN_DENSE, RUN_COUNTS_UBM, RUN_SIM_UBM, RUN_EVAL_RANGE, RUN_EVAL_COUNT };
 struct TopkHostOut { int32_t* song; double* score; int32_t* len; };   // RUN_TOPK: caller buffers the finished slices are copied into
 // RUN_DENSE: where the fp64 rows go.  ALL: out[u][s] for every test user (mr_score_dense).  USERS: out[i][s] for the listed users
 // (DIST getRanks1 granularity).  SONGS: d_out[i][u] for the listed songs, gathered on the device (DIST getRanks2 granularity).
 struct DenseOut { enum Kind { ALL, USERS, SONGS } kind; double* out; const int32_t* ids; int n_ids; const int* d_ids; double* d_out; };
 
-int eval_slice(mr_handle* h, RunMode mode, const BlendParams& bp, const long long* su, const long long* si, const uint64_t* sel, int u0, int n,
-               cudaStream_t st) {
-  if (mode == RUN_EVAL_RANGE)
-    MR_LAUNCH(h, launch_eval_range(bp, su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->d_eval_mm, st));
-  else
-    MR_LAUNCH(h, launch_eval_count(bp, su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->ec, st));
+// A model set (DESIGN.md §4.6): the entries one scoring of the shard serves.  The single-model calls run a set of one.
+constexpr int kMaxSet = 16;
+struct ModelSet {
+  int n = 0;
+  BlendParams bp[kMaxSet];
+  int* out_song[kMaxSet] = {}; double* out_score[kMaxSet] = {}; int* out_len[kMaxSet] = {};   // RUN_TOPK: each entry's device result
+  // eval modes: the entries grouped for the fused consumers; grp_stoch[g] = the STOCH entry whose select plane group g reads, or -1
+  int n_groups = 0; EvalGroup grp[kMaxSet]; int grp_stoch[kMaxSet] = {};
+  int n_stoch = 0;
+  bool needs(int panel_model) const {   // UBM panel: some entry is not IBM; IBM panel: some entry is not UBM
+    for (int i = 0; i < n; ++i) if (bp[i].model != (panel_model == MODEL_UBM ? MODEL_IBM : MODEL_UBM)) return true;
+    return false;
+  }
+};
+
+// The consumers of one masked slice: per entry the select (after its blend's select plane), or per group the fused eval kernels (after
+// the group's STOCH plane; plane_resident: the plane of the set's only STOCH entry is still in place from the range pass).
+int consume_slice(mr_handle* h, const ModelSet& set, RunMode mode, int k, long long* su, long long* si, uint64_t* sel, int u0, int n,
+                  cudaStream_t st, bool plane_resident) {
+  if (mode == RUN_TOPK) {
+    for (int e = 0; e < set.n; ++e) {
+      const BlendParams& bp = set.bp[e];
+      const bool blend_sel = bp.model == MODEL_AGG || bp.model == MODEL_STOCH;
+      if (blend_sel) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
+      MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, bp.model != MODEL_IBM ? su : nullptr, bp.model != MODEL_UBM ? si : nullptr, h->spitch,
+                               blend_sel ? sel : nullptr, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, k, set.out_song[e],
+                               set.out_score[e], set.out_len[e], st));
+    }
+    return MR_OK;
+  }
+  for (int g = 0; g < set.n_groups; ++g) {
+    const int se = set.grp_stoch[g];
+    if (se >= 0 && !plane_resident)
+      MR_LAUNCH(h, launch_select_bits(set.bp[se], h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
+    if (mode == RUN_EVAL_RANGE) {
+      MR_LAUNCH(h, launch_eval_range(set.grp[g], su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->d_eval_mm, st));
+    } else {
+      EvalCounts ec = h->ec;
+      if (g > 0) ec.nlab = nullptr;   // label counts do not depend on the model: the first group takes them
+      MR_LAUNCH(h, launch_eval_count(set.grp[g], su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, ec, st));
+    }
+  }
   return MR_OK;
 }
 
-int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode mode, void* host_out) {
-  const bool need_ubm = model != MODEL_IBM;
-  const bool need_ibm = model != MODEL_UBM && mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM;
+int run_batches(mr_handle* h, const ModelSet& set, int k, RunMode mode, void* host_out) {
+  const bool need_ubm = set.needs(MODEL_UBM);
+  const bool need_ibm = set.needs(MODEL_IBM) && mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM;
+  const int model = set.bp[0].model;   // RUN_DENSE runs a set of one
+  const int pure = need_ubm && need_ibm ? -1 : (need_ubm ? MODEL_UBM : MODEL_IBM);   // the one panel the set needs, if only one
   const bool eval = mode == RUN_EVAL_RANGE || mode == RUN_EVAL_COUNT;
   const bool ranked = mode == RUN_TOPK || eval;      // per-slice consumers of the masked panels: top-k select or evaluation
   const bool item_space = h->space == MR_SPACE_ITEM && (mode == RUN_DENSE || ranked);
@@ -724,7 +766,8 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
   // What it buys is the kernel boundaries (the next kernel's CTAs start while the previous grid drains): 727 -> 701 ms for the two
   // models of the one-GPU job.  Making the kernels truly share the SMs was measured and is WORSE (profiles/r02_summary.md §8): the head
   // pass lives on every resident CTA working on the same song tile out of L2, and a select streaming 48 GB through L2 beside it breaks that.
-  const bool pipelined = item_space && ranked && (model == MODEL_UBM || model == MODEL_IBM) && !(h->flags & MR_PROFILE) &&
+  // A set that needs both panels (a blend, or UBM and IBM entries) cannot alternate them across batches: it takes the alternating slices.
+  const bool pipelined = item_space && ranked && pure >= 0 && !(h->flags & MR_PROFILE) &&
                          h->U > batch && !getenv("MRSCORE_NO_PIPELINE");
   // Every other item-space top-k (one batch, e.g. a GPU's share of a song-partitioned job, or a blend) puts consecutive slices on two
   // alternating streams instead: same idea, the boundaries between the slices' kernels (107.6 -> 105.1 ms for both models of a 1/8 song
@@ -738,12 +781,13 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
     const int nb = std::min(batch, h->U - b0);
     if (item_space) {
       const int models = (need_ubm ? 1 : 0) | (need_ibm ? 2 : 0);
-      const int par = pipelined ? ((b0 / batch) & 1) ^ (model == MODEL_IBM ? 1 : 0) : 0;   // panel of this batch: 0 = d_sint_u, 1 = d_sint_i
+      const int par = pipelined ? ((b0 / batch) & 1) ^ (pure == MODEL_IBM ? 1 : 0) : 0;   // panel of this batch: 0 = d_sint_u, 1 = d_sint_i
       // the panels of this batch by role (pipelined: the pure model's panel alternates between the two allocations)
       long long* const panel = par ? h->d_sint_i : h->d_sint_u;
-      long long* const pu = pipelined ? (model == MODEL_UBM ? panel : nullptr) : h->d_sint_u;
-      long long* const pi = pipelined ? (model == MODEL_IBM ? panel : nullptr) : h->d_sint_i;
+      long long* const pu = pipelined ? (pure == MODEL_UBM ? panel : nullptr) : h->d_sint_u;
+      long long* const pi = pipelined ? (pure == MODEL_IBM ? panel : nullptr) : h->d_sint_i;
       if (!reuse) {
+        ++h->passes;
         PhaseTimer t(h, MR_T_HEAD_ROWSUM);
         const int bi = b0 / batch;
         const int4* grp = h->d_grp_hdr + static_cast<long long>(bi) * h->n_groups;
@@ -778,7 +822,9 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       const long long sub_fit = static_cast<long long>(kTailSubBatch) * round_up(h->S, 32) / h->spitch / (2 * h->num_sms) * (2 * h->num_sms);
       const int tail_sub = tail_sub_env ? tail_sub_env : static_cast<int>(std::max<long long>(kTailSubBatch, std::min<long long>(sub_fit, 1 << 20)));
       const int tail_lanes = 2LL * h->n_cols >= h->S ? 32 : (4LL * h->n_cols >= h->S ? 16 : 8);
-      const bool sel_needed = model == MODEL_AGG || model == MODEL_STOCH;
+      // the select plane: the blends' bits for the top-k, STOCH's for the fused eval kernels (AGG's pick there is its split column)
+      bool sel_needed = false;
+      for (int e = 0; e < set.n; ++e) sel_needed = sel_needed || set.bp[e].model == MODEL_STOCH || (!eval && set.bp[e].model == MODEL_AGG);
       const TopkHostOut* ho = mode == RUN_TOPK ? static_cast<const TopkHostOut*>(host_out) : nullptr;
       for (int s0 = 0; s0 < nb; s0 += tail_sub) {
         const int sn = std::min(tail_sub, nb - s0);
@@ -795,17 +841,8 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
         long long* si = need_ibm ? pi + static_cast<long long>(s0) * h->spitch : nullptr;
         uint64_t* sel = sel_needed ? h->d_sel + static_cast<long long>(s0) * h->sel_pitch : nullptr;
         const int u0 = b0 + s0;
-        if (!reuse) {
-          MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
-          if (sel_needed) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, sn, h->n_cols, sel, h->sel_pitch, ts));
-        }
-        if (eval) {
-          const int rc = eval_slice(h, mode, bp, su, si, sel, u0, sn, ts);
-          if (rc) return rc;
-          continue;
-        }
-        MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, su, si, h->spitch, sel, h->sel_pitch, u0, sn, h->n_cols, h->d_rsa, h->d_rsd, k, h->d_out_song,
-                                 h->d_out_score, h->d_out_len, ts));
+        if (!reuse) MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
+        if (const int rc = consume_slice(h, set, mode, k, su, si, sel, u0, sn, ts, reuse && set.n_stoch == 1)) return rc;
         if (ho) {
           MR_CUDA(h, cudaEventRecord(h->ev_slice, ts));
           MR_CUDA(h, cudaStreamWaitEvent(h->copy_stream, h->ev_slice, 0));
@@ -828,6 +865,7 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       }
       if (mode != RUN_DENSE) continue;   // the batch is finished; RUN_DENSE continues below on the whole batch
     } else if (need_ubm) {
+      if (mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM) ++h->passes;
       int rc = count_ubm_batch(h, b0, nb);
       if (rc) return rc;
       if (mode == RUN_COUNTS_UBM || mode == RUN_SIM_UBM) {
@@ -851,6 +889,7 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
       AggItems items{h->d_item_song, h->d_item_begin, h->d_item_len, h->d_item_split, h->n_items};
       MR_LAUNCH(h, launch_aggregate_ubm(items, h->d_csc_idx, h->d_qv, h->d_ct, h->T, h->d_sint_u, h->spitch, h->num_sms, h->stream));
     }
+    if (!item_space && !need_ubm) ++h->passes;
     if (item_space) {
       // both models were produced above
     } else if (need_ibm && h->engine == MR_ENGINE_SPARSE) {
@@ -903,17 +942,9 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
         MR_CUDA(h, cudaStreamSynchronize(h->stream));
       }
     } else {
-      if (model == MODEL_AGG || model == MODEL_STOCH)
-        MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, b0, nb, h->n_cols, h->d_sel, h->sel_pitch, h->stream));
-      if (eval) {
-        const int rc = eval_slice(h, mode, bp, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr,
-                                  (model == MODEL_AGG || model == MODEL_STOCH) ? h->d_sel : nullptr, b0, nb, h->stream);
-        if (rc) return rc;
-        continue;
-      }
-      MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr, h->spitch,
-                               (model == MODEL_AGG || model == MODEL_STOCH) ? h->d_sel : nullptr, h->sel_pitch, b0, nb, h->n_cols, h->d_rsa,
-                               h->d_rsd, k, h->d_out_song, h->d_out_score, h->d_out_len, h->stream));
+      const int rc = consume_slice(h, set, mode, k, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr, h->d_sel, b0, nb,
+                                   h->stream, false);
+      if (rc) return rc;
     }
   }
   if (need_ibm && !item_space && h->engine == MR_ENGINE_SPARSE) {
@@ -925,6 +956,15 @@ int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode m
         return fail(h, MR_ERR_OOM, "IBM weighted-count carry list overflowed (%u events > capacity %u)", h->h_carry_seen[i], h->carry_cap);
   }
   return MR_OK;
+}
+
+
+// a set of one: the single-model calls
+int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode mode, void* host_out) {
+  ModelSet set;
+  set.n = 1; set.bp[0] = bp; set.bp[0].model = model;
+  set.out_song[0] = h->d_out_song; set.out_score[0] = h->d_out_score; set.out_len[0] = h->d_out_len;
+  return run_batches(h, set, k, mode, host_out);
 }
 
 int make_blend_params(mr_handle* h, int model, double param, uint64_t seed, long long n_total, BlendParams* bp) {
@@ -1212,7 +1252,7 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
     if ((rc = dev_upload(h, &h->d_head_lst_ptr, lst_ptr.data(), lst_ptr.size(), h->allocs))) return rc;
   }
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
-  h->loaded = true;
+  h->loaded = true; h->passes = 0;
   if (n_test > 0) return mr_set_test_users(h, n_test, te_rowptr, te_col, deg_test, 0, 0);
   return MR_OK;
 }
@@ -1236,7 +1276,7 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   MR_CUDA(h, cudaSetDevice(h->device));
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   lap("check_csr + sync");
-  h->have_test = false; h->have_topk = false; h->out_k = 0; ++h->gen;
+  h->have_test = false; h->have_topk = false; h->out_k = 0; h->multi_n = 0; ++h->gen;
   const int U = n_test; const long long nnz = te_rowptr[U];
   h->U = U; h->nnz_te = nnz;
   h->h_te_ptr.assign(te_rowptr, te_rowptr + U + 1);
@@ -1779,56 +1819,129 @@ void join_slice_streams(mr_handle* h) {   // an eval call that fails inside the 
     if (s && cudaEventRecord(h->ev_join, s) == cudaSuccess) cudaStreamWaitEvent(h->stream, h->ev_join, 0);
 }
 
-int eval_params(mr_handle* h, int model, double param, uint64_t seed, BlendParams* bp) {
-  int rc = require_test(h);
-  if (rc) return rc;
-  // min / max are taken on the bit patterns of non-negative scores, as in getTopK (documented deviation, DESIGN.md §3)
-  if (model == MR_LC && !(param >= 0 && param <= 1))
-    return fail(h, MR_ERR_PARAM_RANGE, "evaluation: alpha of the linear combination must be between 0 and 1");
-  if ((rc = make_blend_params(h, model, param, seed, h->n_pairs_total, bp))) return rc;
-  bp->pair_base = h->d_pair_base;
-  bp->stats = nullptr;
-  if (model != MR_UBM && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
-  return MR_OK;
-}
-}  // namespace
-
-int mr_eval_cutoffs(double mn, double mx, int n_thresholds, double* out) {
-  if (!out || (n_thresholds != 10 && n_thresholds != 11)) return MR_ERR_BAD_ARG;
-  eval_cutoffs(mn, mx, n_thresholds, out);
-  return MR_OK;
-}
-
-int mr_eval_range(mr_handle* h, int model, double param, uint64_t seed, double* out_min, double* out_max) {
-  if (!h) return MR_ERR_STATE;
-  if (!out_min || !out_max) return fail(h, MR_ERR_BAD_ARG, "null output");
-  BlendParams bp;
-  int rc = eval_params(h, model, param, seed, &bp);
-  if (rc) return rc;
-  if ((rc = slot_alloc(h, mr_handle::SL_EVAL_MM, &h->d_eval_mm, 2))) return rc;
-  const unsigned long long init[2] = {~0ULL, 0ULL};
-  MR_CUDA(h, cudaMemcpyAsync(h->d_eval_mm, init, sizeof init, cudaMemcpyHostToDevice, h->stream));
-  if ((rc = run_batches(h, model, bp, 0, RUN_EVAL_RANGE, nullptr))) { join_slice_streams(h); return rc; }
-  unsigned long long mm[2];
-  MR_CUDA(h, cudaMemcpyAsync(mm, h->d_eval_mm, sizeof mm, cudaMemcpyDeviceToHost, h->stream));
-  MR_CUDA(h, cudaStreamSynchronize(h->stream));
-  h->eval_gen = h->gen; h->eval_model = model; h->eval_param = param; h->eval_seed = seed;
-  if (mm[0] == ~0ULL) {   // no emitted pair
-    *out_min = std::numeric_limits<double>::infinity(); *out_max = -std::numeric_limits<double>::infinity();
-  } else {
-    memcpy(out_min, &mm[0], 8); memcpy(out_max, &mm[1], 8);
+// A model set from the caller's parallel arrays, every entry checked before any GPU work (what: the caller's name in the messages;
+// name_entries: the message names the first bad entry, as the set calls do).  The LC alpha must be in [0, 1]: the select and the
+// evaluator rank IEEE bit patterns of non-negative scores (documented deviation, DESIGN.md §3).
+int make_set(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, const char* what, bool name_entries,
+             ModelSet* set) {
+  if (n < 1 || n > kMaxSet) return fail(h, MR_ERR_BAD_ARG, "%s: n_models = %d outside 1..%d", what, n, kMaxSet);
+  if (!models || !params || !seeds) return fail(h, MR_ERR_BAD_ARG, "%s: null model arrays", what);
+  set->n = n; set->n_stoch = 0;
+  for (int i = 0; i < n; ++i) {
+    int rc;
+    if (models[i] == MR_LC && !(params[i] >= 0 && params[i] <= 1))
+      rc = fail(h, MR_ERR_PARAM_RANGE, "%s: alpha of the linear combination must be between 0 and 1", what);
+    else
+      rc = make_blend_params(h, models[i], params[i], seeds[i], h->n_pairs_total, &set->bp[i]);
+    if (rc) {
+      if (name_entries) h->err = "entry " + std::to_string(i) + ": " + h->err;
+      return rc;
+    }
+    set->bp[i].pair_base = h->d_pair_base;
+    if (models[i] == MR_STOCH) ++set->n_stoch;
   }
   return MR_OK;
 }
 
-int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double mn, double mx, int n_thresholds, const int64_t* lab_rowptr,
-                   const int32_t* lab_col, const int32_t* new_songs, int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab) {
-  if (!h) return MR_ERR_STATE;
-  if (n_thresholds != 10 && n_thresholds != 11) return fail(h, MR_ERR_BAD_ARG, "n_thresholds must be 10 (MR:590) or 11 (DIST:395)");
-  if (!lab_rowptr || !new_songs || n_new <= 0 || !out_pred || !out_tp || !out_nlab) return fail(h, MR_ERR_BAD_ARG, "null / empty arguments");
-  BlendParams bp;
-  int rc = eval_params(h, model, param, seed, &bp);
+// The evaluation form of a set: checks, the Gram workspace, the AGG split columns (one [U] array per AGG entry, on the library stream)
+// and the consumer groups.  Each STOCH entry heads a group of its own (the group reads the one select plane); the other entries fill
+// the groups in entry order, kEvalGroupMax to a launch.
+int eval_set(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, bool name_entries, ModelSet* set) {
+  int rc = require_test(h);
   if (rc) return rc;
+  if ((rc = make_set(h, n, models, params, seeds, "evaluation", name_entries, set))) return rc;
+  int n_agg = 0; bool ibm_side = false;
+  for (int e = 0; e < n; ++e) { set->bp[e].stats = nullptr; n_agg += set->bp[e].model == MODEL_AGG; ibm_side = ibm_side || set->bp[e].model != MODEL_UBM; }
+  if (ibm_side && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
+  int* d_split = nullptr;
+  if (n_agg && (rc = slot_alloc(h, mr_handle::SL_AGG_SPLIT, &d_split, static_cast<size_t>(n_agg) * h->U))) return rc;
+  set->n_groups = 0;
+  auto add = [&](int g, int e) {
+    EvalGroup& G = set->grp[g];
+    const int m = G.n++;
+    G.model[m] = set->bp[e].model; G.alpha[m] = set->bp[e].alpha; G.oma[m] = set->bp[e].one_minus_alpha; G.out[m] = e; G.split[m] = nullptr;
+    for (unsigned long long& c : G.cut[m]) c = ~0ULL;
+  };
+  auto open_group = [&](int stoch) { const int g = set->n_groups++; memset(&set->grp[g], 0, sizeof(EvalGroup)); set->grp_stoch[g] = stoch; return g; };
+  for (int e = 0; e < n; ++e)
+    if (set->bp[e].model == MODEL_STOCH) add(open_group(e), e);
+  for (int e = 0, j = 0; e < n; ++e) {
+    if (set->bp[e].model == MODEL_STOCH) continue;
+    int g = 0;
+    while (g < set->n_groups && set->grp[g].n == kEvalGroupMax) ++g;
+    if (g == set->n_groups) open_group(-1);
+    add(g, e);
+    if (set->bp[e].model == MODEL_AGG) {
+      int* split = d_split + static_cast<size_t>(j++) * h->U;
+      set->grp[g].split[set->grp[g].n - 1] = split;
+      MR_LAUNCH(h, launch_agg_split(set->bp[e], h->d_te_ptr, h->d_te_col, h->U, h->n_cols, split, h->stream));
+    }
+  }
+  return MR_OK;
+}
+
+void remember_eval_set(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds) {
+  h->eval_gen = h->gen; h->eval_n = n;
+  for (int i = 0; i < n; ++i) { h->eval_models[i] = models[i]; h->eval_params[i] = params[i]; h->eval_seeds[i] = seeds[i]; }
+}
+bool same_eval_set(const mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds) {
+  if (h->eval_gen != h->gen || h->eval_n != n) return false;
+  for (int i = 0; i < n; ++i)
+    if (h->eval_models[i] != models[i] || memcmp(&h->eval_params[i], &params[i], sizeof(double)) != 0 || h->eval_seeds[i] != seeds[i]) return false;
+  return true;
+}
+
+int eval_range_impl(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, bool name_entries, double* out_min,
+                    double* out_max) {
+  if (!h) return MR_ERR_STATE;
+  if (!out_min || !out_max) return fail(h, MR_ERR_BAD_ARG, "null output");
+  ModelSet set;
+  int rc = eval_set(h, n, models, params, seeds, name_entries, &set);
+  if (rc) return rc;
+  if ((rc = slot_alloc(h, mr_handle::SL_EVAL_MM, &h->d_eval_mm, 2 * static_cast<size_t>(n)))) return rc;
+  std::vector<unsigned long long> mm(2 * static_cast<size_t>(n));
+  for (int e = 0; e < n; ++e) { mm[2 * e] = ~0ULL; mm[2 * e + 1] = 0ULL; }
+  MR_CUDA(h, cudaMemcpyAsync(h->d_eval_mm, mm.data(), mm.size() * 8, cudaMemcpyHostToDevice, h->stream));
+  if ((rc = run_batches(h, set, 0, RUN_EVAL_RANGE, nullptr))) { join_slice_streams(h); return rc; }
+  MR_CUDA(h, cudaMemcpyAsync(mm.data(), h->d_eval_mm, mm.size() * 8, cudaMemcpyDeviceToHost, h->stream));
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  remember_eval_set(h, n, models, params, seeds);
+  for (int e = 0; e < n; ++e) {
+    if (mm[2 * e] == ~0ULL) {   // no emitted pair
+      out_min[e] = std::numeric_limits<double>::infinity(); out_max[e] = -std::numeric_limits<double>::infinity();
+    } else {
+      memcpy(&out_min[e], &mm[2 * e], 8); memcpy(&out_max[e], &mm[2 * e + 1], 8);
+    }
+  }
+  return MR_OK;
+}
+
+// MRSCORE_DEBUG_TIMING: the host stages of a count call on stderr
+struct HostStages {
+  bool on = getenv("MRSCORE_DEBUG_TIMING") != nullptr;
+  std::chrono::steady_clock::time_point t = std::chrono::steady_clock::now();
+  std::string line;
+  void mark(const char* stage) {
+    if (!on) return;
+    const auto now = std::chrono::steady_clock::now();
+    char buf[64];
+    snprintf(buf, sizeof buf, " %s=%.2f", stage, std::chrono::duration<double, std::milli>(now - t).count());
+    line += buf; t = now;
+  }
+  void print(int n) const { if (on) fprintf(stderr, "[mrscore] eval_counts host stages (ms), %d model(s):%s\n", n, line.c_str()); }
+};
+
+int eval_counts_impl(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, bool name_entries, const double* mn,
+                     const double* mx, int n_thresholds, const int64_t* lab_rowptr, const int32_t* lab_col, const int32_t* new_songs, int n_new,
+                     int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab) {
+  if (!h) return MR_ERR_STATE;
+  HostStages hs;
+  if (n_thresholds != 10 && n_thresholds != 11) return fail(h, MR_ERR_BAD_ARG, "n_thresholds must be 10 (MR:590) or 11 (DIST:395)");
+  if (!lab_rowptr || !new_songs || n_new <= 0 || !out_pred || !out_tp || !out_nlab || !mn || !mx) return fail(h, MR_ERR_BAD_ARG, "null / empty arguments");
+  ModelSet set;
+  int rc = eval_set(h, n, models, params, seeds, name_entries, &set);
+  if (rc) return rc;
+  hs.mark("set");
   const int U = h->U;
   const long long n_lab = lab_rowptr[U];
   if (lab_rowptr[0] != 0 || n_lab < 0 || (n_lab > 0 && !lab_col)) return fail(h, MR_ERR_BAD_ARG, "bad label CSR");
@@ -1840,20 +1953,35 @@ int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double 
   if (new_songs[0] < 0) return fail(h, MR_ERR_BAD_ARG, "new_songs: negative song id");
   for (int i = 1; i < n_new; ++i)
     if (new_songs[i] <= new_songs[i - 1]) return fail(h, MR_ERR_BAD_ARG, "new_songs not strictly ascending at %d", i);
-  for (long long i = 0; i < n_lab; ++i)
-    if (!std::binary_search(new_songs, new_songs + n_new, lab_col[i]))
-      return fail(h, MR_ERR_BAD_ARG, "new_songs lacks label song %d", lab_col[i]);
-  if (mx - mn > 0 && !(mn >= 0)) return fail(h, MR_ERR_BAD_ARG, "mn must be >= 0 (scores are non-negative)");
-  double cut[11];
-  eval_cutoffs(mn, mx, n_thresholds, cut);
+  {   // every label song is in new_songs: a membership table over [0, largest new song] (a binary search per label was 270 ms at MSD scale)
+    std::vector<uint8_t> in_new(static_cast<size_t>(new_songs[n_new - 1]) + 1, 0);
+    for (int i = 0; i < n_new; ++i) in_new[new_songs[i]] = 1;
+    for (long long i = 0; i < n_lab; ++i)
+      if (static_cast<size_t>(lab_col[i]) >= in_new.size() || !in_new[lab_col[i]])
+        return fail(h, MR_ERR_BAD_ARG, "new_songs lacks label song %d", lab_col[i]);
+  }
+  for (int e = 0; e < n; ++e)
+    if (mx[e] - mn[e] > 0 && !(mn[e] >= 0)) {
+      rc = fail(h, MR_ERR_BAD_ARG, "mn must be >= 0 (scores are non-negative)");
+      if (name_entries) h->err = "entry " + std::to_string(e) + ": " + h->err;
+      return rc;
+    }
+  hs.mark("label_checks");
+  for (int g = 0; g < set.n_groups; ++g) {
+    EvalGroup& G = set.grp[g];
+    for (int m = 0; m < G.n; ++m) {
+      double cut[11];
+      eval_cutoffs(mn[G.out[m]], mx[G.out[m]], n_thresholds, cut);
+      for (int t = 0; t < n_thresholds; ++t) memcpy(&G.cut[m][t], &cut[t], 8);
+    }
+  }
   EvalCounts& ec = h->ec;
   ec = EvalCounts{};
-  for (int t = 0; t < n_thresholds; ++t) memcpy(&ec.cut[t], &cut[t], 8);
   ec.n_thresholds = n_thresholds; ec.col_lo = h->win_lo;
   std::vector<int> colmap(h->n_cols, -1);   // scored column -> label-song index
   for (int i = 0; i < n_new; ++i)
     if (new_songs[i] >= h->win_lo && new_songs[i] < h->win_lo + h->n_cols) colmap[new_songs[i] - h->win_lo] = i;
-  const size_t per = static_cast<size_t>(n_new) * n_thresholds, n_cnt = 2 * per + n_new;
+  const size_t per = static_cast<size_t>(n_new) * n_thresholds, n_cnt = 2 * per * n + n_new;
   int* d_colmap = nullptr; long long* d_lp = nullptr; int* d_lc = nullptr; unsigned long long* d_cnt = nullptr;
   if ((rc = slot_upload(h, mr_handle::SL_EVAL_COLMAP, &d_colmap, colmap.data(), colmap.size())) ||
       (rc = slot_upload(h, mr_handle::SL_LAB_PTR, &d_lp, reinterpret_cast<const long long*>(lab_rowptr), static_cast<size_t>(U) + 1)) ||
@@ -1861,24 +1989,64 @@ int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double 
       (rc = slot_alloc(h, mr_handle::SL_EVAL_CNT, &d_cnt, n_cnt)))
     return rc;
   MR_CUDA(h, cudaMemsetAsync(d_cnt, 0, n_cnt * sizeof(unsigned long long), h->stream));
-  ec.colmap = d_colmap; ec.lab_ptr = d_lp; ec.lab_col = d_lc; ec.pred_b = d_cnt; ec.tp_b = d_cnt + per; ec.nlab = d_cnt + 2 * per;
-  // resident reuse: a single-batch item-space shard whose panels the range pass of the same model has just filled
-  bool reuse = h->space == MR_SPACE_ITEM && h->U <= h->batch_rows && h->eval_gen == h->gen && h->eval_model == model &&
-               memcmp(&h->eval_param, &param, sizeof param) == 0 && h->eval_seed == seed;
-  if ((rc = run_batches(h, model, bp, 0, RUN_EVAL_COUNT, &reuse))) { join_slice_streams(h); return rc; }
+  ec.colmap = d_colmap; ec.lab_ptr = d_lp; ec.lab_col = d_lc; ec.pred_b = d_cnt; ec.tp_b = d_cnt + per;
+  ec.model_stride = static_cast<long long>(2 * per); ec.nlab = d_cnt + 2 * per * n;
+  hs.mark("uploads");
+  // resident reuse: a single-batch item-space shard whose panels the range pass of the same set has just filled
+  bool reuse = h->space == MR_SPACE_ITEM && h->U <= h->batch_rows && same_eval_set(h, n, models, params, seeds);
+  if ((rc = run_batches(h, set, 0, RUN_EVAL_COUNT, &reuse))) { join_slice_streams(h); return rc; }
+  hs.mark("enqueue");
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  hs.mark("gpu_wait");
   std::vector<unsigned long long> cnt(n_cnt);
   MR_CUDA(h, cudaMemcpyAsync(cnt.data(), d_cnt, n_cnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
-  for (int c = 0; c < n_new; ++c) {   // bucket counts -> counts per threshold: predicted at t <=> bucket > t
-    long long p = 0, q = 0;
-    for (int t = n_thresholds - 1; t >= 0; --t) {
-      const size_t i = static_cast<size_t>(c) * n_thresholds + t;
-      p += static_cast<long long>(cnt[i]); q += static_cast<long long>(cnt[per + i]);
-      out_pred[i] = p; out_tp[i] = q;
+  hs.mark("copy_back");
+  for (int e = 0; e < n; ++e) {
+    const unsigned long long* pb = cnt.data() + 2 * per * e;
+    int64_t* op = out_pred + per * e; int64_t* ot = out_tp + per * e;
+    for (int c = 0; c < n_new; ++c) {   // bucket counts -> counts per threshold: predicted at t <=> bucket > t
+      long long p = 0, q = 0;
+      for (int t = n_thresholds - 1; t >= 0; --t) {
+        const size_t i = static_cast<size_t>(c) * n_thresholds + t;
+        p += static_cast<long long>(pb[i]); q += static_cast<long long>(pb[per + i]);
+        op[i] = p; ot[i] = q;
+      }
     }
-    out_nlab[c] = static_cast<long long>(cnt[2 * per + c]);
   }
+  for (int c = 0; c < n_new; ++c) out_nlab[c] = static_cast<long long>(cnt[2 * per * n + c]);
+  hs.mark("suffix_sums");
+  hs.print(n);
   return MR_OK;
+}
+}  // namespace
+
+int mr_eval_cutoffs(double mn, double mx, int n_thresholds, double* out) {
+  if (!out || (n_thresholds != 10 && n_thresholds != 11)) return MR_ERR_BAD_ARG;
+  eval_cutoffs(mn, mx, n_thresholds, out);
+  return MR_OK;
+}
+
+int mr_eval_range(mr_handle* h, int model, double param, uint64_t seed, double* out_min, double* out_max) {
+  return eval_range_impl(h, 1, &model, &param, &seed, false, out_min, out_max);
+}
+
+int mr_eval_counts(mr_handle* h, int model, double param, uint64_t seed, double mn, double mx, int n_thresholds, const int64_t* lab_rowptr,
+                   const int32_t* lab_col, const int32_t* new_songs, int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab) {
+  return eval_counts_impl(h, 1, &model, &param, &seed, false, &mn, &mx, n_thresholds, lab_rowptr, lab_col, new_songs, n_new, out_pred, out_tp,
+                          out_nlab);
+}
+
+int mr_eval_range_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, double* out_min,
+                        double* out_max) {
+  return eval_range_impl(h, n_models, models, params, seeds, true, out_min, out_max);
+}
+
+int mr_eval_counts_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, const double* mn,
+                         const double* mx, int n_thresholds, const int64_t* lab_rowptr, const int32_t* lab_col, const int32_t* new_songs,
+                         int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab) {
+  return eval_counts_impl(h, n_models, models, params, seeds, true, mn, mx, n_thresholds, lab_rowptr, lab_col, new_songs, n_new, out_pred,
+                          out_tp, out_nlab);
 }
 
 // fp64 in exactly the operation order of eval_ap_kernel and mr_evaluate_dense; no contraction into FMAs
@@ -2004,6 +2172,74 @@ int mr_topk(mr_handle* h, int model, double param, uint64_t seed, int k, int32_t
   return topk_impl(h, model, param, seed, k, &ho);
 }
 
+int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k must be in [1,1024], got %d", k);
+  ModelSet set;
+  if ((rc = make_set(h, n_models, models, params, seeds, "getTopK", true, &set))) return rc;
+  // one block (song | score | len) per entry in a grow-only slot of its own: the single-model result (mr_topk_fetch, mr_map_at_k) stays
+  const size_t song_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * k * 4, 16)), score_b = static_cast<size_t>(h->U) * k * 8,
+               len_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * 4, 16)), stride = song_b + score_b + len_b;
+  const size_t need = stride * static_cast<size_t>(n_models);
+  h->multi_n = 0;
+  // it must fit inside the caller's reserve that the batch plan leaves free, and be free now; the plan is not changed for it
+  size_t avail = kCallerReserve;
+  if (h->slot_cap[mr_handle::SL_MULTI_OUT] < need) {
+    size_t free_b = 0, total_b = 0;
+    MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
+    avail = std::min(avail, free_b + h->slot_cap[mr_handle::SL_MULTI_OUT]);
+  }
+  if (need > avail)
+    return fail(h, MR_ERR_OOM, "mr_topk_multi: %d top-%d results of %d users need %zu bytes, more than the %zu bytes of the caller's reserve "
+                "that are free", n_models, k, h->U, need, avail);
+  char* base = nullptr;
+  if ((rc = slot_alloc(h, mr_handle::SL_MULTI_OUT, &base, need, true))) return rc;
+  for (int e = 0; e < n_models; ++e) {
+    char* b = base + stride * e;
+    set.out_song[e] = reinterpret_cast<int*>(b); set.out_score[e] = reinterpret_cast<double*>(b + song_b); set.out_len[e] = reinterpret_cast<int*>(b + song_b + score_b);
+  }
+  bool ibm_side = false;
+  for (int e = 0; e < n_models; ++e) ibm_side = ibm_side || set.bp[e].model != MODEL_UBM;
+  if (ibm_side && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
+  if ((rc = run_batches(h, set, k, RUN_TOPK, nullptr))) return rc;
+  h->multi_n = n_models; h->multi_k = k; h->multi_stride = stride;
+  return MR_OK;
+}
+
+int mr_topk_multi_ptrs(mr_handle* h, int i, int k, void** song, void** score, void** len) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (h->multi_n == 0 || h->multi_k != k) return fail(h, MR_ERR_STATE, "no top-%d set result on the device (call mr_topk_multi_device first)", k);
+  if (i < 0 || i >= h->multi_n) return fail(h, MR_ERR_BAD_ARG, "entry %d outside the set of %d", i, h->multi_n);
+  char* b = static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]) + h->multi_stride * i;
+  const size_t song_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * k * 4, 16)), score_b = static_cast<size_t>(h->U) * k * 8;
+  if (song) *song = b;
+  if (score) *score = b + song_b;
+  if (len) *len = b + song_b + score_b;
+  return MR_OK;
+}
+
+int mr_topk_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k, int32_t* const* out_song,
+                  double* const* out_score, int32_t* const* out_len) {
+  if (!h) return MR_ERR_STATE;
+  if (n_models < 1 || n_models > kMaxSet) return fail(h, MR_ERR_BAD_ARG, "getTopK: n_models = %d outside 1..%d", n_models, kMaxSet);
+  if (!out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null output");
+  for (int e = 0; e < n_models; ++e)
+    if (!out_song[e] || !out_score[e] || !out_len[e]) return fail(h, MR_ERR_BAD_ARG, "entry %d: null output", e);
+  int rc = mr_topk_multi_device(h, n_models, models, params, seeds, k);
+  if (rc) return rc;
+  for (int e = 0; e < n_models; ++e) {
+    void *s = nullptr, *v = nullptr, *l = nullptr;
+    if ((rc = mr_topk_multi_ptrs(h, e, k, &s, &v, &l))) return rc;
+    MR_CUDA(h, cudaMemcpyAsync(out_song[e], s, static_cast<size_t>(h->U) * k * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    MR_CUDA(h, cudaMemcpyAsync(out_score[e], v, static_cast<size_t>(h->U) * k * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    MR_CUDA(h, cudaMemcpyAsync(out_len[e], l, static_cast<size_t>(h->U) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+  }
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MR_OK;
+}
+
 int mr_get_timing(mr_handle* h, double* ms_out, int n) {
   if (!h || !ms_out) return MR_ERR_BAD_ARG;
   for (int i = 0; i < n && i < MR_T_N; ++i) ms_out[i] = h->t_ms[i];
@@ -2018,10 +2254,10 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[19] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[20] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
-                         h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2]};
-  for (int i = 0; i < n && i < 19; ++i) out[i] = v[i];
+                         h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes};
+  for (int i = 0; i < n && i < 20; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

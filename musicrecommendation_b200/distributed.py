@@ -190,6 +190,33 @@ def evaluate_reference_map(mr, model: int, param: float = 0.5, seed: int = 0, n_
     return eval_finish(c[:n * k].reshape(n, k), c[n * k:2 * n * k].reshape(n, k), c[2 * n * k:], n_thresholds)
 
 
+def evaluate_reference_map_multi(mr, specs, n_thresholds: int = 10, new_songs=None, group=None, labels: Dataset | None = None) -> list[float]:
+    """evaluate_reference_map for every entry (model, param, seed) of a model set, from one scoring per batch on every rank: one MIN
+    all-reduce of the 2 M values (mn, -mx), one sum all-reduce of the M count blocks and nlab, and a finish per entry.  One mAP per entry,
+    each with the bits of evaluate_reference_map for that entry."""
+    import torch
+    import torch.distributed as dist
+    from .recommender import eval_finish
+    dev = _collective_device(group)
+    lab = labels if labels is not None else mr.ds
+    if new_songs is None:
+        new_songs = global_label_songs(lab.lab_col, group)
+    mn, mx = mr.eval_range_multi(specs)
+    m = len(mn)
+    r = torch.from_numpy(np.concatenate([np.asarray(mn, np.float64), -np.asarray(mx, np.float64)])).to(dev)
+    dist.all_reduce(r, op=dist.ReduceOp.MIN, group=group)
+    r = r.cpu().numpy()
+    mn, mx = r[:m].copy(), -r[m:]
+    pred, tp, nlab = mr.eval_counts_multi(specs, mn, mx, new_songs, n_thresholds, lab)
+    c = torch.from_numpy(np.concatenate([np.asarray(pred).reshape(m, -1), np.asarray(tp).reshape(m, -1)], axis=1).ravel())
+    c = torch.cat([c, torch.from_numpy(np.asarray(nlab, np.int64))]).to(dev)
+    dist.all_reduce(c, group=group)
+    c = c.cpu().numpy()
+    n, k = len(nlab), n_thresholds
+    blocks, nl = c[:2 * m * n * k].reshape(m, 2, n, k), c[2 * m * n * k:]
+    return [eval_finish(blocks[i, 0], blocks[i, 1], nl, n_thresholds) for i in range(m)]
+
+
 def split_train_users(ds: Dataset, rank: int, world: int) -> Dataset:
     """K-split of the item-item Gram (BASELINE configs[4]): rank r keeps the train users of its contiguous range, every song.
     deg_song stays global — the cosine denominators count all listeners (MR:237)."""

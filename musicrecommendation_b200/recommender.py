@@ -309,6 +309,34 @@ class MusicRecommender:
         self._check(self._lib.mr_topk(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), k, _p(song), _p(score), _p(ln)))
         return song, score, ln
 
+    def getTopKMulti(self, specs, k: int = 500):
+        """getTopK for every entry of a model set (model, param, seed) from one scoring of the shard (mr_topk_multi, DESIGN.md §4.6):
+        one (song [U,k] int32, score [U,k] f64, len [U]) per entry, each equal to getTopK(model, k, param, seed)."""
+        models, params, seeds = model_set_arrays(specs)
+        U, n = self.ds.U, len(models)
+        out = [(np.empty((U, k), np.int32), np.empty((U, k), np.float64), np.empty(U, np.int32)) for _ in range(n)]
+        tab = lambda j: (C.c_void_p * n)(*[o[j].ctypes.data for o in out])      # noqa: E731
+        self._check(self._lib.mr_topk_multi(self._h, n, _p(models), _p(params), _p(seeds), k, tab(0), tab(1), tab(2)))
+        return out
+
+    def topk_multi_device(self, specs, k: int = 500):
+        """mr_topk_multi_device: the set's lists stay in HBM (topk_multi_device_tensors reads them)."""
+        models, params, seeds = model_set_arrays(specs)
+        self._check(self._lib.mr_topk_multi_device(self._h, len(models), _p(models), _p(params), _p(seeds), k))
+
+    def topk_multi_device_tensors(self, i: int, k: int):
+        """torch views (no copy) of entry i of the last set top-k on the device: (song int32 [U,k], score f64 [U,k], len int32 [U])."""
+        import torch
+        ps, pv, pl = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        self._check(self._lib.mr_topk_multi_ptrs(self._h, i, k, C.byref(ps), C.byref(pv), C.byref(pl)))
+        U = self.ds.U
+
+        class _Arr:
+            def __init__(self, ptr, shape, typestr):
+                self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
+        return (torch.as_tensor(_Arr(ps.value, (U, k), "<i4"), device="cuda"), torch.as_tensor(_Arr(pv.value, (U, k), "<f8"), device="cuda"),
+                torch.as_tensor(_Arr(pl.value, (U,), "<i4"), device="cuda"))
+
     def prepare(self):
         """Build the item-space head rows now (one-off per train set) instead of lazily."""
         self._check(self._lib.mr_prepare(self._h))
@@ -456,10 +484,11 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 19)()
-        self._lib.mr_get_info(self._h, v, 19)
+        v = (C.c_int64 * 20)()
+        self._lib.mr_get_info(self._h, v, 20)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
-                         "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects", "topk_short_rows", "topk_degenerate_rows"], list(v)))
+                         "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
+                         "topk_short_rows", "topk_degenerate_rows", "scoring_passes"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -523,6 +552,71 @@ class MusicRecommender:
         new_songs = np.unique(np.asarray(lab.lab_col, np.int32))
         pred, tp, nlab = self.eval_counts(model, mn, mx, new_songs, param, seed, n_thresholds, lab)
         return eval_finish(pred, tp, nlab, n_thresholds)
+
+    # ---- a model set from one scoring per batch (include/mrscore.h mr_eval_*_multi, DESIGN.md §4.6)
+    def eval_range_multi(self, specs) -> tuple[np.ndarray, np.ndarray]:
+        """(min [M], max [M]) of each entry of the model set, as eval_range per entry, from one scoring of the shard."""
+        models, params, seeds = model_set_arrays(specs)
+        mn, mx = np.empty(len(models), np.float64), np.empty(len(models), np.float64)
+        self._check(self._lib.mr_eval_range_multi(self._h, len(models), _p(models), _p(params), _p(seeds), _p(mn), _p(mx)))
+        return mn, mx
+
+    def eval_counts_multi(self, specs, mn, mx, new_songs, n_thresholds: int = 10, labels: Dataset | None = None):
+        """eval_counts for every entry of the model set under its global (mn[i], mx[i]): (pred [M, n_new, n_thr], tp [M, n_new, n_thr],
+        nlab [n_new]) int64."""
+        models, params, seeds = model_set_arrays(specs)
+        n = len(models)
+        mn = np.ascontiguousarray(mn, np.float64)
+        mx = np.ascontiguousarray(mx, np.float64)
+        if mn.shape != (n,) or mx.shape != (n,):
+            raise ValueError(f"mn and mx must hold one value per entry of the set ({n})")
+        lab = labels if labels is not None else self.ds
+        lp = np.ascontiguousarray(lab.lab_ptr, np.int64)
+        lc = np.ascontiguousarray(lab.lab_col, np.int32)
+        if len(lp) != self.ds.U + 1 or len(lc) < (lp[-1] if len(lp) else 0):
+            raise ValueError(f"labels must hold {self.ds.U} label rows (the current shard's users), got {len(lp) - 1}")
+        ns = np.ascontiguousarray(new_songs, np.int32)
+        pred = np.zeros((n, len(ns), n_thresholds), np.int64)
+        tp = np.zeros((n, len(ns), n_thresholds), np.int64)
+        nlab = np.zeros(len(ns), np.int64)
+        self._check(self._lib.mr_eval_counts_multi(self._h, n, _p(models), _p(params), _p(seeds), _p(mn), _p(mx), n_thresholds, _p(lp), _p(lc),
+                                                   _p(ns), len(ns), _p(pred), _p(tp), _p(nlab)))
+        return pred, tp, nlab
+
+    def evaluateAllOnDevice(self, specs, n_thresholds: int = 10, labels: Dataset | None = None) -> list[float]:
+        """evaluateOnDevice for every entry of a model set, from two scorings of the shard (one on a single-batch item-space shard): one
+        mAP per entry, each with the bits of evaluateOnDevice(model, param, seed).  The same whole-model guards as evaluateOnDevice."""
+        if self.song_window != (0, self.ds.S):
+            raise ValueError("evaluateAllOnDevice needs the whole model: this handle scores a song window (use "
+                             "distributed.evaluate_reference_map_multi)")
+        if not self._whole_test_set:
+            raise ValueError("evaluateAllOnDevice needs the whole model: this handle holds a shard of the test users (set_test_users with a "
+                             "pair index base / total); use distributed.evaluate_reference_map_multi")
+        lab = labels if labels is not None else self.ds
+        mn, mx = self.eval_range_multi(specs)
+        new_songs = np.unique(np.asarray(lab.lab_col, np.int32))
+        pred, tp, nlab = self.eval_counts_multi(specs, mn, mx, new_songs, n_thresholds, lab)
+        return [eval_finish(pred[i], tp[i], nlab, n_thresholds) for i in range(len(pred))]
+
+
+MAX_MODEL_SET = 16
+
+
+def model_set_arrays(specs):
+    """A model set [(model, param, seed), ...] of 1..16 entries as the parallel arrays of the C-ABI (int32, float64, uint64).  The shape
+    is checked here; parameter ranges are checked by the library, which names the first bad entry."""
+    specs = list(specs)
+    if not 1 <= len(specs) <= MAX_MODEL_SET:
+        raise ValueError(f"a model set holds 1..{MAX_MODEL_SET} entries, got {len(specs)}")
+    for i, e in enumerate(specs):
+        if len(e) != 3:
+            raise ValueError(f"entry {i}: expected (model, param, seed), got {e!r}")
+        if int(e[0]) != e[0] or not 0 <= int(e[0]) <= _lib.MR_STOCH:
+            raise ValueError(f"entry {i}: unknown model selector {e[0]!r}")
+    models = np.array([int(e[0]) for e in specs], np.int32)
+    params = np.array([float(e[1]) for e in specs], np.float64)
+    seeds = np.array([int(e[2]) & (2**64 - 1) for e in specs], np.uint64)
+    return models, params, seeds
 
 
 def _string_table(names, n):

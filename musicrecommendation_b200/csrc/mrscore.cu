@@ -21,6 +21,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <optional>
 #include <string>
 #include <queue>
 #include <mutex>
@@ -38,6 +39,8 @@ constexpr int kPreStreams = 4;          // streams of the in-place head-row buil
 constexpr int kPreExtraStreams = 3;     // at most 1 + 3 (MRSCORE_PRE_STREAMS)
 constexpr int kMaxDegIbm = 1801439;     // (2e-5 * 2^26)^2 = 1 801 439.85
 constexpr size_t kCallerReserve = 6ULL << 30;   // HBM the item-space batch plan leaves for the caller's context and small workspaces
+
+struct TopkOut { int32_t* song; double* score; int32_t* len; };   // one top-k result: song [U][k], score [U][k], len [U]
 
 }  // namespace
 
@@ -112,9 +115,9 @@ struct mr_handle {
   uint64_t* d_sel = nullptr; long long sel_pitch = 0; int32_t* d_g = nullptr; size_t g_bytes = 0; size_t aj_bytes = 0;
   double* d_dense = nullptr; int32_t* d_cnt = nullptr; float* d_simf = nullptr;
   // results
-  int *d_out_song = nullptr, *d_out_len = nullptr; double* d_out_score = nullptr; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;
-  // results of the last mr_topk_multi_device: entry i's block starts at multi_stride * i in the SL_MULTI_OUT slot (song | score | len)
-  int multi_n = 0, multi_k = 0; size_t multi_stride = 0;
+  TopkOut out{}; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;   // the single-model result, a TopkBlock in SL_OUT_PACK
+  // results of the last mr_topk_multi_device: entry i is the i-th TopkBlock of the SL_MULTI_OUT slot
+  int multi_n = 0, multi_k = 0;
   long long passes = 0;   // scoring passes since mr_load: batches whose score panels were built
   // streamed evaluation (mr_eval_range* / mr_eval_counts*).  gen counts the calls that may rewrite the score panels; after a range pass
   // over a single-batch item-space shard the panels still hold the masked numerators of the model set (eval_n entries of eval_models,
@@ -693,11 +696,28 @@ int plan_item_batches(mr_handle* h, const std::vector<long long>& hu_ptr) {
   }
 }
 
-// RUN_EVAL_RANGE / RUN_EVAL_COUNT: the streamed evaluateModel passes (DESIGN.md §4.5) in place of the top-k select of each slice;
-// host_out is null / points to a bool "the panels already hold this set's masked numerators" (resident reuse, mr_eval_counts*).
-enum RunMode { RUN_TOPK, RUN_DENSE, RUN_COUNTS_UBM, RUN_SIM_UBM, RUN_EVAL_RANGE, RUN_EVAL_COUNT };
-struct TopkHostOut { int32_t* song; double* score; int32_t* len; };   // RUN_TOPK: caller buffers the finished slices are copied into
-// RUN_DENSE: where the fp64 rows go.  ALL: out[u][s] for every test user (mr_score_dense).  USERS: out[i][s] for the listed users
+// The layout of one top-k result block: song i32[U][k] | score f64[U][k] | len i32[U], the song and len parts rounded up to 16 bytes, so
+// that a caller can ship a whole result with a single transfer (mr_topk_packed).
+struct TopkBlock {
+  size_t score_off, len_off, bytes;
+  TopkBlock(int U, int k)
+      : score_off(static_cast<size_t>(round_up(static_cast<long long>(U) * k * 4, 16))), len_off(score_off + static_cast<size_t>(U) * k * 8),
+        bytes(len_off + static_cast<size_t>(round_up(static_cast<long long>(U) * 4, 16))) {}
+  TopkOut at(char* base) const {
+    return {reinterpret_cast<int32_t*>(base), reinterpret_cast<double*>(base + score_off), reinterpret_cast<int32_t*>(base + len_off)};
+  }
+};
+
+// Enqueue on st the copy of users [u0, u0 + n) of the device result src into the caller's host buffers dst (both indexed by user).
+int copy_topk(mr_handle* h, const TopkOut& dst, const TopkOut& src, int k, int u0, int n, cudaStream_t st) {
+  const size_t o = static_cast<size_t>(u0) * k, m = static_cast<size_t>(n) * k;
+  MR_CUDA(h, cudaMemcpyAsync(dst.song + o, src.song + o, m * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  MR_CUDA(h, cudaMemcpyAsync(dst.score + o, src.score + o, m * sizeof(double), cudaMemcpyDeviceToHost, st));
+  MR_CUDA(h, cudaMemcpyAsync(dst.len + u0, src.len + u0, static_cast<size_t>(n) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  return MR_OK;
+}
+
+// DENSE: where the fp64 rows go.  ALL: out[u][s] for every test user (mr_score_dense).  USERS: out[i][s] for the listed users
 // (DIST getRanks1 granularity).  SONGS: d_out[i][u] for the listed songs, gathered on the device (DIST getRanks2 granularity).
 struct DenseOut { enum Kind { ALL, USERS, SONGS } kind; double* out; const int32_t* ids; int n_ids; const int* d_ids; double* d_out; };
 
@@ -706,36 +726,51 @@ constexpr int kMaxSet = 16;
 struct ModelSet {
   int n = 0;
   BlendParams bp[kMaxSet];
-  int* out_song[kMaxSet] = {}; double* out_score[kMaxSet] = {}; int* out_len[kMaxSet] = {};   // RUN_TOPK: each entry's device result
-  // eval modes: the entries grouped for the fused consumers; grp_stoch[g] = the STOCH entry whose select plane group g reads, or -1
+  TopkOut out[kMaxSet] = {};   // TOPK: each entry's device result
+  // eval consumers: the entries grouped for the fused kernels; grp_stoch[g] = the STOCH entry whose select plane group g reads, or -1
   int n_groups = 0; EvalGroup grp[kMaxSet]; int grp_stoch[kMaxSet] = {};
   int n_stoch = 0;
   bool needs(int panel_model) const {   // UBM panel: some entry is not IBM; IBM panel: some entry is not UBM
     for (int i = 0; i < n; ++i) if (bp[i].model != (panel_model == MODEL_UBM ? MODEL_IBM : MODEL_UBM)) return true;
     return false;
   }
+  ModelSet() = default;
+  explicit ModelSet(int model) : n(1) { memset(&bp[0], 0, sizeof bp[0]); bp[0].model = model; }   // one model without blend parameters
+};
+
+// What a scoring run hands the masked panels to: the top-k select, the fp64 rows, or the streamed evaluateModel passes (DESIGN.md §4.5).
+enum class Consumer { TOPK, DENSE, EVAL_RANGE, EVAL_COUNT };
+struct Run {
+  ModelSet set;
+  Consumer what = Consumer::TOPK;
+  int k = 0;                            // TOPK: list length
+  const DenseOut* dense = nullptr;      // DENSE: where the rows go
+  const TopkOut* topk_host = nullptr;   // TOPK in item space: the caller's buffers, filled slice by slice from entry 0 on copy_stream
+  bool reuse = false;                   // EVAL_COUNT: the panels hold this set's masked numerators (resident reuse): no scoring at all
+  bool eval() const { return what == Consumer::EVAL_RANGE || what == Consumer::EVAL_COUNT; }
 };
 
 // The consumers of one masked slice: per entry the select (after its blend's select plane), or per group the fused eval kernels (after
-// the group's STOCH plane; plane_resident: the plane of the set's only STOCH entry is still in place from the range pass).
-int consume_slice(mr_handle* h, const ModelSet& set, RunMode mode, int k, long long* su, long long* si, uint64_t* sel, int u0, int n,
-                  cudaStream_t st, bool plane_resident) {
-  if (mode == RUN_TOPK) {
+// the group's STOCH plane, unless the plane of the set's only STOCH entry is still in place from the range pass).
+int consume_slice(mr_handle* h, const Run& run, long long* su, long long* si, uint64_t* sel, int u0, int n, cudaStream_t st) {
+  const ModelSet& set = run.set;
+  if (run.what == Consumer::TOPK) {
     for (int e = 0; e < set.n; ++e) {
       const BlendParams& bp = set.bp[e];
       const bool blend_sel = bp.model == MODEL_AGG || bp.model == MODEL_STOCH;
       if (blend_sel) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
       MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, bp.model != MODEL_IBM ? su : nullptr, bp.model != MODEL_UBM ? si : nullptr, h->spitch,
-                               blend_sel ? sel : nullptr, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, k, set.out_song[e],
-                               set.out_score[e], set.out_len[e], st));
+                               blend_sel ? sel : nullptr, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, run.k, set.out[e].song,
+                               set.out[e].score, set.out[e].len, st));
     }
     return MR_OK;
   }
+  const bool plane_resident = run.reuse && set.n_stoch == 1;
   for (int g = 0; g < set.n_groups; ++g) {
     const int se = set.grp_stoch[g];
     if (se >= 0 && !plane_resident)
       MR_LAUNCH(h, launch_select_bits(set.bp[se], h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
-    if (mode == RUN_EVAL_RANGE) {
+    if (run.what == Consumer::EVAL_RANGE) {
       MR_LAUNCH(h, launch_eval_range(set.grp[g], su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, h->d_eval_mm, st));
     } else {
       EvalCounts ec = h->ec;
@@ -746,17 +781,128 @@ int consume_slice(mr_handle* h, const ModelSet& set, RunMode mode, int k, long l
   return MR_OK;
 }
 
-int run_batches(mr_handle* h, const ModelSet& set, int k, RunMode mode, void* host_out) {
-  const bool need_ubm = set.needs(MODEL_UBM);
-  const bool need_ibm = set.needs(MODEL_IBM) && mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM;
-  const int model = set.bp[0].model;   // RUN_DENSE runs a set of one
+// Item space, the head pass of batch bi (users [b0, b0 + nb)) on the library stream into pu (models bit 0, UBM) / pi (bit 1, IBM), after
+// the event release of the slices that last read these panels (or null): zero the split rows, head_rowsum, exception fixup.
+int head_pass(mr_handle* h, int bi, int b0, int nb, int models, long long* pu, long long* pi, cudaEvent_t release) {
+  PhaseTimer t(h, MR_T_HEAD_ROWSUM);
+  if (release) MR_CUDA(h, cudaStreamWaitEvent(h->stream, release, 0));
+  const int4* grp = h->d_grp_hdr + static_cast<long long>(bi) * h->n_groups;
+  const int sp0 = h->h_split_ptr[bi], n_split = h->h_split_ptr[bi + 1] - sp0;
+  for (int m = 1; m <= 2; ++m) {
+    if (!(models & m)) continue;
+    long long* const panel = m == 1 ? pu : pi;
+    if (n_split) MR_LAUNCH(h, launch_zero_rows(h->d_split_rows + sp0, n_split, panel, h->spitch, h->stream));
+    MR_LAUNCH(h, launch_head_rowsum(m, m == 1 ? h->head_words_u : h->head_words_i, h->head_threads, grp, h->n_groups, h->d_seg, h->d_ge_row,
+                                    h->d_ge_q, h->seg_cap, h->ent_cap, h->d_g16, h->d_gq32, h->spitch, h->n_cols, panel, h->spitch, h->stream));
+  }
+  if (h->n_ex > 0)
+    MR_LAUNCH(h, launch_head_fixup(models, h->d_hu_ptr, h->d_hu_row, h->d_hu_song, h->d_hu_q, b0, nb, h->d_ex_ptr, h->d_ex_song, h->d_ex_g,
+                                   h->d_ex_gq, pu, pi, h->spitch, h->stream));
+  return MR_OK;
+}
+
+// How a call cuts the item-space batches into slices: panels (as head_pass), users per slice, tail-scatter lanes, whether the consumers
+// read the select plane (the blends' bits for the top-k, STOCH's for the eval kernels; AGG's pick there is its split column), and the two
+// streams consecutive slices alternate between.  Per slice the atomics of one tail-scatter launch stay within a few GB of the Sint panels
+// (measured optimum 300-600 users; kTailSubBatch users of whole rows = ~1.8 GB of a panel; a song partition's rows are shorter).
+struct Slicing { int models, users, lanes; bool sel; cudaStream_t st[2]; };
+
+// Item space, the slices of batch b0: tail scatter, then (DENSE takes the whole batch) mask, consumers and the streamed host copy.
+int item_slices(mr_handle* h, const Run& run, const Slicing& sl, int b0, int nb, long long* pu, long long* pi) {
+  for (int s0 = 0; s0 < nb; s0 += sl.users) {
+    const int sn = std::min(sl.users, nb - s0), u0 = b0 + s0;
+    cudaStream_t const ts = sl.st[(s0 / sl.users) & 1];
+    if (!run.reuse) {
+      PhaseTimer t(h, MR_T_TAIL_SCATTER);
+      const long long e0 = h->h_tu_ptr[u0], e1 = h->h_tu_ptr[u0 + sn];
+      MR_LAUNCH(h, launch_tail_scatter(sl.models, h->d_tu_user, h->d_tu_song, h->d_tu_lptr, e0, e1, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr,
+                                       h->d_tr_end, h->d_tr_col, h->d_qv, h->d_qd, b0, pu, pi, h->spitch, h->h_tu_lptr[e1] - h->h_tu_lptr[e0],
+                                       sl.lanes, ts));
+    }
+    if (run.what == Consumer::DENSE) continue;
+    PhaseTimer t(h, run.eval() ? MR_T_OTHER : MR_T_TOPK);
+    long long* su = (sl.models & 1) ? pu + static_cast<long long>(s0) * h->spitch : nullptr;
+    long long* si = (sl.models & 2) ? pi + static_cast<long long>(s0) * h->spitch : nullptr;
+    uint64_t* sel = sl.sel ? h->d_sel + static_cast<long long>(s0) * h->sel_pitch : nullptr;
+    if (!run.reuse) MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
+    if (const int rc = consume_slice(h, run, su, si, sel, u0, sn, ts)) return rc;
+    if (run.topk_host) {
+      MR_CUDA(h, cudaEventRecord(h->ev_slice, ts));
+      MR_CUDA(h, cudaStreamWaitEvent(h->copy_stream, h->ev_slice, 0));
+      if (const int rc = copy_topk(h, *run.topk_host, run.set.out[0], run.k, u0, sn, h->copy_stream)) return rc;
+    }
+  }
+  return MR_OK;
+}
+
+// User space, K1 + K2 of the 128-user batch b0 into d_sint_u (UBM) and d_sint_i (IBM: sparse weighted counts, or the batch's Gram rows).
+int user_panels(mr_handle* h, int b0, int nb, bool need_ubm, bool need_ibm) {
+  const AggItems items{h->d_item_song, h->d_item_begin, h->d_item_len, h->d_item_split, h->n_items};
+  if (need_ubm) {
+    if (const int rc = count_ubm_batch(h, b0, nb)) return rc;
+    PhaseTimer t(h, MR_T_AGG_UBM);
+    MR_CUDA(h, cudaMemsetAsync(h->d_sint_u, 0, static_cast<size_t>(kUserBatch) * h->spitch * sizeof(long long), h->stream));
+    MR_LAUNCH(h, launch_aggregate_ubm(items, h->d_csc_idx, h->d_qv, h->d_ct, h->T, h->d_sint_u, h->spitch, h->num_sms, h->stream));
+  }
+  if (!need_ibm) return MR_OK;
+  if (h->engine == MR_ENGINE_SPARSE) {
+    // user-space formulation: weighted intersection counts, then the same inverted-index gather as UBM
+    CarryList carry{h->d_carry_count, h->d_carry_events, h->carry_cap};
+    {
+      PhaseTimer t(h, MR_T_COUNT);
+      MR_LAUNCH(h, launch_sparse_wcount_u32(h->d_te_ptr, h->d_te_col, b0, nb, h->d_csc_ptr, h->d_csc_idx, h->d_qd, h->d_wi, h->T, carry, h->stream));
+    }
+    PhaseTimer t(h, MR_T_AGG_IBM);
+    MR_CUDA(h, cudaMemsetAsync(h->d_sint_i, 0, static_cast<size_t>(kUserBatch) * h->spitch * sizeof(long long), h->stream));
+    MR_LAUNCH(h, launch_aggregate_w32(items, h->d_csc_idx, h->d_wi, h->T, h->d_sint_i, h->spitch, h->num_sms, h->stream));
+    MR_LAUNCH(h, launch_carry_fixup(carry, h->d_tr_ptr, h->d_tr_col, h->d_sint_i, h->spitch, h->stream));
+    MR_CUDA(h, cudaMemcpyAsync(h->h_carry_seen + (b0 / kUserBatch) % 4096, h->d_carry_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
+    return MR_OK;
+  }
+  const int bi = b0 / kUserBatch;
+  const long long r_off = h->batch_row_off[bi];
+  const int n_rows = static_cast<int>(h->batch_row_off[bi + 1] - r_off);
+  int rc;
+  if (n_rows > 0 && (rc = gram_rows(h, h->d_rows + r_off, n_rows))) return rc;
+  PhaseTimer t(h, MR_T_AGG_IBM);
+  MR_LAUNCH(h, launch_aggregate_ibm(h->d_te_ptr, h->d_te_col, h->d_te_grow, h->d_qd, b0, nb, h->d_g, h->ldg, h->S, h->d_sint_i, h->spitch, h->stream));
+  return MR_OK;
+}
+
+// DENSE: the masked panel rows of batch b0 as fp64 scores of model, kDenseChunk users at a time, to where d says.
+int dense_out(mr_handle* h, int model, const long long* panel, const DenseOut& d, int b0, int nb) {
+  for (int c0 = 0; c0 < nb; c0 += kDenseChunk) {
+    const int cn = std::min(kDenseChunk, nb - c0), r0 = b0 + c0;
+    MR_LAUNCH(h, launch_dense_scores(model, panel + static_cast<long long>(c0) * h->spitch, h->spitch, r0, cn, h->n_cols, h->d_rsa, h->d_rsd,
+                                     h->d_dense, h->stream));
+    if (d.kind == DenseOut::ALL) {
+      MR_CUDA(h, cudaMemcpyAsync(d.out + static_cast<long long>(r0) * h->n_cols, h->d_dense, static_cast<size_t>(cn) * h->n_cols * sizeof(double),
+                                 cudaMemcpyDeviceToHost, h->stream));
+    } else if (d.kind == DenseOut::USERS) {
+      for (int i = 0; i < d.n_ids; ++i) {
+        const int r = d.ids[i] - r0;
+        if (r < 0 || r >= cn) continue;
+        MR_CUDA(h, cudaMemcpyAsync(d.out + static_cast<long long>(i) * h->n_cols, h->d_dense + static_cast<long long>(r) * h->n_cols,
+                                   static_cast<size_t>(h->n_cols) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+      }
+    } else {
+      MR_LAUNCH(h, launch_gather_columns(h->d_dense, cn, h->n_cols, d.d_ids, d.n_ids, d.d_out, h->U, r0, h->stream));
+    }
+    MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  }
+  return MR_OK;
+}
+
+// One scoring of the shard (DESIGN.md §4.2): per batch, build the score panels the set needs, mask them, and hand them to run.what.
+int run_batches(mr_handle* h, const Run& run) {
+  const bool need_ubm = run.set.needs(MODEL_UBM), need_ibm = run.set.needs(MODEL_IBM);
   const int pure = need_ubm && need_ibm ? -1 : (need_ubm ? MODEL_UBM : MODEL_IBM);   // the one panel the set needs, if only one
-  const bool eval = mode == RUN_EVAL_RANGE || mode == RUN_EVAL_COUNT;
-  const bool ranked = mode == RUN_TOPK || eval;      // per-slice consumers of the masked panels: top-k select or evaluation
-  const bool item_space = h->space == MR_SPACE_ITEM && (mode == RUN_DENSE || ranked);
-  const bool reuse = mode == RUN_EVAL_COUNT && *static_cast<const bool*>(host_out);   // skip head pass, tail scatter, mask and select
-  if (!reuse) ++h->gen;
-  if (item_space) { int rc = ensure_head_rows(h); if (rc) return rc; }
+  const bool item_space = h->space == MR_SPACE_ITEM;
+  int rc;
+  // the Gram workspace of the user-space IBM panel (allocated in item space too, which does not read it: it counts in device_bytes)
+  if (need_ibm && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
+  if (!run.reuse) ++h->gen;
+  if (item_space && (rc = ensure_head_rows(h))) return rc;
   const int batch = item_space ? h->batch_rows : kUserBatch;
   // Batch pipeline (item-space top-k of a pure model over >= 2 batches; not under MR_PROFILE, whose phase timers serialise the
   // stream): the head pass of batch b + 1 is issued on the library stream while the tail scatter, mask and select of batch b run on
@@ -767,186 +913,72 @@ int run_batches(mr_handle* h, const ModelSet& set, int k, RunMode mode, void* ho
   // models of the one-GPU job.  Making the kernels truly share the SMs was measured and is WORSE (profiles/r02_summary.md §8): the head
   // pass lives on every resident CTA working on the same song tile out of L2, and a select streaming 48 GB through L2 beside it breaks that.
   // A set that needs both panels (a blend, or UBM and IBM entries) cannot alternate them across batches: it takes the alternating slices.
-  const bool pipelined = item_space && ranked && pure >= 0 && !(h->flags & MR_PROFILE) &&
+  const bool pipelined = item_space && run.what != Consumer::DENSE && pure >= 0 && !(h->flags & MR_PROFILE) &&
                          h->U > batch && !getenv("MRSCORE_NO_PIPELINE");
   // Every other item-space top-k (one batch, e.g. a GPU's share of a song-partitioned job, or a blend) puts consecutive slices on two
   // alternating streams instead: same idea, the boundaries between the slices' kernels (107.6 -> 105.1 ms for both models of a 1/8 song
   // partition; next to the batch pipeline it adds nothing).  The two streams' kernels have different shared-memory carve-outs and never
   // share an SM; asking for matched carve-outs makes them do so and is slower (profiles/r02_summary.md §8).
-  const bool alternating = item_space && ranked && !pipelined && !(h->flags & MR_PROFILE) && !getenv("MRSCORE_NO_PIPELINE");
+  const bool alternating = item_space && run.what != Consumer::DENSE && !pipelined && !(h->flags & MR_PROFILE) && !getenv("MRSCORE_NO_PIPELINE");
   const bool streamed = pipelined || alternating;   // the slices run off the library stream and are joined back into it
-  cudaStream_t const hs = h->stream;
-  cudaStream_t const sl[2] = {streamed ? h->slice_stream : h->stream, alternating ? h->slice_stream2 : (streamed ? h->slice_stream : h->stream)};
+  // On an error return from the streamed region the library stream is still ordered behind both slice streams, so that nothing the
+  // failed call left on them races the next call on the library stream.
+  struct JoinOnError {
+    mr_handle* h; bool armed;
+    ~JoinOnError() {
+      for (cudaStream_t s : {h->slice_stream, h->slice_stream2})
+        if (armed && s && cudaEventRecord(h->ev_join, s) == cudaSuccess) cudaStreamWaitEvent(h->stream, h->ev_join, 0);
+    }
+  } join{h, streamed};
+  Slicing sl{(need_ubm ? 1 : 0) | (need_ibm ? 2 : 0), 0, 0, false, {h->stream, h->stream}};
+  const long long sub_fit = static_cast<long long>(kTailSubBatch) * round_up(h->S, 32) / h->spitch / (2 * h->num_sms) * (2 * h->num_sms);
+  sl.users = static_cast<int>(std::max<long long>(kTailSubBatch, std::min<long long>(sub_fit, 1 << 20)));
+  sl.lanes = 2LL * h->n_cols >= h->S ? 32 : (4LL * h->n_cols >= h->S ? 16 : 8);
+  for (int e = 0; e < run.set.n; ++e) sl.sel = sl.sel || run.set.bp[e].model == MODEL_STOCH || (!run.eval() && run.set.bp[e].model == MODEL_AGG);
+  if (streamed) { sl.st[0] = h->slice_stream; sl.st[1] = alternating ? h->slice_stream2 : h->slice_stream; }
   for (int b0 = 0; b0 < h->U; b0 += batch) {
-    const int nb = std::min(batch, h->U - b0);
+    const int bi = b0 / batch, nb = std::min(batch, h->U - b0);
+    if (!run.reuse) ++h->passes;
     if (item_space) {
-      const int models = (need_ubm ? 1 : 0) | (need_ibm ? 2 : 0);
-      const int par = pipelined ? ((b0 / batch) & 1) ^ (pure == MODEL_IBM ? 1 : 0) : 0;   // panel of this batch: 0 = d_sint_u, 1 = d_sint_i
+      const int par = pipelined ? (bi & 1) ^ (pure == MODEL_IBM ? 1 : 0) : 0;   // panel of this batch: 0 = d_sint_u, 1 = d_sint_i
       // the panels of this batch by role (pipelined: the pure model's panel alternates between the two allocations)
       long long* const panel = par ? h->d_sint_i : h->d_sint_u;
       long long* const pu = pipelined ? (pure == MODEL_UBM ? panel : nullptr) : h->d_sint_u;
       long long* const pi = pipelined ? (pure == MODEL_IBM ? panel : nullptr) : h->d_sint_i;
-      if (!reuse) {
-        ++h->passes;
-        PhaseTimer t(h, MR_T_HEAD_ROWSUM);
-        const int bi = b0 / batch;
-        const int4* grp = h->d_grp_hdr + static_cast<long long>(bi) * h->n_groups;
-        const int sp0 = h->h_split_ptr[bi], n_split = h->h_split_ptr[bi + 1] - sp0;
-        // the slices that last used this panel (two batches ago in the batch pipeline, else the previous batch) have left it
-        if (streamed && b0 >= (pipelined ? 2 : 1) * batch) MR_CUDA(h, cudaStreamWaitEvent(hs, h->ev_done[par], 0));
-        if (need_ubm) {
-          if (n_split) MR_LAUNCH(h, launch_zero_rows(h->d_split_rows + sp0, n_split, pu, h->spitch, hs));
-          MR_LAUNCH(h, launch_head_rowsum(1, h->head_words_u, h->head_threads, grp, h->n_groups, h->d_seg, h->d_ge_row, h->d_ge_q, h->seg_cap, h->ent_cap, h->d_g16, h->d_gq32,
-                                          h->spitch, h->n_cols, pu, h->spitch, hs));
-        }
-        if (need_ibm) {
-          if (n_split) MR_LAUNCH(h, launch_zero_rows(h->d_split_rows + sp0, n_split, pi, h->spitch, hs));
-          MR_LAUNCH(h, launch_head_rowsum(2, h->head_words_i, h->head_threads, grp, h->n_groups, h->d_seg, h->d_ge_row, h->d_ge_q, h->seg_cap, h->ent_cap, h->d_g16, h->d_gq32,
-                                          h->spitch, h->n_cols, pi, h->spitch, hs));
-        }
-        if (h->n_ex > 0)
-          MR_LAUNCH(h, launch_head_fixup(models, h->d_hu_ptr, h->d_hu_row, h->d_hu_song, h->d_hu_q, b0, nb, h->d_ex_ptr, h->d_ex_song, h->d_ex_g,
-                                         h->d_ex_gq, pu, pi, h->spitch, hs));
-      }
+      // the slices that last used this panel (two batches ago in the batch pipeline, else the previous batch) must have left it
+      cudaEvent_t const release = streamed && bi >= (pipelined ? 2 : 1) ? h->ev_done[par] : nullptr;
+      if (!run.reuse && (rc = head_pass(h, bi, b0, nb, sl.models, pu, pi, release))) return rc;
       if (streamed) {
-        MR_CUDA(h, cudaEventRecord(h->ev_head[par], hs));
-        MR_CUDA(h, cudaStreamWaitEvent(sl[0], h->ev_head[par], 0));
-        if (alternating) MR_CUDA(h, cudaStreamWaitEvent(sl[1], h->ev_head[par], 0));
+        MR_CUDA(h, cudaEventRecord(h->ev_head[par], h->stream));
+        MR_CUDA(h, cudaStreamWaitEvent(sl.st[0], h->ev_head[par], 0));
+        if (alternating) MR_CUDA(h, cudaStreamWaitEvent(sl.st[1], h->ev_head[par], 0));
       }
-      // per slice of users so that the atomics of one launch stay within a few GB of the Sint panels (measured optimum: 300-600 users);
-      // in top-k mode the slice is masked and selected right away, and its rows of the result go to the caller's buffers on the copy
-      // stream while the next slice computes
-      // (kTailSubBatch users of whole rows = ~1.8 GB of a panel; the rows of a song partition are shorter, so a slice holds more of them
-      // — fewer, larger launches of the tail / mask / select kernels)
-      static const int tail_sub_env = getenv("MRSCORE_TAIL_SUB") ? std::max(8, atoi(getenv("MRSCORE_TAIL_SUB"))) : 0;
-      const long long sub_fit = static_cast<long long>(kTailSubBatch) * round_up(h->S, 32) / h->spitch / (2 * h->num_sms) * (2 * h->num_sms);
-      const int tail_sub = tail_sub_env ? tail_sub_env : static_cast<int>(std::max<long long>(kTailSubBatch, std::min<long long>(sub_fit, 1 << 20)));
-      const int tail_lanes = 2LL * h->n_cols >= h->S ? 32 : (4LL * h->n_cols >= h->S ? 16 : 8);
-      // the select plane: the blends' bits for the top-k, STOCH's for the fused eval kernels (AGG's pick there is its split column)
-      bool sel_needed = false;
-      for (int e = 0; e < set.n; ++e) sel_needed = sel_needed || set.bp[e].model == MODEL_STOCH || (!eval && set.bp[e].model == MODEL_AGG);
-      const TopkHostOut* ho = mode == RUN_TOPK ? static_cast<const TopkHostOut*>(host_out) : nullptr;
-      for (int s0 = 0; s0 < nb; s0 += tail_sub) {
-        const int sn = std::min(tail_sub, nb - s0);
-        cudaStream_t const ts = sl[(s0 / tail_sub) & 1];
-        if (!reuse) {
-          PhaseTimer t(h, MR_T_TAIL_SCATTER);
-          const long long e0 = h->h_tu_ptr[b0 + s0], e1 = h->h_tu_ptr[b0 + s0 + sn];
-          MR_LAUNCH(h, launch_tail_scatter(models, h->d_tu_user, h->d_tu_song, h->d_tu_lptr, e0, e1, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr,
-                                           h->d_tr_end, h->d_tr_col, h->d_qv, h->d_qd, b0, pu, pi, h->spitch, h->h_tu_lptr[e1] - h->h_tu_lptr[e0], tail_lanes, ts));
-        }
-        if (mode == RUN_DENSE) continue;
-        PhaseTimer t(h, eval ? MR_T_OTHER : MR_T_TOPK);
-        long long* su = need_ubm ? pu + static_cast<long long>(s0) * h->spitch : nullptr;
-        long long* si = need_ibm ? pi + static_cast<long long>(s0) * h->spitch : nullptr;
-        uint64_t* sel = sel_needed ? h->d_sel + static_cast<long long>(s0) * h->sel_pitch : nullptr;
-        const int u0 = b0 + s0;
-        if (!reuse) MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
-        if (const int rc = consume_slice(h, set, mode, k, su, si, sel, u0, sn, ts, reuse && set.n_stoch == 1)) return rc;
-        if (ho) {
-          MR_CUDA(h, cudaEventRecord(h->ev_slice, ts));
-          MR_CUDA(h, cudaStreamWaitEvent(h->copy_stream, h->ev_slice, 0));
-          const size_t o = static_cast<size_t>(u0) * k, n = static_cast<size_t>(sn) * k;
-          MR_CUDA(h, cudaMemcpyAsync(ho->song + o, h->d_out_song + o, n * sizeof(int32_t), cudaMemcpyDeviceToHost, h->copy_stream));
-          MR_CUDA(h, cudaMemcpyAsync(ho->score + o, h->d_out_score + o, n * sizeof(double), cudaMemcpyDeviceToHost, h->copy_stream));
-          MR_CUDA(h, cudaMemcpyAsync(ho->len + u0, h->d_out_len + u0, static_cast<size_t>(sn) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->copy_stream));
-        }
-      }
+      if ((rc = item_slices(h, run, sl, b0, nb, pu, pi))) return rc;
       if (streamed) {
-        if (alternating) {   // the batch's slices end on sl[0]
-          MR_CUDA(h, cudaEventRecord(h->ev_join, sl[1]));
-          MR_CUDA(h, cudaStreamWaitEvent(sl[0], h->ev_join, 0));
+        if (alternating) {   // the batch's slices end on st[0]
+          MR_CUDA(h, cudaEventRecord(h->ev_join, sl.st[1]));
+          MR_CUDA(h, cudaStreamWaitEvent(sl.st[0], h->ev_join, 0));
         }
-        MR_CUDA(h, cudaEventRecord(h->ev_done[par], sl[0]));
+        MR_CUDA(h, cudaEventRecord(h->ev_done[par], sl.st[0]));
         if (b0 + batch >= h->U) {   // last batch: the library stream joins the slices (of the last two batches in the batch pipeline)
           MR_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_done[par], 0));
           if (pipelined) MR_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_done[par ^ 1], 0));
         }
       }
-      if (mode != RUN_DENSE) continue;   // the batch is finished; RUN_DENSE continues below on the whole batch
-    } else if (need_ubm) {
-      if (mode != RUN_COUNTS_UBM && mode != RUN_SIM_UBM) ++h->passes;
-      int rc = count_ubm_batch(h, b0, nb);
-      if (rc) return rc;
-      if (mode == RUN_COUNTS_UBM || mode == RUN_SIM_UBM) {
-        PhaseTimer t(h, MR_T_OTHER);
-        if (mode == RUN_COUNTS_UBM) {
-          ct_to_i32_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_cnt);
-          h->launches++;
-          MR_CUDA(h, cudaMemcpyAsync(static_cast<int32_t*>(host_out) + static_cast<long long>(b0) * h->T, h->d_cnt,
-                                     static_cast<size_t>(nb) * h->T * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-        } else {
-          ct_to_cos_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_rsa_f + b0, h->d_rsv_f, h->d_simf);
-          h->launches++;
-          MR_CUDA(h, cudaMemcpyAsync(static_cast<float*>(host_out) + static_cast<long long>(b0) * h->T, h->d_simf,
-                                     static_cast<size_t>(nb) * h->T * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-        }
-        MR_CUDA(h, cudaStreamSynchronize(h->stream));
-        continue;
-      }
-      PhaseTimer t(h, MR_T_AGG_UBM);
-      MR_CUDA(h, cudaMemsetAsync(h->d_sint_u, 0, static_cast<size_t>(kUserBatch) * h->spitch * sizeof(long long), h->stream));
-      AggItems items{h->d_item_song, h->d_item_begin, h->d_item_len, h->d_item_split, h->n_items};
-      MR_LAUNCH(h, launch_aggregate_ubm(items, h->d_csc_idx, h->d_qv, h->d_ct, h->T, h->d_sint_u, h->spitch, h->num_sms, h->stream));
+      if (run.what != Consumer::DENSE) continue;   // the slices have consumed the batch
+    } else if ((rc = user_panels(h, b0, nb, need_ubm, need_ibm))) {
+      return rc;
     }
-    if (!item_space && !need_ubm) ++h->passes;
-    if (item_space) {
-      // both models were produced above
-    } else if (need_ibm && h->engine == MR_ENGINE_SPARSE) {
-      // user-space formulation: weighted intersection counts, then the same inverted-index gather as UBM
-      CarryList carry{h->d_carry_count, h->d_carry_events, h->carry_cap};
-      {
-        PhaseTimer t(h, MR_T_COUNT);
-        MR_LAUNCH(h, launch_sparse_wcount_u32(h->d_te_ptr, h->d_te_col, b0, nb, h->d_csc_ptr, h->d_csc_idx, h->d_qd, h->d_wi, h->T, carry, h->stream));
-      }
-      PhaseTimer t(h, MR_T_AGG_IBM);
-      MR_CUDA(h, cudaMemsetAsync(h->d_sint_i, 0, static_cast<size_t>(kUserBatch) * h->spitch * sizeof(long long), h->stream));
-      AggItems items{h->d_item_song, h->d_item_begin, h->d_item_len, h->d_item_split, h->n_items};
-      MR_LAUNCH(h, launch_aggregate_w32(items, h->d_csc_idx, h->d_wi, h->T, h->d_sint_i, h->spitch, h->num_sms, h->stream));
-      MR_LAUNCH(h, launch_carry_fixup(carry, h->d_tr_ptr, h->d_tr_col, h->d_sint_i, h->spitch, h->stream));
-      MR_CUDA(h, cudaMemcpyAsync(h->h_carry_seen + (b0 / kUserBatch) % 4096, h->d_carry_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
-    } else if (need_ibm) {
-      const int bi = b0 / kUserBatch;
-      const long long r_off = h->batch_row_off[bi];
-      const int n_rows = static_cast<int>(h->batch_row_off[bi + 1] - r_off);
-      if (n_rows > 0) {
-        int rc = gram_rows(h, h->d_rows + r_off, n_rows);
-        if (rc) return rc;
-      }
-      PhaseTimer t(h, MR_T_AGG_IBM);
-      MR_LAUNCH(h, launch_aggregate_ibm(h->d_te_ptr, h->d_te_col, h->d_te_grow, h->d_qd, b0, nb, h->d_g, h->ldg, h->S, h->d_sint_i,
-                                        h->spitch, h->stream));
-    }
-    PhaseTimer t(h, eval ? MR_T_OTHER : MR_T_TOPK);
-    MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, need_ubm ? h->d_sint_u : nullptr,
-                                      need_ibm ? h->d_sint_i : nullptr, h->spitch, h->stream));
-    if (mode == RUN_DENSE) {
-      for (int c0 = 0; c0 < nb; c0 += kDenseChunk) {
-        const int cn = std::min(kDenseChunk, nb - c0);
-        MR_LAUNCH(h, launch_dense_scores(model, (need_ubm ? h->d_sint_u : h->d_sint_i) + static_cast<long long>(c0) * h->spitch, h->spitch, b0 + c0, cn,
-                                         h->n_cols, h->d_rsa, h->d_rsd, h->d_dense, h->stream));
-        const DenseOut* dout = static_cast<const DenseOut*>(host_out);
-        if (dout->kind == DenseOut::ALL) {
-          MR_CUDA(h, cudaMemcpyAsync(dout->out + static_cast<long long>(b0 + c0) * h->n_cols, h->d_dense,
-                                     static_cast<size_t>(cn) * h->n_cols * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-        } else if (dout->kind == DenseOut::USERS) {
-          for (int i = 0; i < dout->n_ids; ++i) {
-            const int r = dout->ids[i] - (b0 + c0);
-            if (r < 0 || r >= cn) continue;
-            MR_CUDA(h, cudaMemcpyAsync(dout->out + static_cast<long long>(i) * h->n_cols, h->d_dense + static_cast<long long>(r) * h->n_cols,
-                                       static_cast<size_t>(h->n_cols) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-          }
-        } else {
-          MR_LAUNCH(h, launch_gather_columns(h->d_dense, cn, h->n_cols, dout->d_ids, dout->n_ids, dout->d_out, h->U, b0 + c0, h->stream));
-        }
-        MR_CUDA(h, cudaStreamSynchronize(h->stream));
-      }
-    } else {
-      const int rc = consume_slice(h, set, mode, k, need_ubm ? h->d_sint_u : nullptr, need_ibm ? h->d_sint_i : nullptr, h->d_sel, b0, nb,
-                                   h->stream, false);
-      if (rc) return rc;
-    }
+    // the whole batch on the library stream (user space; the dense rows in item space): mask, then the dense rows or the consumers
+    long long* const su = need_ubm ? h->d_sint_u : nullptr;
+    long long* const si = need_ibm ? h->d_sint_i : nullptr;
+    PhaseTimer t(h, run.eval() ? MR_T_OTHER : MR_T_TOPK);
+    MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, su, si, h->spitch, h->stream));
+    rc = run.what == Consumer::DENSE ? dense_out(h, run.set.bp[0].model, su ? su : si, *run.dense, b0, nb)
+                                     : consume_slice(h, run, su, si, h->d_sel, b0, nb, h->stream);
+    if (rc) return rc;
   }
+  join.armed = false;
   if (need_ibm && !item_space && h->engine == MR_ENGINE_SPARSE) {
     // the carry list of the u32 weighted-count panel must not have overflowed (it never does on real data: an event needs
     // more than ~64 songs shared between one test user and one train user)
@@ -956,15 +988,6 @@ int run_batches(mr_handle* h, const ModelSet& set, int k, RunMode mode, void* ho
         return fail(h, MR_ERR_OOM, "IBM weighted-count carry list overflowed (%u events > capacity %u)", h->h_carry_seen[i], h->carry_cap);
   }
   return MR_OK;
-}
-
-
-// a set of one: the single-model calls
-int run_batches(mr_handle* h, int model, const BlendParams& bp, int k, RunMode mode, void* host_out) {
-  ModelSet set;
-  set.n = 1; set.bp[0] = bp; set.bp[0].model = model;
-  set.out_song[0] = h->d_out_song; set.out_score[0] = h->d_out_score; set.out_len[0] = h->d_out_len;
-  return run_batches(h, set, k, mode, host_out);
 }
 
 int make_blend_params(mr_handle* h, int model, double param, uint64_t seed, long long n_total, BlendParams* bp) {
@@ -1396,37 +1419,41 @@ static int require_test(mr_handle* h) {
   return MR_OK;
 }
 
-int mr_counts_ubm(mr_handle* h, int32_t* out_UxT) {
+// The UBM parity probes, not scoring: per 128-user batch the counts Ct as int32 (out_cnt) or cosines (out_sim; on the tensor engine
+// c / (sqrt|I_u| * sqrt|I_v|), MR:147-148, in the GEMM epilogue) to the caller's [U][T].  They bump gen: a later count pass scores anew.
+static int ubm_probe(mr_handle* h, int32_t* out_cnt, float* out_sim) {
   int rc = require_test(h);
   if (rc) return rc;
-  if (!out_UxT) return fail(h, MR_ERR_BAD_ARG, "null output");
-  if ((rc = slot_alloc(h, mr_handle::SL_CNT, &h->d_cnt, static_cast<size_t>(kUserBatch) * h->T))) return rc;
-  BlendParams bp; memset(&bp, 0, sizeof bp);
-  return run_batches(h, MODEL_UBM, bp, 0, RUN_COUNTS_UBM, out_UxT);
-}
-
-int mr_similarity_ubm(mr_handle* h, float* out_UxT) {
-  int rc = require_test(h);
-  if (rc) return rc;
-  if (!out_UxT) return fail(h, MR_ERR_BAD_ARG, "null output");
-  if (h->engine == MR_ENGINE_TENSOR) {
-    // cosine normalisation fused into the GEMM epilogue: out[b][v] = c / (sqrt|I_u| * sqrt|I_v|)   (MR:147-148)
-    if ((rc = slot_alloc(h, mr_handle::SL_SIMF, &h->d_simf, static_cast<size_t>(kUserBatch) * h->T))) return rc;
-    for (int b0 = 0; b0 < h->U; b0 += kUserBatch) {
-      const int nb = std::min(kUserBatch, h->U - b0);
+  if (!out_cnt && !out_sim) return fail(h, MR_ERR_BAD_ARG, "null output");
+  const size_t ws = static_cast<size_t>(kUserBatch) * h->T;
+  if ((rc = out_cnt ? slot_alloc(h, mr_handle::SL_CNT, &h->d_cnt, ws) : slot_alloc(h, mr_handle::SL_SIMF, &h->d_simf, ws))) return rc;
+  ++h->gen;
+  const bool fused = out_sim && h->engine == MR_ENGINE_TENSOR;
+  for (int b0 = 0; b0 < h->U; b0 += kUserBatch) {
+    const int nb = std::min(kUserBatch, h->U - b0);
+    const long long off = static_cast<long long>(b0) * h->T;
+    std::optional<PhaseTimer> t;   // the conversion and the copy-out; the fused GEMM is not timed
+    if (fused) {
       MR_LAUNCH(h, launch_expand_rows(h->d_te_ptr, h->d_te_col, nullptr, b0, nb, kUserBatch, h->pitchS, h->d_Ate, h->stream));
       MR_LAUNCH(h, launch_count_gemm(h->d_Ate, kUserBatch, h->d_Atr, h->T, h->pitchS, nb, h->T, EPI_COS_F32, h->d_simf, h->T,
                                      h->d_rsa_f + b0, h->d_rsv_f, h->num_sms, h->stream));
-      MR_CUDA(h, cudaMemcpyAsync(out_UxT + static_cast<long long>(b0) * h->T, h->d_simf, static_cast<size_t>(nb) * h->T * sizeof(float),
-                                 cudaMemcpyDeviceToHost, h->stream));
-      MR_CUDA(h, cudaStreamSynchronize(h->stream));
+    } else {
+      if ((rc = count_ubm_batch(h, b0, nb))) return rc;
+      t.emplace(h, MR_T_OTHER);
+      if (out_cnt) ct_to_i32_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_cnt);
+      else ct_to_cos_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_rsa_f + b0, h->d_rsv_f, h->d_simf);
+      h->launches++;
     }
-    return MR_OK;
+    MR_CUDA(h, cudaMemcpyAsync(out_cnt ? static_cast<void*>(out_cnt + off) : static_cast<void*>(out_sim + off),   // both are 4-byte elements
+                               out_cnt ? static_cast<const void*>(h->d_cnt) : static_cast<const void*>(h->d_simf), static_cast<size_t>(nb) * h->T * 4,
+                               cudaMemcpyDeviceToHost, h->stream));
+    MR_CUDA(h, cudaStreamSynchronize(h->stream));
   }
-  if ((rc = slot_alloc(h, mr_handle::SL_SIMF, &h->d_simf, static_cast<size_t>(kUserBatch) * h->T))) return rc;
-  BlendParams bp; memset(&bp, 0, sizeof bp);
-  return run_batches(h, MODEL_UBM, bp, 0, RUN_SIM_UBM, out_UxT);
+  return MR_OK;
 }
+
+int mr_counts_ubm(mr_handle* h, int32_t* out_UxT) { return ubm_probe(h, out_UxT, nullptr); }
+int mr_similarity_ubm(mr_handle* h, float* out_UxT) { return ubm_probe(h, nullptr, out_UxT); }
 
 static int gram_range(mr_handle* h, int s0, int s1, int32_t* out_i32, float* out_f32) {
   int rc = require_test(h);
@@ -1600,10 +1627,9 @@ int mr_score_dense(mr_handle* h, int model, double* out_UxS) {
   if (model != MR_UBM && model != MR_IBM) return fail(h, MR_ERR_BAD_ARG, "mr_score_dense: model must be MR_UBM or MR_IBM");
   if (!out_UxS) return fail(h, MR_ERR_BAD_ARG, "null output");
   if ((rc = slot_alloc(h, mr_handle::SL_DENSE, &h->d_dense, static_cast<size_t>(std::min(h->batch_rows, kDenseChunk)) * h->n_cols))) return rc;
-  if (model == MR_IBM && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
-  BlendParams bp; memset(&bp, 0, sizeof bp); bp.model = model; bp.te_end = h->d_te_end; bp.song_off = h->win_lo;
-  DenseOut dout{DenseOut::ALL, out_UxS, nullptr, 0, nullptr, nullptr};
-  return run_batches(h, model, bp, 0, RUN_DENSE, &dout);
+  const DenseOut dout{DenseOut::ALL, out_UxS, nullptr, 0, nullptr, nullptr};
+  Run run{ModelSet(model), Consumer::DENSE, 0, &dout};
+  return run_batches(h, run);
 }
 
 static int score_subset(mr_handle* h, int model, const int32_t* ids, int n, double* out, bool songs) {
@@ -1616,8 +1642,6 @@ static int score_subset(mr_handle* h, int model, const int32_t* ids, int n, doub
     if (ids[i] < first || ids[i] >= limit) return fail(h, MR_ERR_BAD_ARG, "%s id %d out of range [%d,%d)", songs ? "song" : "test user", ids[i], first, limit);
   if (n == 0) return MR_OK;
   if ((rc = slot_alloc(h, mr_handle::SL_DENSE, &h->d_dense, static_cast<size_t>(std::min(h->batch_rows, kDenseChunk)) * h->n_cols))) return rc;
-  if (model == MR_IBM && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
-  BlendParams bp; memset(&bp, 0, sizeof bp); bp.model = model; bp.te_end = h->d_te_end; bp.song_off = h->win_lo;
   std::vector<void*> tmp;
   DenseOut dout{songs ? DenseOut::SONGS : DenseOut::USERS, out, ids, n, nullptr, nullptr};
   if (songs) {
@@ -1627,7 +1651,8 @@ static int score_subset(mr_handle* h, int model, const int32_t* ids, int n, doub
     if ((rc = dev_upload(h, &d_ids, cols.data(), static_cast<size_t>(n), tmp)) || (rc = dev_alloc(h, &dout.d_out, static_cast<size_t>(n) * h->U, tmp))) { free_list(tmp); return rc; }
     dout.d_ids = d_ids;
   }
-  rc = run_batches(h, model, bp, 0, RUN_DENSE, &dout);
+  Run run{ModelSet(model), Consumer::DENSE, 0, &dout};
+  rc = run_batches(h, run);
   if (!rc && songs) {
     cudaError_t e = cudaMemcpyAsync(out, dout.d_out, static_cast<size_t>(n) * h->U * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
@@ -1658,7 +1683,7 @@ int mr_map_at_k(mr_handle* h, int k, const int32_t* top_song, const int32_t* top
   int rc;
   if (!top_song) {   // rank the device-resident result of the last mr_topk_device / mr_topk
     if (!h->have_topk || h->out_k != k || n_users != h->U) return fail(h, MR_ERR_STATE, "no top-%d result of %d users on the device", k, n_users);
-    d_song = h->d_out_song; d_len = h->d_out_len;
+    d_song = h->out.song; d_len = h->out.len;
   } else {
     int *ds = nullptr, *dl = nullptr;
     if ((rc = dev_upload(h, &ds, top_song, static_cast<size_t>(n_users) * k, tmp)) || (rc = dev_upload(h, &dl, top_len, static_cast<size_t>(n_users), tmp))) { free_list(tmp); return rc; }
@@ -1814,14 +1839,11 @@ void eval_cutoffs(double mn, double mx, int n_thresholds, double* out) {
   }
 }
 
-void join_slice_streams(mr_handle* h) {   // an eval call that fails inside the streamed region leaves no work behind h->stream's back
-  for (cudaStream_t s : {h->slice_stream, h->slice_stream2})
-    if (s && cudaEventRecord(h->ev_join, s) == cudaSuccess) cudaStreamWaitEvent(h->stream, h->ev_join, 0);
-}
-
 // A model set from the caller's parallel arrays, every entry checked before any GPU work (what: the caller's name in the messages;
 // name_entries: the message names the first bad entry, as the set calls do).  The LC alpha must be in [0, 1]: the select and the
-// evaluator rank IEEE bit patterns of non-negative scores (documented deviation, DESIGN.md §3).
+// evaluator rank IEEE bit patterns of non-negative scores.  The reference's linear combination accepts any alpha (MR:317-330 has no
+// range check) and mr_blend_dense follows it, but outside [0,1] a blended score can be negative, which has no place in a ranking of
+// cosine sums (documented deviation, DESIGN.md §3).
 int make_set(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, const char* what, bool name_entries,
              ModelSet* set) {
   if (n < 1 || n > kMaxSet) return fail(h, MR_ERR_BAD_ARG, "%s: n_models = %d outside 1..%d", what, n, kMaxSet);
@@ -1843,16 +1865,15 @@ int make_set(mr_handle* h, int n, const int* models, const double* params, const
   return MR_OK;
 }
 
-// The evaluation form of a set: checks, the Gram workspace, the AGG split columns (one [U] array per AGG entry, on the library stream)
+// The evaluation form of a set: checks, the AGG split columns (one [U] array per AGG entry, on the library stream)
 // and the consumer groups.  Each STOCH entry heads a group of its own (the group reads the one select plane); the other entries fill
 // the groups in entry order, kEvalGroupMax to a launch.
 int eval_set(mr_handle* h, int n, const int* models, const double* params, const uint64_t* seeds, bool name_entries, ModelSet* set) {
   int rc = require_test(h);
   if (rc) return rc;
   if ((rc = make_set(h, n, models, params, seeds, "evaluation", name_entries, set))) return rc;
-  int n_agg = 0; bool ibm_side = false;
-  for (int e = 0; e < n; ++e) { set->bp[e].stats = nullptr; n_agg += set->bp[e].model == MODEL_AGG; ibm_side = ibm_side || set->bp[e].model != MODEL_UBM; }
-  if (ibm_side && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
+  int n_agg = 0;
+  for (int e = 0; e < n; ++e) { set->bp[e].stats = nullptr; n_agg += set->bp[e].model == MODEL_AGG; }
   int* d_split = nullptr;
   if (n_agg && (rc = slot_alloc(h, mr_handle::SL_AGG_SPLIT, &d_split, static_cast<size_t>(n_agg) * h->U))) return rc;
   set->n_groups = 0;
@@ -1895,14 +1916,14 @@ int eval_range_impl(mr_handle* h, int n, const int* models, const double* params
                     double* out_max) {
   if (!h) return MR_ERR_STATE;
   if (!out_min || !out_max) return fail(h, MR_ERR_BAD_ARG, "null output");
-  ModelSet set;
-  int rc = eval_set(h, n, models, params, seeds, name_entries, &set);
+  Run run{ModelSet{}, Consumer::EVAL_RANGE};
+  int rc = eval_set(h, n, models, params, seeds, name_entries, &run.set);
   if (rc) return rc;
   if ((rc = slot_alloc(h, mr_handle::SL_EVAL_MM, &h->d_eval_mm, 2 * static_cast<size_t>(n)))) return rc;
   std::vector<unsigned long long> mm(2 * static_cast<size_t>(n));
   for (int e = 0; e < n; ++e) { mm[2 * e] = ~0ULL; mm[2 * e + 1] = 0ULL; }
   MR_CUDA(h, cudaMemcpyAsync(h->d_eval_mm, mm.data(), mm.size() * 8, cudaMemcpyHostToDevice, h->stream));
-  if ((rc = run_batches(h, set, 0, RUN_EVAL_RANGE, nullptr))) { join_slice_streams(h); return rc; }
+  if ((rc = run_batches(h, run))) return rc;
   MR_CUDA(h, cudaMemcpyAsync(mm.data(), h->d_eval_mm, mm.size() * 8, cudaMemcpyDeviceToHost, h->stream));
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   remember_eval_set(h, n, models, params, seeds);
@@ -1938,8 +1959,8 @@ int eval_counts_impl(mr_handle* h, int n, const int* models, const double* param
   HostStages hs;
   if (n_thresholds != 10 && n_thresholds != 11) return fail(h, MR_ERR_BAD_ARG, "n_thresholds must be 10 (MR:590) or 11 (DIST:395)");
   if (!lab_rowptr || !new_songs || n_new <= 0 || !out_pred || !out_tp || !out_nlab || !mn || !mx) return fail(h, MR_ERR_BAD_ARG, "null / empty arguments");
-  ModelSet set;
-  int rc = eval_set(h, n, models, params, seeds, name_entries, &set);
+  Run run{ModelSet{}, Consumer::EVAL_COUNT};
+  int rc = eval_set(h, n, models, params, seeds, name_entries, &run.set);
   if (rc) return rc;
   hs.mark("set");
   const int U = h->U;
@@ -1967,8 +1988,8 @@ int eval_counts_impl(mr_handle* h, int n, const int* models, const double* param
       return rc;
     }
   hs.mark("label_checks");
-  for (int g = 0; g < set.n_groups; ++g) {
-    EvalGroup& G = set.grp[g];
+  for (int g = 0; g < run.set.n_groups; ++g) {
+    EvalGroup& G = run.set.grp[g];
     for (int m = 0; m < G.n; ++m) {
       double cut[11];
       eval_cutoffs(mn[G.out[m]], mx[G.out[m]], n_thresholds, cut);
@@ -1993,8 +2014,8 @@ int eval_counts_impl(mr_handle* h, int n, const int* models, const double* param
   ec.model_stride = static_cast<long long>(2 * per); ec.nlab = d_cnt + 2 * per * n;
   hs.mark("uploads");
   // resident reuse: a single-batch item-space shard whose panels the range pass of the same set has just filled
-  bool reuse = h->space == MR_SPACE_ITEM && h->U <= h->batch_rows && same_eval_set(h, n, models, params, seeds);
-  if ((rc = run_batches(h, set, 0, RUN_EVAL_COUNT, &reuse))) { join_slice_streams(h); return rc; }
+  run.reuse = h->space == MR_SPACE_ITEM && h->U <= h->batch_rows && same_eval_set(h, n, models, params, seeds);
+  if ((rc = run_batches(h, run))) return rc;
   hs.mark("enqueue");
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   hs.mark("gpu_wait");
@@ -2078,33 +2099,23 @@ int mr_eval_finish(const int64_t* pred, const int64_t* tp, const int64_t* nlab, 
   return MR_OK;
 }
 
-static int topk_impl(mr_handle* h, int model, double param, uint64_t seed, int k, const TopkHostOut* ho) {
+// The single-model top-k: a set of one whose result keeps its own slot (SL_OUT_PACK), so that it survives a set call.
+static int topk_impl(mr_handle* h, int model, double param, uint64_t seed, int k, const TopkOut* ho) {
   int rc = require_test(h);
   if (rc) return rc;
   if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k must be in [1,1024], got %d", k);
-  // The select ranks IEEE bit patterns of non-negative scores.  The reference's linear combination accepts any alpha (MR:317-330 has
-  // no range check) and mr_blend_dense follows it, but outside [0,1] a blended score can be negative, which has no place in a ranking
-  // of cosine sums: getTopK rejects it (documented deviation, DESIGN.md §3).
-  if (model == MR_LC && !(param >= 0 && param <= 1))
-    return fail(h, MR_ERR_PARAM_RANGE, "getTopK: alpha of the linear combination must be between 0 and 1");
-  BlendParams bp;
-  if ((rc = make_blend_params(h, model, param, seed, h->n_pairs_total, &bp))) return rc;
-  bp.pair_base = h->d_pair_base;
-  {  // one packed block (song | score | len) so that a caller can ship the whole result with a single transfer (mr_topk_packed)
-    const size_t song_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * k * 4, 16)), score_b = static_cast<size_t>(h->U) * k * 8,
-                 len_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * 4, 16));
-    char* base = nullptr;
-    if ((rc = slot_alloc(h, mr_handle::SL_OUT_PACK, &base, song_b + score_b + len_b))) return rc;
-    h->d_out_song = reinterpret_cast<int*>(base);
-    h->d_out_score = reinterpret_cast<double*>(base + song_b);
-    h->d_out_len = reinterpret_cast<int*>(base + song_b + score_b);
-    h->out_pack_bytes = song_b + score_b + len_b;
-  }
+  Run run{ModelSet(), Consumer::TOPK, k};
+  if ((rc = make_set(h, 1, &model, &param, &seed, "getTopK", false, &run.set))) return rc;
+  const TopkBlock blk(h->U, k);
+  char* base = nullptr;
+  if ((rc = slot_alloc(h, mr_handle::SL_OUT_PACK, &base, blk.bytes))) return rc;
+  h->out = run.set.out[0] = blk.at(base);
+  h->out_pack_bytes = blk.bytes;
   h->out_k = k;
-  if (model != MR_UBM && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
   h->have_topk = false;
   const bool streamed = ho && h->space == MR_SPACE_ITEM;          // the item-space pipeline copies slice by slice
-  rc = run_batches(h, model, bp, k, RUN_TOPK, streamed ? const_cast<TopkHostOut*>(ho) : nullptr);
+  if (streamed) run.topk_host = ho;
+  rc = run_batches(h, run);
   if (streamed) { cudaError_t e = cudaStreamSynchronize(h->copy_stream); if (!rc && e != cudaSuccess) rc = fail(h, MR_ERR_CUDA, "result copy: %s", cudaGetErrorString(e)); }
   if (rc) return rc;
   h->have_topk = true;
@@ -2120,9 +2131,7 @@ int mr_topk_fetch(mr_handle* h, int k, int32_t* out_song, double* out_score, int
   if (rc) return rc;
   if (!h->have_topk || h->out_k != k) return fail(h, MR_ERR_STATE, "no top-%d result on the device (call mr_topk_device first)", k);
   if (!out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null output");
-  MR_CUDA(h, cudaMemcpyAsync(out_song, h->d_out_song, static_cast<size_t>(h->U) * k * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-  MR_CUDA(h, cudaMemcpyAsync(out_score, h->d_out_score, static_cast<size_t>(h->U) * k * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-  MR_CUDA(h, cudaMemcpyAsync(out_len, h->d_out_len, static_cast<size_t>(h->U) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+  if ((rc = copy_topk(h, TopkOut{out_song, out_score, out_len}, h->out, k, 0, h->U, h->stream))) return rc;
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   return MR_OK;
 }
@@ -2131,9 +2140,9 @@ int mr_topk_device_ptrs(mr_handle* h, int k, void** song, void** score, void** l
   int rc = require_test(h);
   if (rc) return rc;
   if (!h->have_topk || h->out_k != k) return fail(h, MR_ERR_STATE, "no top-%d result on the device (call mr_topk_device first)", k);
-  if (song) *song = h->d_out_song;
-  if (score) *score = h->d_out_score;
-  if (len) *len = h->d_out_len;
+  if (song) *song = h->out.song;
+  if (score) *score = h->out.score;
+  if (len) *len = h->out.len;
   return MR_OK;
 }
 
@@ -2141,10 +2150,10 @@ int mr_topk_packed(mr_handle* h, int k, void** base, uint64_t* bytes, uint64_t* 
   int rc = require_test(h);
   if (rc) return rc;
   if (!h->have_topk || h->out_k != k) return fail(h, MR_ERR_STATE, "no top-%d result on the device (call mr_topk_device first)", k);
-  if (base) *base = h->d_out_song;
+  if (base) *base = h->out.song;
   if (bytes) *bytes = h->out_pack_bytes;
-  if (score_offset) *score_offset = static_cast<uint64_t>(reinterpret_cast<char*>(h->d_out_score) - reinterpret_cast<char*>(h->d_out_song));
-  if (len_offset) *len_offset = static_cast<uint64_t>(reinterpret_cast<char*>(h->d_out_len) - reinterpret_cast<char*>(h->d_out_song));
+  if (score_offset) *score_offset = static_cast<uint64_t>(reinterpret_cast<char*>(h->out.score) - reinterpret_cast<char*>(h->out.song));
+  if (len_offset) *len_offset = static_cast<uint64_t>(reinterpret_cast<char*>(h->out.len) - reinterpret_cast<char*>(h->out.song));
   return MR_OK;
 }
 
@@ -2168,7 +2177,7 @@ int mr_topk_merge(mr_handle* h, int k, int n_parts, int n_users, const int32_t* 
 
 int mr_topk(mr_handle* h, int model, double param, uint64_t seed, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
   if (!out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null output");
-  const TopkHostOut ho{out_song, out_score, out_len};
+  const TopkOut ho{out_song, out_score, out_len};
   return topk_impl(h, model, param, seed, k, &ho);
 }
 
@@ -2176,12 +2185,11 @@ int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const do
   int rc = require_test(h);
   if (rc) return rc;
   if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k must be in [1,1024], got %d", k);
-  ModelSet set;
-  if ((rc = make_set(h, n_models, models, params, seeds, "getTopK", true, &set))) return rc;
-  // one block (song | score | len) per entry in a grow-only slot of its own: the single-model result (mr_topk_fetch, mr_map_at_k) stays
-  const size_t song_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * k * 4, 16)), score_b = static_cast<size_t>(h->U) * k * 8,
-               len_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * 4, 16)), stride = song_b + score_b + len_b;
-  const size_t need = stride * static_cast<size_t>(n_models);
+  Run run{ModelSet(), Consumer::TOPK, k};
+  if ((rc = make_set(h, n_models, models, params, seeds, "getTopK", true, &run.set))) return rc;
+  // one block per entry in a grow-only slot of its own: the single-model result (mr_topk_fetch, mr_map_at_k) stays
+  const TopkBlock blk(h->U, k);
+  const size_t need = blk.bytes * static_cast<size_t>(n_models);
   h->multi_n = 0;
   // it must fit inside the caller's reserve that the batch plan leaves free, and be free now; the plan is not changed for it
   size_t avail = kCallerReserve;
@@ -2195,15 +2203,9 @@ int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const do
                 "that are free", n_models, k, h->U, need, avail);
   char* base = nullptr;
   if ((rc = slot_alloc(h, mr_handle::SL_MULTI_OUT, &base, need, true))) return rc;
-  for (int e = 0; e < n_models; ++e) {
-    char* b = base + stride * e;
-    set.out_song[e] = reinterpret_cast<int*>(b); set.out_score[e] = reinterpret_cast<double*>(b + song_b); set.out_len[e] = reinterpret_cast<int*>(b + song_b + score_b);
-  }
-  bool ibm_side = false;
-  for (int e = 0; e < n_models; ++e) ibm_side = ibm_side || set.bp[e].model != MODEL_UBM;
-  if (ibm_side && h->engine != MR_ENGINE_SPARSE && (rc = ensure_gram_ws(h, h->max_batch_rows))) return rc;
-  if ((rc = run_batches(h, set, k, RUN_TOPK, nullptr))) return rc;
-  h->multi_n = n_models; h->multi_k = k; h->multi_stride = stride;
+  for (int e = 0; e < n_models; ++e) run.set.out[e] = blk.at(base + blk.bytes * e);
+  if ((rc = run_batches(h, run))) return rc;
+  h->multi_n = n_models; h->multi_k = k;
   return MR_OK;
 }
 
@@ -2212,11 +2214,11 @@ int mr_topk_multi_ptrs(mr_handle* h, int i, int k, void** song, void** score, vo
   if (rc) return rc;
   if (h->multi_n == 0 || h->multi_k != k) return fail(h, MR_ERR_STATE, "no top-%d set result on the device (call mr_topk_multi_device first)", k);
   if (i < 0 || i >= h->multi_n) return fail(h, MR_ERR_BAD_ARG, "entry %d outside the set of %d", i, h->multi_n);
-  char* b = static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]) + h->multi_stride * i;
-  const size_t song_b = static_cast<size_t>(round_up(static_cast<long long>(h->U) * k * 4, 16)), score_b = static_cast<size_t>(h->U) * k * 8;
-  if (song) *song = b;
-  if (score) *score = b + song_b;
-  if (len) *len = b + song_b + score_b;
+  const TopkBlock blk(h->U, k);
+  const TopkOut o = blk.at(static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]) + blk.bytes * i);
+  if (song) *song = o.song;
+  if (score) *score = o.score;
+  if (len) *len = o.len;
   return MR_OK;
 }
 
@@ -2229,13 +2231,10 @@ int mr_topk_multi(mr_handle* h, int n_models, const int* models, const double* p
     if (!out_song[e] || !out_score[e] || !out_len[e]) return fail(h, MR_ERR_BAD_ARG, "entry %d: null output", e);
   int rc = mr_topk_multi_device(h, n_models, models, params, seeds, k);
   if (rc) return rc;
-  for (int e = 0; e < n_models; ++e) {
-    void *s = nullptr, *v = nullptr, *l = nullptr;
-    if ((rc = mr_topk_multi_ptrs(h, e, k, &s, &v, &l))) return rc;
-    MR_CUDA(h, cudaMemcpyAsync(out_song[e], s, static_cast<size_t>(h->U) * k * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    MR_CUDA(h, cudaMemcpyAsync(out_score[e], v, static_cast<size_t>(h->U) * k * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    MR_CUDA(h, cudaMemcpyAsync(out_len[e], l, static_cast<size_t>(h->U) * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-  }
+  const TopkBlock blk(h->U, k);
+  char* const base = static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]);
+  for (int e = 0; e < n_models; ++e)
+    if ((rc = copy_topk(h, TopkOut{out_song[e], out_score[e], out_len[e]}, blk.at(base + blk.bytes * e), k, 0, h->U, h->stream))) return rc;
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   return MR_OK;
 }

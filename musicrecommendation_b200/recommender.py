@@ -70,6 +70,15 @@ def _p(a):
     return C.c_void_p(a.ctypes.data) if a is not None else C.c_void_p(0)
 
 
+def _cuda_view(ptr, shape, typestr):
+    """A torch view (no copy) of device memory the library owns."""
+    import torch
+
+    class _Arr:
+        __cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False), "version": 2}
+    return torch.as_tensor(_Arr(), device="cuda")
+
+
 def parse_triplets(stream):
     """One TSV stream -> (users list, songs list) exactly as MR:32-42 accepts it: 3 tab-separated fields, third ignored.
     Java's String.split drops trailing empty strings; a line without exactly 3 fields raises (scala.MatchError, MR:34-35)."""
@@ -326,16 +335,10 @@ class MusicRecommender:
 
     def topk_multi_device_tensors(self, i: int, k: int):
         """torch views (no copy) of entry i of the last set top-k on the device: (song int32 [U,k], score f64 [U,k], len int32 [U])."""
-        import torch
         ps, pv, pl = C.c_void_p(), C.c_void_p(), C.c_void_p()
         self._check(self._lib.mr_topk_multi_ptrs(self._h, i, k, C.byref(ps), C.byref(pv), C.byref(pl)))
         U = self.ds.U
-
-        class _Arr:
-            def __init__(self, ptr, shape, typestr):
-                self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
-        return (torch.as_tensor(_Arr(ps.value, (U, k), "<i4"), device="cuda"), torch.as_tensor(_Arr(pv.value, (U, k), "<f8"), device="cuda"),
-                torch.as_tensor(_Arr(pl.value, (U,), "<i4"), device="cuda"))
+        return _cuda_view(ps.value, (U, k), "<i4"), _cuda_view(pv.value, (U, k), "<f8"), _cuda_view(pl.value, (U,), "<i4")
 
     def prepare(self):
         """Build the item-space head rows now (one-off per train set) instead of lazily."""
@@ -382,16 +385,10 @@ class MusicRecommender:
 
     def topk_device_tensors(self, k: int):
         """torch views (no copy) of the last mr_topk_device result in this GPU's HBM: (song int32 [U,k], score f64 [U,k], len int32 [U])."""
-        import torch
         ps, pv, pl = C.c_void_p(), C.c_void_p(), C.c_void_p()
         self._check(self._lib.mr_topk_device_ptrs(self._h, k, C.byref(ps), C.byref(pv), C.byref(pl)))
         U = self.ds.U
-
-        class _Arr:
-            def __init__(self, ptr, shape, typestr):
-                self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
-        return (torch.as_tensor(_Arr(ps.value, (U, k), "<i4"), device="cuda"), torch.as_tensor(_Arr(pv.value, (U, k), "<f8"), device="cuda"),
-                torch.as_tensor(_Arr(pl.value, (U,), "<i4"), device="cuda"))
+        return _cuda_view(ps.value, (U, k), "<i4"), _cuda_view(pv.value, (U, k), "<f8"), _cuda_view(pl.value, (U,), "<i4")
 
     def mergeTopK(self, parts_song, parts_score, parts_len, out_song, out_score, out_len):
         """Join the ranked lists of several song partitions for the same users (mr_topk_merge; the `.collect` + ranking of
@@ -405,13 +402,9 @@ class MusicRecommender:
     def topk_packed_tensor(self, k: int):
         """The last top-k result as ONE uint8 torch view of device memory plus the byte offsets of its parts:
         (block, score_offset, len_offset); song int32 [U,k] starts at 0."""
-        import torch
         base, nbytes, so, lo = C.c_void_p(), C.c_uint64(), C.c_uint64(), C.c_uint64()
         self._check(self._lib.mr_topk_packed(self._h, k, C.byref(base), C.byref(nbytes), C.byref(so), C.byref(lo)))
-
-        class _Arr:
-            __cuda_array_interface__ = {"shape": (int(nbytes.value),), "typestr": "|u1", "data": (base.value, False), "version": 2}
-        return torch.as_tensor(_Arr(), device="cuda"), int(so.value), int(lo.value)
+        return _cuda_view(base.value, (int(nbytes.value),), "|u1"), int(so.value), int(lo.value)
 
     # ------------------------------------------------------------------ parity probes / similarity products
     def counts_ubm(self) -> np.ndarray:
@@ -426,13 +419,9 @@ class MusicRecommender:
 
     def gram_rows_device(self, s0: int, s1: int):
         """Rows [s0,s1) of this handle's (partial) train co-occurrence matrix as a torch int32 view [s1-s0, ld] of device memory."""
-        import torch
         ptr, ld = C.c_void_p(), C.c_int64()
         self._check(self._lib.mr_gram_rows_device(self._h, s0, s1, C.byref(ptr), C.byref(ld)))
-
-        class _Arr:
-            __cuda_array_interface__ = {"shape": (s1 - s0, ld.value), "typestr": "<i4", "data": (ptr.value, False), "version": 2}
-        return torch.as_tensor(_Arr(), device="cuda")
+        return _cuda_view(ptr.value, (s1 - s0, ld.value), "<i4")
 
     # ---- fused K-split reduce-scatter (GEMM epilogue stores into the owners' receive slots, local or NVLink peer memory)
     def peer_alloc(self, nbytes: int):
@@ -518,16 +507,31 @@ class MusicRecommender:
         self._check(self._lib.mr_eval_range(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), C.byref(mn), C.byref(mx)))
         return float(mn.value), float(mx.value)
 
-    def eval_counts(self, model: int, mn: float, mx: float, new_songs, param: float = 0.5, seed: int = 0, n_thresholds: int = 10,
-                    labels: Dataset | None = None):
-        """Confusion counts of this handle's part of the model under the global (mn, mx): (pred [n_new, n_thr], tp [n_new, n_thr],
-        nlab [n_new]) int64, row c for new_songs[c] (all test users' distinct label songs, ascending).  labels: the data set whose
-        label rows belong to the current shard's users (default: the handle's)."""
+    def _label_csr(self, labels: Dataset | None):
+        """The label CSR (row offsets int64, songs int32) of labels (default: the handle's data set) for the count pass, whose rows must be
+        the current shard's users."""
         lab = labels if labels is not None else self.ds
         lp = np.ascontiguousarray(lab.lab_ptr, np.int64)
         lc = np.ascontiguousarray(lab.lab_col, np.int32)
         if len(lp) != self.ds.U + 1 or len(lc) < (lp[-1] if len(lp) else 0):   # mr_eval_counts reads U + 1 row offsets
             raise ValueError(f"labels must hold {self.ds.U} label rows (the current shard's users), got {len(lp) - 1}")
+        return lp, lc
+
+    def _require_whole_model(self, caller: str, combine: str):
+        """caller evaluates the whole model: no song window, and test users that are the whole test set; a partitioned job combines
+        its handles' parts with distributed.<combine> instead."""
+        if self.song_window != (0, self.ds.S):
+            raise ValueError(f"{caller} needs the whole model: this handle scores a song window (use distributed.{combine})")
+        if not self._whole_test_set:
+            raise ValueError(f"{caller} needs the whole model: this handle holds a shard of the test users (set_test_users with a "
+                             f"pair index base / total); use distributed.{combine}")
+
+    def eval_counts(self, model: int, mn: float, mx: float, new_songs, param: float = 0.5, seed: int = 0, n_thresholds: int = 10,
+                    labels: Dataset | None = None):
+        """Confusion counts of this handle's part of the model under the global (mn, mx): (pred [n_new, n_thr], tp [n_new, n_thr],
+        nlab [n_new]) int64, row c for new_songs[c] (all test users' distinct label songs, ascending).  labels: the data set whose
+        label rows belong to the current shard's users (default: the handle's)."""
+        lp, lc = self._label_csr(labels)
         ns = np.ascontiguousarray(new_songs, np.int32)
         pred = np.zeros((len(ns), n_thresholds), np.int64)
         tp = np.zeros((len(ns), n_thresholds), np.int64)
@@ -542,11 +546,7 @@ class MusicRecommender:
         Same bits as evaluateModel(getXxxModel()) on shapes where that fits.  The handle must hold the whole model: no song window, and
         test users that are the whole test set (ValueError otherwise); a partitioned job combines its handles' parts with
         distributed.evaluate_reference_map."""
-        if self.song_window != (0, self.ds.S):
-            raise ValueError("evaluateOnDevice needs the whole model: this handle scores a song window (use distributed.evaluate_reference_map)")
-        if not self._whole_test_set:
-            raise ValueError("evaluateOnDevice needs the whole model: this handle holds a shard of the test users (set_test_users with a "
-                             "pair index base / total); use distributed.evaluate_reference_map")
+        self._require_whole_model("evaluateOnDevice", "evaluate_reference_map")
         lab = labels if labels is not None else self.ds
         mn, mx = self.eval_range(model, param, seed)
         new_songs = np.unique(np.asarray(lab.lab_col, np.int32))
@@ -570,11 +570,7 @@ class MusicRecommender:
         mx = np.ascontiguousarray(mx, np.float64)
         if mn.shape != (n,) or mx.shape != (n,):
             raise ValueError(f"mn and mx must hold one value per entry of the set ({n})")
-        lab = labels if labels is not None else self.ds
-        lp = np.ascontiguousarray(lab.lab_ptr, np.int64)
-        lc = np.ascontiguousarray(lab.lab_col, np.int32)
-        if len(lp) != self.ds.U + 1 or len(lc) < (lp[-1] if len(lp) else 0):
-            raise ValueError(f"labels must hold {self.ds.U} label rows (the current shard's users), got {len(lp) - 1}")
+        lp, lc = self._label_csr(labels)
         ns = np.ascontiguousarray(new_songs, np.int32)
         pred = np.zeros((n, len(ns), n_thresholds), np.int64)
         tp = np.zeros((n, len(ns), n_thresholds), np.int64)
@@ -586,12 +582,7 @@ class MusicRecommender:
     def evaluateAllOnDevice(self, specs, n_thresholds: int = 10, labels: Dataset | None = None) -> list[float]:
         """evaluateOnDevice for every entry of a model set, from two scorings of the shard (one on a single-batch item-space shard): one
         mAP per entry, each with the bits of evaluateOnDevice(model, param, seed).  The same whole-model guards as evaluateOnDevice."""
-        if self.song_window != (0, self.ds.S):
-            raise ValueError("evaluateAllOnDevice needs the whole model: this handle scores a song window (use "
-                             "distributed.evaluate_reference_map_multi)")
-        if not self._whole_test_set:
-            raise ValueError("evaluateAllOnDevice needs the whole model: this handle holds a shard of the test users (set_test_users with a "
-                             "pair index base / total); use distributed.evaluate_reference_map_multi")
+        self._require_whole_model("evaluateAllOnDevice", "evaluate_reference_map_multi")
         lab = labels if labels is not None else self.ds
         mn, mx = self.eval_range_multi(specs)
         new_songs = np.unique(np.asarray(lab.lab_col, np.int32))

@@ -32,6 +32,8 @@ trait MrScore extends Library {
   // join of the partitions' ranked lists (device pointers; the driver-side collect + ranking of distributed.scala:461, 479)
   def mr_topk_merge(h: Pointer, k: Int, nParts: Int, nUsers: Int, partSong: Array[Pointer], partScore: Array[Pointer], partLen: Array[Pointer],
                     outSong: Pointer, outScore: Pointer, outLen: Pointer): Int
+  // songs like each query song: the k co-listened songs of highest item-item cosine (MusicRecommender.scala:230-239), [n][k] / [n]
+  def mr_similar_songs(h: Pointer, songIds: Array[Int], n: Int, k: Int, outSong: Array[Int], outScore: Array[Double], outLen: Array[Int]): Int
   def mr_ingest_tsv(device: Int, train: Array[Byte], trainLen: Long, test: Array[Byte], testLen: Long, labels: Array[Byte],
                     labelsLen: Long, out: PointerByReference): Int
   def mr_ingest_error(g: Pointer): String

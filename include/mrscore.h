@@ -219,6 +219,24 @@ int mr_eval_counts_multi(mr_handle* h, int n_models, const int* models, const do
                          const double* mn, const double* mx, int n_thresholds, const int64_t* lab_rowptr, const int32_t* lab_col,
                          const int32_t* new_songs, int n_new, int64_t* out_pred, int64_t* out_tp, int64_t* out_nlab);
 
+/* ---- similar songs: the reference's item-item cosine ranked per song (DESIGN.md §4.7) -------------------------------------------------
+ * For each query song i = song_ids[r] (any ids in [0, S), any order, duplicates allowed), the k songs s with the highest
+ *   sim(i, s) = g(i, s) / (sqrt((double) d_i) * sqrt((double) d_s))      (cosineSimilarity, MR:230-239)
+ * with g(i, s) = |U_i^train ∩ U_s^train| over train listeners only (MR:232) and d = deg_song_all as handed to mr_load (train plus test-visible
+ * listeners, MR:237), evaluated in that operation order with correctly rounded steps: every score has the bits of the CPU formula.
+ * Candidates are the co-listened songs only (s != i, g(i, s) > 0) — unlike getTopK, which ranks every unlistened song and so lists 0.0 scores,
+ * a song that shares no train listener with i is never listed.  Order: score descending, then song id ascending (as mr_topk).
+ * Outputs (host arrays): out_song / out_score [n][k], out_len [n]; row r belongs to song_ids[r]; out_len[r] = min(k, #candidates), song -1 /
+ * score 0.0 past it.  A song without train listeners gets out_len 0.  1 <= k <= 1024.  Needs mr_load only (n_test may be 0; the test shard
+ * plays no part).  MR_ERR_BAD_ARG names the first query id out of range; MR_ERR_STATE before mr_load and on a handle with a song window.
+ * Rows whose work E_i = sum over the train listeners v of i of |I_v^train| is small are answered in shared memory (short path, timed as
+ * MR_T_OTHER together with the E_i count); the others from exact count rows of the count engine in chunks of up to 1024 rows (MR_T_COUNT,
+ * MR_T_EXPAND on the tensor engine) and a select over each chunk (MR_T_TOPK).  mr_get_info values 21 / 22 count the rows each path answered.
+ * The call leaves every result and resident state of the scoring calls as it was (top-k results, score panels, head rows, the resident
+ * reuse of mr_eval_counts) and returns with all its work complete.  MR_ERR_OOM, stating the bytes, when not even one chunk of count rows
+ * fits in the free device memory. */
+int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -292,7 +310,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  scored columns (= songs of the window), first song of the window,
                                                                  top-k select since mr_load: rows its sampled fast path handed to the exact path, short rows
                                                                  (exact path by design), degenerate rows (radix select),
-                                                                 scoring passes since mr_load (batches whose score panels were built)] */
+                                                                 scoring passes since mr_load (batches whose score panels were built),
+                                                                 mr_similar_songs rows since mr_load: answered by the short path, by the long path] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

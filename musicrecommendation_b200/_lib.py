@@ -24,7 +24,8 @@ SYMBOLS = ["mr_create", "mr_destroy", "mr_last_error", "mr_load", "mr_set_test_u
            "mr_topk_fetch", "mr_topk_device_ptrs", "mr_set_option", "mr_invalidate_prepared", "mr_score_users", "mr_score_songs", "mr_map_at_k", "mr_write_model", "mr_format_double", "mr_topk_packed", "mr_topk_merge", "mr_gram_rows_scatter_async", "mr_peer_signal", "mr_peer_wait", "mr_sync", "mr_get_timing", "mr_reset_timing", "mr_set_profile", "mr_get_info", "mr_stream",
            "mr_ingest_tsv", "mr_ingest_error", "mr_ingest_dims", "mr_ingest_get", "mr_ingest_free",
            "mr_eval_range", "mr_eval_counts", "mr_eval_finish", "mr_eval_cutoffs",
-           "mr_topk_multi", "mr_topk_multi_device", "mr_topk_multi_ptrs", "mr_eval_range_multi", "mr_eval_counts_multi"]
+           "mr_topk_multi", "mr_topk_multi_device", "mr_topk_multi_ptrs", "mr_eval_range_multi", "mr_eval_counts_multi",
+           "mr_similar_songs"]
 
 _lib = None
 
@@ -107,5 +108,6 @@ def load():
     lib.mr_topk_multi_ptrs.argtypes = [vp, i32, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
     lib.mr_eval_range_multi.argtypes = [vp, i32, vp, vp, vp, vp, vp]
     lib.mr_eval_counts_multi.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp, vp, vp, i32, vp, vp, vp]
+    lib.mr_similar_songs.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     _lib = lib
     return lib

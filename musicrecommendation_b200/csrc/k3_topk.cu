@@ -186,24 +186,6 @@ struct KeyCtx {
   const long long* su; const long long* si; const double* rsd; const uint64_t* sel;
 };
 
-// digit d (0 = most significant) of the 96-bit composite (kb : 64, ~song : 32), 8 bits each
-__device__ __forceinline__ uint32_t key_digit(unsigned long long kb, uint32_t inv_song, int d) {
-  return d < 8 ? static_cast<uint32_t>(kb >> (56 - 8 * d)) & 255u : (inv_song >> (24 - 8 * (d - 8))) & 255u;
-}
-// compare the first nd digits of (kb, inv) against the prefix: -1 below, 0 equal, +1 above
-__device__ __forceinline__ int prefix_cmp(unsigned long long kb, uint32_t inv, unsigned long long phi, uint32_t plo, int nd) {
-  if (nd == 0) return 0;
-  if (nd <= 8) {
-    const int sh = 64 - 8 * nd;
-    const unsigned long long a = kb >> sh, b = phi >> sh;
-    return a < b ? -1 : (a > b ? 1 : 0);
-  }
-  if (kb != phi) return kb < phi ? -1 : 1;
-  const int sh = 32 - 8 * (nd - 8);
-  const uint32_t a = inv >> sh, b = plo >> sh;
-  return a < b ? -1 : (a > b ? 1 : 0);
-}
-
 // L2 prefetches.  The select streams a row in dependent rounds (a thread has one or two 32-byte loads in flight, then computes), so a
 // round costs a full DRAM latency.  Short rows (a song partition: a few hundred KB per user) are pulled into L2 whole by a handful of
 // bulk prefetches when the CTA starts — the sampled passes and the collect pass then hit L2, and the row crosses HBM once instead of
@@ -257,20 +239,6 @@ __device__ __forceinline__ void scan_row(const KeyCtx& c, int n_songs, F&& f, in
       f(s + t, kb, ok);
     }
   }
-}
-
-// warp-aggregated shared-memory histogram increment: peel the two most common bins of the warp with ballots
-__device__ __forceinline__ void hist_add(int* hist, uint32_t bin, bool ok, int lane) {
-  uint32_t pending = __ballot_sync(0xffffffffu, ok);
-#pragma unroll 1
-  for (int round = 0; round < 2 && pending; ++round) {
-    const int leader = __ffs(pending) - 1;
-    const uint32_t lb = __shfl_sync(0xffffffffu, bin, leader);
-    const uint32_t same = __ballot_sync(0xffffffffu, ok && bin == lb) & pending;
-    if (lane == leader) atomicAdd(&hist[lb], __popc(same));
-    pending &= ~same;
-  }
-  if ((pending >> lane) & 1u) atomicAdd(&hist[bin], 1);
 }
 
 // ---- fast path helpers.  "Proxy" p of a song: the integer numerator (pure UBM) or the fp64 score bits (every other model); the

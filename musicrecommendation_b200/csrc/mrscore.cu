@@ -102,7 +102,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard and its results: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -125,6 +125,8 @@ struct mr_handle {
   unsigned long long gen = 0, eval_gen = ~0ULL; int eval_n = 0; int eval_models[16] = {}; double eval_params[16] = {}; uint64_t eval_seeds[16] = {};
   unsigned long long* d_eval_mm = nullptr;   // [2] min / max bit patterns of the range pass
   EvalCounts ec{};                           // device state of the count pass
+  // similar songs (mr_similar_songs): sqrt(deg_song_all) per song, built on the first call; rows answered by each path since mr_load
+  double* d_sim_sqd = nullptr; long long sim_short_rows = 0, sim_long_rows = 0;
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -1621,6 +1623,135 @@ int mr_similarity_ibm(mr_handle* h, int s0, int s1, float* out_rows) {
   return gram_range(h, s0, s1, nullptr, out_rows);
 }
 
+// ---- similar songs (DESIGN.md §4.7, k8_similar.cu).  Uses only the train replica and its own slots: the score panels, the select plane,
+// the head rows, the top-k blocks and gen stay as they are; the count rows of the long path go to the Gram workspace (ensure_gram_ws).
+static constexpr int kSimClassCap[] = {256, 1024, 4096, kSimShortMax};   // short-path launches by E_i: 12 * cap bytes of shared memory per CTA
+static constexpr size_t kSimWindowBytes = 256ULL << 20;   // short-path results: the query list in windows of rows whose block fits this
+static constexpr size_t kSimMargin = 512ULL << 20;        // device memory the long path's chunk sizing leaves free
+
+int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
+  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
+  if (h->windowed) return fail(h, MR_ERR_STATE, "similar songs are not available on a handle with a song window (its song ids are rotated)");
+  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k = %d outside [1, 1024]", k);
+  if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
+  if (n == 0) return MR_OK;
+  if (!song_ids || !out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
+  for (int r = 0; r < n; ++r)
+    if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "query %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
+  MR_CUDA(h, cudaSetDevice(h->device));
+  cudaStream_t st = h->stream;
+  int rc;
+  int* d_ids = nullptr;
+  if (!h->d_sim_sqd) {   // sqrt(d_s), correctly rounded on the device, once per handle
+    double* sq = nullptr;
+    if ((rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_ids, h->deg_song.data(), static_cast<size_t>(h->S))) ||
+        (rc = dev_alloc(h, &sq, static_cast<size_t>(h->S), h->allocs))) return rc;
+    MR_LAUNCH(h, launch_sqrt_deg(d_ids, h->S, sq, st));
+    h->d_sim_sqd = sq;
+  }
+  // E_i per query, read back to split the queries into short and long rows
+  long long* d_ev = nullptr;
+  if ((rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_ids, song_ids, static_cast<size_t>(n))) ||
+      (rc = slot_alloc(h, mr_handle::SL_SIM_EV, &d_ev, static_cast<size_t>(n)))) return rc;
+  std::vector<long long> ev(static_cast<size_t>(n));
+  {
+    PhaseTimer t(h, MR_T_OTHER);
+    MR_LAUNCH(h, launch_sim_events(d_ids, n, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, d_ev, st));
+  }
+  MR_CUDA(h, cudaMemcpyAsync(ev.data(), d_ev, static_cast<size_t>(n) * sizeof(long long), cudaMemcpyDeviceToHost, st));
+  MR_CUDA(h, cudaStreamSynchronize(st));
+  long long short_max = kSimShortMax;   // MRSCORE_SIM_SHORT_MAX can lower the limit (0: every row long), never raise it
+  if (const char* e = getenv("MRSCORE_SIM_SHORT_MAX")) short_max = std::max(0LL, std::min<long long>(kSimShortMax, atoll(e)));
+
+  // short rows: the query list in windows of W rows; one launch per size class; the window's block goes to out rows [r0, r1) in one copy.
+  // The block's rows of long queries hold nothing meaningful; the long path below overwrites them on the host.
+  constexpr int kClasses = static_cast<int>(sizeof kSimClassCap / sizeof kSimClassCap[0]);
+  const size_t row_bytes = static_cast<size_t>(k) * 12 + 4;
+  size_t w_rows = std::min<size_t>(static_cast<size_t>(n), kSimWindowBytes / row_bytes);
+  if (const char* e = getenv("MRSCORE_SIM_WINDOW")) w_rows = std::min<size_t>(w_rows, static_cast<size_t>(std::max(1LL, atoll(e))));   // test aid: many windows
+  const int W = static_cast<int>(std::max<size_t>(1, w_rows));
+  std::vector<int> long_rows;
+  {
+    const TopkBlock blk(W, k);
+    char* base = nullptr; int* d_q = nullptr;
+    if ((rc = slot_alloc(h, mr_handle::SL_SIM_OUT, &base, blk.bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_Q, &d_q, 2 * static_cast<size_t>(W)))) return rc;
+    const TopkOut dev = blk.at(base);
+    std::vector<int> q(2 * static_cast<size_t>(W));   // songs [0, W), window rows [W, 2W), grouped by class
+    for (int r0 = 0; r0 < n; r0 += W) {
+      const int r1 = std::min(n, r0 + W);
+      int cnt[kClasses] = {}, off[kClasses + 1] = {};
+      auto cls = [&](long long e) { int c = 0; while (c < kClasses - 1 && kSimClassCap[c] < e) ++c; return c; };
+      for (int r = r0; r < r1; ++r)
+        if (ev[r] <= short_max) ++cnt[cls(ev[r])]; else long_rows.push_back(r);
+      for (int c = 0; c < kClasses; ++c) off[c + 1] = off[c] + cnt[c];
+      const int n_short = off[kClasses];
+      if (n_short == 0) continue;
+      int fill[kClasses];
+      std::copy(off, off + kClasses, fill);
+      for (int r = r0; r < r1; ++r)
+        if (ev[r] <= short_max) { const int p = fill[cls(ev[r])]++; q[p] = song_ids[r]; q[W + p] = r - r0; }
+      MR_CUDA(h, cudaMemcpyAsync(d_q, q.data(), static_cast<size_t>(n_short) * sizeof(int), cudaMemcpyHostToDevice, st));
+      MR_CUDA(h, cudaMemcpyAsync(d_q + W, q.data() + W, static_cast<size_t>(n_short) * sizeof(int), cudaMemcpyHostToDevice, st));
+      {
+        PhaseTimer t(h, MR_T_OTHER);
+        for (int c = 0; c < kClasses; ++c)
+          if (cnt[c]) MR_LAUNCH(h, launch_similar_short(d_q + off[c], d_q + W + off[c], cnt[c], kSimClassCap[c], h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr,
+                                                        h->d_tr_col, h->d_sim_sqd, k, dev.song, dev.score, dev.len, st));
+      }
+      const size_t o = static_cast<size_t>(r0) * k;
+      if ((rc = copy_topk(h, TopkOut{out_song + o, out_score + o, out_len + r0}, dev, k, 0, r1 - r0, st))) return rc;
+      h->sim_short_rows += n_short;
+    }
+  }
+  // long rows: exact count rows in chunks (count GEMM or inverted-index counts), the select over each chunk, then the rows to the caller
+  if (!long_rows.empty()) {
+    const int n_long = static_cast<int>(long_rows.size());
+    const bool tensor = h->engine == MR_ENGINE_TENSOR;
+    const size_t ws_row = static_cast<size_t>(h->ldg) * sizeof(int32_t) + (tensor ? static_cast<size_t>(h->pitchT) : 0);
+    long long have = static_cast<long long>(h->g_bytes / (static_cast<size_t>(h->ldg) * sizeof(int32_t)));   // rows the workspace holds already
+    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->aj_bytes / h->pitchT));
+    size_t free_b = 0, total_b = 0;
+    MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
+    const long long grow = static_cast<long long>((free_b > kSimMargin ? free_b - kSimMargin : 0) / (ws_row + row_bytes)) / 128 * 128;
+    long long chunk = std::min<long long>(1024, std::max(have, grow));
+    if (const char* e = getenv("MRSCORE_SIM_CHUNK")) chunk = std::min(chunk, std::max(1LL, atoll(e)));   // test aid: force a multi-chunk run
+    chunk = std::min<long long>(chunk, n_long);
+    if (chunk < 1)
+      return fail(h, MR_ERR_OOM, "similar songs: one chunk of 128 count rows needs %zu bytes of device memory beyond a %zu-byte margin, %zu are free",
+                  128 * (ws_row + row_bytes), kSimMargin, free_b);
+    const int C = static_cast<int>(chunk);
+    if ((rc = ensure_gram_ws(h, C))) return rc;
+    const TopkBlock blk(C, k);
+    char* base = nullptr; int* d_rows = nullptr;
+    if ((rc = slot_alloc(h, mr_handle::SL_SIM_LOUT, &base, blk.bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_LIDS, &d_rows, static_cast<size_t>(C)))) return rc;
+    const TopkOut dev = blk.at(base);
+    std::vector<int> rows(static_cast<size_t>(C));
+    std::vector<int32_t> hs(static_cast<size_t>(C) * k), hl(static_cast<size_t>(C));
+    std::vector<double> hv(static_cast<size_t>(C) * k);
+    for (int c0 = 0; c0 < n_long; c0 += C) {
+      const int nc = std::min(C, n_long - c0);
+      for (int j = 0; j < nc; ++j) rows[j] = song_ids[long_rows[c0 + j]];
+      MR_CUDA(h, cudaMemcpyAsync(d_rows, rows.data(), static_cast<size_t>(nc) * sizeof(int), cudaMemcpyHostToDevice, st));
+      if ((rc = gram_rows(h, d_rows, nc))) return rc;
+      {
+        PhaseTimer t(h, MR_T_TOPK);
+        MR_LAUNCH(h, launch_similar_rows(d_rows, nc, h->d_g, h->ldg, h->S, h->d_sim_sqd, k, dev.song, dev.score, dev.len, st));
+      }
+      if ((rc = copy_topk(h, TopkOut{hs.data(), hv.data(), hl.data()}, dev, k, 0, nc, st))) return rc;
+      MR_CUDA(h, cudaStreamSynchronize(st));
+      for (int j = 0; j < nc; ++j) {
+        const size_t r = static_cast<size_t>(long_rows[c0 + j]);
+        memcpy(out_song + r * k, hs.data() + static_cast<size_t>(j) * k, static_cast<size_t>(k) * sizeof(int32_t));
+        memcpy(out_score + r * k, hv.data() + static_cast<size_t>(j) * k, static_cast<size_t>(k) * sizeof(double));
+        out_len[r] = hl[j];
+      }
+    }
+    h->sim_long_rows += n_long;
+  }
+  MR_CUDA(h, cudaStreamSynchronize(st));
+  return MR_OK;
+}
+
 int mr_score_dense(mr_handle* h, int model, double* out_UxS) {
   int rc = require_test(h);
   if (rc) return rc;
@@ -2253,10 +2384,11 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[20] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[22] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
-                         h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes};
-  for (int i = 0; i < n && i < 20; ++i) out[i] = v[i];
+                         h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
+                         h->sim_short_rows, h->sim_long_rows};
+  for (int i = 0; i < n && i < 22; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

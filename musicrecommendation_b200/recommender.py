@@ -318,6 +318,18 @@ class MusicRecommender:
         self._check(self._lib.mr_topk(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), k, _p(song), _p(score), _p(ln)))
         return song, score, ln
 
+    def getSimilarSongs(self, songs=None, k: int = 100):
+        """Songs like each of `songs` (default: all S songs): the k co-listened songs of highest item-item cosine (MR:230-239), score
+        descending then song id ascending (mr_similar_songs, DESIGN.md §4.7).  Returns (song [n, k] int32, score [n, k] float64,
+        len [n] int32); row r belongs to songs[r], song -1 / score 0.0 past len[r]."""
+        ids = np.arange(self.ds.S, dtype=np.int32) if songs is None else np.ascontiguousarray(songs, np.int32).reshape(-1)
+        n = len(ids)
+        song = np.empty((n, k), np.int32)
+        score = np.empty((n, k), np.float64)
+        ln = np.empty(n, np.int32)
+        self._check(self._lib.mr_similar_songs(self._h, _p(ids), n, k, _p(song), _p(score), _p(ln)))
+        return song, score, ln
+
     def getTopKMulti(self, specs, k: int = 500):
         """getTopK for every entry of a model set (model, param, seed) from one scoring of the shard (mr_topk_multi, DESIGN.md §4.6):
         one (song [U,k] int32, score [U,k] f64, len [U]) per entry, each equal to getTopK(model, k, param, seed)."""
@@ -473,11 +485,11 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 20)()
-        self._lib.mr_get_info(self._h, v, 20)
+        v = (C.c_int64 * 22)()
+        self._lib.mr_get_info(self._h, v, 22)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
-                         "topk_short_rows", "topk_degenerate_rows", "scoring_passes"], list(v)))
+                         "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -710,6 +722,41 @@ def eval_counts_host(scores: np.ndarray, ds: Dataset, lo: int, mn: float, mx: fl
         tp[idx, t] = (p & lab).sum(0)
     nlab[idx] = lab.sum(0)
     return pred, tp, nlab
+
+
+def similar_songs_host(ds: Dataset, songs, k: int):
+    """numpy mirror of mr_similar_songs: per query song i, the train histories of i's train listeners concatenated, their distinct songs
+    s != i with counts g (np.unique), sim = g / (sqrt(d_i) * sqrt(d_s)) in that operation order (0 where the denominator is 0, as the
+    reference's cosineSimilarity), ranked by score descending then song id ascending.  Returns (song [n, k], score [n, k], len [n])."""
+    songs = np.asarray(songs, np.int64).reshape(-1)
+    n = len(songs)
+    out_song = np.full((n, k), -1, np.int32)
+    out_score = np.zeros((n, k), np.float64)
+    out_len = np.zeros(n, np.int32)
+    tr_ptr = np.asarray(ds.tr_ptr, np.int64)
+    tr_col = np.asarray(ds.tr_col, np.int64)
+    owner = np.repeat(np.arange(ds.T), np.diff(tr_ptr))                    # train user of every train entry
+    order = np.argsort(tr_col, kind="stable")                              # inverted index: listeners of a song, ascending
+    csc_ptr = np.concatenate([[0], np.cumsum(np.bincount(tr_col, minlength=ds.S))])
+    listeners = owner[order]
+    deg = np.asarray(ds.deg_song, np.int64)
+    for r, i in enumerate(songs):
+        users = listeners[csc_ptr[i]:csc_ptr[i + 1]]
+        if len(users) == 0:
+            continue
+        hist = np.concatenate([tr_col[tr_ptr[v]:tr_ptr[v + 1]] for v in users])
+        s, g = np.unique(hist, return_counts=True)
+        keep = s != i
+        s, g = s[keep], g[keep]
+        den = np.sqrt(np.float64(deg[i])) * np.sqrt(deg[s].astype(np.float64))
+        with np.errstate(divide="ignore", invalid="ignore"):
+            sim = np.where(den != 0, g.astype(np.float64) / den, 0.0)
+        rank = np.lexsort((s, -sim))
+        m = min(k, len(rank))
+        out_song[r, :m] = s[rank[:m]]
+        out_score[r, :m] = sim[rank[:m]]
+        out_len[r] = m
+    return out_song, out_score, out_len
 
 
 def evaluate_map(scores: np.ndarray, ds: Dataset, n_thresholds: int = 10) -> float:

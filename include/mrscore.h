@@ -304,7 +304,7 @@ enum { MR_T_EXPAND = 0, MR_T_COUNT = 1, MR_T_AGG_UBM = 2, MR_T_AGG_IBM = 3, MR_T
 int mr_get_timing(mr_handle* h, double* ms_out, int n);      /* accumulated CUDA-event ms per phase since the last reset */
 int mr_reset_timing(mr_handle* h);
 int mr_set_profile(mr_handle* h, int on);                   /* toggle MR_PROFILE at run time (it synchronises after every phase) */
-int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel launches so far, dense operand bytes, n_items, num_sms, device bytes allocated, space, n_head songs,
+int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel launches so far, dense operand bytes, n_items, num_sms, device bytes the handle holds now, space, n_head songs,
                                                                  test entries on head songs, test entries on tail songs, head-row exceptions,
                                                                  test users per batch, head_rowsum work groups per batch, users split over groups,
                                                                  scored columns (= songs of the window), first song of the window,

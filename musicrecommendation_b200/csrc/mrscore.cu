@@ -16,6 +16,7 @@
 #include <algorithm>
 #include <chrono>
 #include <cmath>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -55,7 +56,7 @@ struct mr_handle {
   cudaStream_t slice_stream2 = nullptr; cudaEvent_t ev_join = nullptr;   // single-batch calls alternate their slices between the two slice streams
   std::string err;
   long long launches = 0; size_t dev_bytes = 0;
-  std::vector<void*> allocs;          // everything freed in mr_destroy
+  std::vector<void*> allocs;          // allocated once per handle (mr_load, the sqrt table of similar songs, peer buffers), freed in mr_destroy
   // train
   int T = 0, S = 0; long long nnz_tr = 0; bool loaded = false;
   long long *d_tr_ptr = nullptr, *d_csc_ptr = nullptr; int *d_tr_col = nullptr, *d_csc_idx = nullptr;
@@ -91,8 +92,8 @@ struct mr_handle {
   int4 *d_seg = nullptr, *d_grp_hdr = nullptr; int *d_ge_row = nullptr, *d_split_rows = nullptr; uint32_t* d_ge_q = nullptr; int seg_cap = 1, ent_cap = 1;
   std::vector<int> h_split_ptr;   // balanced work groups per batch
   std::vector<int> head_index;         // song -> head row or -1
-  int* d_head_song = nullptr; long long* d_head_lst_ptr = nullptr; uint16_t* d_g16 = nullptr; uint32_t* d_gq32 = nullptr;
-  size_t head_rows_cap = 0;            // entries the packed-row allocations hold (kept across mr_invalidate_prepared)
+  int* d_head_song = nullptr; long long* d_head_lst_ptr = nullptr;
+  uint16_t* d_g16 = nullptr; uint32_t* d_gq32 = nullptr;   // packed head rows, slots SL_HEAD_G16 / SL_HEAD_GQ32 (kept across mr_invalidate_prepared)
   int n_head_staged = 0;               // rows [0, n_head_staged) are built in a 64-bit staging area and packed; the rest directly in place
   long long opt_head_min_deg = 0;      // mr_set_option(MR_OPT_HEAD_MIN_DEG): 0 = default rule
   long long* d_ex_ptr = nullptr; int* d_ex_song = nullptr; uint32_t* d_ex_g = nullptr; unsigned long long* d_ex_gq = nullptr; long long n_ex = 0;
@@ -100,9 +101,9 @@ struct mr_handle {
   int *d_tu_user = nullptr, *d_tu_song = nullptr; long long* d_tu_lptr = nullptr; std::vector<long long> h_tu_ptr, h_tu_lptr; long long n_head_entries = 0, n_tail_entries = 0;
   // test shard (freed / reallocated by mr_set_test_users)
   int U = 0; long long nnz_te = 0; bool have_test = false;
-  // grow-only device buffers of the test shard and its results: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
+  // grow-only device buffers of the test shard, its results and the workspaces: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -112,7 +113,7 @@ struct mr_handle {
   uint8_t *d_Ate = nullptr, *d_Aj = nullptr; uint16_t* d_ct = nullptr; long long *d_sint_u = nullptr, *d_sint_i = nullptr;
   uint32_t* d_wi = nullptr;             // IBM user-space weighted counts u32[T][128] (sparse engine)
   unsigned int* d_carry_count = nullptr; uint2* d_carry_events = nullptr; unsigned int carry_cap = 1u << 20; unsigned int* h_carry_seen = nullptr;
-  uint64_t* d_sel = nullptr; long long sel_pitch = 0; int32_t* d_g = nullptr; size_t g_bytes = 0; size_t aj_bytes = 0;
+  uint64_t* d_sel = nullptr; long long sel_pitch = 0; int32_t* d_g = nullptr;   // d_g / d_Aj: the Gram workspace, slots SL_GRAM_G / SL_GRAM_A
   double* d_dense = nullptr; int32_t* d_cnt = nullptr; float* d_simf = nullptr;
   // results
   TopkOut out{}; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;   // the single-model result, a TopkBlock in SL_OUT_PACK
@@ -199,6 +200,35 @@ int dev_upload(mr_handle* h, Tp** out, const Tp* src, size_t count, std::vector<
   return MR_OK;
 }
 
+// The temporaries of one call, counted in dev_bytes while they live.  They are freed when the owner goes out of scope, on every return
+// path, once the stream they are used on has drained.
+struct Scratch {
+  mr_handle* h; cudaStream_t st;
+  std::vector<void*> bufs; size_t bytes = 0;
+  Scratch(mr_handle* hh, cudaStream_t s) : h(hh), st(s) {}
+  Scratch(const Scratch&) = delete;
+  Scratch& operator=(const Scratch&) = delete;
+  ~Scratch() {
+    if (bufs.empty()) return;
+    cudaStreamSynchronize(st);
+    for (void* p : bufs) cudaFree(p);
+    h->dev_bytes -= bytes;
+  }
+  template <class Tp>
+  int alloc(Tp** out, size_t count) {
+    const int rc = dev_alloc(h, out, count, bufs);
+    if (!rc) bytes += std::max<size_t>(count, 1) * sizeof(Tp);
+    return rc;
+  }
+  template <class Tp>
+  int upload(Tp** out, const Tp* src, size_t count) {
+    const int rc = alloc(out, count);
+    if (rc) return rc;
+    if (count) MR_CUDA(h, cudaMemcpyAsync(*out, src, count * sizeof(Tp), cudaMemcpyHostToDevice, st));
+    return MR_OK;
+  }
+};
+
 inline uint32_t q_of(int32_t deg, double scale) { return deg <= 0 ? 0u : static_cast<uint32_t>(llrint(scale / std::sqrt(static_cast<double>(deg)))); }
 inline double rs_of(int32_t deg, double inv) { return deg <= 0 ? 0.0 : inv / std::sqrt(static_cast<double>(deg)); }
 inline float rsf_of(int32_t deg) { return deg <= 0 ? 0.0f : static_cast<float>(1.0 / std::sqrt(static_cast<double>(deg))); }
@@ -242,7 +272,7 @@ int check_csr(mr_handle* h, const char* what, int n_rows, int n_cols, const int6
   });
   const Bad& b = best;
   if (b.row >= 0 && b.kind == 1) return fail(h, MR_ERR_BAD_ARG, "%s: column id %d out of range at row %d", what, b.col, b.row);
-  if (b.row >= 0) return fail(h, MR_ERR_BAD_ARG, "%s: row %d not ascending/unique", what, b.row);
+  if (b.row >= 0) return fail(h, MR_ERR_BAD_ARG, "%s row %d not ascending/unique", what, b.row);
   return MR_OK;
 }
 
@@ -289,11 +319,6 @@ __global__ void iota_kernel(int* p, int start, int n) {
   if (i < n) p[i] = start + i;
 }
 
-void free_list(std::vector<void*>& v) {
-  for (void* p : v) cudaFree(p);
-  v.clear();
-}
-
 // ---- K1 for one batch of test users -> Ct u16[T][128]
 int count_ubm_batch(mr_handle* h, int b0, int nb) {
   if (h->engine == MR_ENGINE_TENSOR) {
@@ -334,21 +359,10 @@ int gram_rows(mr_handle* h, const int* d_rows, int n_rows) {
 }
 
 int ensure_gram_ws(mr_handle* h, int n_rows) {
-  const size_t need_g = static_cast<size_t>(round_up(std::max(n_rows, 1), 128)) * h->ldg * sizeof(int32_t);
-  if (need_g > h->g_bytes) {
-    int32_t* p; int rc = dev_alloc(h, &p, need_g / sizeof(int32_t), h->allocs);
-    if (rc) return rc;
-    h->d_g = p; h->g_bytes = need_g;
-  }
-  if (h->engine == MR_ENGINE_TENSOR) {
-    const size_t need_a = static_cast<size_t>(round_up(std::max(n_rows, 1), 128)) * h->pitchT;
-    if (need_a > h->aj_bytes) {
-      uint8_t* p; int rc = dev_alloc(h, &p, need_a, h->allocs);
-      if (rc) return rc;
-      h->d_Aj = p; h->aj_bytes = need_a;
-    }
-  }
-  return MR_OK;
+  const size_t rows = static_cast<size_t>(round_up(std::max(n_rows, 1), 128));
+  const int rc = slot_alloc(h, mr_handle::SL_GRAM_G, &h->d_g, rows * h->ldg, true);
+  if (rc || h->engine != MR_ENGINE_TENSOR) return rc;
+  return slot_alloc(h, mr_handle::SL_GRAM_A, &h->d_Aj, rows * h->pitchT, true);
 }
 
 // Item-space: compute the rows G[h][:], Gq[h][:] of the head songs once per train set (lazily, on first use, or mr_prepare).
@@ -376,16 +390,8 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
   auto now = [] { return std::chrono::steady_clock::now(); };
   auto ms_since = [&](std::chrono::steady_clock::time_point t) { return std::chrono::duration<double, std::milli>(now() - t).count(); };
   auto t_start = now();
-  const size_t n = static_cast<size_t>(std::max(h->n_head, 1)) * h->spitch;
-  if (h->head_rows_cap < n) {   // allocated once per handle; a failed or invalidated precompute reuses it
-    if (h->d_g16) { cudaFree(h->d_g16); h->d_g16 = nullptr; }
-    if (h->d_gq32) { cudaFree(h->d_gq32); h->d_gq32 = nullptr; }
-    h->dev_bytes -= h->head_rows_cap * 6; h->head_rows_cap = 0;
-    MR_CUDA(h, cudaMalloc(reinterpret_cast<void**>(&h->d_g16), n * sizeof(uint16_t)));
-    cudaError_t em = cudaMalloc(reinterpret_cast<void**>(&h->d_gq32), n * sizeof(uint32_t));
-    if (em != cudaSuccess) { cudaFree(h->d_g16); h->d_g16 = nullptr; return fail(h, MR_ERR_OOM, "head rows: %s", cudaGetErrorString(em)); }
-    h->head_rows_cap = n; h->dev_bytes += n * 6;
-  }
+  const size_t n = static_cast<size_t>(std::max(h->n_head, 1)) * h->spitch;   // allocated once per handle; a failed or invalidated precompute reuses it
+  if ((rc = slot_alloc(h, mr_handle::SL_HEAD_G16, &h->d_g16, n, true)) || (rc = slot_alloc(h, mr_handle::SL_HEAD_GQ32, &h->d_gq32, n, true))) return rc;
   const bool tensor = h->engine == MR_ENGINE_TENSOR && h->n_head > 0 && h->T < (1 << 23);
   const int n_staged = tensor ? h->n_head : h->n_head_staged;
   // number of byte planes the weights q_24(|I_v|) need (3 when every train user has >= 2 songs: q < 2^24)
@@ -408,7 +414,7 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
   // every step of a job that counts the model build) does no cudaMalloc / cudaFree — next to 100+ GB of live allocations those cost
   // tens to hundreds of milliseconds, more than the kernels of a song partition's precompute.  Only the tensor engine's dense operands
   // (small shapes) are temporary.
-  std::vector<void*> tmp;
+  Scratch tmp(h, st);
   uint32_t* g_stage = nullptr; unsigned long long* gq_stage = nullptr;
   HeadExceptions ex{};
   ex.capacity = n_staged > 0 ? (1u << 24) : 1u;
@@ -424,24 +430,23 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
     ex.song = reinterpret_cast<int*>(xb + 16 + cap * 12);
     ex.g_extra = reinterpret_cast<uint32_t*>(xb + 16 + cap * 16);
   }
-  auto bail = [&](int code) { cudaStreamSynchronize(st); free_list(tmp); return code; };
   cudaError_t e = cudaMemsetAsync(ex.count, 0, sizeof(unsigned int), st);
-  if (e != cudaSuccess) return bail(fail(h, MR_ERR_CUDA, "memset: %s", cudaGetErrorString(e)));
+  if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "memset: %s", cudaGetErrorString(e));
   uint8_t *a_rows = nullptr, *b_plane = nullptr;
   if (tensor) {
-    if ((rc = dev_alloc(h, &a_rows, static_cast<size_t>(chunk) * h->pitchT, tmp)) ||
-        (rc = dev_alloc(h, &b_plane, static_cast<size_t>(h->S) * h->pitchT * n_planes, tmp))) { free_list(tmp); return rc; }
+    if ((rc = tmp.alloc(&a_rows, static_cast<size_t>(chunk) * h->pitchT)) ||
+        (rc = tmp.alloc(&b_plane, static_cast<size_t>(h->S) * h->pitchT * n_planes))) return rc;
     // the GEMM epilogues write only the columns < S: the pad columns of the staging rows must not hold garbage (pack reads the full pitch)
     e = cudaMemsetAsync(g_stage, 0, stage_entries * sizeof(uint32_t), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(gq_stage, 0, stage_entries * sizeof(unsigned long long), st);
-    if (e != cudaSuccess) return bail(fail(h, MR_ERR_CUDA, "memset: %s", cudaGetErrorString(e)));
+    if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "memset: %s", cudaGetErrorString(e));
     // the byte planes of q_24(|I_v|) as weighted B operands (built once, reused by every chunk)
     PhaseTimer t(h, MR_T_EXPAND, st);
     for (int plane = 0; plane < n_planes; ++plane) {
       int lrc = launch_expand_rows_weighted(h->d_csc_ptr, h->d_csc_idx, h->d_qv, plane, h->S, h->pitchT,
                                             b_plane + static_cast<size_t>(plane) * h->S * h->pitchT, st);
       h->launches++;
-      if (lrc) return bail(fail(h, MR_ERR_CUDA, "launch_expand_rows_weighted failed"));
+      if (lrc) return fail(h, MR_ERR_CUDA, "launch_expand_rows_weighted failed");
     }
   }
   if (dbg) { cudaStreamSynchronize(st); fprintf(stderr, "[mrscore] precompute: allocations %.1f ms (staged rows %d in chunks of %lld, direct rows %d)\n", ms_since(t_start), n_staged, chunk, h->n_head - n_staged); }
@@ -455,7 +460,7 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
         PhaseTimer t(h, MR_T_EXPAND, st);
         int lrc = launch_expand_rows(h->d_csc_ptr, h->d_csc_idx, h->d_head_song + r0, 0, nr, n_pad, h->pitchT, a_rows, st);
         h->launches++;
-        if (lrc) return bail(fail(h, MR_ERR_CUDA, "launch_expand_rows failed"));
+        if (lrc) return fail(h, MR_ERR_CUDA, "launch_expand_rows failed");
       }
       PhaseTimer t(h, MR_T_COUNT, st);
       int lrc = launch_count_gemm(a_rows, n_pad, h->d_AtrT, h->S, h->pitchT, nr, h->S, EPI_I32, g_stage, h->spitch, nullptr, nullptr, h->num_sms, st);
@@ -465,18 +470,18 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
                                 gq_stage, h->spitch, nullptr, nullptr, h->num_sms, st, 8 * plane, plane > 0);
         h->launches++;
       }
-      if (lrc) return bail(fail(h, MR_ERR_CUDA, "launch_count_gemm failed: rc=%d (%s)", lrc, cudaGetErrorString(cudaGetLastError())));
+      if (lrc) return fail(h, MR_ERR_CUDA, "launch_count_gemm failed: rc=%d (%s)", lrc, cudaGetErrorString(cudaGetLastError()));
     } else {
       PhaseTimer t(h, MR_T_PRECOMPUTE, st);
       int lrc = launch_gram_head_scatter(h->d_head_song, h->d_head_lst_ptr, r0, r0 + nr, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_end,
                                          h->d_tr_col, h->d_qv, g_stage, gq_stage, h->spitch, packed ? 1 : 0, h->num_sms, st);
       h->launches++;
-      if (lrc) return bail(fail(h, MR_ERR_CUDA, "launch_gram_head_scatter failed"));
+      if (lrc) return fail(h, MR_ERR_CUDA, "launch_gram_head_scatter failed");
     }
     PhaseTimer t(h, MR_T_PRECOMPUTE, st);
     int lrc = launch_pack_head_rows(g_stage, gq_stage, packed ? 1 : 0, r0, nr, h->spitch, h->n_cols, h->d_g16, h->d_gq32, ex, h->num_sms, st);
     h->launches++;
-    if (lrc) return bail(fail(h, MR_ERR_CUDA, "launch_pack_head_rows failed"));
+    if (lrc) return fail(h, MR_ERR_CUDA, "launch_pack_head_rows failed");
   }
   if (dbg) { cudaStreamSynchronize(st); fprintf(stderr, "[mrscore] precompute: staged rows %.1f ms\n", ms_since(t_loop)); }
   if (n_staged < h->n_head) {
@@ -495,7 +500,7 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
     auto sync_extra = [&] { for (int i = 0; i < kPreExtraStreams; ++i) cudaStreamSynchronize(h->pre_extra[i]); };
     for (int i = 0; i + 1 < n_streams; ++i) {
       if ((e = cudaEventRecord(h->ev_pre_extra[i], st)) != cudaSuccess || (e = cudaStreamWaitEvent(h->pre_extra[i], h->ev_pre_extra[i], 0)) != cudaSuccess)
-        return bail(fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e)));
+        return fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e));
     }
     int ci = 0;
     for (int r0 = n_staged; r0 < h->n_head; r0 += static_cast<int>(dchunk), ++ci) {
@@ -504,20 +509,19 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
       int lrc = launch_gram_head_direct(h->d_head_song, h->d_head_lst_ptr, r0, r0 + nr, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_end,
                                         h->d_tr_col, h->d_qv, h->d_g16, h->d_gq32, h->spitch, h->num_sms, si ? h->pre_extra[si - 1] : st);
       h->launches++;
-      if (lrc) { sync_extra(); return bail(fail(h, MR_ERR_CUDA, "launch_gram_head_direct failed")); }
+      if (lrc) { sync_extra(); return fail(h, MR_ERR_CUDA, "launch_gram_head_direct failed"); }
     }
     for (int i = 0; i + 1 < n_streams; ++i) {   // `st` joins the extra streams
       if ((e = cudaEventRecord(h->ev_pre_extra[i], h->pre_extra[i])) != cudaSuccess || (e = cudaStreamWaitEvent(st, h->ev_pre_extra[i], 0)) != cudaSuccess) {
         sync_extra();
-        return bail(fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e)));
+        return fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e));
       }
     }
   }
   // the exception count travels to pinned host memory behind the kernels; finish_head_rows picks it up
   e = cudaMemcpyAsync(h->h_n_ex, ex.count, sizeof(unsigned int), cudaMemcpyDeviceToHost, st);
   if (e == cudaSuccess) e = cudaEventRecord(h->ev_pre, st);
-  if (e != cudaSuccess) return bail(fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e)));
-  if (!tmp.empty()) { cudaStreamSynchronize(st); free_list(tmp); }     // tensor engine only: its dense operands are temporary
+  if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "head-row precompute: %s", cudaGetErrorString(e));
   if (dbg) fprintf(stderr, "[mrscore] precompute: launched after %.1f ms\n", ms_since(t_start));
   h->pend_ex = ex;
   h->head_pending = true;
@@ -588,7 +592,7 @@ int plan_item_batches_once(mr_handle* h, const std::vector<long long>& hu_ptr, i
     const size_t per_row = static_cast<size_t>(h->spitch) * 16 + static_cast<size_t>(h->sel_pitch) * 8;
     size_t avail = free_b + h->slot_cap[mr_handle::SL_SINT_U] + h->slot_cap[mr_handle::SL_SINT_I] + h->slot_cap[mr_handle::SL_SEL];
     size_t reserve = kCallerReserve;   // left for the caller's context (torch, NCCL buffers, gathered top-k blocks) and small workspaces
-    if (!h->head_ready && h->head_rows_cap == 0) reserve += static_cast<size_t>(std::max(h->n_head, 1)) * h->spitch * 6 + (1ULL << 30);   // head rows + staging come later
+    if (!h->head_ready && h->slot_cap[mr_handle::SL_HEAD_G16] == 0) reserve += static_cast<size_t>(std::max(h->n_head, 1)) * h->spitch * 6 + (1ULL << 30);   // head rows + staging come later
     long long max_rows = avail > reserve ? static_cast<long long>((avail - reserve) / per_row) : 0;
     max_rows = std::max<long long>(max_rows, kUserBatch);
     if (h->item_batch_cap > 0) max_rows = std::min<long long>(max_rows, h->item_batch_cap);
@@ -1081,9 +1085,7 @@ void mr_destroy(mr_handle* h) {
   for (int i = 0; i < 2; ++i) { if (h->ev_head[i]) cudaEventDestroy(h->ev_head[i]); if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]); }
   if (h->h_n_ex) cudaFreeHost(h->h_n_ex);
   for (int i = 0; i < mr_handle::SL_N; ++i) if (h->slot_p[i]) cudaFree(h->slot_p[i]);
-  if (h->d_g16) cudaFree(h->d_g16);
-  if (h->d_gq32) cudaFree(h->d_gq32);
-  free_list(h->allocs);
+  for (void* p : h->allocs) cudaFree(p);
   if (h->h_carry_seen) cudaFreeHost(h->h_carry_seen);
   if (h->ev[0]) cudaEventDestroy(h->ev[0]);
   if (h->ev[1]) cudaEventDestroy(h->ev[1]);
@@ -1413,12 +1415,17 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   return MR_OK;
 }
 
-static int require_test(mr_handle* h) {
-  if (!h) return MR_ERR_STATE;
-  if (!h->loaded || !h->have_test) return fail(h, MR_ERR_STATE, "no data loaded (mr_load / mr_set_test_users)");
+static int require_loaded(mr_handle* h) {
+  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
   cudaError_t e = cudaSetDevice(h->device);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
   return MR_OK;
+}
+
+static int require_test(mr_handle* h) {
+  if (!h) return MR_ERR_STATE;
+  if (!h->loaded || !h->have_test) return fail(h, MR_ERR_STATE, "no data loaded (mr_load / mr_set_test_users)");
+  return require_loaded(h);
 }
 
 // The UBM parity probes, not scoring: per 128-user batch the counts Ct as int32 (out_cnt) or cosines (out_sim; on the tensor engine
@@ -1458,23 +1465,21 @@ int mr_counts_ubm(mr_handle* h, int32_t* out_UxT) { return ubm_probe(h, out_UxT,
 int mr_similarity_ubm(mr_handle* h, float* out_UxT) { return ubm_probe(h, nullptr, out_UxT); }
 
 static int gram_range(mr_handle* h, int s0, int s1, int32_t* out_i32, float* out_f32) {
-  int rc = require_test(h);
-  if (rc == MR_ERR_STATE && h && h->loaded) rc = MR_OK;   // Gram rows need only the train replica
+  int rc = require_loaded(h);   // Gram rows need only the train replica
   if (rc) return rc;
-  MR_CUDA(h, cudaSetDevice(h->device));
   if (h->windowed) return fail(h, MR_ERR_STATE, "Gram rows are not available on a handle with a song window (its song ids are rotated)");
   if (s0 < 0 || s1 > h->S || s0 > s1) return fail(h, MR_ERR_BAD_ARG, "song range [%d,%d) outside [0,%d)", s0, s1, h->S);
   const int chunk = 1024;
   int* d_ids = nullptr; float* d_f = nullptr;
-  std::vector<void*> tmp;
-  if ((rc = dev_alloc(h, &d_ids, chunk, tmp))) return rc;
-  if (out_f32 && (rc = dev_alloc(h, &d_f, static_cast<size_t>(chunk) * h->S, tmp))) { free_list(tmp); return rc; }
-  if ((rc = ensure_gram_ws(h, chunk))) { free_list(tmp); return rc; }
+  Scratch tmp(h, h->stream);
+  if ((rc = tmp.alloc(&d_ids, chunk))) return rc;
+  if (out_f32 && (rc = tmp.alloc(&d_f, static_cast<size_t>(chunk) * h->S))) return rc;
+  if ((rc = ensure_gram_ws(h, chunk))) return rc;
   for (int r0 = s0; r0 < s1; r0 += chunk) {
     const int n = std::min(chunk, s1 - r0);
     iota_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(d_ids, r0, n);
     h->launches++;
-    if ((rc = gram_rows(h, d_ids, n))) { free_list(tmp); return rc; }
+    if ((rc = gram_rows(h, d_ids, n))) return rc;
     cudaError_t e;
     if (out_i32) {
       e = cudaMemcpy2DAsync(out_i32 + static_cast<long long>(r0 - s0) * h->S, static_cast<size_t>(h->S) * 4, h->d_g,
@@ -1486,21 +1491,19 @@ static int gram_range(mr_handle* h, int s0, int s1, int32_t* out_i32, float* out
                           cudaMemcpyDeviceToHost, h->stream);
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) { free_list(tmp); return fail(h, MR_ERR_CUDA, "gram rows copy-out: %s", cudaGetErrorString(e)); }
+    if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "gram rows copy-out: %s", cudaGetErrorString(e));
   }
-  free_list(tmp);
   return MR_OK;
 }
 
 int mr_gram_rows_device(mr_handle* h, int s0, int s1, int32_t** dev_out, int64_t* ld) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
+  int rc = require_loaded(h);
+  if (rc) return rc;
   if (!dev_out || !ld) return fail(h, MR_ERR_BAD_ARG, "null output");
-  MR_CUDA(h, cudaSetDevice(h->device));
   if (h->windowed) return fail(h, MR_ERR_STATE, "Gram rows are not available on a handle with a song window (its song ids are rotated)");
   if (s0 < 0 || s1 > h->S || s0 >= s1) return fail(h, MR_ERR_BAD_ARG, "song range [%d,%d) outside [0,%d)", s0, s1, h->S);
   const int n = s1 - s0;
-  int rc = ensure_gram_ws(h, n);
-  if (rc) return rc;
+  if ((rc = ensure_gram_ws(h, n))) return rc;
   int* d_ids = nullptr;
   if ((rc = slot_alloc(h, mr_handle::SL_GRAM_IDS, &d_ids, static_cast<size_t>(n)))) return rc;
   iota_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(d_ids, s0, n);
@@ -1581,23 +1584,17 @@ int mr_sync(mr_handle* h) {
 }
 
 static int gram_rows_scatter_impl(mr_handle* h, int s0, int s1, void* const* slot_ptrs, int n_owners, int rows_per_owner, int64_t ld, bool sync) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
+  int rc = require_loaded(h);
+  if (rc) return rc;
   if (h->engine != MR_ENGINE_TENSOR) return fail(h, MR_ERR_STATE, "mr_gram_rows_scatter needs the tensor engine (the scatter is the GEMM epilogue)");
-  MR_CUDA(h, cudaSetDevice(h->device));
   if (h->windowed) return fail(h, MR_ERR_STATE, "Gram rows are not available on a handle with a song window (its song ids are rotated)");
   if (s0 < 0 || s1 > h->S || s0 >= s1) return fail(h, MR_ERR_BAD_ARG, "song range [%d,%d) outside [0,%d)", s0, s1, h->S);
   const int n = s1 - s0;
   if (!slot_ptrs || n_owners < 1 || n_owners > 8 || rows_per_owner < 1 || static_cast<long long>(n_owners) * rows_per_owner < n || ld < h->S)
     return fail(h, MR_ERR_BAD_ARG, "bad slot table (owners %d, rows per owner %d, ld %lld)", n_owners, rows_per_owner, static_cast<long long>(ld));
   const int rows_pad = static_cast<int>(round_up(n, 128));
-  const size_t need_a = static_cast<size_t>(rows_pad) * h->pitchT;
-  if (need_a > h->aj_bytes) {
-    uint8_t* pa; int rc = dev_alloc(h, &pa, need_a, h->allocs);
-    if (rc) return rc;
-    h->d_Aj = pa; h->aj_bytes = need_a;
-  }
+  if ((rc = slot_alloc(h, mr_handle::SL_GRAM_A, &h->d_Aj, static_cast<size_t>(rows_pad) * h->pitchT, true))) return rc;   // no G: the GEMM scatters
   int* d_ids = nullptr;
-  int rc;
   if ((rc = slot_alloc(h, mr_handle::SL_GRAM_IDS, &d_ids, static_cast<size_t>(n)))) return rc;
   iota_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(d_ids, s0, n);
   h->launches++;
@@ -1630,7 +1627,8 @@ static constexpr size_t kSimWindowBytes = 256ULL << 20;   // short-path results:
 static constexpr size_t kSimMargin = 512ULL << 20;        // device memory the long path's chunk sizing leaves free
 
 int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
+  int rc = require_loaded(h);
+  if (rc) return rc;
   if (h->windowed) return fail(h, MR_ERR_STATE, "similar songs are not available on a handle with a song window (its song ids are rotated)");
   if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k = %d outside [1, 1024]", k);
   if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
@@ -1638,9 +1636,7 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
   if (!song_ids || !out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
   for (int r = 0; r < n; ++r)
     if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "query %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
-  MR_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t st = h->stream;
-  int rc;
   int* d_ids = nullptr;
   if (!h->d_sim_sqd) {   // sqrt(d_s), correctly rounded on the device, once per handle
     double* sq = nullptr;
@@ -1708,8 +1704,8 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
     const int n_long = static_cast<int>(long_rows.size());
     const bool tensor = h->engine == MR_ENGINE_TENSOR;
     const size_t ws_row = static_cast<size_t>(h->ldg) * sizeof(int32_t) + (tensor ? static_cast<size_t>(h->pitchT) : 0);
-    long long have = static_cast<long long>(h->g_bytes / (static_cast<size_t>(h->ldg) * sizeof(int32_t)));   // rows the workspace holds already
-    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->aj_bytes / h->pitchT));
+    long long have = static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_G] / (static_cast<size_t>(h->ldg) * sizeof(int32_t)));   // rows the workspace holds already
+    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_A] / h->pitchT));
     size_t free_b = 0, total_b = 0;
     MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
     const long long grow = static_cast<long long>((free_b > kSimMargin ? free_b - kSimMargin : 0) / (ws_row + row_bytes)) / 128 * 128;
@@ -1773,24 +1769,23 @@ static int score_subset(mr_handle* h, int model, const int32_t* ids, int n, doub
     if (ids[i] < first || ids[i] >= limit) return fail(h, MR_ERR_BAD_ARG, "%s id %d out of range [%d,%d)", songs ? "song" : "test user", ids[i], first, limit);
   if (n == 0) return MR_OK;
   if ((rc = slot_alloc(h, mr_handle::SL_DENSE, &h->d_dense, static_cast<size_t>(std::min(h->batch_rows, kDenseChunk)) * h->n_cols))) return rc;
-  std::vector<void*> tmp;
+  Scratch tmp(h, h->stream);
   DenseOut dout{songs ? DenseOut::SONGS : DenseOut::USERS, out, ids, n, nullptr, nullptr};
   if (songs) {
     int* d_ids = nullptr;
     std::vector<int> cols(ids, ids + n);
     for (int& c : cols) c -= h->win_lo;
-    if ((rc = dev_upload(h, &d_ids, cols.data(), static_cast<size_t>(n), tmp)) || (rc = dev_alloc(h, &dout.d_out, static_cast<size_t>(n) * h->U, tmp))) { free_list(tmp); return rc; }
+    if ((rc = tmp.upload(&d_ids, cols.data(), static_cast<size_t>(n))) || (rc = tmp.alloc(&dout.d_out, static_cast<size_t>(n) * h->U))) return rc;
     dout.d_ids = d_ids;
   }
   Run run{ModelSet(model), Consumer::DENSE, 0, &dout};
-  rc = run_batches(h, run);
-  if (!rc && songs) {
+  if ((rc = run_batches(h, run))) return rc;
+  if (songs) {
     cudaError_t e = cudaMemcpyAsync(out, dout.d_out, static_cast<size_t>(n) * h->U * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) rc = fail(h, MR_ERR_CUDA, "mr_score_songs copy-out: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_score_songs copy-out: %s", cudaGetErrorString(e));
   }
-  free_list(tmp);
-  return rc;
+  return MR_OK;
 }
 
 int mr_score_users(mr_handle* h, int model, const int32_t* user_idx, int n, double* out_nxS) { return score_subset(h, model, user_idx, n, out_nxS, false); }
@@ -1801,29 +1796,24 @@ int mr_map_at_k(mr_handle* h, int k, const int32_t* top_song, const int32_t* top
   if (!h || !h->stream) return MR_ERR_STATE;
   if (k < 1 || n_users <= 0 || !lab_rowptr || !out_map) return fail(h, MR_ERR_BAD_ARG, "null / empty arguments");
   if ((top_song == nullptr) != (top_len == nullptr)) return fail(h, MR_ERR_BAD_ARG, "top_song and top_len must both be given or both be null");
+  int rc = check_csr(h, "label", n_users, INT_MAX, lab_rowptr, lab_col);   // song ids are only compared: any id >= 0 is in range
+  if (rc) return rc;
   const long long n_lab = lab_rowptr[n_users];
-  if (lab_rowptr[0] != 0 || n_lab < 0 || (n_lab > 0 && !lab_col)) return fail(h, MR_ERR_BAD_ARG, "bad label CSR");
-  for (int u = 0; u < n_users; ++u) {
-    if (lab_rowptr[u + 1] < lab_rowptr[u]) return fail(h, MR_ERR_BAD_ARG, "label rowptr not monotone at row %d", u);
-    for (long long i = lab_rowptr[u] + 1; i < lab_rowptr[u + 1]; ++i)
-      if (lab_col[i] <= lab_col[i - 1]) return fail(h, MR_ERR_BAD_ARG, "label row %d not ascending/unique", u);
-  }
   MR_CUDA(h, cudaSetDevice(h->device));
   const int* d_song = nullptr; const int* d_len = nullptr;
-  std::vector<void*> tmp;
-  int rc;
+  Scratch tmp(h, h->stream);
   if (!top_song) {   // rank the device-resident result of the last mr_topk_device / mr_topk
     if (!h->have_topk || h->out_k != k || n_users != h->U) return fail(h, MR_ERR_STATE, "no top-%d result of %d users on the device", k, n_users);
     d_song = h->out.song; d_len = h->out.len;
   } else {
     int *ds = nullptr, *dl = nullptr;
-    if ((rc = dev_upload(h, &ds, top_song, static_cast<size_t>(n_users) * k, tmp)) || (rc = dev_upload(h, &dl, top_len, static_cast<size_t>(n_users), tmp))) { free_list(tmp); return rc; }
+    if ((rc = tmp.upload(&ds, top_song, static_cast<size_t>(n_users) * k)) || (rc = tmp.upload(&dl, top_len, static_cast<size_t>(n_users)))) return rc;
     d_song = ds; d_len = dl;
   }
   std::vector<long long> lp(lab_rowptr, lab_rowptr + n_users + 1);
   long long* d_lp = nullptr; int* d_lc = nullptr; double* d_ap = nullptr;
-  if ((rc = dev_upload(h, &d_lp, lp.data(), lp.size(), tmp)) || (rc = dev_upload(h, &d_lc, lab_col, static_cast<size_t>(n_lab), tmp)) ||
-      (rc = dev_alloc(h, &d_ap, static_cast<size_t>(n_users), tmp))) { free_list(tmp); return rc; }
+  if ((rc = tmp.upload(&d_lp, lp.data(), lp.size())) || (rc = tmp.upload(&d_lc, lab_col, static_cast<size_t>(n_lab))) ||
+      (rc = tmp.alloc(&d_ap, static_cast<size_t>(n_users)))) return rc;
   int lrc;
   {
     PhaseTimer t(h, MR_T_OTHER);
@@ -1833,7 +1823,6 @@ int mr_map_at_k(mr_handle* h, int k, const int32_t* top_song, const int32_t* top
   std::vector<double> ap(n_users);
   cudaError_t e = lrc ? cudaErrorLaunchFailure : cudaMemcpyAsync(ap.data(), d_ap, static_cast<size_t>(n_users) * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  free_list(tmp);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_map_at_k: %s", cudaGetErrorString(e));
   double total = 0.0; long long n_eval = 0;
   for (int u = 0; u < n_users; ++u) {
@@ -1869,9 +1858,9 @@ int mr_set_option(mr_handle* h, int option, int64_t value) {
 }
 
 int mr_invalidate_prepared(mr_handle* h) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
-  cudaError_t e = cudaSetDevice(h->device);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  const int rc = require_loaded(h);
+  if (rc) return rc;
+  const cudaError_t e = cudaStreamSynchronize(h->stream);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_invalidate_prepared: %s", cudaGetErrorString(e));
   if (h->head_pending) { cudaEventSynchronize(h->ev_pre); h->head_pending = false; }   // a build in flight is abandoned once it has drained
   h->head_ready = false; h->n_ex = 0; ++h->gen;
@@ -1888,9 +1877,9 @@ int mr_blend_dense(mr_handle* h, int kind, double param, uint64_t seed, const do
   if (rc) return rc;
   if (n_pairs == 0) return MR_OK;
   MR_CUDA(h, cudaSetDevice(h->device));
-  std::vector<void*> tmp;
+  Scratch tmp(h, h->stream);
   double *du = nullptr, *di = nullptr, *dout = nullptr;
-  if ((rc = dev_alloc(h, &du, n_pairs, tmp)) || (rc = dev_alloc(h, &di, n_pairs, tmp)) || (rc = dev_alloc(h, &dout, n_pairs, tmp))) { free_list(tmp); return rc; }
+  if ((rc = tmp.alloc(&du, n_pairs)) || (rc = tmp.alloc(&di, n_pairs)) || (rc = tmp.alloc(&dout, n_pairs))) return rc;
   cudaError_t e = cudaMemcpyAsync(du, ubm, n_pairs * sizeof(double), cudaMemcpyHostToDevice, h->stream);
   if (e == cudaSuccess) e = cudaMemcpyAsync(di, ibm, n_pairs * sizeof(double), cudaMemcpyHostToDevice, h->stream);
   if (e == cudaSuccess) {
@@ -1901,7 +1890,6 @@ int mr_blend_dense(mr_handle* h, int kind, double param, uint64_t seed, const do
   }
   if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, n_pairs * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  free_list(tmp);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_blend_dense: %s", cudaGetErrorString(e));
   return MR_OK;
 }
@@ -1913,21 +1901,19 @@ int mr_evaluate_dense(mr_handle* h, const double* scores_UxS, int n_users, int n
   if (n_thresholds != 10 && n_thresholds != 11) return fail(h, MR_ERR_BAD_ARG, "n_thresholds must be 10 (MR:590) or 11 (DIST:395)");
   const long long n_lab = lab_rowptr[n_users];
   if (n_lab <= 0 || !lab_col) return fail(h, MR_ERR_BAD_ARG, "empty label set");
-  for (int u = 0; u < n_users; ++u)
-    for (long long i = lab_rowptr[u] + 1; i < lab_rowptr[u + 1]; ++i)
-      if (lab_col[i] <= lab_col[i - 1]) return fail(h, MR_ERR_BAD_ARG, "label row %d not ascending/unique", u);
+  int rc = check_csr(h, "label", n_users, INT_MAX, lab_rowptr, lab_col);   // eval_ap_kernel scores only ids < n_songs
+  if (rc) return rc;
   MR_CUDA(h, cudaSetDevice(h->device));
   std::vector<int> new_songs(lab_col, lab_col + n_lab);                       // newSongs = distinct label songs (MR:72, 79)
   std::sort(new_songs.begin(), new_songs.end());
   new_songs.erase(std::unique(new_songs.begin(), new_songs.end()), new_songs.end());
   const int n_new = static_cast<int>(new_songs.size());
   std::vector<long long> lp(lab_rowptr, lab_rowptr + n_users + 1);
-  std::vector<void*> tmp;
+  Scratch tmp(h, h->stream);
   double *d_scores = nullptr, *d_ap = nullptr; long long* d_lp = nullptr; int *d_lc = nullptr, *d_new = nullptr; unsigned long long* d_mm = nullptr;
-  int rc;
-  if ((rc = dev_upload(h, &d_scores, scores_UxS, static_cast<size_t>(n_users) * n_songs, tmp)) || (rc = dev_upload(h, &d_lp, lp.data(), lp.size(), tmp)) ||
-      (rc = dev_upload(h, &d_lc, lab_col, static_cast<size_t>(n_lab), tmp)) || (rc = dev_upload(h, &d_new, new_songs.data(), new_songs.size(), tmp)) ||
-      (rc = dev_alloc(h, &d_ap, static_cast<size_t>(n_new), tmp)) || (rc = dev_alloc(h, &d_mm, 2, tmp))) { free_list(tmp); return rc; }
+  if ((rc = tmp.upload(&d_scores, scores_UxS, static_cast<size_t>(n_users) * n_songs)) || (rc = tmp.upload(&d_lp, lp.data(), lp.size())) ||
+      (rc = tmp.upload(&d_lc, lab_col, static_cast<size_t>(n_lab))) || (rc = tmp.upload(&d_new, new_songs.data(), new_songs.size())) ||
+      (rc = tmp.alloc(&d_ap, static_cast<size_t>(n_new))) || (rc = tmp.alloc(&d_mm, 2))) return rc;
   int lrc;
   {
     PhaseTimer t(h, MR_T_OTHER);
@@ -1937,7 +1923,6 @@ int mr_evaluate_dense(mr_handle* h, const double* scores_UxS, int n_users, int n
   std::vector<double> ap(n_new);
   cudaError_t e = lrc ? cudaErrorLaunchFailure : cudaMemcpyAsync(ap.data(), d_ap, n_new * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  free_list(tmp);
   if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_evaluate_dense: %s", cudaGetErrorString(e));
   double total = 0.0;
   for (int c = 0; c < n_new; ++c) total += ap[c];                              // foldLeft(0.0)(_+_), MR:626
@@ -2095,13 +2080,8 @@ int eval_counts_impl(mr_handle* h, int n, const int* models, const double* param
   if (rc) return rc;
   hs.mark("set");
   const int U = h->U;
+  if ((rc = check_csr(h, "label", U, INT_MAX, lab_rowptr, lab_col))) return rc;   // ids beyond the songs are checked against new_songs below
   const long long n_lab = lab_rowptr[U];
-  if (lab_rowptr[0] != 0 || n_lab < 0 || (n_lab > 0 && !lab_col)) return fail(h, MR_ERR_BAD_ARG, "bad label CSR");
-  for (int u = 0; u < U; ++u) {
-    if (lab_rowptr[u + 1] < lab_rowptr[u]) return fail(h, MR_ERR_BAD_ARG, "label rowptr not monotone at row %d", u);
-    for (long long i = lab_rowptr[u]; i < lab_rowptr[u + 1]; ++i)
-      if (lab_col[i] < 0 || (i > lab_rowptr[u] && lab_col[i] <= lab_col[i - 1])) return fail(h, MR_ERR_BAD_ARG, "label row %d not ascending/unique", u);
-  }
   if (new_songs[0] < 0) return fail(h, MR_ERR_BAD_ARG, "new_songs: negative song id");
   for (int i = 1; i < n_new; ++i)
     if (new_songs[i] <= new_songs[i - 1]) return fail(h, MR_ERR_BAD_ARG, "new_songs not strictly ascending at %d", i);
@@ -2392,18 +2372,15 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
-  cudaError_t e = cudaSetDevice(h->device);
-  if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
+  const int rc = require_loaded(h);
+  if (rc) return rc;
   return start_head_rows(h, h->pre_stream);
 }
 
 int mr_prepare(mr_handle* h) {
-  if (!h || !h->loaded) return fail(h, MR_ERR_STATE, "mr_load has not succeeded on this handle");
-  cudaError_t e = cudaSetDevice(h->device);
-  if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "cudaSetDevice: %s", cudaGetErrorString(e));
-  int rc = ensure_head_rows(h);
+  int rc = require_loaded(h);
   if (rc) return rc;
+  if ((rc = ensure_head_rows(h))) return rc;
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   return MR_OK;
 }

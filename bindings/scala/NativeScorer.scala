@@ -34,6 +34,8 @@ trait MrScore extends Library {
                     outSong: Pointer, outScore: Pointer, outLen: Pointer): Int
   // songs like each query song: the k co-listened songs of highest item-item cosine (MusicRecommender.scala:230-239), [n][k] / [n]
   def mr_similar_songs(h: Pointer, songIds: Array[Int], n: Int, k: Int, outSong: Array[Int], outScore: Array[Double], outLen: Array[Int]): Int
+  // listeners like each query test user (indices into the current shard): the k train users of highest user-user cosine (MR:140-149)
+  def mr_similar_users(h: Pointer, userIdx: Array[Int], n: Int, k: Int, outUser: Array[Int], outScore: Array[Double], outLen: Array[Int]): Int
   def mr_ingest_tsv(device: Int, train: Array[Byte], trainLen: Long, test: Array[Byte], testLen: Long, labels: Array[Byte],
                     labelsLen: Long, out: PointerByReference): Int
   def mr_ingest_error(g: Pointer): String

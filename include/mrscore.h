@@ -237,6 +237,22 @@ int mr_eval_counts_multi(mr_handle* h, int n_models, const int* models, const do
  * fits in the free device memory. */
 int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len);
 
+/* ---- similar users: the reference's user-user cosine ranked per test user (DESIGN.md §4.8) -----------------------------------------------
+ * For each query u = user_idx[r] (indices into the CURRENT test shard, as mr_score_users: any order, duplicates allowed), the k train users v
+ * with the highest
+ *   w(u, v) = c / (sqrt((double) deg_test[u]) * sqrt((double) deg_train[v]))      (cosineSimilarity, MR:140-149)
+ * with c = |I_u ∩ I_v| over u's visible test row and v's train row, and the degrees as handed to mr_load / mr_set_test_users (MR:147),
+ * evaluated in that operation order with correctly rounded steps: every score has the bits of the CPU formula (the weight UBM sums, MR:159-166).
+ * Candidates are the train users with c > 0 only: a train user who shares no song with u is never listed.  Order: score descending, then
+ * train-user id ascending.  Outputs (host arrays): out_user / out_score [n][k], out_len [n]; row r belongs to user_idx[r]; out_len[r] =
+ * min(k, #candidates), user -1 / score 0.0 past it.  A test user with an empty visible row gets out_len 0.  1 <= k <= 1024; n = 0 returns
+ * MR_OK.  MR_ERR_BAD_ARG names the first query index outside [0, U); MR_ERR_STATE before mr_load and without test users.
+ * Works on a handle with a song window and gives the same lists there (user ids are not rotated; the handle keeps whole rows).
+ * Paths, phase timers and chunking as mr_similar_songs; mr_get_info values 23 / 24 count the rows each path answered.  The call leaves
+ * every result and resident state of the scoring calls as it was and returns with all its work complete.  MR_ERR_OOM, stating the bytes,
+ * when not even one chunk of count rows fits in the free device memory. */
+int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_t* out_user, double* out_score, int32_t* out_len);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -311,7 +327,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  top-k select since mr_load: rows its sampled fast path handed to the exact path, short rows
                                                                  (exact path by design), degenerate rows (radix select),
                                                                  scoring passes since mr_load (batches whose score panels were built),
-                                                                 mr_similar_songs rows since mr_load: answered by the short path, by the long path] */
+                                                                 mr_similar_songs rows since mr_load: answered by the short path, by the long path,
+                                                                 mr_similar_users rows since mr_load: answered by the short path, by the long path] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

@@ -1,17 +1,20 @@
-// k8_similar.cu — similar songs: the exact top-k of the reference's item-item cosine (MusicRecommender.scala:230-239) for a list of
-// query songs (mr_similar_songs, DESIGN.md §4.7).
+// k8_similar.cu — the exact top-k of the reference's two cosines for a list of queries (DESIGN.md §4.7, §4.8):
+//   similar songs (mr_similar_songs):  sim(i, s) = g(i, s) / (sqrt((double) d_i) * sqrt((double) d_s))   g = |U_i^train ∩ U_s^train| (MR:232),
+//                                      d = deg_song_all (MR:237); candidates s != i
+//   similar users (mr_similar_users):  w(u, v) = c(u, v) / (sqrt((double) |I_u|) * sqrt((double) |I_v|))   c = |I_u^test ∩ I_v^train| (MR:142-145),
+//                                      the degrees as handed to mr_load / mr_set_test_users (MR:147); candidates are train users v
+// in the operation order of the CPU formula (the reference's cosineSimilarity, MR:147-148 and MR:237-238), every step correctly rounded
+// (__dsqrt_rn, __dmul_rn, __ddiv_rn; the library is built with --fmad=false), so every score has the bits of the CPU formula.  Candidates
+// have a count > 0; order: score descending, then candidate id ascending — the composite key (score bits : 64, ~id : 32) of k3_topk.cu.
 //
-//   sim(i, s) = g(i, s) / (sqrt((double) d_i) * sqrt((double) d_s))        g = |U_i^train ∩ U_s^train| (MR:232), d = deg_song_all (MR:237)
-//
-// in the operation order of the CPU formula (the reference's cosineSimilarity, MR:237-238), every step correctly rounded (__dsqrt_rn, __dmul_rn,
-// __ddiv_rn; the library is built with --fmad=false), so every score has the bits of the CPU formula.  Candidates are the co-listened songs
-// (g > 0) other than i; order: score descending, then song id ascending — the composite key (score bits : 64, ~song : 32) of k3_topk.cu.
-//
-// The work of query i is E_i = sum over its train listeners v of |I_v^train| events.  Two row paths:
-//   short rows (E_i <= kSimShortMax): one CTA per query gathers the co-listened song ids into shared memory, sorts them, run-lengths them
-//     into (s, g), scores each distinct s and sorts the candidates by key; the row never touches HBM and no global atomics are used;
-//   long rows: exact int32 count rows from the count engines (mrscore.cu gram_rows), then similar_row_topk_kernel, one CTA per row: the
+// Both query kinds are one two-level walk (SimLists): query q -> its items q_idx[q_ptr[q] .. q_ptr[q + 1]) -> the candidates of each item
+// c_idx[c_ptr[j] .. c_ptr[j + 1]).  Songs: song -> train listeners (inverted index) -> their train histories.  Users: test user -> visible
+// songs -> train listeners.  The work of query q is E_q = the number of (item, candidate) events.  Two row paths:
+//   short rows (E_q <= kSimShortMax): one CTA per query gathers the candidate ids into shared memory, sorts them, run-lengths them into
+//     (id, count), scores each distinct id and sorts the candidates by key; the row never touches HBM and no global atomics are used;
+//   long rows: exact int32 count rows from the count engines (mrscore.cu count_rows), then similar_row_topk_kernel, one CTA per row: the
 //     exact path of topk_kernel (maximum, linear histogram, bin of the k-th key, MSD radix select inside a crowded bin, collect, bitonic sort).
+// kSelf: similar songs exclude the query song from its own list; a train user is never the test user asking, so similar users exclude none.
 #include <climits>
 
 #include "mr_common.cuh"
@@ -21,7 +24,7 @@ namespace mr {
 
 __device__ __forceinline__ double sim_score(int g, double sq_i, double sq_s) {
   const double den = __dmul_rn(sq_i, sq_s);
-  return den != 0.0 ? __ddiv_rn(static_cast<double>(g), den) : 0.0;   // naive_ibm_cos: denominator != 0 ? numerator / denominator : 0
+  return den != 0.0 ? __ddiv_rn(static_cast<double>(g), den) : 0.0;   // naive_*_cos: denominator != 0 ? numerator / denominator : 0
 }
 
 __device__ __forceinline__ unsigned long long key_bits(double x) { return static_cast<unsigned long long>(__double_as_longlong(x)); }
@@ -70,50 +73,50 @@ int launch_sqrt_deg(const int* deg, int n, double* out, cudaStream_t st) {
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
-// E_i of every query, one warp per query
-__global__ void sim_events_kernel(const int* __restrict__ songs, int n, const long long* __restrict__ csc_ptr, const int* __restrict__ csc_idx,
-                                  const long long* __restrict__ tr_ptr, long long* __restrict__ events) {
+// E_q of every query, one warp per query
+__global__ void sim_events_kernel(const int* __restrict__ ids, int n, const long long* __restrict__ q_ptr, const int* __restrict__ q_idx,
+                                  const long long* __restrict__ c_ptr, long long* __restrict__ events) {
   const int q = static_cast<int>((blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x) >> 5), lane = threadIdx.x & 31;
   if (q >= n) return;
-  const int i = songs[q];
+  const int i = ids[q];
   long long e = 0;
-  for (long long l = csc_ptr[i] + lane; l < csc_ptr[i + 1]; l += 32) { const int v = csc_idx[l]; e += tr_ptr[v + 1] - tr_ptr[v]; }
+  for (long long l = q_ptr[i] + lane; l < q_ptr[i + 1]; l += 32) { const int j = q_idx[l]; e += c_ptr[j + 1] - c_ptr[j]; }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
   if (lane == 0) events[q] = e;
 }
 
-int launch_sim_events(const int* songs, int n, const long long* csc_ptr, const int* csc_idx, const long long* tr_ptr, long long* events,
-                      cudaStream_t st) {
+int launch_sim_events(const int* ids, int n, const SimLists& l, long long* events, cudaStream_t st) {
   if (n <= 0) return 0;
-  sim_events_kernel<<<(n + 7) / 8, 256, 0, st>>>(songs, n, csc_ptr, csc_idx, tr_ptr, events);
+  sim_events_kernel<<<(n + 7) / 8, 256, 0, st>>>(ids, n, l.q_ptr, l.q_idx, l.c_ptr, events);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
 // ---------------------------------------------------------------- short rows: one CTA per query, everything in shared memory
-// Dynamic shared memory: key u64[cap] | ids i32[cap], cap a power of two >= E_i of every query of the launch (12 * cap bytes).
+// Dynamic shared memory: key u64[cap] | ids i32[cap], cap a power of two >= E_q of every query of the launch (12 * cap bytes).
 // Positions per thread (cap / blockDim.x) must be <= 32: the candidate flags of a thread live in one register mask.
-__global__ void similar_short_kernel(const int* __restrict__ q_song, const int* __restrict__ q_row, int cap, const long long* __restrict__ csc_ptr,
-                                     const int* __restrict__ csc_idx, const long long* __restrict__ tr_ptr, const int* __restrict__ tr_col,
-                                     const double* __restrict__ sqd, int k, int* __restrict__ out_song, double* __restrict__ out_score,
-                                     int* __restrict__ out_len) {
+template <bool kSelf>
+__global__ void similar_short_kernel(const int* __restrict__ q_ids, const int* __restrict__ q_row, int cap, const long long* __restrict__ q_ptr,
+                                     const int* __restrict__ q_idx, const long long* __restrict__ c_ptr, const int* __restrict__ c_idx,
+                                     const double* __restrict__ sq_q, const double* __restrict__ sq_c, int k, int* __restrict__ out_song,
+                                     double* __restrict__ out_score, int* __restrict__ out_len) {
   extern __shared__ unsigned long long s_dyn[];
   unsigned long long* s_key = s_dyn;
   int* s_ids = reinterpret_cast<int*>(s_dyn + cap);
   __shared__ int s_n, s_cand;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, n_warps = blockDim.x >> 5;
-  const int i = q_song[blockIdx.x], row = q_row[blockIdx.x];
+  const int i = q_ids[blockIdx.x], row = q_row[blockIdx.x];
   if (tid == 0) { s_n = 0; s_cand = 0; }
   __syncthreads();
-  // gather the train histories of i's train listeners, one warp per listener
-  for (long long l = csc_ptr[i] + warp; l < csc_ptr[i + 1]; l += n_warps) {
-    const int v = csc_idx[l];
-    const long long b = tr_ptr[v];
-    const int len = static_cast<int>(tr_ptr[v + 1] - b);
+  // gather the candidate lists of i's items, one warp per item (songs: the train histories of i's train listeners)
+  for (long long l = q_ptr[i] + warp; l < q_ptr[i + 1]; l += n_warps) {
+    const int j = q_idx[l];
+    const long long b = c_ptr[j];
+    const int len = static_cast<int>(c_ptr[j + 1] - b);
     int base = 0;
     if (lane == 0) base = atomicAdd(&s_n, len);
     base = __shfl_sync(0xffffffffu, base, 0);
-    for (int m = lane; m < len; m += 32) s_ids[base + m] = __ldg(tr_col + b + m);
+    for (int m = lane; m < len; m += 32) s_ids[base + m] = __ldg(c_idx + b + m);
   }
   __syncthreads();
   const int n = s_n;
@@ -121,16 +124,16 @@ __global__ void similar_short_kernel(const int* __restrict__ q_song, const int* 
   while (n_pad < n) n_pad <<= 1;
   for (int p = n + tid; p < n_pad; p += blockDim.x) s_ids[p] = INT_MAX;
   bitonic_ints(s_ids, n_pad);
-  // run-length: the first position of each run of equal ids is a candidate (s, g = run length) unless s == i
-  const double sq_i = sqd[i];
+  // run-length: the first position of each run of equal ids is a candidate (s, g = run length), unless kSelf and s == i
+  const double sq_i = sq_q[i];
   uint32_t cand = 0;
   int n_mine = 0;
   for (int p = tid, j = 0; p < n; p += blockDim.x, ++j) {
     const int s = s_ids[p];
-    if (s == i || (p > 0 && s_ids[p - 1] == s)) continue;
+    if ((kSelf && s == i) || (p > 0 && s_ids[p - 1] == s)) continue;
     int lo = p + 1, hi = n;                       // end of the run: first position with a larger id
     while (lo < hi) { const int m = (lo + hi) >> 1; if (s_ids[m] <= s) lo = m + 1; else hi = m; }
-    s_key[p] = key_bits(sim_score(lo - p, sq_i, __ldg(sqd + s)));
+    s_key[p] = key_bits(sim_score(lo - p, sq_i, __ldg(sq_c + s)));
     cand |= 1u << j;
     ++n_mine;
   }
@@ -150,8 +153,8 @@ __global__ void similar_short_kernel(const int* __restrict__ q_song, const int* 
   if (tid == 0) out_len[row] = need;
 }
 
-int launch_similar_short(const int* q_song, const int* q_row, int n_q, int cap, const long long* csc_ptr, const int* csc_idx, const long long* tr_ptr,
-                         const int* tr_col, const double* sqd, int k, int* out_song, double* out_score, int* out_len, cudaStream_t st) {
+int launch_similar_short(const int* q_ids, const int* q_row, int n_q, int cap, const SimLists& l, int k, int* out_song, double* out_score,
+                         int* out_len, cudaStream_t st) {
   if (n_q <= 0) return 0;
   if (cap < 64 || cap > kSimShortMax || (cap & (cap - 1))) return -2;
   const int threads = cap <= 1024 ? 128 : 256;
@@ -159,8 +162,9 @@ int launch_similar_short(const int* q_song, const int* q_row, int n_q, int cap, 
   const size_t smem = static_cast<size_t>(cap) * 12;
   // the attribute is per device (handles may live on several GPUs of one process); setting it is cheap, so no caching.  Always set: the
   // 48 KB default counts the static shared memory too, which the 4 k class (48 KB dynamic) already exceeds
-  if (cudaFuncSetAttribute(similar_short_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSimShortMax * 12) != cudaSuccess) return -3;
-  similar_short_kernel<<<n_q, threads, smem, st>>>(q_song, q_row, cap, csc_ptr, csc_idx, tr_ptr, tr_col, sqd, k, out_song, out_score, out_len);
+  auto kern = l.self ? similar_short_kernel<true> : similar_short_kernel<false>;
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSimShortMax * 12) != cudaSuccess) return -3;
+  kern<<<n_q, threads, smem, st>>>(q_ids, q_row, cap, l.q_ptr, l.q_idx, l.c_ptr, l.c_idx, l.sq_q, l.sq_c, k, out_song, out_score, out_len);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
@@ -170,8 +174,8 @@ constexpr int kSimCap = 2048;     // candidate buffer, bitonic-sorted in shared 
 constexpr int kSimBins = 2048;
 
 // f(song, key bits, candidate) for 4 songs per thread per step, the same number of times by every thread (f may use warp collectives)
-template <class F>
-__device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n_songs, int self, double sq_i, const double* __restrict__ sqd, F&& f) {
+template <bool kSelf, class F>
+__device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n_songs, int self, double sq_i, const double* __restrict__ sq_c, F&& f) {
   for (int base0 = 0; base0 < n_songs; base0 += 4 * kSimThreads) {
     const int s = base0 + 4 * static_cast<int>(threadIdx.x);
     int4 v = make_int4(0, 0, 0, 0);
@@ -179,16 +183,18 @@ __device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n
     const int c[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
-      const bool ok = s + t < n_songs && c[t] > 0 && s + t != self;
-      const unsigned long long kb = ok ? key_bits(sim_score(c[t], sq_i, __ldg(sqd + s + t))) : 0ULL;
+      const bool ok = s + t < n_songs && c[t] > 0 && (!kSelf || s + t != self);
+      const unsigned long long kb = ok ? key_bits(sim_score(c[t], sq_i, __ldg(sq_c + s + t))) : 0ULL;
       f(s + t, kb, ok);
     }
   }
 }
 
+template <bool kSelf>
 __global__ void __launch_bounds__(kSimThreads, 2)
 similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t* __restrict__ g, long long ldg, int n_songs,
-                        const double* __restrict__ sqd, int k, int* __restrict__ out_song, double* __restrict__ out_score, int* __restrict__ out_len) {
+                        const double* __restrict__ sq_q, const double* __restrict__ sq_c, int k, int* __restrict__ out_song,
+                        double* __restrict__ out_score, int* __restrict__ out_len) {
   __shared__ unsigned long long s_key[kSimCap];
   __shared__ int s_song[kSimCap];
   __shared__ int s_hist[kSimBins];
@@ -199,7 +205,7 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
   if (r >= n_rows) return;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int self = rows[r];
-  const double sq_i = sqd[self];
+  const double sq_i = sq_q[self];
   const int32_t* row = g + static_cast<long long>(r) * ldg;
   int* o_song = out_song + static_cast<long long>(r) * k;
   double* o_score = out_score + static_cast<long long>(r) * k;
@@ -207,7 +213,7 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
   if (tid == 0) { s_valid = 0; s_count = 0; }
   __syncthreads();
   unsigned long long mx = 0; int nv = 0;
-  scan_counts(row, n_songs, self, sq_i, sqd, [&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
+  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xffffffffu, mx, o); mx = other > mx ? other : mx; nv += __shfl_xor_sync(0xffffffffu, nv, o); }
   if (lane == 0) { s_max[warp] = mx; atomicAdd(&s_valid, nv); }
@@ -228,7 +234,7 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
     return static_cast<uint32_t>(d > kSimBins - 1 ? kSimBins - 1 : d);
   };
   // ---- linear histogram of the candidates, then the bin holding the need-th best key (warp 0, suffix search)
-  scan_counts(row, n_songs, self, sq_i, sqd, [&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
+  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
   __syncthreads();
   if (warp == 0) {
     int part = 0;
@@ -255,7 +261,7 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
       __syncthreads();
       for (int i = tid; i < 256; i += kSimThreads) s_hist[i] = 0;
       __syncthreads();
-      scan_counts(row, n_songs, self, sq_i, sqd, [&](int s, unsigned long long kb, bool ok) {
+      scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int s, unsigned long long kb, bool ok) {
         const uint32_t inv = ~static_cast<uint32_t>(s);
         ok = ok && bin_of(kb) == cbin && prefix_cmp(kb, inv, phi, plo, nd) == 0;
         hist_add(s_hist, ok ? key_digit(kb, inv, nd) : 0u, ok, lane);
@@ -281,7 +287,7 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
   }
   // ---- collect every key in a higher bin, plus the keys of bin cbin at or above the radix prefix
   __syncthreads();
-  scan_counts(row, n_songs, self, sq_i, sqd, [&](int s, unsigned long long kb, bool ok) {
+  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int s, unsigned long long kb, bool ok) {
     if (ok) {
       const uint32_t bn = bin_of(kb);
       ok = bn > cbin || (bn == cbin && prefix_cmp(kb, ~static_cast<uint32_t>(s), phi, plo, nd) >= 0);
@@ -310,11 +316,12 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
   if (tid == 0) out_len[r] = need;
 }
 
-int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_songs, const double* sqd, int k, int* out_song,
+int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_cols, const SimLists& l, int k, int* out_song,
                         double* out_score, int* out_len, cudaStream_t st) {
   if (n_rows <= 0) return 0;
   if (k <= 0 || k > kSimCap / 2) return -2;
-  similar_row_topk_kernel<<<n_rows, kSimThreads, 0, st>>>(rows, n_rows, g, ldg, n_songs, sqd, k, out_song, out_score, out_len);
+  auto kern = l.self ? similar_row_topk_kernel<true> : similar_row_topk_kernel<false>;
+  kern<<<n_rows, kSimThreads, 0, st>>>(rows, n_rows, g, ldg, n_cols, l.sq_q, l.sq_c, k, out_song, out_score, out_len);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

@@ -171,18 +171,25 @@ int launch_agg_split(const BlendParams& bp, const long long* te_ptr, const int* 
 int launch_map_at_k(const int* top_song, const int* top_len, int n_users, int k, const long long* lab_ptr, const int* lab_col,
                     double* ap_out, cudaStream_t st);
 
-// ---- similar songs (k8_similar.cu, DESIGN.md §4.7)
-// kSimShortMax: events E_i (co-listened song ids with repeats) a short row gathers into shared memory: 12 bytes each (id + sort key),
+// ---- similar songs and similar users (k8_similar.cu, DESIGN.md §4.7, §4.8)
+// kSimShortMax: events E_q (candidate ids with repeats) a short row gathers into shared memory: 12 bytes each (id + sort key),
 // 96 KB at the limit, two CTAs per SM
 constexpr int kSimShortMax = 8192;
+// A query kind: query q -> items q_idx[q_ptr[q] .. q_ptr[q + 1]) -> candidates c_idx[c_ptr[j] .. c_ptr[j + 1]) of each item j; the score of
+// (q, c) with count n is n / (sq_q[q] * sq_c[c]); self: c == q is no candidate (similar songs)
+struct SimLists {
+  const long long* q_ptr; const int* q_idx;
+  const long long* c_ptr; const int* c_idx;
+  const double* sq_q; const double* sq_c;
+  bool self;
+};
 int launch_sqrt_deg(const int* deg, int n, double* out, cudaStream_t st);
-int launch_sim_events(const int* songs, int n, const long long* csc_ptr, const int* csc_idx, const long long* tr_ptr, long long* events,
-                      cudaStream_t st);
-// cap: a power of two in [64, kSimShortMax], >= E_i of every query of the launch; query q writes row q_row[q] of the outputs ([row][k])
-int launch_similar_short(const int* q_song, const int* q_row, int n_q, int cap, const long long* csc_ptr, const int* csc_idx, const long long* tr_ptr,
-                         const int* tr_col, const double* sqd, int k, int* out_song, double* out_score, int* out_len, cudaStream_t st);
-// row r of g (count row of song rows[r], ldg apart) -> row r of the outputs
-int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_songs, const double* sqd, int k, int* out_song,
+int launch_sim_events(const int* ids, int n, const SimLists& l, long long* events, cudaStream_t st);
+// cap: a power of two in [64, kSimShortMax], >= E_q of every query of the launch; query q writes row q_row[q] of the outputs ([row][k])
+int launch_similar_short(const int* q_ids, const int* q_row, int n_q, int cap, const SimLists& l, int k, int* out_song, double* out_score,
+                         int* out_len, cudaStream_t st);
+// row r of g (count row of query rows[r] over n_cols candidates, ldg apart, padded to 32) -> row r of the outputs
+int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_cols, const SimLists& l, int k, int* out_song,
                         double* out_score, int* out_len, cudaStream_t st);
 
 }  // namespace mr

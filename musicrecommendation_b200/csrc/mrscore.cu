@@ -56,7 +56,7 @@ struct mr_handle {
   cudaStream_t slice_stream2 = nullptr; cudaEvent_t ev_join = nullptr;   // single-batch calls alternate their slices between the two slice streams
   std::string err;
   long long launches = 0; size_t dev_bytes = 0;
-  std::vector<void*> allocs;          // allocated once per handle (mr_load, the sqrt table of similar songs, peer buffers), freed in mr_destroy
+  std::vector<void*> allocs;          // allocated once per handle (mr_load, the sqrt tables of similar songs / users, peer buffers), freed in mr_destroy
   // train
   int T = 0, S = 0; long long nnz_tr = 0; bool loaded = false;
   long long *d_tr_ptr = nullptr, *d_csc_ptr = nullptr; int *d_tr_col = nullptr, *d_csc_idx = nullptr;
@@ -103,7 +103,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard, its results and the workspaces: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -128,6 +128,10 @@ struct mr_handle {
   EvalCounts ec{};                           // device state of the count pass
   // similar songs (mr_similar_songs): sqrt(deg_song_all) per song, built on the first call; rows answered by each path since mr_load
   double* d_sim_sqd = nullptr; long long sim_short_rows = 0, sim_long_rows = 0;
+  // similar users (mr_similar_users): sqrt(deg_train) per train user, built on the first call; sqrt(deg_test) per test user of the shard
+  // (slot SL_SIM_SQU), rebuilt on the first call after each mr_set_test_users; rows answered by each path since mr_load
+  std::vector<int32_t> deg_train, deg_test;
+  double *d_simu_sqt = nullptr, *d_simu_squ = nullptr; bool simu_squ_ok = false; long long simu_short_rows = 0, simu_long_rows = 0;
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -336,33 +340,48 @@ int count_ubm_batch(mr_handle* h, int b0, int nb) {
   return MR_OK;
 }
 
-// ---- K1 for a list of Gram rows (device array of song ids) -> G i32[n_rows][ldg]
-int gram_rows(mr_handle* h, const int* d_rows, int n_rows) {
+// Exact intersection-count rows of one query kind: G[r][c] = |items(rows[r]) ∩ items(c)| for the n_cols candidates c, rows ld apart, in
+// the Gram workspace.  Tensor engine: the query rows expanded to 0/1 rows of `pitch` bytes, times the candidates' dense operand B (n_cols
+// rows).  Sparse engine: the walk query -> items (q_ptr / q_idx) -> candidates (c_ptr / c_idx), one atomic per event.
+//   Gram rows (song x song):        q = inverted index, c = train rows, B = A_tr^T, pitch = pitchT, n_cols = S, ld = ldg
+//   user rows (test x train user):  q = test rows, c = inverted index, B = A_tr, pitch = pitchS, n_cols = T, ld = T padded to 32
+struct CountRows {
+  const long long* q_ptr; const int* q_idx; const long long* c_ptr; const int* c_idx;
+  const uint8_t* B; long long pitch; int n_cols; long long ld;
+};
+CountRows song_count_rows(const mr_handle* h) { return {h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_col, h->d_AtrT, h->pitchT, h->S, h->ldg}; }
+CountRows user_count_rows(const mr_handle* h) { return {h->d_te_ptr, h->d_te_col, h->d_csc_ptr, h->d_csc_idx, h->d_Atr, h->pitchS, h->T, round_up(h->T, 32)}; }
+
+int count_rows(mr_handle* h, const CountRows& cr, const int* d_rows, int n_rows) {
   if (h->engine == MR_ENGINE_TENSOR) {
     const int rows_pad = static_cast<int>(round_up(n_rows, 128));
     {
       PhaseTimer t(h, MR_T_EXPAND);
-      MR_LAUNCH(h, launch_expand_rows(h->d_csc_ptr, h->d_csc_idx, d_rows, 0, n_rows, rows_pad, h->pitchT, h->d_Aj, h->stream));
+      MR_LAUNCH(h, launch_expand_rows(cr.q_ptr, cr.q_idx, d_rows, 0, n_rows, rows_pad, cr.pitch, h->d_Aj, h->stream));
     }
     PhaseTimer t(h, MR_T_COUNT);
-    MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, h->d_AtrT, h->S, h->pitchT, n_rows, h->S, EPI_I32, h->d_g, h->ldg, nullptr,
+    MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, cr.B, cr.n_cols, cr.pitch, n_rows, cr.n_cols, EPI_I32, h->d_g, cr.ld, nullptr,
                                    nullptr, h->num_sms, h->stream));
   } else {
     PhaseTimer t(h, MR_T_COUNT);
     for (int r0 = 0; r0 < n_rows; r0 += 32768) {
       const int n = std::min(32768, n_rows - r0);
-      MR_LAUNCH(h, launch_sparse_gram_rows(d_rows + r0, n, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_col,
-                                           h->d_g + static_cast<long long>(r0) * h->ldg, h->ldg, h->stream));
+      MR_LAUNCH(h, launch_sparse_gram_rows(d_rows + r0, n, cr.q_ptr, cr.q_idx, cr.c_ptr, cr.c_idx, h->d_g + static_cast<long long>(r0) * cr.ld,
+                                           cr.ld, h->stream));
     }
   }
   return MR_OK;
 }
 
-int ensure_gram_ws(mr_handle* h, int n_rows) {
+// ---- K1 for a list of Gram rows (device array of song ids) -> G i32[n_rows][ldg]
+int gram_rows(mr_handle* h, const int* d_rows, int n_rows) { return count_rows(h, song_count_rows(h), d_rows, n_rows); }
+
+// the Gram workspace for n_rows count rows of a kind (default: Gram rows): ld ints per row, and on the tensor engine the expanded query rows
+int ensure_gram_ws(mr_handle* h, int n_rows, long long ld = 0, long long a_pitch = 0) {
   const size_t rows = static_cast<size_t>(round_up(std::max(n_rows, 1), 128));
-  const int rc = slot_alloc(h, mr_handle::SL_GRAM_G, &h->d_g, rows * h->ldg, true);
+  const int rc = slot_alloc(h, mr_handle::SL_GRAM_G, &h->d_g, rows * (ld ? ld : h->ldg), true);
   if (rc || h->engine != MR_ENGINE_TENSOR) return rc;
-  return slot_alloc(h, mr_handle::SL_GRAM_A, &h->d_Aj, rows * h->pitchT, true);
+  return slot_alloc(h, mr_handle::SL_GRAM_A, &h->d_Aj, rows * (a_pitch ? a_pitch : h->pitchT), true);
 }
 
 // Item-space: compute the rows G[h][:], Gq[h][:] of the head songs once per train set (lazily, on first use, or mr_prepare).
@@ -1142,6 +1161,7 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
   h->pitchS = round_up(S, 128); h->pitchT = round_up(T, 128);
   h->spitch = round_up(h->n_cols, 32); h->ldg = round_up(S, 32);
   h->deg_song.assign(deg_song_all, deg_song_all + S);
+  h->deg_train.assign(deg_train, deg_train + T);
   h->deg_song_train.assign(S, 0);
   for (long long i = 0; i < nnz; ++i) h->deg_song_train[tr_col[i]]++;
 
@@ -1306,6 +1326,7 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   h->have_test = false; h->have_topk = false; h->out_k = 0; h->multi_n = 0; ++h->gen;
   const int U = n_test; const long long nnz = te_rowptr[U];
   h->U = U; h->nnz_te = nnz;
+  h->deg_test.assign(deg_test, deg_test + U); h->simu_squ_ok = false;
   h->h_te_ptr.assign(te_rowptr, te_rowptr + U + 1);
   if (h->windowed) h->h_te_col.resize(static_cast<size_t>(nnz)); else h->h_te_col.assign(te_col, te_col + nnz);   // a window rewrites every row below
   std::vector<double> rsa(U); std::vector<float> rsaf(U);
@@ -1620,39 +1641,43 @@ int mr_similarity_ibm(mr_handle* h, int s0, int s1, float* out_rows) {
   return gram_range(h, s0, s1, nullptr, out_rows);
 }
 
-// ---- similar songs (DESIGN.md §4.7, k8_similar.cu).  Uses only the train replica and its own slots: the score panels, the select plane,
-// the head rows, the top-k blocks and gen stay as they are; the count rows of the long path go to the Gram workspace (ensure_gram_ws).
-static constexpr int kSimClassCap[] = {256, 1024, 4096, kSimShortMax};   // short-path launches by E_i: 12 * cap bytes of shared memory per CTA
+// ---- similar songs and similar users (DESIGN.md §4.7, §4.8, k8_similar.cu).  Both use only the train replica (and the test shard's rows)
+// and their own slots: the score panels, the select plane, the head rows, the top-k blocks and gen stay as they are; the count rows of the
+// long path go to the Gram workspace (ensure_gram_ws).
+static constexpr int kSimClassCap[] = {256, 1024, 4096, kSimShortMax};   // short-path launches by E_q: 12 * cap bytes of shared memory per CTA
 static constexpr size_t kSimWindowBytes = 256ULL << 20;   // short-path results: the query list in windows of rows whose block fits this
 static constexpr size_t kSimMargin = 512ULL << 20;        // device memory the long path's chunk sizing leaves free
 
-int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
-  int rc = require_loaded(h);
+// One query kind of the similar-items driver: the two-level lists and sqrt tables of the kernels, the count rows of the long path and
+// the counters of mr_get_info.
+struct SimKind {
+  const char* name;   // "similar songs" / "similar users", for messages
+  SimLists lists;
+  CountRows counts;
+  long long *short_rows, *long_rows;
+};
+
+// the sqrt of n degrees, correctly rounded on the device, into out (the degrees pass through the SL_SIM_IDS slot)
+static int sqrt_table(mr_handle* h, const int32_t* deg, int n, double* out) {
+  int* d_deg = nullptr;
+  const int rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_deg, deg, static_cast<size_t>(n));
   if (rc) return rc;
-  if (h->windowed) return fail(h, MR_ERR_STATE, "similar songs are not available on a handle with a song window (its song ids are rotated)");
-  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k = %d outside [1, 1024]", k);
-  if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
-  if (n == 0) return MR_OK;
-  if (!song_ids || !out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
-  for (int r = 0; r < n; ++r)
-    if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "query %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
+  MR_LAUNCH(h, launch_sqrt_deg(d_deg, n, out, h->stream));
+  return MR_OK;
+}
+
+// The query ids are checked by the caller.  E_q of every query is read back to split the queries into short and long rows.
+static int similar_lists(mr_handle* h, const SimKind& kind, const int32_t* ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
   cudaStream_t st = h->stream;
+  int rc;
   int* d_ids = nullptr;
-  if (!h->d_sim_sqd) {   // sqrt(d_s), correctly rounded on the device, once per handle
-    double* sq = nullptr;
-    if ((rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_ids, h->deg_song.data(), static_cast<size_t>(h->S))) ||
-        (rc = dev_alloc(h, &sq, static_cast<size_t>(h->S), h->allocs))) return rc;
-    MR_LAUNCH(h, launch_sqrt_deg(d_ids, h->S, sq, st));
-    h->d_sim_sqd = sq;
-  }
-  // E_i per query, read back to split the queries into short and long rows
   long long* d_ev = nullptr;
-  if ((rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_ids, song_ids, static_cast<size_t>(n))) ||
+  if ((rc = slot_upload(h, mr_handle::SL_SIM_IDS, &d_ids, ids, static_cast<size_t>(n))) ||
       (rc = slot_alloc(h, mr_handle::SL_SIM_EV, &d_ev, static_cast<size_t>(n)))) return rc;
   std::vector<long long> ev(static_cast<size_t>(n));
   {
     PhaseTimer t(h, MR_T_OTHER);
-    MR_LAUNCH(h, launch_sim_events(d_ids, n, h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, d_ev, st));
+    MR_LAUNCH(h, launch_sim_events(d_ids, n, kind.lists, d_ev, st));
   }
   MR_CUDA(h, cudaMemcpyAsync(ev.data(), d_ev, static_cast<size_t>(n) * sizeof(long long), cudaMemcpyDeviceToHost, st));
   MR_CUDA(h, cudaStreamSynchronize(st));
@@ -1672,7 +1697,7 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
     char* base = nullptr; int* d_q = nullptr;
     if ((rc = slot_alloc(h, mr_handle::SL_SIM_OUT, &base, blk.bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_Q, &d_q, 2 * static_cast<size_t>(W)))) return rc;
     const TopkOut dev = blk.at(base);
-    std::vector<int> q(2 * static_cast<size_t>(W));   // songs [0, W), window rows [W, 2W), grouped by class
+    std::vector<int> q(2 * static_cast<size_t>(W));   // query ids [0, W), window rows [W, 2W), grouped by class
     for (int r0 = 0; r0 < n; r0 += W) {
       const int r1 = std::min(n, r0 + W);
       int cnt[kClasses] = {}, off[kClasses + 1] = {};
@@ -1685,27 +1710,28 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
       int fill[kClasses];
       std::copy(off, off + kClasses, fill);
       for (int r = r0; r < r1; ++r)
-        if (ev[r] <= short_max) { const int p = fill[cls(ev[r])]++; q[p] = song_ids[r]; q[W + p] = r - r0; }
+        if (ev[r] <= short_max) { const int p = fill[cls(ev[r])]++; q[p] = ids[r]; q[W + p] = r - r0; }
       MR_CUDA(h, cudaMemcpyAsync(d_q, q.data(), static_cast<size_t>(n_short) * sizeof(int), cudaMemcpyHostToDevice, st));
       MR_CUDA(h, cudaMemcpyAsync(d_q + W, q.data() + W, static_cast<size_t>(n_short) * sizeof(int), cudaMemcpyHostToDevice, st));
       {
         PhaseTimer t(h, MR_T_OTHER);
         for (int c = 0; c < kClasses; ++c)
-          if (cnt[c]) MR_LAUNCH(h, launch_similar_short(d_q + off[c], d_q + W + off[c], cnt[c], kSimClassCap[c], h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr,
-                                                        h->d_tr_col, h->d_sim_sqd, k, dev.song, dev.score, dev.len, st));
+          if (cnt[c]) MR_LAUNCH(h, launch_similar_short(d_q + off[c], d_q + W + off[c], cnt[c], kSimClassCap[c], kind.lists, k, dev.song, dev.score,
+                                                        dev.len, st));
       }
       const size_t o = static_cast<size_t>(r0) * k;
       if ((rc = copy_topk(h, TopkOut{out_song + o, out_score + o, out_len + r0}, dev, k, 0, r1 - r0, st))) return rc;
-      h->sim_short_rows += n_short;
+      *kind.short_rows += n_short;
     }
   }
   // long rows: exact count rows in chunks (count GEMM or inverted-index counts), the select over each chunk, then the rows to the caller
   if (!long_rows.empty()) {
     const int n_long = static_cast<int>(long_rows.size());
+    const CountRows& cr = kind.counts;
     const bool tensor = h->engine == MR_ENGINE_TENSOR;
-    const size_t ws_row = static_cast<size_t>(h->ldg) * sizeof(int32_t) + (tensor ? static_cast<size_t>(h->pitchT) : 0);
-    long long have = static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_G] / (static_cast<size_t>(h->ldg) * sizeof(int32_t)));   // rows the workspace holds already
-    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_A] / h->pitchT));
+    const size_t ws_row = static_cast<size_t>(cr.ld) * sizeof(int32_t) + (tensor ? static_cast<size_t>(cr.pitch) : 0);
+    long long have = static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_G] / (static_cast<size_t>(cr.ld) * sizeof(int32_t)));   // rows the workspace holds already
+    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_A] / cr.pitch));
     size_t free_b = 0, total_b = 0;
     MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
     const long long grow = static_cast<long long>((free_b > kSimMargin ? free_b - kSimMargin : 0) / (ws_row + row_bytes)) / 128 * 128;
@@ -1713,10 +1739,10 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
     if (const char* e = getenv("MRSCORE_SIM_CHUNK")) chunk = std::min(chunk, std::max(1LL, atoll(e)));   // test aid: force a multi-chunk run
     chunk = std::min<long long>(chunk, n_long);
     if (chunk < 1)
-      return fail(h, MR_ERR_OOM, "similar songs: one chunk of 128 count rows needs %zu bytes of device memory beyond a %zu-byte margin, %zu are free",
-                  128 * (ws_row + row_bytes), kSimMargin, free_b);
+      return fail(h, MR_ERR_OOM, "%s: one chunk of 128 count rows needs %zu bytes of device memory beyond a %zu-byte margin, %zu are free",
+                  kind.name, 128 * (ws_row + row_bytes), kSimMargin, free_b);
     const int C = static_cast<int>(chunk);
-    if ((rc = ensure_gram_ws(h, C))) return rc;
+    if ((rc = ensure_gram_ws(h, C, cr.ld, cr.pitch))) return rc;
     const TopkBlock blk(C, k);
     char* base = nullptr; int* d_rows = nullptr;
     if ((rc = slot_alloc(h, mr_handle::SL_SIM_LOUT, &base, blk.bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_LIDS, &d_rows, static_cast<size_t>(C)))) return rc;
@@ -1726,12 +1752,12 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
     std::vector<double> hv(static_cast<size_t>(C) * k);
     for (int c0 = 0; c0 < n_long; c0 += C) {
       const int nc = std::min(C, n_long - c0);
-      for (int j = 0; j < nc; ++j) rows[j] = song_ids[long_rows[c0 + j]];
+      for (int j = 0; j < nc; ++j) rows[j] = ids[long_rows[c0 + j]];
       MR_CUDA(h, cudaMemcpyAsync(d_rows, rows.data(), static_cast<size_t>(nc) * sizeof(int), cudaMemcpyHostToDevice, st));
-      if ((rc = gram_rows(h, d_rows, nc))) return rc;
+      if ((rc = count_rows(h, cr, d_rows, nc))) return rc;
       {
         PhaseTimer t(h, MR_T_TOPK);
-        MR_LAUNCH(h, launch_similar_rows(d_rows, nc, h->d_g, h->ldg, h->S, h->d_sim_sqd, k, dev.song, dev.score, dev.len, st));
+        MR_LAUNCH(h, launch_similar_rows(d_rows, nc, h->d_g, cr.ld, cr.n_cols, kind.lists, k, dev.song, dev.score, dev.len, st));
       }
       if ((rc = copy_topk(h, TopkOut{hs.data(), hv.data(), hl.data()}, dev, k, 0, nc, st))) return rc;
       MR_CUDA(h, cudaStreamSynchronize(st));
@@ -1742,10 +1768,54 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
         out_len[r] = hl[j];
       }
     }
-    h->sim_long_rows += n_long;
+    *kind.long_rows += n_long;
   }
   MR_CUDA(h, cudaStreamSynchronize(st));
   return MR_OK;
+}
+
+int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
+  int rc = require_loaded(h);
+  if (rc) return rc;
+  if (h->windowed) return fail(h, MR_ERR_STATE, "similar songs are not available on a handle with a song window (its song ids are rotated)");
+  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k = %d outside [1, 1024]", k);
+  if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
+  if (n == 0) return MR_OK;
+  if (!song_ids || !out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
+  for (int r = 0; r < n; ++r)
+    if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "query %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
+  if (!h->d_sim_sqd) {   // sqrt(d_s), once per handle
+    double* sq = nullptr;
+    if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->S), h->allocs)) || (rc = sqrt_table(h, h->deg_song.data(), h->S, sq))) return rc;
+    h->d_sim_sqd = sq;
+  }
+  const SimKind kind{"similar songs", SimLists{h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_col, h->d_sim_sqd, h->d_sim_sqd, true},
+                     song_count_rows(h), &h->sim_short_rows, &h->sim_long_rows};
+  return similar_lists(h, kind, song_ids, n, k, out_song, out_score, out_len);
+}
+
+int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_t* out_user, double* out_score, int32_t* out_len) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k = %d outside [1, 1024]", k);
+  if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
+  if (n == 0) return MR_OK;
+  if (!user_idx || !out_user || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
+  for (int r = 0; r < n; ++r)
+    if (user_idx[r] < 0 || user_idx[r] >= h->U) return fail(h, MR_ERR_BAD_ARG, "query %d: test user index %d outside [0,%d)", r, user_idx[r], h->U);
+  if (!h->d_simu_sqt) {   // sqrt(|I_v|) of the train users, once per handle
+    double* sq = nullptr;
+    if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->T), h->allocs)) || (rc = sqrt_table(h, h->deg_train.data(), h->T, sq))) return rc;
+    h->d_simu_sqt = sq;
+  }
+  if (!h->simu_squ_ok) {   // sqrt(|I_u|) of the test users, once per shard
+    if ((rc = slot_alloc(h, mr_handle::SL_SIM_SQU, &h->d_simu_squ, static_cast<size_t>(h->U))) ||
+        (rc = sqrt_table(h, h->deg_test.data(), h->U, h->d_simu_squ))) return rc;
+    h->simu_squ_ok = true;
+  }
+  const SimKind kind{"similar users", SimLists{h->d_te_ptr, h->d_te_col, h->d_csc_ptr, h->d_csc_idx, h->d_simu_squ, h->d_simu_sqt, false},
+                     user_count_rows(h), &h->simu_short_rows, &h->simu_long_rows};
+  return similar_lists(h, kind, user_idx, n, k, out_user, out_score, out_len);
 }
 
 int mr_score_dense(mr_handle* h, int model, double* out_UxS) {
@@ -2364,11 +2434,11 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[22] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[24] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
                          h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
-                         h->sim_short_rows, h->sim_long_rows};
-  for (int i = 0; i < n && i < 22; ++i) out[i] = v[i];
+                         h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows};
+  for (int i = 0; i < n && i < 24; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

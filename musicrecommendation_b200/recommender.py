@@ -330,6 +330,18 @@ class MusicRecommender:
         self._check(self._lib.mr_similar_songs(self._h, _p(ids), n, k, _p(song), _p(score), _p(ln)))
         return song, score, ln
 
+    def getSimilarUsers(self, users=None, k: int = 100):
+        """Listeners like each of `users` (indices into the current test shard, default: all of them): the k train users of highest
+        user-user cosine (MR:140-149), score descending then train-user id ascending (mr_similar_users, DESIGN.md §4.8).  Returns
+        (user [n, k] int32, score [n, k] float64, len [n] int32); row r belongs to users[r], user -1 / score 0.0 past len[r]."""
+        ids = np.arange(self.ds.U, dtype=np.int32) if users is None else np.ascontiguousarray(users, np.int32).reshape(-1)
+        n = len(ids)
+        user = np.empty((n, k), np.int32)
+        score = np.empty((n, k), np.float64)
+        ln = np.empty(n, np.int32)
+        self._check(self._lib.mr_similar_users(self._h, _p(ids), n, k, _p(user), _p(score), _p(ln)))
+        return user, score, ln
+
     def getTopKMulti(self, specs, k: int = 500):
         """getTopK for every entry of a model set (model, param, seed) from one scoring of the shard (mr_topk_multi, DESIGN.md §4.6):
         one (song [U,k] int32, score [U,k] f64, len [U]) per entry, each equal to getTopK(model, k, param, seed)."""
@@ -485,11 +497,12 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 22)()
-        self._lib.mr_get_info(self._h, v, 22)
+        v = (C.c_int64 * 24)()
+        self._lib.mr_get_info(self._h, v, 24)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
-                         "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows"], list(v)))
+                         "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows",
+                         "similar_user_short_rows", "similar_user_long_rows"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -757,6 +770,45 @@ def similar_songs_host(ds: Dataset, songs, k: int):
         out_score[r, :m] = sim[rank[:m]]
         out_len[r] = m
     return out_song, out_score, out_len
+
+
+def similar_users_host(ds: Dataset, users, k: int):
+    """numpy mirror of mr_similar_users: per query test user u, the train listeners of u's visible songs concatenated, their distinct
+    train users v with counts c (np.unique), w = c / (sqrt(deg_te[u]) * sqrt(deg_tr[v])) in that operation order (0 where the
+    denominator is 0, as the reference's cosineSimilarity), ranked by score descending then train-user id ascending.
+    Returns (user [n, k], score [n, k], len [n])."""
+    users = np.asarray(users, np.int64).reshape(-1)
+    n = len(users)
+    out_user = np.full((n, k), -1, np.int32)
+    out_score = np.zeros((n, k), np.float64)
+    out_len = np.zeros(n, np.int32)
+    tr_ptr = np.asarray(ds.tr_ptr, np.int64)
+    tr_col = np.asarray(ds.tr_col, np.int64)
+    te_ptr = np.asarray(ds.te_ptr, np.int64)
+    te_col = np.asarray(ds.te_col, np.int64)
+    owner = np.repeat(np.arange(ds.T), np.diff(tr_ptr))                    # train user of every train entry
+    order = np.argsort(tr_col, kind="stable")                              # inverted index: listeners of a song, ascending
+    csc_ptr = np.concatenate([[0], np.cumsum(np.bincount(tr_col, minlength=ds.S))])
+    listeners = owner[order]
+    deg_tr = np.asarray(ds.deg_tr, np.int64)
+    deg_te = np.asarray(ds.deg_te, np.int64)
+    for r, u in enumerate(users):
+        songs = te_col[te_ptr[u]:te_ptr[u + 1]]
+        if len(songs) == 0:
+            continue
+        hist = np.concatenate([listeners[csc_ptr[j]:csc_ptr[j + 1]] for j in songs])
+        if len(hist) == 0:
+            continue
+        v, c = np.unique(hist, return_counts=True)
+        den = np.sqrt(np.float64(deg_te[u])) * np.sqrt(deg_tr[v].astype(np.float64))
+        with np.errstate(divide="ignore", invalid="ignore"):
+            w = np.where(den != 0, c.astype(np.float64) / den, 0.0)
+        rank = np.lexsort((v, -w))
+        m = min(k, len(rank))
+        out_user[r, :m] = v[rank[:m]]
+        out_score[r, :m] = w[rank[:m]]
+        out_len[r] = m
+    return out_user, out_score, out_len
 
 
 def evaluate_map(scores: np.ndarray, ds: Dataset, n_thresholds: int = 10) -> float:

@@ -177,9 +177,7 @@ int launch_agg_split(const BlendParams& bp, const long long* te_ptr, const int* 
 //   degenerate rows (thousands of exact ties such as all-zero rows, or a bin more crowded than the candidate buffer): exact
 //                           most-significant-digit radix select (8-bit digits of the 96-bit key) inside the chosen bin
 // The collected keys (<= 2048) are bitonic-sorted exactly in shared memory: key descending, song ascending.
-constexpr int kTopkThreads = 512;   // per CTA = per test user, 2 CTAs per SM (64 registers); 256 x 4 measured the same on whole rows and on 48 k-song rows
-constexpr int kTopkCap = 2048;    // candidate buffer (>= 2 * k); bitonic-sorted in shared memory
-constexpr int kTopkBins = 2048;
+// The exact select (bin search, radix select, collect, sort, write-out) is shared with similar_row_topk_kernel (mr_common.cuh).
 
 struct KeyCtx {
   int model; double rsu, alpha, oma;
@@ -401,27 +399,11 @@ __device__ __forceinline__ bool topk_fast_path(const KeyCtx& c, int n_songs, int
     }
   });
   __syncthreads();
-  // ---- the cut: highest bin with at least `want` sampled keys in it or above (warp 0); bins >= 2 only, so the threshold is a real proxy value
-  if (warp == 0) {
-    // keys aimed at above the cut: k plus 3 sigma of the sampling noise (every 8th chunk: sigma of the full-row count ~ sqrt(8 * want)
-    // ~ 75 for k = 500) — 730 for k = 500, so that the collected keys land in [~520, ~950]: at least k, and the final sort stays at 1024 slots
-    const int want = (k + (46 * k) / 100 + stride - 1) / stride;
-    int part = 0;
-    for (int i = 0; i < kTopkBins / 32; ++i) part += s_hist[lane * (kTopkBins / 32) + i];
-    int above_lane = 0;
-    for (int l = 0; l < 32; ++l) { const int pp = __shfl_sync(0xffffffffu, part, l); if (l > lane) above_lane += pp; }
-    if (lane == 0) s_ctl[0] = 0;
-    __syncwarp();
-    if (above_lane < want && above_lane + part >= want) {
-      int cum = above_lane, chosen = lane * (kTopkBins / 32);
-      for (int i = kTopkBins / 32 - 1; i >= 0; --i) {
-        const int bin = lane * (kTopkBins / 32) + i;
-        if (cum + s_hist[bin] >= want) { chosen = bin; break; }
-        cum += s_hist[bin];
-      }
-      s_ctl[0] = chosen;
-    }
-  }
+  // ---- the cut: highest bin with at least `want` sampled keys in it or above, bin 0 when the sample holds fewer; bins >= 2 only, so the
+  // threshold is a real proxy value.  Keys aimed at above the cut: k plus 3 sigma of the sampling noise (every 8th chunk: sigma of the
+  // full-row count ~ sqrt(8 * want) ~ 75 for k = 500) — 730 for k = 500, so that the collected keys land in [~520, ~950]: at least k, and
+  // the final sort stays at 1024 slots
+  if (warp == 0) find_bin(s_hist, (k + (46 * k) / 100 + stride - 1) / stride, false, s_ctl);
   __syncthreads();
   const int cut = s_ctl[0];
   if (cut < 2) return false;                     // too few positive keys in the sample: let the exact path decide
@@ -500,7 +482,6 @@ __device__ __noinline__ int trim_candidates(unsigned long long* s_key, int* s_so
   for (int i = 0; i < kTopkThreads / 32; ++i) kmax = s_max[i] > kmax ? s_max[i] : kmax;
   __syncthreads();
   if (lane == 0) s_max[warp] = kmin;                   // the minimum through a second round on the same scratch array
-  if (tid == 0) { s_ctl[0] = 0; s_ctl[1] = 0; }        // "no bin chosen" reads as kept = 0 below
   __syncthreads();
   kmin = ~0ULL;
   for (int i = 0; i < kTopkThreads / 32; ++i) kmin = s_max[i] < kmin ? s_max[i] : kmin;
@@ -515,23 +496,9 @@ __device__ __noinline__ int trim_candidates(unsigned long long* s_key, int* s_so
     if (tid + e * kTopkThreads < n_cand) atomicAdd(&s_hist[tb[e]], 1);
   }
   __syncthreads();
-  if (warp == 0) {                                     // the highest bin with at least `need` keys in it or above
-    int part = 0;
-    for (int i = 0; i < kTopkBins / 32; ++i) part += s_hist[lane * (kTopkBins / 32) + i];
-    int above_lane = 0;
-    for (int l = 0; l < 32; ++l) { const int pp = __shfl_sync(0xffffffffu, part, l); if (l > lane) above_lane += pp; }
-    if (above_lane < need && above_lane + part >= need) {
-      int cum = above_lane, chosen = lane * (kTopkBins / 32);
-      for (int i = kTopkBins / 32 - 1; i >= 0; --i) {
-        const int bin = lane * (kTopkBins / 32) + i;
-        if (cum + s_hist[bin] >= need) { chosen = bin; break; }
-        cum += s_hist[bin];
-      }
-      s_ctl[0] = chosen; s_ctl[1] = cum + s_hist[chosen];
-    }
-  }
+  if (warp == 0) find_bin(s_hist, need, false, s_ctl);   // the highest bin with at least `need` keys in it or above (n_cand >= need)
   __syncthreads();
-  const int tbin = s_ctl[0], kept = s_ctl[1];
+  const int tbin = s_ctl[0], kept = s_ctl[1] + s_ctl[2];
   if (kept < need || kept > kTopkThreads) return n_cand;   // (uniform) a crowded bin: keep the whole buffer
   __syncthreads();
   if (tid == 0) *s_count = 0;
@@ -602,134 +569,42 @@ topk_kernel(BlendParams bp, const long long* __restrict__ te_ptr, const long lon
     const int d = __double2int_rz(__dmul_rn(__longlong_as_double(static_cast<long long>(kb)), scale));
     return static_cast<uint32_t>(d > kTopkBins - 1 ? kTopkBins - 1 : d);
   };
-  // suffix search over the 2048-bin histogram by warp 0: the highest bin such that `want` keys lie in it or above
-  auto find_bin = [&](int want_or_k, bool clamp_to_total) {
-    if (warp == 0) {
-      int part = 0;
-      for (int i = 0; i < kTopkBins / 32; ++i) part += s_hist[lane * (kTopkBins / 32) + i];
-      int total = part;
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xffffffffu, total, o);
-      int above_lane = 0;   // keys in bins owned by higher lanes
-      for (int l = 0; l < 32; ++l) { const int pp = __shfl_sync(0xffffffffu, part, l); if (l > lane) above_lane += pp; }
-      const int want = clamp_to_total ? min(want_or_k, total) : want_or_k;
-      if (lane == 0) { s_ctl[3] = want; if (want > total) { s_ctl[0] = 0; s_ctl[1] = total - s_hist[0]; s_ctl[2] = s_hist[0]; } }
-      const bool mine = want > 0 && above_lane < want && above_lane + part >= want;
-      if (mine) {
-        int cum = above_lane, chosen = lane * (kTopkBins / 32);
-        for (int i = kTopkBins / 32 - 1; i >= 0; --i) {
-          const int bin = lane * (kTopkBins / 32) + i;
-          if (cum + s_hist[bin] >= want) { chosen = bin; break; }
-          cum += s_hist[bin];
-        }
-        s_ctl[0] = chosen; s_ctl[1] = cum; s_ctl[2] = s_hist[chosen];
-      }
-    }
-  };
-  uint32_t cbin = 0; unsigned long long phi = 0; uint32_t plo = 0; int nd = 0;
+  auto scan = [&](auto&& f) { scan_row(c, n_songs, f); };
   if (!collected) {
     if (tid == 0 && bp.stats) atomicAdd(bp.stats + (stride > 1 ? 0 : 1), 1u);   // rows the fast path handed back / short rows
     // ---- exact histogram over the whole row
     for (int i = tid; i < kTopkBins; i += kTopkThreads) s_hist[i] = 0;
-    if (tid == 0) s_count = 0;
     __syncthreads();
-    scan_row(c, n_songs, [&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
+    scan([&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
     __syncthreads();
-  }
-  if (!collected) {
     // ---- exact path: the bin holding the k-th best key from the full histogram
-    find_bin(k, true);
+    if (warp == 0) {
+      const int want = find_bin(s_hist, k, true, s_ctl);
+      if (lane == 0) s_ctl[3] = want;
+    }
     __syncthreads();
     need = s_ctl[3];
     if (need > 0) {
-      cbin = static_cast<uint32_t>(s_ctl[0]);
+      const uint32_t cbin = static_cast<uint32_t>(s_ctl[0]);
       int above = s_ctl[1];                 // keys strictly better than everything still undecided
+      unsigned long long phi = 0; uint32_t plo = 0; int nd = 0;
       if (above + s_ctl[2] > kTopkCap) {
-        if (tid == 0 && bp.stats) atomicAdd(bp.stats + 2, 1u);
-        // degenerate row: exact radix select of the (need - above) best keys inside bin cbin
-        for (;;) {
-          __syncthreads();
-          for (int i = tid; i < 256; i += kTopkThreads) s_hist[i] = 0;
-          __syncthreads();
-          scan_row(c, n_songs, [&](int s, unsigned long long kb, bool ok) {
-            const uint32_t inv = ~static_cast<uint32_t>(s);
-            ok = ok && bin_of(kb) == cbin && prefix_cmp(kb, inv, phi, plo, nd) == 0;
-            hist_add(s_hist, ok ? key_digit(kb, inv, nd) : 0u, ok, lane);
-          });
-          __syncthreads();
-          if (tid == 0) {
-            const int want = need - above;
-            int cum = 0, chosen = 0;
-            for (int d = 255; d >= 0; --d) {
-              if (cum + s_hist[d] >= want) { chosen = d; break; }
-              cum += s_hist[d];
-            }
-            s_ctl[0] = chosen; s_ctl[1] = above + cum; s_ctl[2] = s_hist[chosen];
-          }
-          __syncthreads();
-          const int chosen = s_ctl[0];
-          above = s_ctl[1];
-          if (nd < 8) phi |= static_cast<unsigned long long>(chosen) << (56 - 8 * nd);
-          else plo |= static_cast<uint32_t>(chosen) << (24 - 8 * (nd - 8));
-          ++nd;
-          if (above + s_ctl[2] <= kTopkCap || nd == 12) break;
-        }
+        if (tid == 0 && bp.stats) atomicAdd(bp.stats + 2, 1u);   // degenerate rows
+        radix_refine(scan, bin_of, cbin, need, above, phi, plo, nd, s_hist, s_ctl);
       }
-      // pass C: collect every key in a higher bin, plus the keys of bin cbin at or above the radix prefix
-      __syncthreads();
-      if (tid == 0) s_count = 0;
-      __syncthreads();
-      scan_row(c, n_songs, [&](int s, unsigned long long kb, bool ok) {
-        if (ok) {
-          const uint32_t bn = bin_of(kb);
-          ok = bn > cbin || (bn == cbin && prefix_cmp(kb, ~static_cast<uint32_t>(s), phi, plo, nd) >= 0);
-        }
-        const uint32_t m = __ballot_sync(0xffffffffu, ok);
-        if (m) {
-          int base = 0;
-          if (lane == 0) base = atomicAdd(&s_count, __popc(m));
-          base = __shfl_sync(0xffffffffu, base, 0);
-          if (ok) {
-            const int pos = base + __popc(m & ((1u << lane) - 1));
-            if (pos < kTopkCap) { s_key[pos] = kb; s_song[pos] = s; }
-          }
-        }
-      });
+      collect_keys(scan, bin_of, cbin, phi, plo, nd, s_key, s_song, &s_count);   // pass C
     }
   }
   if (need == 0) {
-    for (int i = tid; i < k; i += kTopkThreads) { o_song[i] = -1; o_score[i] = 0.0; }
-    if (tid == 0) out_len[u] = 0;
+    write_list(s_key, s_song, 0, k, 0, o_song, o_score, out_len + u);
     return;
   }
   __syncthreads();
   int n_cand = min(s_count, kTopkCap);
   if (n_cand > kTopkThreads && n_cand <= 2 * kTopkThreads && need <= kTopkThreads)
     n_cand = trim_candidates(s_key, s_song, s_hist, s_max, s_ctl, &s_count, n_cand, need);
-  int n_sort = 1;
-  while (n_sort < n_cand) n_sort <<= 1;
-  for (int i = n_cand + tid; i < n_sort; i += kTopkThreads) { s_key[i] = 0; s_song[i] = 0x7fffffff; }   // sorts last
-  __syncthreads();
-  // bitonic sort, "better first": key descending, then song ascending
-  for (int size = 2; size <= n_sort; size <<= 1) {
-    for (int stride = size >> 1; stride > 0; stride >>= 1) {
-      for (int i = tid; i < n_sort / 2; i += kTopkThreads) {
-        const int lo = 2 * i - (i & (stride - 1));
-        const int hi = lo + stride;
-        const bool desc_block = (lo & size) == 0;   // first-half blocks keep the better element at the lower index
-        const unsigned long long ka = s_key[lo], kb2 = s_key[hi];
-        const int sa = s_song[lo], sb = s_song[hi];
-        const bool a_better = ka > kb2 || (ka == kb2 && sa < sb);
-        if (a_better != desc_block) { s_key[lo] = kb2; s_key[hi] = ka; s_song[lo] = sb; s_song[hi] = sa; }
-      }
-      __syncthreads();
-    }
-  }
-  for (int i = tid; i < k; i += kTopkThreads) {
-    if (i < need) { o_song[i] = s_song[i] + bp.song_off; o_score[i] = __longlong_as_double(static_cast<long long>(s_key[i])); }
-    else { o_song[i] = -1; o_score[i] = 0.0; }
-  }
-  if (tid == 0) out_len[u] = need;
+  sort_keys(s_key, s_song, n_cand);
+  write_list(s_key, s_song, need, k, bp.song_off, o_song, o_score, out_len + u);
 }
 
 int launch_topk(const BlendParams& bp, const long long* te_ptr, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,

@@ -12,8 +12,9 @@
 // songs -> train listeners.  The work of query q is E_q = the number of (item, candidate) events.  Two row paths:
 //   short rows (E_q <= kSimShortMax): one CTA per query gathers the candidate ids into shared memory, sorts them, run-lengths them into
 //     (id, count), scores each distinct id and sorts the candidates by key; the row never touches HBM and no global atomics are used;
-//   long rows: exact int32 count rows from the count engines (mrscore.cu count_rows), then similar_row_topk_kernel, one CTA per row: the
-//     exact path of topk_kernel (maximum, linear histogram, bin of the k-th key, MSD radix select inside a crowded bin, collect, bitonic sort).
+//   long rows: exact int32 count rows from the count engines (mrscore.cu count_rows), then similar_row_topk_kernel, one CTA per row:
+//     maximum, linear histogram, then the exact select topk_kernel runs too (mr_common.cuh: bin of the k-th key, MSD radix select inside
+//     a crowded bin, collect, bitonic sort, write-out).
 // kSelf: similar songs exclude the query song from its own list; a train user is never the test user asking, so similar users exclude none.
 #include <climits>
 
@@ -38,23 +39,6 @@ __device__ void bitonic_ints(int* a, int n_pad) {
         const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
         const int x = a[lo], y = a[hi];
         if ((x > y) == ((lo & size) == 0)) { a[lo] = y; a[hi] = x; }
-      }
-      __syncthreads();
-    }
-  }
-}
-
-// bitonic sort of n_pad (key, song) pairs, "better first": key descending, then song ascending
-__device__ void bitonic_keys(unsigned long long* key, int* song, int n_pad) {
-  __syncthreads();
-  for (int size = 2; size <= n_pad; size <<= 1) {
-    for (int stride = size >> 1; stride > 0; stride >>= 1) {
-      for (int i = threadIdx.x; i < n_pad / 2; i += blockDim.x) {
-        const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
-        const unsigned long long ka = key[lo], kb = key[hi];
-        const int sa = song[lo], sb = song[hi];
-        const bool a_better = ka > kb || (ka == kb && sa < sb);
-        if (a_better != ((lo & size) == 0)) { key[lo] = kb; key[hi] = ka; song[lo] = sb; song[hi] = sa; }
       }
       __syncthreads();
     }
@@ -169,14 +153,10 @@ int launch_similar_short(const int* q_ids, const int* q_row, int n_q, int cap, c
 }
 
 // ---------------------------------------------------------------- long rows: select over exact int32 count rows, one CTA per row
-constexpr int kSimThreads = 512;
-constexpr int kSimCap = 2048;     // candidate buffer, bitonic-sorted in shared memory
-constexpr int kSimBins = 2048;
-
 // f(song, key bits, candidate) for 4 songs per thread per step, the same number of times by every thread (f may use warp collectives)
 template <bool kSelf, class F>
 __device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n_songs, int self, double sq_i, const double* __restrict__ sq_c, F&& f) {
-  for (int base0 = 0; base0 < n_songs; base0 += 4 * kSimThreads) {
+  for (int base0 = 0; base0 < n_songs; base0 += 4 * kTopkThreads) {
     const int s = base0 + 4 * static_cast<int>(threadIdx.x);
     int4 v = make_int4(0, 0, 0, 0);
     if (s < n_songs) v = __ldg(reinterpret_cast<const int4*>(g + s));   // rows are padded to 32 songs
@@ -191,14 +171,14 @@ __device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n
 }
 
 template <bool kSelf>
-__global__ void __launch_bounds__(kSimThreads, 2)
+__global__ void __launch_bounds__(kTopkThreads, 2)
 similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t* __restrict__ g, long long ldg, int n_songs,
                         const double* __restrict__ sq_q, const double* __restrict__ sq_c, int k, int* __restrict__ out_song,
                         double* __restrict__ out_score, int* __restrict__ out_len) {
-  __shared__ unsigned long long s_key[kSimCap];
-  __shared__ int s_song[kSimCap];
-  __shared__ int s_hist[kSimBins];
-  __shared__ unsigned long long s_max[kSimThreads / 32];
+  __shared__ unsigned long long s_key[kTopkCap];
+  __shared__ int s_song[kTopkCap];
+  __shared__ int s_hist[kTopkBins];
+  __shared__ unsigned long long s_max[kTopkThreads / 32];
   __shared__ int s_count, s_valid;
   __shared__ int s_ctl[3];     // 0: chosen bin / digit, 1: keys strictly above it, 2: keys in it
   const int r = blockIdx.x;
@@ -209,119 +189,52 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
   const int32_t* row = g + static_cast<long long>(r) * ldg;
   int* o_song = out_song + static_cast<long long>(r) * k;
   double* o_score = out_score + static_cast<long long>(r) * k;
+  auto scan = [&](auto&& f) { scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, f); };
   // ---- maximum key and number of candidates
-  if (tid == 0) { s_valid = 0; s_count = 0; }
+  if (tid == 0) s_valid = 0;
   __syncthreads();
   unsigned long long mx = 0; int nv = 0;
-  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
+  scan([&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xffffffffu, mx, o); mx = other > mx ? other : mx; nv += __shfl_xor_sync(0xffffffffu, nv, o); }
   if (lane == 0) { s_max[warp] = mx; atomicAdd(&s_valid, nv); }
-  for (int i = tid; i < kSimBins; i += kSimThreads) s_hist[i] = 0;
+  for (int i = tid; i < kTopkBins; i += kTopkThreads) s_hist[i] = 0;
   __syncthreads();
   mx = 0;
-  for (int i = 0; i < kSimThreads / 32; ++i) mx = s_max[i] > mx ? s_max[i] : mx;
+  for (int i = 0; i < kTopkThreads / 32; ++i) mx = s_max[i] > mx ? s_max[i] : mx;
   const int need = min(k, s_valid);
   if (need == 0) {
-    for (int i = tid; i < k; i += kSimThreads) { o_song[i] = -1; o_score[i] = 0.0; }
-    if (tid == 0) out_len[r] = 0;
+    write_list(s_key, s_song, 0, k, 0, o_song, o_score, out_len + r);
     return;
   }
   const double max_score = __longlong_as_double(static_cast<long long>(mx));
-  const double scale = max_score > 0.0 ? __ddiv_rn(static_cast<double>(kSimBins - 1), max_score) : 0.0;
+  const double scale = max_score > 0.0 ? __ddiv_rn(static_cast<double>(kTopkBins - 1), max_score) : 0.0;
   auto bin_of = [&](unsigned long long kb) -> uint32_t {   // monotone in the key
     const int d = __double2int_rz(__dmul_rn(__longlong_as_double(static_cast<long long>(kb)), scale));
-    return static_cast<uint32_t>(d > kSimBins - 1 ? kSimBins - 1 : d);
+    return static_cast<uint32_t>(d > kTopkBins - 1 ? kTopkBins - 1 : d);
   };
-  // ---- linear histogram of the candidates, then the bin holding the need-th best key (warp 0, suffix search)
-  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
+  // ---- linear histogram of the candidates, then the shared exact select (mr_common.cuh)
+  scan([&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
   __syncthreads();
-  if (warp == 0) {
-    int part = 0;
-    for (int i = 0; i < kSimBins / 32; ++i) part += s_hist[lane * (kSimBins / 32) + i];
-    int above_lane = 0;
-    for (int l = 0; l < 32; ++l) { const int pp = __shfl_sync(0xffffffffu, part, l); if (l > lane) above_lane += pp; }
-    if (above_lane < need && above_lane + part >= need) {
-      int cum = above_lane, chosen = lane * (kSimBins / 32);
-      for (int i = kSimBins / 32 - 1; i >= 0; --i) {
-        const int bin = lane * (kSimBins / 32) + i;
-        if (cum + s_hist[bin] >= need) { chosen = bin; break; }
-        cum += s_hist[bin];
-      }
-      s_ctl[0] = chosen; s_ctl[1] = cum; s_ctl[2] = s_hist[chosen];
-    }
-  }
+  if (warp == 0) find_bin(s_hist, need, false, s_ctl);
   __syncthreads();
   const uint32_t cbin = static_cast<uint32_t>(s_ctl[0]);
   int above = s_ctl[1];
   unsigned long long phi = 0; uint32_t plo = 0; int nd = 0;
-  if (above + s_ctl[2] > kSimCap) {
-    // crowded bin (thousands of exact ties, e.g. g = 1 against songs of one degree): MSD radix select of the (need - above) best keys in it
-    for (;;) {
-      __syncthreads();
-      for (int i = tid; i < 256; i += kSimThreads) s_hist[i] = 0;
-      __syncthreads();
-      scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int s, unsigned long long kb, bool ok) {
-        const uint32_t inv = ~static_cast<uint32_t>(s);
-        ok = ok && bin_of(kb) == cbin && prefix_cmp(kb, inv, phi, plo, nd) == 0;
-        hist_add(s_hist, ok ? key_digit(kb, inv, nd) : 0u, ok, lane);
-      });
-      __syncthreads();
-      if (tid == 0) {
-        const int want = need - above;
-        int cum = 0, chosen = 0;
-        for (int d = 255; d >= 0; --d) {
-          if (cum + s_hist[d] >= want) { chosen = d; break; }
-          cum += s_hist[d];
-        }
-        s_ctl[0] = chosen; s_ctl[1] = above + cum; s_ctl[2] = s_hist[chosen];
-      }
-      __syncthreads();
-      const int chosen = s_ctl[0];
-      above = s_ctl[1];
-      if (nd < 8) phi |= static_cast<unsigned long long>(chosen) << (56 - 8 * nd);
-      else plo |= static_cast<uint32_t>(chosen) << (24 - 8 * (nd - 8));
-      ++nd;
-      if (above + s_ctl[2] <= kSimCap || nd == 12) break;
-    }
-  }
-  // ---- collect every key in a higher bin, plus the keys of bin cbin at or above the radix prefix
+  // a crowded bin: thousands of exact ties, e.g. g = 1 against songs of one degree
+  if (above + s_ctl[2] > kTopkCap) radix_refine(scan, bin_of, cbin, need, above, phi, plo, nd, s_hist, s_ctl);
+  collect_keys(scan, bin_of, cbin, phi, plo, nd, s_key, s_song, &s_count);
   __syncthreads();
-  scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, [&](int s, unsigned long long kb, bool ok) {
-    if (ok) {
-      const uint32_t bn = bin_of(kb);
-      ok = bn > cbin || (bn == cbin && prefix_cmp(kb, ~static_cast<uint32_t>(s), phi, plo, nd) >= 0);
-    }
-    const uint32_t m = __ballot_sync(0xffffffffu, ok);
-    if (m) {
-      int base = 0;
-      if (lane == 0) base = atomicAdd(&s_count, __popc(m));
-      base = __shfl_sync(0xffffffffu, base, 0);
-      if (ok) {
-        const int pos = base + __popc(m & ((1u << lane) - 1));
-        if (pos < kSimCap) { s_key[pos] = kb; s_song[pos] = s; }
-      }
-    }
-  });
-  __syncthreads();
-  const int n_cand = min(s_count, kSimCap);
-  int n_sort = 1;
-  while (n_sort < n_cand) n_sort <<= 1;
-  for (int i = n_cand + tid; i < n_sort; i += kSimThreads) { s_key[i] = 0; s_song[i] = INT_MAX; }   // sorts last
-  bitonic_keys(s_key, s_song, n_sort);
-  for (int i = tid; i < k; i += kSimThreads) {
-    if (i < need) { o_song[i] = s_song[i]; o_score[i] = __longlong_as_double(static_cast<long long>(s_key[i])); }
-    else { o_song[i] = -1; o_score[i] = 0.0; }
-  }
-  if (tid == 0) out_len[r] = need;
+  sort_keys(s_key, s_song, min(s_count, kTopkCap));
+  write_list(s_key, s_song, need, k, 0, o_song, o_score, out_len + r);
 }
 
 int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_cols, const SimLists& l, int k, int* out_song,
                         double* out_score, int* out_len, cudaStream_t st) {
   if (n_rows <= 0) return 0;
-  if (k <= 0 || k > kSimCap / 2) return -2;
+  if (k <= 0 || k > kTopkCap / 2) return -2;
   auto kern = l.self ? similar_row_topk_kernel<true> : similar_row_topk_kernel<false>;
-  kern<<<n_rows, kSimThreads, 0, st>>>(rows, n_rows, g, ldg, n_cols, l.sq_q, l.sq_c, k, out_song, out_score, out_len);
+  kern<<<n_rows, kTopkThreads, 0, st>>>(rows, n_rows, g, ldg, n_cols, l.sq_q, l.sq_c, k, out_song, out_score, out_len);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

@@ -36,6 +36,10 @@ trait MrScore extends Library {
   def mr_similar_songs(h: Pointer, songIds: Array[Int], n: Int, k: Int, outSong: Array[Int], outScore: Array[Double], outLen: Array[Int]): Int
   // listeners like each query test user (indices into the current shard): the k train users of highest user-user cosine (MR:140-149)
   def mr_similar_users(h: Pointer, userIdx: Array[Int], n: Int, k: Int, outUser: Array[Int], outScore: Array[Double], outLen: Array[Int]): Int
+  // why song songIds(r) scores what it does for test user userIdx(r) under MR_UBM / MR_IBM: the m largest contributors ([n][m] ids, cosine
+  // terms, fixed-point terms), their number, the exact numerator and the library's score per pair (DESIGN.md §4.9)
+  def mr_explain(h: Pointer, model: Int, userIdx: Array[Int], songIds: Array[Int], n: Int, m: Int, outId: Array[Int], outTerm: Array[Double],
+                 outNum: Array[Long], outLen: Array[Int], outCount: Array[Int], outTotal: Array[Long], outScore: Array[Double]): Int
   def mr_ingest_tsv(device: Int, train: Array[Byte], trainLen: Long, test: Array[Byte], testLen: Long, labels: Array[Byte],
                     labelsLen: Long, out: PointerByReference): Int
   def mr_ingest_error(g: Pointer): String

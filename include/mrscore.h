@@ -253,6 +253,35 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
  * when not even one chunk of count rows fits in the free device memory. */
 int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_t* out_user, double* out_score, int32_t* out_len);
 
+/* ---- explanations: why a song scores what it scores for a test user (DESIGN.md §4.9) --------------------------------------------------
+ * Pair r is (u = user_idx[r], an index into the CURRENT test shard as in mr_score_users; s = song_ids[r] in [0, S)); any order, duplicates
+ * allowed.  model = MR_UBM or MR_IBM (blends: MR_ERR_BAD_ARG).  The score of DESIGN.md §3 is one integer numerator times one factor, and
+ * each term of the numerator is one contributor:
+ *   MR_UBM: the train listeners v of s with c(u, v) = |I_u ∩ I_v| > 0;
+ *           term = c / (sqrt((double) deg_test[u]) * sqrt((double) deg_train[v]))   (the score mr_similar_users gives (u, v)),
+ *           num = c * q_24(deg_train[v]);
+ *   MR_IBM: u's visible songs j != s with g(s, j) = |U_s^train ∩ U_j^train| > 0;
+ *           term = g / (sqrt((double) d_s) * sqrt((double) d_j)), d = deg_song_all  (the score mr_similar_songs gives (s, j)),
+ *           num = g * q_26(d_j);
+ * each term evaluated in that operation order, correctly rounded.  Contributors are ordered by term descending, then id ascending.
+ * Outputs (host arrays): out_id / out_term / out_num [n][m] hold the first out_len[r] = min(m, out_count[r]) contributors of pair r, then
+ * id -1, term 0.0, num 0; out_count[r] = the number of all contributors; out_total[r] = the sum of num over ALL of them, whatever m;
+ * out_score[r] = (double) out_total[r] * (2^-24 / sqrt(deg_test[u]) for UBM, 2^-26 / sqrt(d_s) for IBM), with the bits mr_topk and
+ * mr_score_users give the pair.  Two exactness statements:
+ *   1. out_total is the library's score numerator Sint[u, s], bit for bit;
+ *   2. the sum of term over all contributors in ascending id is the as-written score of the reference's loops (MR:159-166, 249-257),
+ *      bit for bit.
+ * The two scores (the sum of the terms and out_score) differ within the quantisation bound of DESIGN.md §3: that is expected, not a bug.
+ * A listened pair (s in I_u; the reference emits none, MR:109) gets score NaN, len 0, count 0, total 0; an unlistened pair without
+ * contributors score 0.0 and len 0.  1 <= m <= 1024; n = 0 returns MR_OK.  MR_ERR_BAD_ARG names the first pair with an id out of range, and
+ * covers a bad m or model and null arrays; MR_ERR_STATE before mr_load, without test users and on a handle with a song window.  One count
+ * row serves all pairs of its key (UBM: c(u, .) over the train users, IBM: g(s, .) over the songs), built by the count engine in chunks of up
+ * to 1024 rows (MR_T_COUNT, MR_T_EXPAND on the tensor engine); the contributors of each pair are ranked by one select (MR_T_TOPK).
+ * mr_get_info value 25 counts the count rows built since mr_load.  The call leaves every result and resident state of the scoring calls as it
+ * was and returns with all its work complete.  MR_ERR_OOM, stating the bytes, when not even one chunk of count rows fits. */
+int mr_explain(mr_handle* h, int model, const int32_t* user_idx, const int32_t* song_ids, int n, int m, int32_t* out_id, double* out_term,
+               int64_t* out_num, int32_t* out_len, int32_t* out_count, int64_t* out_total, double* out_score);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -328,7 +357,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  (exact path by design), degenerate rows (radix select),
                                                                  scoring passes since mr_load (batches whose score panels were built),
                                                                  mr_similar_songs rows since mr_load: answered by the short path, by the long path,
-                                                                 mr_similar_users rows since mr_load: answered by the short path, by the long path] */
+                                                                 mr_similar_users rows since mr_load: answered by the short path, by the long path,
+                                                                 mr_explain count rows built since mr_load] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

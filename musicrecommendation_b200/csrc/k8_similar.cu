@@ -16,6 +16,9 @@
 //     maximum, linear histogram, then the exact select topk_kernel runs too (mr_common.cuh: bin of the k-th key, MSD radix select inside
 //     a crowded bin, collect, bitonic sort, write-out).
 // kSelf: similar songs exclude the query song from its own list; a train user is never the test user asking, so similar users exclude none.
+//
+// Explanations (mr_explain, DESIGN.md §4.9) rank the same two cosines restricted to the contributors of one (test user, song) score:
+// explain_pairs_kernel runs the select of the long rows (row_select) over a scan of the pair's contributor list instead of a count row.
 #include <climits>
 
 #include "mr_common.cuh"
@@ -170,42 +173,39 @@ __device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n
   }
 }
 
-template <bool kSelf>
-__global__ void __launch_bounds__(kTopkThreads, 2)
-similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t* __restrict__ g, long long ldg, int n_songs,
-                        const double* __restrict__ sq_q, const double* __restrict__ sq_c, int k, int* __restrict__ out_song,
-                        double* __restrict__ out_score, int* __restrict__ out_len) {
-  __shared__ unsigned long long s_key[kTopkCap];
-  __shared__ int s_song[kTopkCap];
-  __shared__ int s_hist[kTopkBins];
-  __shared__ unsigned long long s_max[kTopkThreads / 32];
-  __shared__ int s_count, s_valid;
-  __shared__ int s_ctl[3];     // 0: chosen bin / digit, 1: keys strictly above it, 2: keys in it
-  const int r = blockIdx.x;
-  if (r >= n_rows) return;
+// Shared memory of one row's exact select
+struct RowSelect {
+  unsigned long long key[kTopkCap];
+  int id[kTopkCap];
+  int hist[kTopkBins];
+  unsigned long long max[kTopkThreads / 32];
+  int count, valid;
+  int ctl[3];     // 0: chosen bin / digit, 1: keys strictly above it, 2: keys in it
+};
+
+// The exact list of one row (similar_row_topk_kernel, explain_pairs_kernel): the maximum key and the number of candidates from the pass
+// first(f), then a linear histogram and the exact select of topk_kernel (mr_common.cuh) over the passes scan(f); write_list stores the
+// first min(k, candidates) entries.  first and scan stream the same candidates (first may also accumulate the caller's own sums).
+// Returns need = min(k, candidates); sm.valid holds the number of candidates, sm.id[0 .. need) the listed ids.
+template <class First, class Scan>
+__device__ __forceinline__ int row_select(First&& first, Scan&& scan, int k, RowSelect& sm, int* o_id, double* o_score, int* o_len) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int self = rows[r];
-  const double sq_i = sq_q[self];
-  const int32_t* row = g + static_cast<long long>(r) * ldg;
-  int* o_song = out_song + static_cast<long long>(r) * k;
-  double* o_score = out_score + static_cast<long long>(r) * k;
-  auto scan = [&](auto&& f) { scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, f); };
   // ---- maximum key and number of candidates
-  if (tid == 0) s_valid = 0;
+  if (tid == 0) sm.valid = 0;
   __syncthreads();
   unsigned long long mx = 0; int nv = 0;
-  scan([&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
+  first([&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xffffffffu, mx, o); mx = other > mx ? other : mx; nv += __shfl_xor_sync(0xffffffffu, nv, o); }
-  if (lane == 0) { s_max[warp] = mx; atomicAdd(&s_valid, nv); }
-  for (int i = tid; i < kTopkBins; i += kTopkThreads) s_hist[i] = 0;
+  if (lane == 0) { sm.max[warp] = mx; atomicAdd(&sm.valid, nv); }
+  for (int i = tid; i < kTopkBins; i += kTopkThreads) sm.hist[i] = 0;
   __syncthreads();
   mx = 0;
-  for (int i = 0; i < kTopkThreads / 32; ++i) mx = s_max[i] > mx ? s_max[i] : mx;
-  const int need = min(k, s_valid);
+  for (int i = 0; i < kTopkThreads / 32; ++i) mx = sm.max[i] > mx ? sm.max[i] : mx;
+  const int need = min(k, sm.valid);
   if (need == 0) {
-    write_list(s_key, s_song, 0, k, 0, o_song, o_score, out_len + r);
-    return;
+    write_list(sm.key, sm.id, 0, k, 0, o_id, o_score, o_len);
+    return 0;
   }
   const double max_score = __longlong_as_double(static_cast<long long>(mx));
   const double scale = max_score > 0.0 ? __ddiv_rn(static_cast<double>(kTopkBins - 1), max_score) : 0.0;
@@ -214,19 +214,35 @@ similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t*
     return static_cast<uint32_t>(d > kTopkBins - 1 ? kTopkBins - 1 : d);
   };
   // ---- linear histogram of the candidates, then the shared exact select (mr_common.cuh)
-  scan([&](int, unsigned long long kb, bool ok) { hist_add(s_hist, ok ? bin_of(kb) : 0u, ok, lane); });
+  scan([&](int, unsigned long long kb, bool ok) { hist_add(sm.hist, ok ? bin_of(kb) : 0u, ok, lane); });
   __syncthreads();
-  if (warp == 0) find_bin(s_hist, need, false, s_ctl);
+  if (warp == 0) find_bin(sm.hist, need, false, sm.ctl);
   __syncthreads();
-  const uint32_t cbin = static_cast<uint32_t>(s_ctl[0]);
-  int above = s_ctl[1];
+  const uint32_t cbin = static_cast<uint32_t>(sm.ctl[0]);
+  int above = sm.ctl[1];
   unsigned long long phi = 0; uint32_t plo = 0; int nd = 0;
   // a crowded bin: thousands of exact ties, e.g. g = 1 against songs of one degree
-  if (above + s_ctl[2] > kTopkCap) radix_refine(scan, bin_of, cbin, need, above, phi, plo, nd, s_hist, s_ctl);
-  collect_keys(scan, bin_of, cbin, phi, plo, nd, s_key, s_song, &s_count);
+  if (above + sm.ctl[2] > kTopkCap) radix_refine(scan, bin_of, cbin, need, above, phi, plo, nd, sm.hist, sm.ctl);
+  collect_keys(scan, bin_of, cbin, phi, plo, nd, sm.key, sm.id, &sm.count);
   __syncthreads();
-  sort_keys(s_key, s_song, min(s_count, kTopkCap));
-  write_list(s_key, s_song, need, k, 0, o_song, o_score, out_len + r);
+  sort_keys(sm.key, sm.id, min(sm.count, kTopkCap));
+  write_list(sm.key, sm.id, need, k, 0, o_id, o_score, o_len);
+  return need;
+}
+
+template <bool kSelf>
+__global__ void __launch_bounds__(kTopkThreads, 2)
+similar_row_topk_kernel(const int* __restrict__ rows, int n_rows, const int32_t* __restrict__ g, long long ldg, int n_songs,
+                        const double* __restrict__ sq_q, const double* __restrict__ sq_c, int k, int* __restrict__ out_song,
+                        double* __restrict__ out_score, int* __restrict__ out_len) {
+  __shared__ RowSelect sm;
+  const int r = blockIdx.x;
+  if (r >= n_rows) return;
+  const int self = rows[r];
+  const double sq_i = sq_q[self];
+  const int32_t* row = g + static_cast<long long>(r) * ldg;
+  auto scan = [&](auto&& f) { scan_counts<kSelf>(row, n_songs, self, sq_i, sq_c, f); };
+  row_select(scan, scan, k, sm, out_song + static_cast<long long>(r) * k, out_score + static_cast<long long>(r) * k, out_len + r);
 }
 
 int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_cols, const SimLists& l, int k, int* out_song,
@@ -235,6 +251,84 @@ int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long
   if (k <= 0 || k > kTopkCap / 2) return -2;
   auto kern = l.self ? similar_row_topk_kernel<true> : similar_row_topk_kernel<false>;
   kern<<<n_rows, kTopkThreads, 0, st>>>(rows, n_rows, g, ldg, n_cols, l.sq_q, l.sq_c, k, out_song, out_score, out_len);
+  return cudaGetLastError() == cudaSuccess ? 0 : -1;
+}
+
+// ---------------------------------------------------------------- explanations: the contributors of one (test user, song) score
+// One CTA per pair p = (count row a.pairs[p].x of the chunk, other id a.pairs[p].y).  The pair's contributor list is scanned straight
+// from the index and each entry's count read from the count row:
+//   UBM (key = test user u, other = song s): the train listeners v of s (inverted index), c(u, v) from the row c(u, .);
+//   IBM (key = song s, other = test user u): u's visible songs j, g(s, j) from the Gram row g(s, .).
+// Since s is not in I_u for an explained pair, j != s holds for every j of I_u.  The first pass also sums num = count * q over all
+// contributors: the exact numerator Sint[u, s] of DESIGN.md §3.
+template <int kModel>
+__global__ void __launch_bounds__(kTopkThreads, 2)
+explain_pairs_kernel(const ExplainArgs a, int n, int m, const ExplainOut o) {
+  __shared__ RowSelect sm;
+  __shared__ unsigned long long s_total;
+  const int p = blockIdx.x;
+  if (p >= n) return;
+  const int tid = threadIdx.x, lane = tid & 31;
+  const int2 pr = a.pairs[p];
+  const int key = a.keys[pr.x];
+  const int u = kModel == MODEL_UBM ? key : pr.y, s = kModel == MODEL_UBM ? pr.y : key;
+  const int32_t* row = a.g + static_cast<long long>(pr.x) * a.ld;
+  int* o_id = o.id + static_cast<long long>(p) * m;
+  double* o_term = o.term + static_cast<long long>(p) * m;
+  long long* o_num = o.num + static_cast<long long>(p) * m;
+  // a listened pair (s in u's ascending test row) is no pair of the model (MR:109)
+  const long long tb = a.te_ptr[u];
+  int lo = 0, hi = static_cast<int>(a.te_ptr[u + 1] - tb);
+  const int n_u = hi;
+  while (lo < hi) { const int mid = (lo + hi) >> 1; if (__ldg(a.te_col + tb + mid) < s) lo = mid + 1; else hi = mid; }
+  if (lo < n_u && __ldg(a.te_col + tb + lo) == s) {
+    for (int i = tid; i < m; i += kTopkThreads) { o_id[i] = -1; o_term[i] = 0.0; o_num[i] = 0; }
+    if (tid == 0) { o.len[p] = 0; o.count[p] = 0; o.total[p] = 0; o.score[p] = __longlong_as_double(0x7ff8000000000000LL); }
+    return;
+  }
+  const int li = kModel == MODEL_UBM ? s : u;
+  const long long lb = a.list_ptr[li];
+  const int len = static_cast<int>(a.list_ptr[li + 1] - lb);
+  const int* list = a.list_idx + lb;
+  const double sq_k = a.sq_key[key];
+  if (tid == 0) s_total = 0;   // row_select synchronises before anyone adds to it
+  long long tot = 0;
+  // f(id, key bits, contributor) for one list entry per thread per step; on(id, count) for each contributor
+  auto walk = [&](auto&& f, auto&& on) {
+    for (int b = 0; b < len; b += kTopkThreads) {
+      const int i = b + tid;
+      int id = 0, c = 0;
+      if (i < len) { id = __ldg(list + i); c = __ldg(row + id); }
+      unsigned long long kb = 0;
+      if (c > 0) { kb = key_bits(sim_score(c, sq_k, __ldg(a.sq_other + id))); on(id, c); }
+      f(id, kb, c > 0);
+    }
+  };
+  auto first = [&](auto&& f) { walk(f, [&](int id, int c) { tot += static_cast<long long>(c) * __ldg(a.q + id); }); };
+  auto scan = [&](auto&& f) { walk(f, [](int, int) {}); };
+  const int need = row_select(first, scan, m, sm, o_id, o_term, o.len + p);
+  for (int i = tid; i < m; i += kTopkThreads) {
+    long long v = 0;
+    if (i < need) { const int id = sm.id[i]; v = static_cast<long long>(__ldg(row + id)) * __ldg(a.q + id); }
+    o_num[i] = v;
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, off);
+  if (lane == 0 && tot) atomicAdd(&s_total, static_cast<unsigned long long>(tot));
+  __syncthreads();
+  if (tid == 0) {
+    const long long total = static_cast<long long>(s_total);
+    o.count[p] = sm.valid;
+    o.total[p] = total;
+    o.score[p] = __dmul_rn(__ll2double_rn(total), a.rs[kModel == MODEL_UBM ? u : s]);
+  }
+}
+
+int launch_explain_pairs(int model, const ExplainArgs& a, int n, int m, const ExplainOut& o, cudaStream_t st) {
+  if (n <= 0) return 0;
+  if (m <= 0 || m > kTopkCap / 2 || (model != MODEL_UBM && model != MODEL_IBM)) return -2;
+  auto kern = model == MODEL_UBM ? explain_pairs_kernel<MODEL_UBM> : explain_pairs_kernel<MODEL_IBM>;
+  kern<<<n, kTopkThreads, 0, st>>>(a, n, m, o);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

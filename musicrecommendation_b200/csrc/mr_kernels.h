@@ -192,4 +192,18 @@ int launch_similar_short(const int* q_ids, const int* q_row, int n_q, int cap, c
 int launch_similar_rows(const int* rows, int n_rows, const int32_t* g, long long ldg, int n_cols, const SimLists& l, int k, int* out_song,
                         double* out_score, int* out_len, cudaStream_t st);
 
+// ---- explanations (k8_similar.cu, DESIGN.md §4.9): the contributors of (test user, song) scores of UBM or IBM from the count rows of a chunk
+struct ExplainArgs {
+  const int* keys;                                   // [rows] key of each count row: test user (UBM) or song (IBM)
+  const int2* pairs;                                 // [n] (count row in the chunk, other id: song (UBM) or test user (IBM))
+  const int32_t* g; long long ld;                    // count rows c(u, .) over the train users (UBM) or g(s, .) over the songs (IBM)
+  const long long* list_ptr; const int* list_idx;    // contributor lists: the inverted index by song (UBM), the test rows (IBM)
+  const long long* te_ptr; const int* te_col;        // test rows (ascending): the listened check
+  const double* sq_key; const double* sq_other;      // sqrt of the degrees: deg_test, deg_train (UBM); deg_song_all, deg_song_all (IBM)
+  const uint32_t* q;                                 // q_24(deg_train) (UBM), q_26(deg_song_all) (IBM)
+  const double* rs;                                  // the score factor: rsa per test user (UBM), rsd per song (IBM)
+};
+struct ExplainOut { int* id; double* term; long long* num; int* len; int* count; long long* total; double* score; };   // [n][m] x 3, [n] x 4
+int launch_explain_pairs(int model, const ExplainArgs& a, int n, int m, const ExplainOut& o, cudaStream_t st);
+
 }  // namespace mr

@@ -22,6 +22,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <numeric>
 #include <optional>
 #include <string>
 #include <queue>
@@ -132,6 +133,7 @@ struct mr_handle {
   // (slot SL_SIM_SQU), rebuilt on the first call after each mr_set_test_users; rows answered by each path since mr_load
   std::vector<int32_t> deg_train, deg_test;
   double *d_simu_sqt = nullptr, *d_simu_squ = nullptr; bool simu_squ_ok = false; long long simu_short_rows = 0, simu_long_rows = 0;
+  long long explain_rows = 0;   // mr_explain: count rows built since mr_load
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -1666,6 +1668,53 @@ static int sqrt_table(mr_handle* h, const int32_t* deg, int n, double* out) {
   return MR_OK;
 }
 
+// Rows per chunk of count rows of kind cr for n_rows rows (the long rows of similar_lists, the keys of mr_explain), each row needing
+// row_bytes of its own besides: up to 1024 rows, as many as the Gram workspace holds already or as fit in the free device memory less
+// kSimMargin, in multiples of 128; MRSCORE_SIM_CHUNK caps it (test aid: force a multi-chunk run).  Sizes the workspace for the chunk.
+static int count_chunk(mr_handle* h, const CountRows& cr, size_t row_bytes, int n_rows, const char* name, int* out) {
+  const bool tensor = h->engine == MR_ENGINE_TENSOR;
+  const size_t ws_row = static_cast<size_t>(cr.ld) * sizeof(int32_t) + (tensor ? static_cast<size_t>(cr.pitch) : 0);
+  long long have = static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_G] / (static_cast<size_t>(cr.ld) * sizeof(int32_t)));   // rows the workspace holds already
+  if (tensor) have = std::min<long long>(have, static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_A] / cr.pitch));
+  size_t free_b = 0, total_b = 0;
+  MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
+  const long long grow = static_cast<long long>((free_b > kSimMargin ? free_b - kSimMargin : 0) / (ws_row + row_bytes)) / 128 * 128;
+  long long chunk = std::min<long long>(1024, std::max(have, grow));
+  if (const char* e = getenv("MRSCORE_SIM_CHUNK")) chunk = std::min(chunk, std::max(1LL, atoll(e)));
+  chunk = std::min<long long>(chunk, n_rows);
+  if (chunk < 1)
+    return fail(h, MR_ERR_OOM, "%s: one chunk of 128 count rows needs %zu bytes of device memory beyond a %zu-byte margin, %zu are free",
+                name, 128 * (ws_row + row_bytes), kSimMargin, free_b);
+  *out = static_cast<int>(chunk);
+  return ensure_gram_ws(h, *out, cr.ld, cr.pitch);
+}
+
+// sqrt(d_s) of every song (similar songs, IBM explanations), once per handle
+static int ensure_sqrt_songs(mr_handle* h) {
+  if (h->d_sim_sqd) return MR_OK;
+  double* sq = nullptr;
+  int rc;
+  if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->S), h->allocs)) || (rc = sqrt_table(h, h->deg_song.data(), h->S, sq))) return rc;
+  h->d_sim_sqd = sq;
+  return MR_OK;
+}
+
+// sqrt(|I_v|) of the train users, once per handle, and sqrt(|I_u|) of the test users, once per shard (similar users, UBM explanations)
+static int ensure_sqrt_users(mr_handle* h) {
+  int rc;
+  if (!h->d_simu_sqt) {
+    double* sq = nullptr;
+    if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->T), h->allocs)) || (rc = sqrt_table(h, h->deg_train.data(), h->T, sq))) return rc;
+    h->d_simu_sqt = sq;
+  }
+  if (!h->simu_squ_ok) {
+    if ((rc = slot_alloc(h, mr_handle::SL_SIM_SQU, &h->d_simu_squ, static_cast<size_t>(h->U))) ||
+        (rc = sqrt_table(h, h->deg_test.data(), h->U, h->d_simu_squ))) return rc;
+    h->simu_squ_ok = true;
+  }
+  return MR_OK;
+}
+
 // The query ids are checked by the caller.  E_q of every query is read back to split the queries into short and long rows.
 static int similar_lists(mr_handle* h, const SimKind& kind, const int32_t* ids, int n, int k, int32_t* out_song, double* out_score, int32_t* out_len) {
   cudaStream_t st = h->stream;
@@ -1728,21 +1777,8 @@ static int similar_lists(mr_handle* h, const SimKind& kind, const int32_t* ids, 
   if (!long_rows.empty()) {
     const int n_long = static_cast<int>(long_rows.size());
     const CountRows& cr = kind.counts;
-    const bool tensor = h->engine == MR_ENGINE_TENSOR;
-    const size_t ws_row = static_cast<size_t>(cr.ld) * sizeof(int32_t) + (tensor ? static_cast<size_t>(cr.pitch) : 0);
-    long long have = static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_G] / (static_cast<size_t>(cr.ld) * sizeof(int32_t)));   // rows the workspace holds already
-    if (tensor) have = std::min<long long>(have, static_cast<long long>(h->slot_cap[mr_handle::SL_GRAM_A] / cr.pitch));
-    size_t free_b = 0, total_b = 0;
-    MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
-    const long long grow = static_cast<long long>((free_b > kSimMargin ? free_b - kSimMargin : 0) / (ws_row + row_bytes)) / 128 * 128;
-    long long chunk = std::min<long long>(1024, std::max(have, grow));
-    if (const char* e = getenv("MRSCORE_SIM_CHUNK")) chunk = std::min(chunk, std::max(1LL, atoll(e)));   // test aid: force a multi-chunk run
-    chunk = std::min<long long>(chunk, n_long);
-    if (chunk < 1)
-      return fail(h, MR_ERR_OOM, "%s: one chunk of 128 count rows needs %zu bytes of device memory beyond a %zu-byte margin, %zu are free",
-                  kind.name, 128 * (ws_row + row_bytes), kSimMargin, free_b);
-    const int C = static_cast<int>(chunk);
-    if ((rc = ensure_gram_ws(h, C, cr.ld, cr.pitch))) return rc;
+    int C = 0;
+    if ((rc = count_chunk(h, cr, row_bytes, n_long, kind.name, &C))) return rc;
     const TopkBlock blk(C, k);
     char* base = nullptr; int* d_rows = nullptr;
     if ((rc = slot_alloc(h, mr_handle::SL_SIM_LOUT, &base, blk.bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_LIDS, &d_rows, static_cast<size_t>(C)))) return rc;
@@ -1784,11 +1820,7 @@ int mr_similar_songs(mr_handle* h, const int32_t* song_ids, int n, int k, int32_
   if (!song_ids || !out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
   for (int r = 0; r < n; ++r)
     if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "query %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
-  if (!h->d_sim_sqd) {   // sqrt(d_s), once per handle
-    double* sq = nullptr;
-    if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->S), h->allocs)) || (rc = sqrt_table(h, h->deg_song.data(), h->S, sq))) return rc;
-    h->d_sim_sqd = sq;
-  }
+  if ((rc = ensure_sqrt_songs(h))) return rc;
   const SimKind kind{"similar songs", SimLists{h->d_csc_ptr, h->d_csc_idx, h->d_tr_ptr, h->d_tr_col, h->d_sim_sqd, h->d_sim_sqd, true},
                      song_count_rows(h), &h->sim_short_rows, &h->sim_long_rows};
   return similar_lists(h, kind, song_ids, n, k, out_song, out_score, out_len);
@@ -1803,19 +1835,113 @@ int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_
   if (!user_idx || !out_user || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null query or output array");
   for (int r = 0; r < n; ++r)
     if (user_idx[r] < 0 || user_idx[r] >= h->U) return fail(h, MR_ERR_BAD_ARG, "query %d: test user index %d outside [0,%d)", r, user_idx[r], h->U);
-  if (!h->d_simu_sqt) {   // sqrt(|I_v|) of the train users, once per handle
-    double* sq = nullptr;
-    if ((rc = dev_alloc(h, &sq, static_cast<size_t>(h->T), h->allocs)) || (rc = sqrt_table(h, h->deg_train.data(), h->T, sq))) return rc;
-    h->d_simu_sqt = sq;
-  }
-  if (!h->simu_squ_ok) {   // sqrt(|I_u|) of the test users, once per shard
-    if ((rc = slot_alloc(h, mr_handle::SL_SIM_SQU, &h->d_simu_squ, static_cast<size_t>(h->U))) ||
-        (rc = sqrt_table(h, h->deg_test.data(), h->U, h->d_simu_squ))) return rc;
-    h->simu_squ_ok = true;
-  }
+  if ((rc = ensure_sqrt_users(h))) return rc;
   const SimKind kind{"similar users", SimLists{h->d_te_ptr, h->d_te_col, h->d_csc_ptr, h->d_csc_idx, h->d_simu_squ, h->d_simu_sqt, false},
                      user_count_rows(h), &h->simu_short_rows, &h->simu_long_rows};
   return similar_lists(h, kind, user_idx, n, k, out_user, out_score, out_len);
+}
+
+// ---- explanations (DESIGN.md §4.9, k8_similar.cu explain_pairs_kernel): the contributors of (test user, song) scores of UBM or IBM.  The
+// pairs are grouped by the key whose count row serves them (UBM: the test user, row c(u, .); IBM: the song, Gram row g(s, .)); the
+// distinct keys go through count_rows in chunks sized as the long rows of similar_lists, and the pairs of each chunk through
+// explain_pairs_kernel in windows whose results fit kSimWindowBytes.  Slots: the keys, pair descriptors and results use the similar
+// calls' SL_SIM_LIDS, SL_SIM_Q and SL_SIM_LOUT (no call keeps anything in them), the count rows the Gram workspace.
+int mr_explain(mr_handle* h, int model, const int32_t* user_idx, const int32_t* song_ids, int n, int m, int32_t* out_id, double* out_term,
+               int64_t* out_num, int32_t* out_len, int32_t* out_count, int64_t* out_total, double* out_score) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (h->windowed) return fail(h, MR_ERR_STATE, "explanations are not available on a handle with a song window (its song ids are rotated)");
+  if (model != MR_UBM && model != MR_IBM) return fail(h, MR_ERR_BAD_ARG, "model %d: explanations exist for MR_UBM and MR_IBM only", model);
+  if (m < 1 || m > 1024) return fail(h, MR_ERR_BAD_ARG, "m = %d outside [1, 1024]", m);
+  if (n < 0) return fail(h, MR_ERR_BAD_ARG, "n = %d < 0", n);
+  if (n == 0) return MR_OK;
+  if (!user_idx || !song_ids || !out_id || !out_term || !out_num || !out_len || !out_count || !out_total || !out_score)
+    return fail(h, MR_ERR_BAD_ARG, "null pair or output array");
+  for (int r = 0; r < n; ++r) {
+    if (user_idx[r] < 0 || user_idx[r] >= h->U) return fail(h, MR_ERR_BAD_ARG, "pair %d: test user index %d outside [0,%d)", r, user_idx[r], h->U);
+    if (song_ids[r] < 0 || song_ids[r] >= h->S) return fail(h, MR_ERR_BAD_ARG, "pair %d: song id %d outside [0,%d)", r, song_ids[r], h->S);
+  }
+  const bool ubm = model == MR_UBM;
+  if ((rc = ubm ? ensure_sqrt_users(h) : ensure_sqrt_songs(h))) return rc;
+  cudaStream_t st = h->stream;
+  const int32_t* key_of = ubm ? user_idx : song_ids;
+  const int32_t* other_of = ubm ? song_ids : user_idx;
+  // the pairs sorted by key; keys[i] is the i-th distinct key, its pairs are order[kbeg[i] .. kbeg[i + 1])
+  std::vector<int> order(static_cast<size_t>(n));
+  std::iota(order.begin(), order.end(), 0);
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return key_of[a] < key_of[b]; });
+  std::vector<int> keys, kbeg;
+  for (int p = 0; p < n; ++p)
+    if (p == 0 || key_of[order[p]] != keys.back()) { keys.push_back(key_of[order[p]]); kbeg.push_back(p); }
+  kbeg.push_back(n);
+  const int n_keys = static_cast<int>(keys.size());
+
+  // results of a window of W pairs: term f64 [W][m] | num i64 [W][m] | total i64 [W] | score f64 [W] | id i32 [W][m] | len i32 [W] | count i32 [W]
+  const size_t pair_bytes = static_cast<size_t>(m) * 20 + 24;
+  const int W = static_cast<int>(std::max<size_t>(1, std::min<size_t>(static_cast<size_t>(n), kSimWindowBytes / pair_bytes)));
+  const size_t Wm = static_cast<size_t>(W) * m;
+  auto at = [&](char* b) {
+    ExplainOut o;
+    o.term = reinterpret_cast<double*>(b);
+    o.num = reinterpret_cast<long long*>(o.term + Wm);
+    o.total = o.num + Wm;
+    o.score = reinterpret_cast<double*>(o.total + W);
+    o.id = reinterpret_cast<int*>(o.score + W);
+    o.len = o.id + Wm;
+    o.count = o.len + W;
+    return o;
+  };
+  char* base = nullptr; int2* d_pairs = nullptr; int* d_keys = nullptr;
+  if ((rc = slot_alloc(h, mr_handle::SL_SIM_LOUT, &base, W * pair_bytes)) || (rc = slot_alloc(h, mr_handle::SL_SIM_Q, &d_pairs, static_cast<size_t>(W))))
+    return rc;
+  const CountRows cr = ubm ? user_count_rows(h) : song_count_rows(h);
+  int C = 0;
+  if ((rc = count_chunk(h, cr, sizeof(int), n_keys, "explanations", &C))) return rc;
+  if ((rc = slot_alloc(h, mr_handle::SL_SIM_LIDS, &d_keys, static_cast<size_t>(C)))) return rc;
+  const ExplainArgs a{d_keys, d_pairs, h->d_g, cr.ld, ubm ? h->d_csc_ptr : h->d_te_ptr, ubm ? h->d_csc_idx : h->d_te_col, h->d_te_ptr,
+                      h->d_te_col, ubm ? h->d_simu_squ : h->d_sim_sqd, ubm ? h->d_simu_sqt : h->d_sim_sqd, ubm ? h->d_qv : h->d_qd,
+                      ubm ? h->d_rsa : h->d_rsd};
+  const ExplainOut dev = at(base);
+  std::vector<char> hb(W * pair_bytes);
+  const ExplainOut hst = at(hb.data());
+  std::vector<int2> desc(static_cast<size_t>(W));
+  for (int k0 = 0; k0 < n_keys; k0 += C) {
+    const int nc = std::min(C, n_keys - k0);
+    MR_CUDA(h, cudaMemcpyAsync(d_keys, keys.data() + k0, static_cast<size_t>(nc) * sizeof(int), cudaMemcpyHostToDevice, st));
+    if ((rc = count_rows(h, cr, d_keys, nc))) return rc;
+    h->explain_rows += nc;
+    int ki = k0;
+    for (int w0 = kbeg[k0]; w0 < kbeg[k0 + nc]; w0 += W) {
+      const int nw = std::min(W, kbeg[k0 + nc] - w0);
+      for (int j = 0; j < nw; ++j) {
+        while (kbeg[ki + 1] <= w0 + j) ++ki;
+        desc[j] = make_int2(ki - k0, other_of[order[w0 + j]]);
+      }
+      MR_CUDA(h, cudaMemcpyAsync(d_pairs, desc.data(), static_cast<size_t>(nw) * sizeof(int2), cudaMemcpyHostToDevice, st));
+      {
+        PhaseTimer t(h, MR_T_TOPK);
+        MR_LAUNCH(h, launch_explain_pairs(model, a, nw, m, dev, st));
+      }
+      const size_t nwm = static_cast<size_t>(nw) * m;
+      MR_CUDA(h, cudaMemcpyAsync(hst.term, dev.term, nwm * sizeof(double), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.num, dev.num, nwm * sizeof(long long), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.id, dev.id, nwm * sizeof(int), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.total, dev.total, static_cast<size_t>(nw) * sizeof(long long), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.score, dev.score, static_cast<size_t>(nw) * sizeof(double), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.len, dev.len, static_cast<size_t>(nw) * sizeof(int), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaMemcpyAsync(hst.count, dev.count, static_cast<size_t>(nw) * sizeof(int), cudaMemcpyDeviceToHost, st));
+      MR_CUDA(h, cudaStreamSynchronize(st));
+      for (int j = 0; j < nw; ++j) {   // into the caller's rows
+        const size_t r = static_cast<size_t>(order[w0 + j]), o = static_cast<size_t>(j) * m;
+        memcpy(out_id + r * m, hst.id + o, static_cast<size_t>(m) * sizeof(int32_t));
+        memcpy(out_term + r * m, hst.term + o, static_cast<size_t>(m) * sizeof(double));
+        memcpy(out_num + r * m, hst.num + o, static_cast<size_t>(m) * sizeof(int64_t));
+        out_len[r] = hst.len[j]; out_count[r] = hst.count[j]; out_total[r] = hst.total[j]; out_score[r] = hst.score[j];
+      }
+    }
+  }
+  MR_CUDA(h, cudaStreamSynchronize(st));
+  return MR_OK;
 }
 
 int mr_score_dense(mr_handle* h, int model, double* out_UxS) {
@@ -2434,11 +2560,11 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[24] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[25] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
                          h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
-                         h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows};
-  for (int i = 0; i < n && i < 24; ++i) out[i] = v[i];
+                         h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows, h->explain_rows};
+  for (int i = 0; i < n && i < 25; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

@@ -20,6 +20,7 @@ import ctypes as C
 import io
 import sys
 from dataclasses import dataclass
+from typing import NamedTuple
 
 import numpy as np
 
@@ -64,6 +65,19 @@ class Model:
         sn = self.songs if self.songs is not None else list(range(self.scores.shape[1]))
         for a, b, c in zip(u.tolist(), s.tolist(), v.tolist()):
             yield un[a], (sn[b], c)
+
+
+class Explanation(NamedTuple):
+    """The contributors of (test user, song) scores (mr_explain, DESIGN.md §4.9), row r for pair r: the first len[r] of count[r]
+    contributors by term descending then id ascending (id -1, term 0.0, num 0 past len[r]); total[r] = the sum of num over all of them, the
+    score's exact numerator; score[r] = the library's score of the pair (NaN for a listened pair)."""
+    id: np.ndarray        # [n, m] int32: train users (UBM) or the user's visible songs (IBM)
+    term: np.ndarray      # [n, m] float64: the cosine weight of the contributor, as the reference computes it
+    num: np.ndarray       # [n, m] int64: the contributor's term of the fixed-point numerator (DESIGN.md §3)
+    len: np.ndarray       # [n] int32
+    count: np.ndarray     # [n] int32
+    total: np.ndarray     # [n] int64
+    score: np.ndarray     # [n] float64
 
 
 def _p(a):
@@ -342,6 +356,20 @@ class MusicRecommender:
         self._check(self._lib.mr_similar_users(self._h, _p(ids), n, k, _p(user), _p(score), _p(ln)))
         return user, score, ln
 
+    def explain(self, model: int, users, songs, m: int = 10) -> Explanation:
+        """Why song songs[r] scores what it does for test user users[r] (indices into the current test shard): the contributors of the
+        UBM score (train listeners of the song who share songs with the user) or of the IBM score (the user's visible songs co-listened
+        with it), each with its cosine weight and its exact fixed-point term, the m largest weights listed (mr_explain, DESIGN.md §4.9)."""
+        u = np.ascontiguousarray(users, np.int32).reshape(-1)
+        s = np.ascontiguousarray(songs, np.int32).reshape(-1)
+        if len(u) != len(s):
+            raise ValueError(f"{len(u)} users but {len(s)} songs")
+        n = len(u)
+        out = Explanation(np.empty((n, m), np.int32), np.empty((n, m), np.float64), np.empty((n, m), np.int64), np.empty(n, np.int32),
+                          np.empty(n, np.int32), np.empty(n, np.int64), np.empty(n, np.float64))
+        self._check(self._lib.mr_explain(self._h, model, _p(u), _p(s), n, m, *[_p(a) for a in out]))
+        return out
+
     def getTopKMulti(self, specs, k: int = 500):
         """getTopK for every entry of a model set (model, param, seed) from one scoring of the shard (mr_topk_multi, DESIGN.md §4.6):
         one (song [U,k] int32, score [U,k] f64, len [U]) per entry, each equal to getTopK(model, k, param, seed)."""
@@ -497,12 +525,12 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 24)()
-        self._lib.mr_get_info(self._h, v, 24)
+        v = (C.c_int64 * 25)()
+        self._lib.mr_get_info(self._h, v, 25)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
                          "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows",
-                         "similar_user_short_rows", "similar_user_long_rows"], list(v)))
+                         "similar_user_short_rows", "similar_user_long_rows", "explain_rows"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -809,6 +837,74 @@ def similar_users_host(ds: Dataset, users, k: int):
         out_score[r, :m] = w[rank[:m]]
         out_len[r] = m
     return out_user, out_score, out_len
+
+
+def explain_host(ds: Dataset, model: int, users, songs, m: int) -> Explanation:
+    """numpy mirror of mr_explain.  UBM: the train listeners v of s with c = |I_u ∩ I_v| > 0, term = c / (sqrt(deg_te[u]) * sqrt(deg_tr[v])),
+    num = c * q_24(deg_tr[v]); IBM: u's visible songs j with g = |U_s^train ∩ U_j^train| > 0, term = g / (sqrt(d_s) * sqrt(d_j)),
+    num = g * q_26(d_j), d = deg_song; each term in that operation order (0 where the denominator is 0), ranked by term descending then id
+    ascending.  q_k(x) = rint(2^k / sqrt(x)) (0 for x = 0) as the oracle's mro_q; score = float(total) * 2^-k / sqrt(deg_te[u] or d_s)."""
+    users = np.asarray(users, np.int64).reshape(-1)
+    songs = np.asarray(songs, np.int64).reshape(-1)
+    n = len(users)
+    out = Explanation(np.full((n, m), -1, np.int32), np.zeros((n, m), np.float64), np.zeros((n, m), np.int64), np.zeros(n, np.int32),
+                      np.zeros(n, np.int32), np.zeros(n, np.int64), np.zeros(n, np.float64))
+    tr_ptr = np.asarray(ds.tr_ptr, np.int64)
+    tr_col = np.asarray(ds.tr_col, np.int64)
+    te_ptr = np.asarray(ds.te_ptr, np.int64)
+    te_col = np.asarray(ds.te_col, np.int64)
+    owner = np.repeat(np.arange(ds.T), np.diff(tr_ptr))                    # train user of every train entry
+    order = np.argsort(tr_col, kind="stable")                              # inverted index: listeners of a song, ascending
+    csc_ptr = np.concatenate([[0], np.cumsum(np.bincount(tr_col, minlength=ds.S))])
+    listeners = owner[order]
+    deg_tr = np.asarray(ds.deg_tr, np.int64)
+    deg_te = np.asarray(ds.deg_te, np.int64)
+    deg = np.asarray(ds.deg_song, np.int64)
+    kq = 24 if model == _lib.MR_UBM else 26
+
+    def q(d):
+        with np.errstate(divide="ignore"):
+            return np.where(d > 0, np.rint(2.0 ** kq / np.sqrt(d.astype(np.float64))), 0).astype(np.int64)
+
+    def rs(d):
+        return (1.0 / 2.0 ** kq) / np.sqrt(np.float64(d)) if d > 0 else 0.0
+
+    for r, (u, s) in enumerate(zip(users, songs)):
+        iu = te_col[te_ptr[u]:te_ptr[u + 1]]
+        if s in iu:                                                        # a listened pair: no element of the model (MR:109)
+            out.score[r] = np.nan
+            continue
+        if model == _lib.MR_UBM:
+            seen = [listeners[csc_ptr[j]:csc_ptr[j + 1]] for j in iu]
+            cnt = np.bincount(np.concatenate(seen) if seen else np.zeros(0, np.int64), minlength=ds.T)
+            ids = listeners[csc_ptr[s]:csc_ptr[s + 1]]
+            c = cnt[ids]
+            den = np.sqrt(np.float64(deg_te[u])) * np.sqrt(deg_tr[ids].astype(np.float64))
+            dq = deg_tr[ids]
+            factor = rs(deg_te[u])
+        else:
+            hist = [tr_col[tr_ptr[v]:tr_ptr[v + 1]] for v in listeners[csc_ptr[s]:csc_ptr[s + 1]]]
+            gram = np.bincount(np.concatenate(hist) if hist else np.zeros(0, np.int64), minlength=ds.S)
+            ids = iu
+            c = gram[ids]
+            den = np.sqrt(np.float64(deg[s])) * np.sqrt(deg[ids].astype(np.float64))
+            dq = deg[ids]
+            factor = rs(deg[s])
+        keep = c > 0
+        ids, c, den, dq = ids[keep], c[keep], den[keep], dq[keep]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            term = np.where(den != 0, c.astype(np.float64) / den, 0.0)
+        num = c.astype(np.int64) * q(dq)
+        rank = np.lexsort((ids, -term))
+        k = min(m, len(rank))
+        out.id[r, :k] = ids[rank[:k]]
+        out.term[r, :k] = term[rank[:k]]
+        out.num[r, :k] = num[rank[:k]]
+        out.len[r] = k
+        out.count[r] = len(ids)
+        out.total[r] = int(num.sum())
+        out.score[r] = np.float64(out.total[r]) * factor
+    return out
 
 
 def evaluate_map(scores: np.ndarray, ds: Dataset, n_thresholds: int = 10) -> float:

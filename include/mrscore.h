@@ -137,8 +137,9 @@ int mr_peer_alloc(mr_handle* h, uint64_t bytes, void** dev_ptr, unsigned char* h
 int mr_peer_open(mr_handle* h, const unsigned char* handle_64, void** dev_ptr);                  /* map a peer's buffer into this process */
 int mr_peer_close(mr_handle* h, void* dev_ptr);
 
-/* Cosine similarities with the normalisation fused into the GEMM epilogue (fp32): user-user MR:140-149 and rows [s0,s1) of
- * item-item MR:230-239 (denominator uses the train+test listener counts, MR:237). */
+/* Cosine similarities in fp32: user-user MR:140-149 and rows [s0,s1) of item-item MR:230-239 (denominator uses the train+test
+ * listener counts, MR:237).  Each entry is float(c) * (rs(a) * rs(b)) for the count c and the degrees a, b of its row and column, with
+ * rs(d) = float(1.0 / sqrt((double) d)) and rs(0) = 0. */
 int mr_similarity_ubm(mr_handle* h, float* out_UxT);
 int mr_similarity_ibm(mr_handle* h, int s0, int s1, float* out_rows);
 

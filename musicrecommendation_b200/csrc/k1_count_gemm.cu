@@ -12,9 +12,8 @@
 //   warp 2   TMEM allocator (2 accumulator stages x BN columns, so the epilogue of tile i overlaps the MMAs of tile i+1)
 //   warps 4-7 epilogue    : tcgen05.ld 32x32b -> registers -> fused output transform -> global
 // Epilogue modes:
-//   EPI_I32      int32 C row-major                      (parity probes mr_counts_*, Gram rows consumed by the IBM aggregation)
+//   EPI_I32      int32 C row-major                      (count rows: IBM aggregation, similar songs / users, explanations, parity probes)
 //   EPI_U16_T    uint16 C^T  (Ct[n][m], m contiguous)   (UBM: train-user-major count panel consumed by the K2 gather)
-//   EPI_COS_F32  float   C[m][n] / (sqrt(da[m]) * sqrt(db[n]))   fused cosine normalisation (similarity products, MR:147-148 / 237-238)
 //   EPI_I32_SCATTER  int32 rows stored into per-owner receive slots (local or NVLink peer memory): the reduce-scatter of the K-split
 //                item-item sweep fused into the epilogue (coalesced 128-byte row segments via a shared-memory transpose)
 //   EPI_ACC_U64  u64 out (+)= C << shift                         byte-plane accumulation of the weighted Gram Gq (item-space head rows)
@@ -46,19 +45,18 @@ struct GemmParams {
   int M, N;            // logical output extent (rows of A / rows of B that are real)
   int num_k_blocks;    // K_pad / 128
   int num_m_tiles, num_n_tiles;
-  void* out;           // int32* / uint16_t* / float*
+  void* out;           // int32* / uint16_t* / unsigned long long*
   long long ld;        // leading dimension of `out` in elements
-  const float* rsa;    // EPI_COS_F32: 1/sqrt(deg) per A row, per B row (0 where deg == 0)
-  const float* rsb;
   int32_t* slots[8];   // EPI_I32_SCATTER: row m goes to slots[m / rows_per_owner] + (m % rows_per_owner) * ld  (peer or local memory)
   int rows_per_owner;
   int shift;           // EPI_ACC_U64: out = (plane 0 ? 0 : out) + (u64(acc) << shift)  (byte-plane weighted Gram)
   int accumulate;
 };
 
+// p is __grid_constant__ so that the run-time index into p.slots reads the parameter bank in place instead of a per-thread local copy of p
 template <int BN, int EPI>
 __global__ void __launch_bounds__(kGemmThreads, 1)
-count_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, GemmParams p) {
+count_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ GemmParams p) {
   using Cfg = GemmCfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   // 128 B swizzle atoms need 1024 B alignment
@@ -211,12 +209,6 @@ count_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                 dst[j] = (p.accumulate ? dst[j] : 0ULL) + (static_cast<unsigned long long>(r[j]) << p.shift);
             }
           }
-        } else {  // EPI_COS_F32
-          if (m < p.M) {
-            const float ra = p.rsa[m];
-            float* dst = reinterpret_cast<float*>(p.out) + static_cast<long long>(m) * p.ld + n0;
-            for (int j = 0; j < 32 && n0 + j < p.N; ++j) dst[j] = static_cast<float>((int)r[j]) * (ra * p.rsb[n0 + j]);
-          }
         }
       }
       tc_fence_before();
@@ -321,7 +313,7 @@ static cudaError_t launch_gemm_t(const CUtensorMap& ta, const CUtensorMap& tb, c
 }
 
 int launch_count_gemm(const uint8_t* A, long long a_rows, const uint8_t* B, long long b_rows, long long pitch, int M, int N,
-                      int epi, void* out, long long ld, const float* rsa, const float* rsb, int num_sms, cudaStream_t st,
+                      int epi, void* out, long long ld, int num_sms, cudaStream_t st,
                       int shift, int accumulate, int32_t* const* slots, int n_slots, int rows_per_owner) {
   if (pitch % kBK != 0 || M <= 0 || N <= 0) return -3;
   const int bn = (N > 128) ? 256 : 128;
@@ -335,7 +327,7 @@ int launch_count_gemm(const uint8_t* A, long long a_rows, const uint8_t* B, long
   p.num_k_blocks = static_cast<int>(pitch / kBK);
   p.num_m_tiles = (M + kBM - 1) / kBM;
   p.num_n_tiles = (N + bn - 1) / bn;
-  p.out = out; p.ld = ld; p.rsa = rsa; p.rsb = rsb; p.shift = shift; p.accumulate = accumulate;
+  p.out = out; p.ld = ld; p.shift = shift; p.accumulate = accumulate;
   for (int i = 0; i < 8; ++i) p.slots[i] = (slots && i < n_slots) ? slots[i] : nullptr;
   p.rows_per_owner = rows_per_owner > 0 ? rows_per_owner : 1;
   if (epi == EPI_I32_SCATTER && (!slots || n_slots < 1 || n_slots > 8 || static_cast<long long>(n_slots) * p.rows_per_owner < M)) return -4;
@@ -344,14 +336,12 @@ int launch_count_gemm(const uint8_t* A, long long a_rows, const uint8_t* B, long
     e = epi == EPI_I32 ? launch_gemm_t<256, EPI_I32>(ta, tb, p, num_sms, st)
       : epi == EPI_U16_T ? launch_gemm_t<256, EPI_U16_T>(ta, tb, p, num_sms, st)
       : epi == EPI_ACC_U64 ? launch_gemm_t<256, EPI_ACC_U64>(ta, tb, p, num_sms, st)
-      : epi == EPI_I32_SCATTER ? launch_gemm_t<256, EPI_I32_SCATTER>(ta, tb, p, num_sms, st)
-                         : launch_gemm_t<256, EPI_COS_F32>(ta, tb, p, num_sms, st);
+                         : launch_gemm_t<256, EPI_I32_SCATTER>(ta, tb, p, num_sms, st);
   } else {
     e = epi == EPI_I32 ? launch_gemm_t<128, EPI_I32>(ta, tb, p, num_sms, st)
       : epi == EPI_U16_T ? launch_gemm_t<128, EPI_U16_T>(ta, tb, p, num_sms, st)
       : epi == EPI_ACC_U64 ? launch_gemm_t<128, EPI_ACC_U64>(ta, tb, p, num_sms, st)
-      : epi == EPI_I32_SCATTER ? launch_gemm_t<128, EPI_I32_SCATTER>(ta, tb, p, num_sms, st)
-                         : launch_gemm_t<128, EPI_COS_F32>(ta, tb, p, num_sms, st);
+                         : launch_gemm_t<128, EPI_I32_SCATTER>(ta, tb, p, num_sms, st);
   }
   return e == cudaSuccess ? 0 : -100 - static_cast<int>(e);
 }

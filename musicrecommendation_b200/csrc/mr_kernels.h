@@ -16,12 +16,12 @@ constexpr int kTailSubBatch = 592; // tail scatter runs per 592 users so its ato
 __host__ __device__ inline long long ct_index(long long T, int v, int b) { (void)T; return static_cast<long long>(v) * kUserBatch + b; }
 __host__ __device__ inline long long wi_index(long long T, int v, int b) { (void)T; return static_cast<long long>(v) * kUserBatch + b; }
 
-enum { EPI_I32 = 0, EPI_U16_T = 1, EPI_COS_F32 = 2, EPI_ACC_U64 = 3, EPI_I32_SCATTER = 4 };
+enum { EPI_I32 = 0, EPI_U16_T = 1, EPI_ACC_U64 = 3, EPI_I32_SCATTER = 4 };
 enum { MODEL_UBM = 0, MODEL_IBM = 1, MODEL_LC = 2, MODEL_AGG = 3, MODEL_STOCH = 4 };
 
 // ---- K1 (k1_count_gemm.cu)
 int launch_count_gemm(const uint8_t* A, long long a_rows, const uint8_t* B, long long b_rows, long long pitch, int M, int N,
-                      int epi, void* out, long long ld, const float* rsa, const float* rsb, int num_sms, cudaStream_t st,
+                      int epi, void* out, long long ld, int num_sms, cudaStream_t st,
                       int shift = 0, int accumulate = 0, int32_t* const* slots = nullptr, int n_slots = 0, int rows_per_owner = 0);
 int launch_expand_rows_weighted(const long long* ptr, const int* idx, const uint32_t* weight, int plane, int n_rows, long long pitch,
                                 uint8_t* out, cudaStream_t st);

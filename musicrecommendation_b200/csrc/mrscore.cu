@@ -23,7 +23,6 @@
 #include <cstring>
 #include <limits>
 #include <numeric>
-#include <optional>
 #include <string>
 #include <queue>
 #include <mutex>
@@ -73,7 +72,7 @@ struct mr_handle {
   cudaStream_t pre_extra[kPreExtraStreams] = {}; cudaEvent_t ev_pre_extra[kPreExtraStreams] = {};   // extra streams of the in-place row build (chunks rotate over them)
   HeadExceptions pend_ex{};
   unsigned int* d_topk_stats = nullptr;   // [3] counters of the top-k select since mr_load (BlendParams::stats)
-  uint32_t *d_qv = nullptr, *d_qd = nullptr; double* d_rsd = nullptr; float *d_rsv_f = nullptr, *d_rsd_f = nullptr, *d_rsd_up = nullptr;
+  uint32_t *d_qv = nullptr, *d_qd = nullptr; double* d_rsd = nullptr; float* d_rsd_up = nullptr;
   std::vector<int32_t> deg_song, deg_song_train;
   struct SongInfo { int head; uint32_t v; };   // head row or -1; v = q_26(d_s) of a head song, train listeners of a tail song
   int2* d_song_info = nullptr;                 // the same records on the device (k7_testlists.cu)
@@ -103,10 +102,10 @@ struct mr_handle {
   // test shard (freed / reallocated by mr_set_test_users)
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard, its results and the workspaces: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
-  enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_RSA_F, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_CNT, SL_SIMF, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
+  enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
-  long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr; float* d_rsa_f = nullptr;
+  long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
   std::vector<long long> batch_row_off; int* d_rows = nullptr; int max_batch_rows = 0;
   long long pair_index_base = 0, n_pairs_total = 0;
@@ -115,7 +114,7 @@ struct mr_handle {
   uint32_t* d_wi = nullptr;             // IBM user-space weighted counts u32[T][128] (sparse engine)
   unsigned int* d_carry_count = nullptr; uint2* d_carry_events = nullptr; unsigned int carry_cap = 1u << 20; unsigned int* h_carry_seen = nullptr;
   uint64_t* d_sel = nullptr; long long sel_pitch = 0; int32_t* d_g = nullptr;   // d_g / d_Aj: the Gram workspace, slots SL_GRAM_G / SL_GRAM_A
-  double* d_dense = nullptr; int32_t* d_cnt = nullptr; float* d_simf = nullptr;
+  double* d_dense = nullptr;
   // results
   TopkOut out{}; int out_k = 0; bool have_topk = false; size_t out_pack_bytes = 0;   // the single-model result, a TopkBlock in SL_OUT_PACK
   // results of the last mr_topk_multi_device: entry i is the i-th TopkBlock of the SL_MULTI_OUT slot
@@ -237,7 +236,6 @@ struct Scratch {
 
 inline uint32_t q_of(int32_t deg, double scale) { return deg <= 0 ? 0u : static_cast<uint32_t>(llrint(scale / std::sqrt(static_cast<double>(deg)))); }
 inline double rs_of(int32_t deg, double inv) { return deg <= 0 ? 0.0 : inv / std::sqrt(static_cast<double>(deg)); }
-inline float rsf_of(int32_t deg) { return deg <= 0 ? 0.0f : static_cast<float>(1.0 / std::sqrt(static_cast<double>(deg))); }
 inline long long round_up(long long x, long long m) { return (x + m - 1) / m * m; }
 
 // f(lo, hi) over disjoint row ranges on a few host threads.  The per-shard host work of mr_set_test_users (CSR validation, id rotation,
@@ -296,28 +294,17 @@ struct PhaseTimer {   // CUDA events on the library stream (or the given one) ar
   }
 };
 
-__global__ void ct_to_i32_kernel(const uint16_t* __restrict__ ct, int n_train, int nb, int32_t* __restrict__ out) {
-  // out[b][v] = Ct[v][b]
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < static_cast<long long>(nb) * n_train;
+// In place over n_rows count rows ld apart: c -> float(c) * (rs(sq_row[rows[r]]) * rs(sq_col[j])) with rs(x) = float(1.0 / x), 0 where x = 0
+// (degree 0).  The sqrt tables are correctly rounded (launch_sqrt_deg) and the build uses --fmad=false, so each value has the bits of
+// the same formula on the host.  An element's int32 and its float share the 4 bytes, read and written by one thread.
+__global__ void count_to_cos_kernel(int32_t* __restrict__ g, long long ld, const int* __restrict__ rows, int n_rows, int n_cols,
+                                    const double* __restrict__ sq_row, const double* __restrict__ sq_col) {
+  auto rs = [](double x) { return x > 0 ? static_cast<float>(1.0 / x) : 0.0f; };
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < static_cast<long long>(n_rows) * n_cols;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int b = static_cast<int>(i / n_train), v = static_cast<int>(i % n_train);
-    out[i] = ct[ct_index(n_train, v, b)];
-  }
-}
-__global__ void ct_to_cos_kernel(const uint16_t* __restrict__ ct, int n_train, int nb, const float* __restrict__ rsa,
-                                 const float* __restrict__ rsv, float* __restrict__ out) {
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < static_cast<long long>(nb) * n_train;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int b = static_cast<int>(i / n_train), v = static_cast<int>(i % n_train);
-    out[i] = static_cast<float>(ct[ct_index(n_train, v, b)]) * (rsa[b] * rsv[v]);
-  }
-}
-__global__ void gram_to_cos_kernel(const int32_t* __restrict__ g, long long ldg, const int* __restrict__ rows, int n_rows, int n_songs,
-                                   const float* __restrict__ rsd, float* __restrict__ out) {
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < static_cast<long long>(n_rows) * n_songs;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int r = static_cast<int>(i / n_songs), s = static_cast<int>(i % n_songs);
-    out[i] = static_cast<float>(g[r * ldg + s]) * (rsd[rows[r]] * rsd[s]);
+    const int r = static_cast<int>(i / n_cols), j = static_cast<int>(i % n_cols);
+    int32_t& e = g[r * ld + j];
+    e = __float_as_int(static_cast<float>(e) * (rs(sq_row[rows[r]]) * rs(sq_col[j])));
   }
 }
 __global__ void iota_kernel(int* p, int start, int n) {
@@ -334,7 +321,7 @@ int count_ubm_batch(mr_handle* h, int b0, int nb) {
     }
     PhaseTimer t(h, MR_T_COUNT);
     MR_LAUNCH(h, launch_count_gemm(h->d_Ate, kUserBatch, h->d_Atr, h->T, h->pitchS, kUserBatch, h->T, EPI_U16_T, h->d_ct, kUserBatch,
-                                   nullptr, nullptr, h->num_sms, h->stream));
+                                   h->num_sms, h->stream));
   } else {
     PhaseTimer t(h, MR_T_COUNT);
     MR_LAUNCH(h, launch_sparse_count_u16t(h->d_te_ptr, h->d_te_col, b0, nb, h->d_csc_ptr, h->d_csc_idx, h->d_ct, h->T, h->stream));
@@ -362,8 +349,8 @@ int count_rows(mr_handle* h, const CountRows& cr, const int* d_rows, int n_rows)
       MR_LAUNCH(h, launch_expand_rows(cr.q_ptr, cr.q_idx, d_rows, 0, n_rows, rows_pad, cr.pitch, h->d_Aj, h->stream));
     }
     PhaseTimer t(h, MR_T_COUNT);
-    MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, cr.B, cr.n_cols, cr.pitch, n_rows, cr.n_cols, EPI_I32, h->d_g, cr.ld, nullptr,
-                                   nullptr, h->num_sms, h->stream));
+    MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, cr.B, cr.n_cols, cr.pitch, n_rows, cr.n_cols, EPI_I32, h->d_g, cr.ld, h->num_sms,
+                                   h->stream));
   } else {
     PhaseTimer t(h, MR_T_COUNT);
     for (int r0 = 0; r0 < n_rows; r0 += 32768) {
@@ -484,11 +471,11 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
         if (lrc) return fail(h, MR_ERR_CUDA, "launch_expand_rows failed");
       }
       PhaseTimer t(h, MR_T_COUNT, st);
-      int lrc = launch_count_gemm(a_rows, n_pad, h->d_AtrT, h->S, h->pitchT, nr, h->S, EPI_I32, g_stage, h->spitch, nullptr, nullptr, h->num_sms, st);
+      int lrc = launch_count_gemm(a_rows, n_pad, h->d_AtrT, h->S, h->pitchT, nr, h->S, EPI_I32, g_stage, h->spitch, h->num_sms, st);
       h->launches++;
       for (int plane = 0; plane < n_planes && !lrc; ++plane) {
         lrc = launch_count_gemm(a_rows, n_pad, b_plane + static_cast<size_t>(plane) * h->S * h->pitchT, h->S, h->pitchT, nr, h->S, EPI_ACC_U64,
-                                gq_stage, h->spitch, nullptr, nullptr, h->num_sms, st, 8 * plane, plane > 0);
+                                gq_stage, h->spitch, h->num_sms, st, 8 * plane, plane > 0);
         h->launches++;
       }
       if (lrc) return fail(h, MR_ERR_CUDA, "launch_count_gemm failed: rc=%d (%s)", lrc, cudaGetErrorString(cudaGetLastError()));
@@ -1180,9 +1167,8 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
   // fixed-point cosine factors
   std::vector<uint32_t> qv(T), qd(S);
   std::vector<double> rsd(S);
-  std::vector<float> rsvf(T), rsdf(S);
-  for (int v = 0; v < T; ++v) { qv[v] = q_of(deg_train[v], kQScaleUbm); rsvf[v] = rsf_of(deg_train[v]); h->max_qv = std::max(h->max_qv, qv[v]); }
-  for (int s = 0; s < S; ++s) { qd[s] = q_of(deg_song_all[s], kQScaleIbm); rsd[s] = rs_of(deg_song_all[s], kQInvIbm); rsdf[s] = rsf_of(deg_song_all[s]); }
+  for (int v = 0; v < T; ++v) { qv[v] = q_of(deg_train[v], kQScaleUbm); h->max_qv = std::max(h->max_qv, qv[v]); }
+  for (int s = 0; s < S; ++s) { qd[s] = q_of(deg_song_all[s], kQScaleIbm); rsd[s] = rs_of(deg_song_all[s], kQInvIbm); }
   h->song_qsum.assign(S, 0);
   for (int s = 0; s < S; ++s)
     for (long long i = csc_ptr[s]; i < csc_ptr[s + 1]; ++i) h->song_qsum[s] += qv[csc_idx[i]];
@@ -1223,8 +1209,6 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
     if ((rc = dev_upload(h, &h->d_rsd_up, up.data(), up.size(), h->allocs))) return rc;
     MR_CUDA(h, cudaStreamSynchronize(h->stream));
   }
-  if ((rc = dev_upload(h, &h->d_rsv_f, rsvf.data(), rsvf.size(), h->allocs))) return rc;
-  if ((rc = dev_upload(h, &h->d_rsd_f, rsdf.data(), rsdf.size(), h->allocs))) return rc;
   if ((rc = dev_upload(h, &h->d_item_song, it_song.data(), it_song.size(), h->allocs))) return rc;
   if ((rc = dev_upload(h, &h->d_item_begin, it_begin.data(), it_begin.size(), h->allocs))) return rc;
   if ((rc = dev_upload(h, &h->d_item_len, it_len.data(), it_len.size(), h->allocs))) return rc;
@@ -1331,10 +1315,10 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   h->deg_test.assign(deg_test, deg_test + U); h->simu_squ_ok = false;
   h->h_te_ptr.assign(te_rowptr, te_rowptr + U + 1);
   if (h->windowed) h->h_te_col.resize(static_cast<size_t>(nnz)); else h->h_te_col.assign(te_col, te_col + nnz);   // a window rewrites every row below
-  std::vector<double> rsa(U); std::vector<float> rsaf(U);
+  std::vector<double> rsa(U);
   std::vector<long long> pair_base(static_cast<size_t>(U) + 1);
   pair_base[0] = pair_index_base;
-  parallel_rows(U, [&](int lo, int hi) { for (int u = lo; u < hi; ++u) { rsa[u] = rs_of(deg_test[u], kQInvUbm); rsaf[u] = rsf_of(deg_test[u]); } });
+  parallel_rows(U, [&](int lo, int hi) { for (int u = lo; u < hi; ++u) rsa[u] = rs_of(deg_test[u], kQInvUbm); });
   for (int u = 0; u < U; ++u) pair_base[u + 1] = pair_base[u] + (h->S - (te_rowptr[u + 1] - te_rowptr[u]));   // unlistened songs of u (MR:109)
   h->pair_index_base = pair_index_base;
   h->n_pairs_total = n_pairs_total > 0 ? n_pairs_total : pair_base[U] - pair_index_base;
@@ -1388,7 +1372,6 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   if ((rc = slot_upload(h, mr_handle::SL_TE_COL, &h->d_te_col, h->h_te_col.data(), static_cast<size_t>(nnz)))) return rc;
   if ((rc = slot_upload(h, mr_handle::SL_TE_GROW, &h->d_te_grow, grow.data(), grow.size()))) return rc;
   if ((rc = slot_upload(h, mr_handle::SL_RSA, &h->d_rsa, rsa.data(), rsa.size()))) return rc;
-  if ((rc = slot_upload(h, mr_handle::SL_RSA_F, &h->d_rsa_f, rsaf.data(), rsaf.size()))) return rc;
   if ((rc = slot_upload(h, mr_handle::SL_PAIR_BASE, &h->d_pair_base, pair_base.data(), pair_base.size()))) return rc;
   if ((rc = slot_upload(h, mr_handle::SL_ROWS, &h->d_rows, rows_all.data(), rows_all.size()))) return rc;
   lap("uploads 1");
@@ -1449,74 +1432,6 @@ static int require_test(mr_handle* h) {
   if (!h) return MR_ERR_STATE;
   if (!h->loaded || !h->have_test) return fail(h, MR_ERR_STATE, "no data loaded (mr_load / mr_set_test_users)");
   return require_loaded(h);
-}
-
-// The UBM parity probes, not scoring: per 128-user batch the counts Ct as int32 (out_cnt) or cosines (out_sim; on the tensor engine
-// c / (sqrt|I_u| * sqrt|I_v|), MR:147-148, in the GEMM epilogue) to the caller's [U][T].  They bump gen: a later count pass scores anew.
-static int ubm_probe(mr_handle* h, int32_t* out_cnt, float* out_sim) {
-  int rc = require_test(h);
-  if (rc) return rc;
-  if (!out_cnt && !out_sim) return fail(h, MR_ERR_BAD_ARG, "null output");
-  const size_t ws = static_cast<size_t>(kUserBatch) * h->T;
-  if ((rc = out_cnt ? slot_alloc(h, mr_handle::SL_CNT, &h->d_cnt, ws) : slot_alloc(h, mr_handle::SL_SIMF, &h->d_simf, ws))) return rc;
-  ++h->gen;
-  const bool fused = out_sim && h->engine == MR_ENGINE_TENSOR;
-  for (int b0 = 0; b0 < h->U; b0 += kUserBatch) {
-    const int nb = std::min(kUserBatch, h->U - b0);
-    const long long off = static_cast<long long>(b0) * h->T;
-    std::optional<PhaseTimer> t;   // the conversion and the copy-out; the fused GEMM is not timed
-    if (fused) {
-      MR_LAUNCH(h, launch_expand_rows(h->d_te_ptr, h->d_te_col, nullptr, b0, nb, kUserBatch, h->pitchS, h->d_Ate, h->stream));
-      MR_LAUNCH(h, launch_count_gemm(h->d_Ate, kUserBatch, h->d_Atr, h->T, h->pitchS, nb, h->T, EPI_COS_F32, h->d_simf, h->T,
-                                     h->d_rsa_f + b0, h->d_rsv_f, h->num_sms, h->stream));
-    } else {
-      if ((rc = count_ubm_batch(h, b0, nb))) return rc;
-      t.emplace(h, MR_T_OTHER);
-      if (out_cnt) ct_to_i32_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_cnt);
-      else ct_to_cos_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_ct, h->T, nb, h->d_rsa_f + b0, h->d_rsv_f, h->d_simf);
-      h->launches++;
-    }
-    MR_CUDA(h, cudaMemcpyAsync(out_cnt ? static_cast<void*>(out_cnt + off) : static_cast<void*>(out_sim + off),   // both are 4-byte elements
-                               out_cnt ? static_cast<const void*>(h->d_cnt) : static_cast<const void*>(h->d_simf), static_cast<size_t>(nb) * h->T * 4,
-                               cudaMemcpyDeviceToHost, h->stream));
-    MR_CUDA(h, cudaStreamSynchronize(h->stream));
-  }
-  return MR_OK;
-}
-
-int mr_counts_ubm(mr_handle* h, int32_t* out_UxT) { return ubm_probe(h, out_UxT, nullptr); }
-int mr_similarity_ubm(mr_handle* h, float* out_UxT) { return ubm_probe(h, nullptr, out_UxT); }
-
-static int gram_range(mr_handle* h, int s0, int s1, int32_t* out_i32, float* out_f32) {
-  int rc = require_loaded(h);   // Gram rows need only the train replica
-  if (rc) return rc;
-  if (h->windowed) return fail(h, MR_ERR_STATE, "Gram rows are not available on a handle with a song window (its song ids are rotated)");
-  if (s0 < 0 || s1 > h->S || s0 > s1) return fail(h, MR_ERR_BAD_ARG, "song range [%d,%d) outside [0,%d)", s0, s1, h->S);
-  const int chunk = 1024;
-  int* d_ids = nullptr; float* d_f = nullptr;
-  Scratch tmp(h, h->stream);
-  if ((rc = tmp.alloc(&d_ids, chunk))) return rc;
-  if (out_f32 && (rc = tmp.alloc(&d_f, static_cast<size_t>(chunk) * h->S))) return rc;
-  if ((rc = ensure_gram_ws(h, chunk))) return rc;
-  for (int r0 = s0; r0 < s1; r0 += chunk) {
-    const int n = std::min(chunk, s1 - r0);
-    iota_kernel<<<(n + 255) / 256, 256, 0, h->stream>>>(d_ids, r0, n);
-    h->launches++;
-    if ((rc = gram_rows(h, d_ids, n))) return rc;
-    cudaError_t e;
-    if (out_i32) {
-      e = cudaMemcpy2DAsync(out_i32 + static_cast<long long>(r0 - s0) * h->S, static_cast<size_t>(h->S) * 4, h->d_g,
-                            static_cast<size_t>(h->ldg) * 4, static_cast<size_t>(h->S) * 4, n, cudaMemcpyDeviceToHost, h->stream);
-    } else {
-      gram_to_cos_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_g, h->ldg, d_ids, n, h->S, h->d_rsd_f, d_f);
-      h->launches++;
-      e = cudaMemcpyAsync(out_f32 + static_cast<long long>(r0 - s0) * h->S, d_f, static_cast<size_t>(n) * h->S * 4,
-                          cudaMemcpyDeviceToHost, h->stream);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "gram rows copy-out: %s", cudaGetErrorString(e));
-  }
-  return MR_OK;
 }
 
 int mr_gram_rows_device(mr_handle* h, int s0, int s1, int32_t** dev_out, int64_t* ld) {
@@ -1628,19 +1543,10 @@ static int gram_rows_scatter_impl(mr_handle* h, int s0, int s1, void* const* slo
   int32_t* slots[8];
   for (int i = 0; i < n_owners; ++i) slots[i] = static_cast<int32_t*>(slot_ptrs[i]);
   PhaseTimer t(h, MR_T_COUNT);
-  MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, h->d_AtrT, h->S, h->pitchT, n, h->S, EPI_I32_SCATTER, nullptr, ld, nullptr, nullptr, h->num_sms,
-                                 h->stream, 0, 0, slots, n_owners, rows_per_owner));
+  MR_LAUNCH(h, launch_count_gemm(h->d_Aj, rows_pad, h->d_AtrT, h->S, h->pitchT, n, h->S, EPI_I32_SCATTER, nullptr, ld, h->num_sms, h->stream, 0, 0,
+                                 slots, n_owners, rows_per_owner));
   if (sync) MR_CUDA(h, cudaStreamSynchronize(h->stream));
   return MR_OK;
-}
-
-int mr_counts_ibm(mr_handle* h, int s0, int s1, int32_t* out_rows) {
-  if (!out_rows) return fail(h, MR_ERR_BAD_ARG, "null output");
-  return gram_range(h, s0, s1, out_rows, nullptr);
-}
-int mr_similarity_ibm(mr_handle* h, int s0, int s1, float* out_rows) {
-  if (!out_rows) return fail(h, MR_ERR_BAD_ARG, "null output");
-  return gram_range(h, s0, s1, nullptr, out_rows);
 }
 
 // ---- similar songs and similar users (DESIGN.md §4.7, §4.8, k8_similar.cu).  Both use only the train replica (and the test shard's rows)
@@ -1839,6 +1745,71 @@ int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_
   const SimKind kind{"similar users", SimLists{h->d_te_ptr, h->d_te_col, h->d_csc_ptr, h->d_csc_idx, h->d_simu_squ, h->d_simu_sqt, false},
                      user_count_rows(h), &h->simu_short_rows, &h->simu_long_rows};
   return similar_lists(h, kind, user_idx, n, k, out_user, out_score, out_len);
+}
+
+// ---- parity probes (mr_counts_*, mr_similarity_*): rows [r0, r1) of count rows cr to the caller's [r1 - r0][n_cols], as int32 (out_i32)
+// or as cosines (out_f32, count_to_cos_kernel over the sqrt tables sq_row / sq_col), in chunks sized as the long rows of similar_lists.
+// Like the similar calls they keep to the Gram workspace and SL_GRAM_IDS: the score panels, the select plane and gen stay as they are.
+static int count_probe(mr_handle* h, const CountRows& cr, int r0, int r1, int32_t* out_i32, float* out_f32, const double* sq_row,
+                       const double* sq_col) {
+  if (r0 == r1) return MR_OK;
+  int C = 0, rc;
+  int* d_ids = nullptr;
+  if ((rc = count_chunk(h, cr, 0, r1 - r0, "parity probe", &C)) || (rc = slot_alloc(h, mr_handle::SL_GRAM_IDS, &d_ids, static_cast<size_t>(C))))
+    return rc;
+  char* out = out_i32 ? reinterpret_cast<char*>(out_i32) : reinterpret_cast<char*>(out_f32);   // both are 4-byte elements
+  const size_t row = static_cast<size_t>(cr.n_cols) * 4;
+  for (int c0 = r0; c0 < r1; c0 += C) {
+    const int nc = std::min(C, r1 - c0);
+    iota_kernel<<<(nc + 255) / 256, 256, 0, h->stream>>>(d_ids, c0, nc);
+    h->launches++;
+    if ((rc = count_rows(h, cr, d_ids, nc))) return rc;
+    if (out_f32) {
+      PhaseTimer t(h, MR_T_OTHER);
+      count_to_cos_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->d_g, cr.ld, d_ids, nc, cr.n_cols, sq_row, sq_col);
+      h->launches++;
+    }
+    MR_CUDA(h, cudaMemcpy2DAsync(out + static_cast<size_t>(c0 - r0) * row, row, h->d_g, static_cast<size_t>(cr.ld) * 4, row, nc,
+                                 cudaMemcpyDeviceToHost, h->stream));
+    MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  }
+  return MR_OK;
+}
+
+int mr_counts_ubm(mr_handle* h, int32_t* out_UxT) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (!out_UxT) return fail(h, MR_ERR_BAD_ARG, "null output");
+  return count_probe(h, user_count_rows(h), 0, h->U, out_UxT, nullptr, nullptr, nullptr);
+}
+
+int mr_similarity_ubm(mr_handle* h, float* out_UxT) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (!out_UxT) return fail(h, MR_ERR_BAD_ARG, "null output");
+  if ((rc = ensure_sqrt_users(h))) return rc;
+  return count_probe(h, user_count_rows(h), 0, h->U, nullptr, out_UxT, h->d_simu_squ, h->d_simu_sqt);
+}
+
+static int check_gram_range(mr_handle* h, int s0, int s1) {
+  int rc = require_loaded(h);   // Gram rows need only the train replica
+  if (rc) return rc;
+  if (h->windowed) return fail(h, MR_ERR_STATE, "Gram rows are not available on a handle with a song window (its song ids are rotated)");
+  if (s0 < 0 || s1 > h->S || s0 > s1) return fail(h, MR_ERR_BAD_ARG, "song range [%d,%d) outside [0,%d)", s0, s1, h->S);
+  return MR_OK;
+}
+
+int mr_counts_ibm(mr_handle* h, int s0, int s1, int32_t* out_rows) {
+  if (!out_rows) return fail(h, MR_ERR_BAD_ARG, "null output");
+  const int rc = check_gram_range(h, s0, s1);
+  return rc ? rc : count_probe(h, song_count_rows(h), s0, s1, out_rows, nullptr, nullptr, nullptr);
+}
+
+int mr_similarity_ibm(mr_handle* h, int s0, int s1, float* out_rows) {
+  if (!out_rows) return fail(h, MR_ERR_BAD_ARG, "null output");
+  int rc = check_gram_range(h, s0, s1);
+  if (rc || (rc = ensure_sqrt_songs(h))) return rc;
+  return count_probe(h, song_count_rows(h), s0, s1, nullptr, out_rows, h->d_sim_sqd, h->d_sim_sqd);
 }
 
 // ---- explanations (DESIGN.md §4.9, k8_similar.cu explain_pairs_kernel): the contributors of (test user, song) scores of UBM or IBM.  The

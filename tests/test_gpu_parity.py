@@ -1,4 +1,5 @@
 """GPU parity tests (-m gpu): the CUDA path, called through the C-ABI (via the host mirror), against the oracle."""
+import dataclasses
 import json
 from pathlib import Path
 
@@ -274,16 +275,49 @@ def test_error_behaviour(mrlib, oracle_lib):
         MusicRecommender(bad)
 
 
-def test_similarity_products(engine, oracle_lib):
-    """Cosine normalisation fused into the count-GEMM epilogue (fp32 products): user-user MR:140-149, item-item MR:230-239."""
-    ds = synth(T=300, U=20, S=2000, seed=1)
+def with_empty_test_user(ds):
+    """ds with one more test user, last, whose visible row is empty (degree 0)."""
+    return dataclasses.replace(ds, U=ds.U + 1, te_ptr=np.append(ds.te_ptr, ds.te_ptr[-1]), lab_ptr=np.append(ds.lab_ptr, ds.lab_ptr[-1]),
+                               deg_te=np.append(ds.deg_te, 0).astype(np.int32))
+
+
+def rs32(deg):
+    """float(1 / sqrt(deg)) rounded from fp64, 0 for degree 0: the fp32 factor of the similarity products."""
+    d = np.asarray(deg, np.float64)
+    with np.errstate(divide="ignore"):
+        return np.where(d > 0, 1.0 / np.sqrt(d), 0.0).astype(np.float32)
+
+
+def check_probes(ds, oracle_lib, engine):
+    """The parity probes: counts bit for bit; cosines user-user MR:140-149 and item-item MR:230-239 within 1e-5 of the fp64 formula and
+    bit for bit float(c) * (rs(a) * rs(b)) in fp32."""
     with MusicRecommender(ds, **engine) as mr:
-        c = oracle_lib.counts_ubm(ds).astype(np.float64)
-        want = c / (np.sqrt(ds.deg_te.astype(np.float64))[:, None] * np.sqrt(ds.deg_tr.astype(np.float64))[None, :])
-        np.testing.assert_allclose(mr.similarity_ubm(), want, rtol=1e-5, atol=0)
-        g = oracle_lib.gram_rows(ds, np.arange(100, 300)).astype(np.float64)
+        c = oracle_lib.counts_ubm(ds)
+        np.testing.assert_array_equal(mr.counts_ubm(), c)
+        g = oracle_lib.gram_rows(ds, np.arange(100, 300))
+        np.testing.assert_array_equal(mr.counts_ibm(100, 300), g)
+        sim_u, sim_i = mr.similarity_ubm(), mr.similarity_ibm(100, 300)
+        du, dv = ds.deg_te.astype(np.float64), ds.deg_tr.astype(np.float64)
+        with np.errstate(invalid="ignore"):
+            want = np.where(du[:, None] > 0, c / (np.sqrt(du)[:, None] * np.sqrt(dv)[None, :]), 0.0)
+        np.testing.assert_allclose(sim_u, want, rtol=1e-5, atol=0)
         d = np.sqrt(ds.deg_song.astype(np.float64))
-        np.testing.assert_allclose(mr.similarity_ibm(100, 300), g / (d[100:300, None] * d[None, :]), rtol=1e-5, atol=0)
+        np.testing.assert_allclose(sim_i, g / (d[100:300, None] * d[None, :]), rtol=1e-5, atol=0)
+        exact_u = c.astype(np.float32) * (rs32(ds.deg_te)[:, None] * rs32(ds.deg_tr)[None, :])
+        rd = rs32(ds.deg_song)
+        exact_i = g.astype(np.float32) * (rd[100:300, None] * rd[None, :])
+        np.testing.assert_array_equal(sim_u.view(np.int32), exact_u.view(np.int32))
+        np.testing.assert_array_equal(sim_i.view(np.int32), exact_i.view(np.int32))
+
+
+def test_similarity_products(engine, oracle_lib):
+    check_probes(with_empty_test_user(synth(T=300, U=20, S=2000, seed=1)), oracle_lib, engine)
+
+
+def test_probes_across_chunks(engine, oracle_lib, monkeypatch):
+    """The same with chunks of 7 count rows (MRSCORE_SIM_CHUNK): every probe crosses chunk boundaries."""
+    monkeypatch.setenv("MRSCORE_SIM_CHUNK", "7")
+    check_probes(with_empty_test_user(synth(T=300, U=20, S=2000, seed=1)), oracle_lib, engine)
 
 
 def test_shard_invariance(oracle_lib):

@@ -162,8 +162,8 @@ def test_train_only_handle(mrlib):
 
 
 def test_scoring_state_is_left_alone(mrlib):
-    """Single-batch item-space shard: device-resident top-k results of both kinds survive the call, host top-k results are unchanged, and
-    range -> similar -> counts still reuses the panels (one scoring pass) with the same mAP bits."""
+    """Single-batch item-space shard: device-resident top-k results of both kinds survive the call and the parity probes, host top-k results
+    are unchanged, and range -> similar + probes -> counts still reuses the panels (one scoring pass) with the same mAP bits."""
     import torch
     ds = synth(**ITEMDS)
     new = np.unique(ds.lab_col)
@@ -180,6 +180,8 @@ def test_scoring_state_is_left_alone(mrlib):
         p0 = mr.info()["scoring_passes"]
         got, n_s, n_l = run_paths(mr, ds, None, 100)
         assert n_s > 0 and n_l > 0
+        mr.counts_ubm()
+        mr.similarity_ibm(0, 50)
         cnt = mr.eval_counts(_lib.MR_IBM, mn, mx, new)
         assert mr.info()["scoring_passes"] == p0                    # the count pass reused the panels of the range pass
         for a, b in zip(dev, mr.topk_device_tensors(50)):

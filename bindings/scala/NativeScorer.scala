@@ -40,6 +40,10 @@ trait MrScore extends Library {
   // terms, fixed-point terms), their number, the exact numerator and the library's score per pair (DESIGN.md §4.9)
   def mr_explain(h: Pointer, model: Int, userIdx: Array[Int], songIds: Array[Int], n: Int, m: Int, outId: Array[Int], outTerm: Array[Double],
                  outNum: Array[Long], outLen: Array[Int], outCount: Array[Int], outTotal: Array[Long], outScore: Array[Double]): Int
+  // who scores each query song highest under a model (any MR_*, as mr_topk): the k test users of the current shard, score descending then
+  // user index ascending, [n][k] / [n] (DESIGN.md §4.10)
+  def mr_song_audience(h: Pointer, model: Int, param: Double, seed: Long, songIds: Array[Int], n: Int, k: Int, outUser: Array[Int],
+                       outScore: Array[Double], outLen: Array[Int]): Int
   def mr_ingest_tsv(device: Int, train: Array[Byte], trainLen: Long, test: Array[Byte], testLen: Long, labels: Array[Byte],
                     labelsLen: Long, out: PointerByReference): Int
   def mr_ingest_error(g: Pointer): String

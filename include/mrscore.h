@@ -283,6 +283,24 @@ int mr_similar_users(mr_handle* h, const int32_t* user_idx, int n, int k, int32_
 int mr_explain(mr_handle* h, int model, const int32_t* user_idx, const int32_t* song_ids, int n, int m, int32_t* out_id, double* out_term,
                int64_t* out_num, int32_t* out_len, int32_t* out_count, int64_t* out_total, double* out_score);
 
+/* ---- song audiences: the test users who score a song highest (DESIGN.md §4.10) ----------------------------------------------------------
+ * For each query song s = song_ids[r] (any order, duplicates allowed), the k test users u of the CURRENT shard with the highest score of
+ * (u, s) under model / param / seed, which mean what they mean in mr_topk (any MR_* selector, blends fused).  Candidates are the test users
+ * who have not listened to s (the reference emits no listened pair, MR:109); a 0.0 score is a candidate, as in mr_topk.  Order: score
+ * descending, then user index ascending.  Every listed score has the bits mr_score_songs (getRanks2) and mr_topk give the pair, AGG and
+ * STOCH under the global pair index of mr_set_test_users included.  User ids are indices into the current shard, as in mr_score_users.
+ * Outputs (host arrays): out_user / out_score [n][k], out_len [n]; out_len[r] = min(k, test users who have not listened to s), user -1 /
+ * score 0.0 past it.  On a handle with a song window the ids must lie in the window; such a handle sees every test user, so its lists are
+ * the global ones.  1 <= k <= 1024; n = 0 returns MR_OK.  MR_ERR_BAD_ARG names the first id outside [0, S) or the window, and covers a bad
+ * k or model and null arrays; MR_ERR_PARAM_RANGE as in mr_topk (LC alpha, AGG / STOCH parameter outside [0, 1] or NaN); MR_ERR_STATE
+ * before mr_load and without test users.  A scoring call: it scores the shard once per batch (mr_get_info value 20 grows by the batches),
+ * ranks each batch's panels by column (MR_T_TOPK) into running per-song lists of n x k x 12 bytes in a grow-only block of their own, and
+ * returns with all its work complete.  The lists must fit in the device memory the batch plan leaves free (MR_ERR_OOM stating the bytes
+ * otherwise; the plan is not changed for it).  It leaves the single-model top-k result and the model-set results untouched.
+ * mr_get_info value 26 counts the query rows answered since mr_load, value 27 the (column, batch) selects that took the radix select. */
+int mr_song_audience(mr_handle* h, int model, double param, uint64_t seed, const int32_t* song_ids, int n, int k, int32_t* out_user,
+                     double* out_score, int32_t* out_len);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -359,7 +377,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  scoring passes since mr_load (batches whose score panels were built),
                                                                  mr_similar_songs rows since mr_load: answered by the short path, by the long path,
                                                                  mr_similar_users rows since mr_load: answered by the short path, by the long path,
-                                                                 mr_explain count rows built since mr_load] */
+                                                                 mr_explain count rows built since mr_load,
+                                                                 mr_song_audience since mr_load: query rows answered, column selects through the radix select] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

@@ -25,7 +25,7 @@ SYMBOLS = ["mr_create", "mr_destroy", "mr_last_error", "mr_load", "mr_set_test_u
            "mr_ingest_tsv", "mr_ingest_error", "mr_ingest_dims", "mr_ingest_get", "mr_ingest_free",
            "mr_eval_range", "mr_eval_counts", "mr_eval_finish", "mr_eval_cutoffs",
            "mr_topk_multi", "mr_topk_multi_device", "mr_topk_multi_ptrs", "mr_eval_range_multi", "mr_eval_counts_multi",
-           "mr_similar_songs", "mr_similar_users", "mr_explain"]
+           "mr_similar_songs", "mr_similar_users", "mr_explain", "mr_song_audience"]
 
 _lib = None
 
@@ -111,5 +111,6 @@ def load():
     lib.mr_similar_songs.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.mr_similar_users.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.mr_explain.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.mr_song_audience.argtypes = [vp, i32, dbl, u64, vp, i32, i32, vp, vp, vp]
     _lib = lib
     return lib

@@ -31,8 +31,6 @@ __device__ __forceinline__ double sim_score(int g, double sq_i, double sq_s) {
   return den != 0.0 ? __ddiv_rn(static_cast<double>(g), den) : 0.0;   // naive_*_cos: denominator != 0 ? numerator / denominator : 0
 }
 
-__device__ __forceinline__ unsigned long long key_bits(double x) { return static_cast<unsigned long long>(__double_as_longlong(x)); }
-
 // ascending bitonic sort of n_pad (a power of two) ints; every thread of the CTA calls it
 __device__ void bitonic_ints(int* a, int n_pad) {
   __syncthreads();
@@ -171,63 +169,6 @@ __device__ __forceinline__ void scan_counts(const int32_t* __restrict__ g, int n
       f(s + t, kb, ok);
     }
   }
-}
-
-// Shared memory of one row's exact select
-struct RowSelect {
-  unsigned long long key[kTopkCap];
-  int id[kTopkCap];
-  int hist[kTopkBins];
-  unsigned long long max[kTopkThreads / 32];
-  int count, valid;
-  int ctl[3];     // 0: chosen bin / digit, 1: keys strictly above it, 2: keys in it
-};
-
-// The exact list of one row (similar_row_topk_kernel, explain_pairs_kernel): the maximum key and the number of candidates from the pass
-// first(f), then a linear histogram and the exact select of topk_kernel (mr_common.cuh) over the passes scan(f); write_list stores the
-// first min(k, candidates) entries.  first and scan stream the same candidates (first may also accumulate the caller's own sums).
-// Returns need = min(k, candidates); sm.valid holds the number of candidates, sm.id[0 .. need) the listed ids.
-template <class First, class Scan>
-__device__ __forceinline__ int row_select(First&& first, Scan&& scan, int k, RowSelect& sm, int* o_id, double* o_score, int* o_len) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  // ---- maximum key and number of candidates
-  if (tid == 0) sm.valid = 0;
-  __syncthreads();
-  unsigned long long mx = 0; int nv = 0;
-  first([&](int, unsigned long long kb, bool ok) { if (ok) { ++nv; mx = kb > mx ? kb : mx; } });
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xffffffffu, mx, o); mx = other > mx ? other : mx; nv += __shfl_xor_sync(0xffffffffu, nv, o); }
-  if (lane == 0) { sm.max[warp] = mx; atomicAdd(&sm.valid, nv); }
-  for (int i = tid; i < kTopkBins; i += kTopkThreads) sm.hist[i] = 0;
-  __syncthreads();
-  mx = 0;
-  for (int i = 0; i < kTopkThreads / 32; ++i) mx = sm.max[i] > mx ? sm.max[i] : mx;
-  const int need = min(k, sm.valid);
-  if (need == 0) {
-    write_list(sm.key, sm.id, 0, k, 0, o_id, o_score, o_len);
-    return 0;
-  }
-  const double max_score = __longlong_as_double(static_cast<long long>(mx));
-  const double scale = max_score > 0.0 ? __ddiv_rn(static_cast<double>(kTopkBins - 1), max_score) : 0.0;
-  auto bin_of = [&](unsigned long long kb) -> uint32_t {   // monotone in the key
-    const int d = __double2int_rz(__dmul_rn(__longlong_as_double(static_cast<long long>(kb)), scale));
-    return static_cast<uint32_t>(d > kTopkBins - 1 ? kTopkBins - 1 : d);
-  };
-  // ---- linear histogram of the candidates, then the shared exact select (mr_common.cuh)
-  scan([&](int, unsigned long long kb, bool ok) { hist_add(sm.hist, ok ? bin_of(kb) : 0u, ok, lane); });
-  __syncthreads();
-  if (warp == 0) find_bin(sm.hist, need, false, sm.ctl);
-  __syncthreads();
-  const uint32_t cbin = static_cast<uint32_t>(sm.ctl[0]);
-  int above = sm.ctl[1];
-  unsigned long long phi = 0; uint32_t plo = 0; int nd = 0;
-  // a crowded bin: thousands of exact ties, e.g. g = 1 against songs of one degree
-  if (above + sm.ctl[2] > kTopkCap) radix_refine(scan, bin_of, cbin, need, above, phi, plo, nd, sm.hist, sm.ctl);
-  collect_keys(scan, bin_of, cbin, phi, plo, nd, sm.key, sm.id, &sm.count);
-  __syncthreads();
-  sort_keys(sm.key, sm.id, min(sm.count, kTopkCap));
-  write_list(sm.key, sm.id, need, k, 0, o_id, o_score, o_len);
-  return need;
 }
 
 template <bool kSelf>

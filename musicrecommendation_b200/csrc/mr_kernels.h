@@ -206,4 +206,17 @@ struct ExplainArgs {
 struct ExplainOut { int* id; double* term; long long* num; int* len; int* count; long long* total; double* score; };   // [n][m] x 3, [n] x 4
 int launch_explain_pairs(int model, const ExplainArgs& a, int n, int m, const ExplainOut& o, cudaStream_t st);
 
+// ---- song audiences (k9_audience.cu, DESIGN.md §4.10): the column select of one masked batch into the running per-song lists
+struct AudienceArgs {
+  int model; double alpha, oma;                      // MODEL_*, LC weights
+  const long long* su; const long long* si;          // the batch's masked panels, row r = test user u0 + r (null where the model reads none)
+  long long spitch;
+  const uint64_t* sel; long long sel_pitch;          // AGG / STOCH select plane of the batch (words per row)
+  const double* rsa; const double* rsd;
+  const int2* q;                                     // [n_q] (column, list row), ascending column
+  int* user; double* score; int* len;                // running lists: [rows][k], [rows][k], [rows]
+  unsigned int* radix_rows;                          // columns that took the radix select, or null
+};
+int launch_audience(const AudienceArgs& a, int n_q, int u0, int nb, int k, cudaStream_t st);
+
 }  // namespace mr

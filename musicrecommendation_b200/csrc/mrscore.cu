@@ -71,7 +71,7 @@ struct mr_handle {
   cudaStream_t pre_stream = nullptr; cudaEvent_t ev_pre = nullptr; bool head_pending = false; unsigned int* h_n_ex = nullptr;
   cudaStream_t pre_extra[kPreExtraStreams] = {}; cudaEvent_t ev_pre_extra[kPreExtraStreams] = {};   // extra streams of the in-place row build (chunks rotate over them)
   HeadExceptions pend_ex{};
-  unsigned int* d_topk_stats = nullptr;   // [3] counters of the top-k select since mr_load (BlendParams::stats)
+  unsigned int* d_topk_stats = nullptr;   // [4] counters since mr_load: [0, 3) of the top-k select (BlendParams::stats), [3] audience columns through the radix select
   uint32_t *d_qv = nullptr, *d_qd = nullptr; double* d_rsd = nullptr; float* d_rsd_up = nullptr;
   std::vector<int32_t> deg_song, deg_song_train;
   struct SongInfo { int head; uint32_t v; };   // head row or -1; v = q_26(d_s) of a head song, train listeners of a tail song
@@ -103,7 +103,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard, its results and the workspaces: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_AUD_OUT, SL_AUD_Q, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -133,6 +133,7 @@ struct mr_handle {
   std::vector<int32_t> deg_train, deg_test;
   double *d_simu_sqt = nullptr, *d_simu_squ = nullptr; bool simu_squ_ok = false; long long simu_short_rows = 0, simu_long_rows = 0;
   long long explain_rows = 0;   // mr_explain: count rows built since mr_load
+  long long audience_rows = 0;  // mr_song_audience: query rows answered since mr_load
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -752,8 +753,9 @@ struct ModelSet {
   explicit ModelSet(int model) : n(1) { memset(&bp[0], 0, sizeof bp[0]); bp[0].model = model; }   // one model without blend parameters
 };
 
-// What a scoring run hands the masked panels to: the top-k select, the fp64 rows, or the streamed evaluateModel passes (DESIGN.md §4.5).
-enum class Consumer { TOPK, DENSE, EVAL_RANGE, EVAL_COUNT };
+// What a scoring run hands the masked panels to: the top-k select, the fp64 rows, the streamed evaluateModel passes (DESIGN.md §4.5), or
+// the column select of song audiences (DESIGN.md §4.10).
+enum class Consumer { TOPK, DENSE, EVAL_RANGE, EVAL_COUNT, AUDIENCE };
 struct Run {
   ModelSet set;
   Consumer what = Consumer::TOPK;
@@ -761,6 +763,8 @@ struct Run {
   const DenseOut* dense = nullptr;      // DENSE: where the rows go
   const TopkOut* topk_host = nullptr;   // TOPK in item space: the caller's buffers, filled slice by slice from entry 0 on copy_stream
   bool reuse = false;                   // EVAL_COUNT: the panels hold this set's masked numerators (resident reuse): no scoring at all
+  const int2* aud_q = nullptr;          // AUDIENCE: [aud_n] device (column, list row), ascending column; the running lists are set.out[0]
+  int aud_n = 0;
   bool eval() const { return what == Consumer::EVAL_RANGE || what == Consumer::EVAL_COUNT; }
 };
 
@@ -768,6 +772,12 @@ struct Run {
 // the group's STOCH plane, unless the plane of the set's only STOCH entry is still in place from the range pass).
 int consume_slice(mr_handle* h, const Run& run, long long* su, long long* si, uint64_t* sel, int u0, int n, cudaStream_t st) {
   const ModelSet& set = run.set;
+  if (run.what == Consumer::AUDIENCE) {   // the column select runs once per batch (audience_columns); a slice only builds its select plane
+    const BlendParams& bp = set.bp[0];
+    if (bp.model == MODEL_AGG || bp.model == MODEL_STOCH)
+      MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
+    return MR_OK;
+  }
   if (run.what == Consumer::TOPK) {
     for (int e = 0; e < set.n; ++e) {
       const BlendParams& bp = set.bp[e];
@@ -792,6 +802,18 @@ int consume_slice(mr_handle* h, const Run& run, long long* su, long long* si, ui
       MR_LAUNCH(h, launch_eval_count(set.grp[g], su, si, h->spitch, sel, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, ec, st));
     }
   }
+  return MR_OK;
+}
+
+// AUDIENCE: the column select of the whole masked batch [b0, b0 + nb) (panels and select plane from row 0 of the batch) on st, after every
+// slice of the batch, into the running lists.
+int audience_columns(mr_handle* h, const Run& run, const long long* su, const long long* si, int b0, int nb, cudaStream_t st) {
+  const BlendParams& bp = run.set.bp[0];
+  const TopkOut& l = run.set.out[0];
+  const AudienceArgs a{bp.model, bp.alpha, bp.one_minus_alpha, su, si, h->spitch, h->d_sel, h->sel_pitch, h->d_rsa, h->d_rsd, run.aud_q,
+                       l.song, l.score, l.len, h->d_topk_stats + 3};
+  PhaseTimer t(h, MR_T_TOPK, st);
+  MR_LAUNCH(h, launch_audience(a, run.aud_n, b0, nb, run.k, st));
   return MR_OK;
 }
 
@@ -968,11 +990,12 @@ int run_batches(mr_handle* h, const Run& run) {
         if (alternating) MR_CUDA(h, cudaStreamWaitEvent(sl.st[1], h->ev_head[par], 0));
       }
       if ((rc = item_slices(h, run, sl, b0, nb, pu, pi))) return rc;
+      if (alternating) {   // the batch's slices end on st[0]
+        MR_CUDA(h, cudaEventRecord(h->ev_join, sl.st[1]));
+        MR_CUDA(h, cudaStreamWaitEvent(sl.st[0], h->ev_join, 0));
+      }
+      if (run.what == Consumer::AUDIENCE && (rc = audience_columns(h, run, pu, pi, b0, nb, sl.st[0]))) return rc;
       if (streamed) {
-        if (alternating) {   // the batch's slices end on st[0]
-          MR_CUDA(h, cudaEventRecord(h->ev_join, sl.st[1]));
-          MR_CUDA(h, cudaStreamWaitEvent(sl.st[0], h->ev_join, 0));
-        }
         MR_CUDA(h, cudaEventRecord(h->ev_done[par], sl.st[0]));
         if (b0 + batch >= h->U) {   // last batch: the library stream joins the slices (of the last two batches in the batch pipeline)
           MR_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_done[par], 0));
@@ -986,11 +1009,14 @@ int run_batches(mr_handle* h, const Run& run) {
     // the whole batch on the library stream (user space; the dense rows in item space): mask, then the dense rows or the consumers
     long long* const su = need_ubm ? h->d_sint_u : nullptr;
     long long* const si = need_ibm ? h->d_sint_i : nullptr;
-    PhaseTimer t(h, run.eval() ? MR_T_OTHER : MR_T_TOPK);
-    MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, su, si, h->spitch, h->stream));
-    rc = run.what == Consumer::DENSE ? dense_out(h, run.set.bp[0].model, su ? su : si, *run.dense, b0, nb)
-                                     : consume_slice(h, run, su, si, h->d_sel, b0, nb, h->stream);
-    if (rc) return rc;
+    {
+      PhaseTimer t(h, run.eval() ? MR_T_OTHER : MR_T_TOPK);   // closed before audience_columns opens its own timer on the same events
+      MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, su, si, h->spitch, h->stream));
+      rc = run.what == Consumer::DENSE ? dense_out(h, run.set.bp[0].model, su ? su : si, *run.dense, b0, nb)
+                                       : consume_slice(h, run, su, si, h->d_sel, b0, nb, h->stream);
+      if (rc) return rc;
+    }
+    if (run.what == Consumer::AUDIENCE && (rc = audience_columns(h, run, su, si, b0, nb, h->stream))) return rc;
   }
   join.armed = false;
   if (need_ibm && !item_space && h->engine == MR_ENGINE_SPARSE) {
@@ -2517,6 +2543,53 @@ int mr_topk_multi(mr_handle* h, int n_models, const int* models, const double* p
   return MR_OK;
 }
 
+int mr_song_audience(mr_handle* h, int model, double param, uint64_t seed, const int32_t* song_ids, int n, int k, int32_t* out_user,
+                     double* out_score, int32_t* out_len) {
+  int rc = require_test(h);
+  if (rc) return rc;
+  if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k must be in [1,1024], got %d", k);
+  Run run{ModelSet(), Consumer::AUDIENCE, k};
+  if ((rc = make_set(h, 1, &model, &param, &seed, "getSongAudience", false, &run.set))) return rc;
+  if (n < 0 || (n > 0 && (!song_ids || !out_user || !out_score || !out_len))) return fail(h, MR_ERR_BAD_ARG, "null song list / output");
+  const int lo = h->win_lo, hi = h->win_lo + h->n_cols;
+  for (int i = 0; i < n; ++i)
+    if (song_ids[i] < lo || song_ids[i] >= hi) return fail(h, MR_ERR_BAD_ARG, "song id %d out of range [%d,%d)", song_ids[i], lo, hi);
+  if (n == 0) return MR_OK;
+  // the running lists, one TopkBlock of n rows in a grow-only slot of their own (the top-k results stay); it must fit inside the caller's
+  // reserve that the batch plan leaves free, and be free now; the plan is not changed for it
+  const TopkBlock blk(n, k);
+  size_t avail = kCallerReserve;
+  if (h->slot_cap[mr_handle::SL_AUD_OUT] < blk.bytes) {
+    size_t free_b = 0, total_b = 0;
+    MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
+    avail = std::min(avail, free_b + h->slot_cap[mr_handle::SL_AUD_OUT]);
+  }
+  if (blk.bytes > avail)
+    return fail(h, MR_ERR_OOM, "mr_song_audience: %d top-%d lists need %zu bytes, more than the %zu bytes of the caller's reserve that are free",
+                n, k, blk.bytes, avail);
+  char* base = nullptr;
+  int2* d_q = nullptr;
+  if ((rc = slot_alloc(h, mr_handle::SL_AUD_OUT, &base, blk.bytes, true))) return rc;
+  // the queries by column (rotated into the window), so that CTAs of adjacent columns run together; each keeps its caller's row
+  std::vector<int2> q(static_cast<size_t>(n));
+  for (int i = 0; i < n; ++i) q[i] = make_int2(song_ids[i] - lo, i);
+  std::sort(q.begin(), q.end(), [](const int2& a, const int2& b) { return a.x != b.x ? a.x < b.x : a.y < b.y; });
+  if ((rc = slot_upload(h, mr_handle::SL_AUD_Q, &d_q, q.data(), q.size()))) return rc;
+  run.set.out[0] = blk.at(base);
+  run.aud_q = d_q; run.aud_n = n;
+  const TopkOut& l = run.set.out[0];
+  MR_CUDA(h, cudaMemsetAsync(l.song, 0xff, static_cast<size_t>(n) * k * sizeof(int32_t), h->stream));   // empty lists: user -1, score 0.0, len 0
+  MR_CUDA(h, cudaMemsetAsync(l.score, 0, static_cast<size_t>(n) * k * sizeof(double), h->stream));
+  MR_CUDA(h, cudaMemsetAsync(l.len, 0, static_cast<size_t>(n) * sizeof(int32_t), h->stream));
+  rc = run_batches(h, run);
+  if (!rc) rc = copy_topk(h, TopkOut{out_user, out_score, out_len}, l, k, 0, n, h->stream);
+  const cudaError_t e = cudaStreamSynchronize(h->stream);   // also keeps the pageable query list alive until its upload has run
+  if (rc) return rc;
+  if (e != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_song_audience: %s", cudaGetErrorString(e));
+  h->audience_rows += n;
+  return MR_OK;
+}
+
 int mr_get_timing(mr_handle* h, double* ms_out, int n) {
   if (!h || !ms_out) return MR_ERR_BAD_ARG;
   for (int i = 0; i < n && i < MR_T_N; ++i) ms_out[i] = h->t_ms[i];
@@ -2531,11 +2604,12 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[25] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[27] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
                          h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
-                         h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows, h->explain_rows};
-  for (int i = 0; i < n && i < 25; ++i) out[i] = v[i];
+                         h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows, h->explain_rows,
+                         h->audience_rows, st[3]};
+  for (int i = 0; i < n && i < 27; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

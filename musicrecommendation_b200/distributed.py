@@ -138,6 +138,53 @@ def exchange_song_partitions(song, score, length, n_users_total: int, world: int
     return tuple(outs)
 
 
+def audience_shard_parts(user, score, length, u0: int, world: int, rank: int, group=None):
+    """The host part of song_audience under test-user sharding: every rank holds, for ALL query songs, the audience lists of its shard
+    (user indices into the shard, -1 past the length).  The ids are made global by adding the shard's first user u0, then
+    exchange_song_partitions hands rank r every rank's lists of ITS rows of the query list (shard_range over the queries): the exchange is
+    row-generic, the rows here are query songs.  Returns (parts_user [world, n_r, k], parts_score, parts_len [world, n_r]); the parts hold
+    disjoint user sets, each ordered by (score descending, user ascending), so their join (mr_topk_merge) is exact."""
+    import torch
+    user = torch.as_tensor(user)
+    user = torch.where(user >= 0, user + int(u0), user)
+    return exchange_song_partitions(user, score, length, user.shape[0], world, rank, group)
+
+
+def song_audience(mr, model: int, k: int, param: float = 0.5, seed: int = 0, songs=None, group=None):
+    """getSongAudience of a job whose ranks each hold one part of the model (DESIGN.md §4.10).  Every rank passes the same query list
+    (default: every song).
+      song partitioning (the handle has a song window, and sees every test user): each rank answers the queries inside its window, and
+        rank 0 gathers them in window order.  Returns (songs, user, score, len) on rank 0, None elsewhere.
+      test-user sharding (mr.ds is the shard [u0, u1) of shard_test_users): each rank ranks its shard for every query, the ids are made
+        global, audience_shard_parts moves the lists by query rows and mr_topk_merge joins them on the GPU.  Returns (songs, user, score,
+        len) of this rank's rows shard_range(n, rank, world) of the query list; user ids index the whole test set."""
+    import torch
+    import torch.distributed as dist
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    lo, hi = mr.song_window
+    ids = np.arange(mr.ds.S, dtype=np.int32) if songs is None else np.ascontiguousarray(songs, np.int32).reshape(-1)
+    if (lo, hi) != (0, mr.ds.S):
+        mine = ids[(ids >= lo) & (ids < hi)]
+        part = (mine,) + tuple(mr.getSongAudience(model, mine, k, param, seed))
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(part, parts, dst=0, group=group)
+        if rank != 0:
+            return None
+        return tuple(np.concatenate([p[i] for p in parts]) for i in range(4))
+    user, score, ln = mr.getSongAudience(model, ids, k, param, seed)
+    dev = _collective_device(group)
+    u0 = mr.ds.meta.get("shard", (0, mr.ds.U))[0]
+    ps, pv, pl = audience_shard_parts(torch.from_numpy(user).to(dev), torch.from_numpy(score).to(dev), torch.from_numpy(ln).to(dev), u0,
+                                      world, rank, group)
+    r0, r1 = shard_range(len(ids), rank, world)
+    ps, pv, pl = ps.cuda(), pv.cuda(), pl.cuda()
+    out = (torch.empty_like(ps[0]), torch.empty_like(pv[0]), torch.empty_like(pl[0]))
+    torch.cuda.synchronize()          # the parts are written on torch's streams, the join runs on the library stream
+    mr.mergeTopK(ps, pv, pl, *out)
+    mr.sync()
+    return (ids[r0:r1],) + tuple(t.cpu().numpy() for t in out)
+
+
 def _collective_device(group):
     import torch
     import torch.distributed as dist

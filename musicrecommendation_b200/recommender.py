@@ -370,6 +370,22 @@ class MusicRecommender:
         self._check(self._lib.mr_explain(self._h, model, _p(u), _p(s), n, m, *[_p(a) for a in out]))
         return out
 
+    def getSongAudience(self, model: int = _lib.MR_UBM, songs=None, k: int = 100, param: float = 0.5, seed: int = 0):
+        """Who scores each of `songs` highest (default: every song of the handle's window, ascending): the k test users of the current
+        shard with the best score of (user, song) under model / param / seed as in getTopK, score descending then user index ascending
+        (mr_song_audience, DESIGN.md §4.10).  Returns (user [n, k] int32, score [n, k] float64, len [n] int32); row r belongs to
+        songs[r], user -1 / score 0.0 past len[r]."""
+        lo, hi = self.song_window
+        ids = np.arange(lo, hi, dtype=np.int32) if songs is None else np.ascontiguousarray(songs, np.int32).reshape(-1)
+        n = len(ids)
+        kk = max(int(k), 0)                 # a k outside 1..1024 is refused by the library (MR_ERR_BAD_ARG), not by numpy
+        user = np.empty((n, kk), np.int32)
+        score = np.empty((n, kk), np.float64)
+        ln = np.empty(n, np.int32)
+        self._check(self._lib.mr_song_audience(self._h, model, float(param), C.c_uint64(seed & (2**64 - 1)), _p(ids), n, k, _p(user),
+                                               _p(score), _p(ln)))
+        return user, score, ln
+
     def getTopKMulti(self, specs, k: int = 500):
         """getTopK for every entry of a model set (model, param, seed) from one scoring of the shard (mr_topk_multi, DESIGN.md §4.6):
         one (song [U,k] int32, score [U,k] f64, len [U]) per entry, each equal to getTopK(model, k, param, seed)."""
@@ -525,12 +541,13 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 25)()
-        self._lib.mr_get_info(self._h, v, 25)
+        v = (C.c_int64 * 27)()
+        self._lib.mr_get_info(self._h, v, 27)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
                          "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows",
-                         "similar_user_short_rows", "similar_user_long_rows", "explain_rows"], list(v)))
+                         "similar_user_short_rows", "similar_user_long_rows", "explain_rows", "audience_rows",
+                         "audience_radix_selects"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -837,6 +854,23 @@ def similar_users_host(ds: Dataset, users, k: int):
         out_score[r, :m] = w[rank[:m]]
         out_len[r] = m
     return out_user, out_score, out_len
+
+
+def song_audience_host(scores: np.ndarray, songs, k: int):
+    """numpy mirror of mr_song_audience over a dense model [U, S] (NaN at listened pairs, as mr_score_dense and the oracle give it): per
+    query song, its column's non-NaN entries ordered by (-score, user), the first k.  Returns (user [n, k] int32, score [n, k] f64,
+    len [n] int32), user -1 / score 0.0 past len."""
+    ids = np.asarray(songs, np.int64).reshape(-1)
+    n = len(ids)
+    cols = np.asarray(scores, np.float64)[:, ids]                      # [U, n]
+    order = np.argsort(-cols, axis=0, kind="stable")[:k].T             # NaN sorts last; equal scores keep user order
+    ln = np.minimum(k, (~np.isnan(cols)).sum(axis=0)).astype(np.int32)
+    user = np.full((n, k), -1, np.int32)
+    score = np.zeros((n, k), np.float64)
+    for r in range(n):
+        user[r, :ln[r]] = order[r, :ln[r]]
+        score[r, :ln[r]] = cols[order[r, :ln[r]], r]
+    return user, score, ln
 
 
 def explain_host(ds: Dataset, model: int, users, songs, m: int) -> Explanation:

@@ -44,6 +44,12 @@ trait MrScore extends Library {
   // user index ascending, [n][k] / [n] (DESIGN.md §4.10)
   def mr_song_audience(h: Pointer, model: Int, param: Double, seed: Long, songIds: Array[Int], n: Int, k: Int, outUser: Array[Int],
                        outScore: Array[Double], outLen: Array[Int]): Int
+  // filtered top-k (DESIGN.md §4.11): an allowed song set (n = -1: every song) and per-user exclusion rows of the current shard (null: none);
+  // then per model-set entry each user's ranking without the filtered songs, truncated to k (outputs as mr_topk's, one array per entry)
+  def mr_set_topk_filter(h: Pointer, allowSongs: Array[Int], nAllow: Int, exRowptr: Array[Long], exCol: Array[Int]): Int
+  def mr_topk_filtered(h: Pointer, nModels: Int, models: Array[Int], params: Array[Double], seeds: Array[Long], k: Int,
+                       outSong: Array[Pointer], outScore: Array[Pointer], outLen: Array[Pointer]): Int
+  def mr_topk_filtered_device(h: Pointer, nModels: Int, models: Array[Int], params: Array[Double], seeds: Array[Long], k: Int): Int
   def mr_ingest_tsv(device: Int, train: Array[Byte], trainLen: Long, test: Array[Byte], testLen: Long, labels: Array[Byte],
                     labelsLen: Long, out: PointerByReference): Int
   def mr_ingest_error(g: Pointer): String

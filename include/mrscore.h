@@ -301,6 +301,30 @@ int mr_explain(mr_handle* h, int model, const int32_t* user_idx, const int32_t* 
 int mr_song_audience(mr_handle* h, int model, double param, uint64_t seed, const int32_t* song_ids, int n, int k, int32_t* out_user,
                      double* out_score, int32_t* out_len);
 
+/* ---- filtered top-k: an allowed song set and per-user exclusions (DESIGN.md §4.11) -------------------------------------------------------
+ * The filter belongs to the handle's CURRENT test shard: an allowed song set A (allow_songs [n_allow], global ids in [0, S), any order,
+ * duplicates ignored; n_allow = -1: every song, 0: the empty set) and exclusion rows E_u (ex_rowptr [U + 1] with ex_rowptr[0] = 0,
+ * non-decreasing, one row per test user of the shard; ex_col ids in [0, S), strictly ascending within a row; ex_rowptr = NULL: none).
+ * The candidates of test user u are the songs of the handle's window that lie in A, that u has not listened to (MR:109) and that are not in
+ * E_u (an excluded listened song changes nothing).  A handle with a song window keeps the in-window part of A and E: ids outside it are no
+ * error, so every rank of a song-partitioned job sets the same global filter.  mr_set_topk_filter(h, NULL, -1, NULL, NULL) clears it;
+ * mr_set_test_users drops it.  MR_ERR_BAD_ARG names the first allowed id out of range or the first bad exclusion row; MR_ERR_STATE before
+ * mr_load and without test users; MR_ERR_OOM (stating the bytes) when the filter's device copy does not fit in the caller's reserve the
+ * batch plan leaves free.  The filter changes no other call: every unfiltered call gives what it gives without one. */
+int mr_set_topk_filter(mr_handle* h, const int32_t* allow_songs, int n_allow, const int64_t* ex_rowptr, const int32_t* ex_col);
+/* The filtered top-k of a model set (arguments, checks and outputs as mr_topk_multi): for every entry, each test user's unfiltered ranking
+ * (score descending, song id ascending) with every non-candidate removed, truncated to k.  Every listed score has the bits mr_topk and
+ * mr_score_users give the pair, AGG and STOCH under the global pair index of mr_set_test_users (a filter removes pairs from the output,
+ * it never renumbers the model).  out_len[u] = min(k, candidates of u), song -1 / score 0.0 past it.  MR_ERR_STATE without a filter.  A
+ * scoring call: the exclusions are written into the score panels as listened pairs (MR_T_TOPK), after which the lists come from the
+ * full-row select with the allowed-column bitmap, or, for an allowed set below 3 % of the window, from a select over the allowed
+ * columns only; mr_get_info values 28 / 29 count the rows (test users x entries) each path answered since mr_load. */
+int mr_topk_filtered(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k,
+                     int32_t* const* out_song, double* const* out_score, int32_t* const* out_len);
+/* The same with the lists kept in HBM as the result of a set call (mr_topk_multi_device, read with mr_topk_multi_ptrs); it replaces the
+ * last set result and leaves the single-model result untouched. */
+int mr_topk_filtered_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k);
+
 /* mAP@k of ranked lists against the hidden (label) half of the test users — north_star's "mAP@500".  The reference has no ranking and
  * no such metric (its evaluateModel is the threshold sweep above); this is the Million Song Dataset Challenge definition:
  * AP@k(u) = (sum_{i<=n} [r_i in L_u] * hits_i / i) / min(|L_u|, k), mean over the test users with at least one label row.
@@ -378,7 +402,8 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  mr_similar_songs rows since mr_load: answered by the short path, by the long path,
                                                                  mr_similar_users rows since mr_load: answered by the short path, by the long path,
                                                                  mr_explain count rows built since mr_load,
-                                                                 mr_song_audience since mr_load: query rows answered, column selects through the radix select] */
+                                                                 mr_song_audience since mr_load: query rows answered, column selects through the radix select,
+                                                                 mr_topk_filtered rows since mr_load: answered by the full-row path, by the candidate path] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

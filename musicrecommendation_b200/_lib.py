@@ -25,7 +25,8 @@ SYMBOLS = ["mr_create", "mr_destroy", "mr_last_error", "mr_load", "mr_set_test_u
            "mr_ingest_tsv", "mr_ingest_error", "mr_ingest_dims", "mr_ingest_get", "mr_ingest_free",
            "mr_eval_range", "mr_eval_counts", "mr_eval_finish", "mr_eval_cutoffs",
            "mr_topk_multi", "mr_topk_multi_device", "mr_topk_multi_ptrs", "mr_eval_range_multi", "mr_eval_counts_multi",
-           "mr_similar_songs", "mr_similar_users", "mr_explain", "mr_song_audience"]
+           "mr_similar_songs", "mr_similar_users", "mr_explain", "mr_song_audience",
+           "mr_set_topk_filter", "mr_topk_filtered", "mr_topk_filtered_device"]
 
 _lib = None
 
@@ -112,5 +113,8 @@ def load():
     lib.mr_similar_users.argtypes = [vp, vp, i32, i32, vp, vp, vp]
     lib.mr_explain.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp]
     lib.mr_song_audience.argtypes = [vp, i32, dbl, u64, vp, i32, i32, vp, vp, vp]
+    lib.mr_set_topk_filter.argtypes = [vp, vp, i32, vp, vp]
+    lib.mr_topk_filtered.argtypes = [vp, i32, vp, vp, vp, i32, vp, vp, vp]
+    lib.mr_topk_filtered_device.argtypes = [vp, i32, vp, vp, vp, i32]
     _lib = lib
     return lib

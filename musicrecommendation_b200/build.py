@@ -9,7 +9,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 SO = PKG / "libmrscore.so"
-SOURCES = ["mrscore.cu", "k1_count_gemm.cu", "k1_sparse_count.cu", "k2_aggregate.cu", "k3_topk.cu", "k4_itemspace.cu", "k5_evaluate.cu", "k6_ingest.cu", "k7_testlists.cu", "k8_similar.cu", "k9_audience.cu", "modelio.cu"]
+SOURCES = ["mrscore.cu", "k1_count_gemm.cu", "k1_sparse_count.cu", "k2_aggregate.cu", "k3_topk.cu", "k4_itemspace.cu", "k5_evaluate.cu", "k6_ingest.cu", "k7_testlists.cu", "k8_similar.cu", "k9_audience.cu", "k10_filter.cu", "modelio.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--fmad=false",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "-cudart", "static"]
 

@@ -182,7 +182,18 @@ int launch_agg_split(const BlendParams& bp, const long long* te_ptr, const int* 
 struct KeyCtx {
   int model; double rsu, alpha, oma;
   const long long* su; const long long* si; const double* rsd; const uint64_t* sel;
+  const uint32_t* allow;   // kAllow: allowed-column bitmap of a filtered top-k (DESIGN.md §4.11), bit c % 32 of word c / 32
 };
+
+// kAllow: a disallowed column reads as a listened pair (-1 in both panels), so every pass below sees fewer candidates and nothing else.
+// The 4 columns s .. s + 3 (s a multiple of 4) share one bitmap word.
+template <bool kAllow>
+__device__ __forceinline__ void drop_disallowed(const KeyCtx& c, int s, long long* a, long long* b) {
+  if (!kAllow) return;
+  const uint32_t w = __ldg(c.allow + (s >> 5)) >> (s & 31);
+#pragma unroll
+  for (int t = 0; t < 4; ++t) if (!((w >> t) & 1u)) { if (a) a[t] = -1; b[t] = -1; }
+}
 
 // L2 prefetches.  The select streams a row in dependent rounds (a thread has one or two 32-byte loads in flight, then computes), so a
 // round costs a full DRAM latency.  Short rows (a song partition: a few hundred KB per user) are pulled into L2 whole by a handful of
@@ -206,7 +217,7 @@ __device__ __forceinline__ void prefetch_row(const long long* row, int n_songs) 
 // thread of the CTA (so f may use warp collectives); valid is false for listened pairs and past the end of the row.
 // ubm_min: for the pure UBM model the score is monotone in the integer numerator, so the caller may pass the smallest numerator
 // worth looking at; rows entries below it are reported as valid with key 0 and cost no fp64 work at all.
-template <class F>
+template <bool kAllow, class F>
 __device__ __forceinline__ void scan_row(const KeyCtx& c, int n_songs, F&& f, int chunk_stride = 1, long long ubm_min = 0) {
   for (int base = 0; base < n_songs; base += 4 * kTopkThreads * chunk_stride) {
     const int s = base + 4 * static_cast<int>(threadIdx.x);
@@ -225,6 +236,7 @@ __device__ __forceinline__ void scan_row(const KeyCtx& c, int n_songs, F&& f, in
         for (int t = 0; t < 4; ++t) rd[t] = s + t < n_songs ? c.rsd[s + t] : 0.0;
       }
       if (c.model >= MODEL_AGG) selw = c.sel[s >> 6] >> (s & 63);
+      drop_disallowed<kAllow>(c, s, a, b);
     }
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
@@ -246,7 +258,7 @@ __device__ __forceinline__ uint32_t logbits_key(unsigned long long kb) { return 
 
 // Visit the row 4 songs per thread per step, two steps in flight: f(song of the first of 4, a[4], b[4], rsd[4], select word) with a = -1 /
 // b = -1 where the model does not use that panel; entries past the end of the row are reported as listened (-1).
-template <bool kInt, class F>
+template <bool kInt, bool kAllow, class F>
 __device__ __forceinline__ void visit_row(const KeyCtx& c, int n_songs, int chunk_stride, F&& f) {
   constexpr int kSteps = kInt ? 2 : 1;                          // steps in flight (the fp64 models already load three arrays per step)
   const int step = 4 * kTopkThreads * chunk_stride;
@@ -291,6 +303,7 @@ __device__ __forceinline__ void visit_row(const KeyCtx& c, int n_songs, int chun
 #pragma unroll
           for (int t = 0; t < 4; ++t) if (s + t >= n_songs) { a[h][t] = -1; b[h][t] = -1; }
         }
+        drop_disallowed<kAllow>(c, s, a[h], b[h]);
       }
     }
 #pragma unroll
@@ -313,6 +326,7 @@ __device__ __forceinline__ unsigned long long proxy_of(const KeyCtx& c, long lon
 // round-up fp32 product bounds the fp64 score from above — float_ru(Sint) * rsd_up[s] (rsd_up = rsd rounded up to fp32, product
 // rounded up) >= the exact product >= its fp64 rounding — and only songs whose bound reaches the threshold (rounded down to fp32)
 // are evaluated exactly.  12 bytes per song instead of 16, no fp64 work per song, and two steps of loads in flight per thread.
+template <bool kAllow>
 __device__ __forceinline__ void ibm_collect_pass(const KeyCtx& c, const float* __restrict__ rsd_up, int n_songs, unsigned long long thr,
                                                  unsigned long long* s_key, int* s_song, int* s_count) {
   const float t_f = __double2float_rd(__longlong_as_double(static_cast<long long>(thr)));
@@ -341,6 +355,7 @@ __device__ __forceinline__ void ibm_collect_pass(const KeyCtx& c, const float* _
 #pragma unroll
           for (int t = 0; t < 4; ++t) { if (s + t < n_songs) r[h][t] = __ldg(rsd_up + s + t); else b[h][t] = -1; }
         }
+        drop_disallowed<kAllow>(c, s, nullptr, b[h]);
       }
     }
 #pragma unroll
@@ -364,13 +379,13 @@ __device__ __forceinline__ void ibm_collect_pass(const KeyCtx& c, const float* _
 
 // Fast path for long rows; returns true when the candidate buffer holds a superset of the top `need` keys (s_count of them).
 // *scale_out = the linear-bin scale of the exact path (from the sampled maximum), so a rejected row continues there.
-template <bool kInt>
+template <bool kInt, bool kAllow>
 __device__ __forceinline__ bool topk_fast_path(const KeyCtx& c, int n_songs, int stride, int k, int need, unsigned long long* s_key, int* s_song,
                                                int* s_hist, unsigned long long* s_max, int* s_count, int* s_ctl, double* max_score_out, const float* __restrict__ rsd_up) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   // ---- A1: sampled maximum of the proxy
   unsigned long long mx = 0;
-  visit_row<kInt>(c, n_songs, stride, [&](int, const long long* a, const long long* b, const double* rd, uint64_t selw) {
+  visit_row<kInt, kAllow>(c, n_songs, stride, [&](int, const long long* a, const long long* b, const double* rd, uint64_t selw) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) { const unsigned long long p = proxy_of<kInt>(c, a[t], b[t], rd[t], (selw >> t) & 1ULL); mx = p > mx ? p : mx; }
   });
@@ -391,7 +406,7 @@ __device__ __forceinline__ bool topk_fast_path(const KeyCtx& c, int n_songs, int
     return static_cast<uint32_t>(d < 1 ? 1 : (d > kTopkBins - 1 ? kTopkBins - 1 : d));
   };
   // ---- A2: histogram over the same chunks
-  visit_row<kInt>(c, n_songs, stride, [&](int, const long long* a, const long long* b, const double* rd, uint64_t selw) {
+  visit_row<kInt, kAllow>(c, n_songs, stride, [&](int, const long long* a, const long long* b, const double* rd, uint64_t selw) {
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
       const unsigned long long p = proxy_of<kInt>(c, a[t], b[t], rd[t], (selw >> t) & 1ULL);
@@ -415,7 +430,7 @@ __device__ __forceinline__ bool topk_fast_path(const KeyCtx& c, int n_songs, int
   else thr = static_cast<unsigned long long>(lb_cut) << 46;
   // ---- B: one full pass, collect every song whose proxy is at or above the threshold
   if (!kInt && c.model == MODEL_IBM && rsd_up) {
-    ibm_collect_pass(c, rsd_up, n_songs, thr, s_key, s_song, s_count);
+    ibm_collect_pass<kAllow>(c, rsd_up, n_songs, thr, s_key, s_song, s_count);
     __syncthreads();
     return *s_count >= need && *s_count <= kTopkCap;
   }
@@ -423,7 +438,7 @@ __device__ __forceinline__ bool topk_fast_path(const KeyCtx& c, int n_songs, int
   // shuffles in the common no-candidate case; the order inside the buffer is irrelevant, it is sorted afterwards).
   // (the integer path keeps the raw numerators in the buffer and converts the few hundred survivors to fp64 after the pass)
   const long long thr_int = static_cast<long long>(thr);            // >= 1: a listened pair (-1) or a zero score never passes
-  visit_row<kInt>(c, n_songs, 1, [&](int s, const long long* a, const long long* b, const double* rd, uint64_t selw) {
+  visit_row<kInt, kAllow>(c, n_songs, 1, [&](int s, const long long* a, const long long* b, const double* rd, uint64_t selw) {
     unsigned long long p[4];
     int n_ok = 0;
 #pragma unroll
@@ -514,6 +529,7 @@ __device__ __noinline__ int trim_candidates(unsigned long long* s_key, int* s_so
   return *s_count;
 }
 
+template <bool kAllow>
 __global__ void __launch_bounds__(kTopkThreads, 2)
 topk_kernel(BlendParams bp, const long long* __restrict__ te_ptr, const long long* __restrict__ sint_u, const long long* __restrict__ sint_i, long long spitch,
             const uint64_t* __restrict__ sel, long long sel_pitch_words, int u0, int n_songs, const double* __restrict__ rsa,
@@ -535,26 +551,29 @@ topk_kernel(BlendParams bp, const long long* __restrict__ te_ptr, const long lon
   c.si = sint_i ? sint_i + static_cast<long long>(b) * spitch : nullptr;
   c.rsd = rsd;
   c.sel = sel ? sel + static_cast<long long>(b) * sel_pitch_words : nullptr;
+  c.allow = bp.allow;
   int* o_song = out_song + static_cast<long long>(u) * k;
   double* o_score = out_score + static_cast<long long>(u) * k;
 
   if (n_songs <= kShortRow) { prefetch_row(c.su, n_songs); prefetch_row(c.si, n_songs); }
   const int stride = n_songs > 16384 ? 8 : 1;   // the rows of a song partition (S / 8 = 48 k songs at MSD scale) take the sampled path too
-  const int n_valid = n_songs - static_cast<int>(bp.te_end[u] - te_ptr[u]);   // scored pairs of this user (MR:109)
+  // scored pairs of this user (MR:109).  Under a filter it over-counts the candidates: the fast path then only hands back (to the exact
+  // path) the rows with fewer than k candidates, whose collected keys cannot reach need
+  const int n_valid = n_songs - static_cast<int>(bp.te_end[u] - te_ptr[u]);
   int need = 0;
   bool collected = false;
   double max_score = 0.0;
   if (stride > 1) {
     need = min(k, n_valid);
     if (c.model == MODEL_UBM && bp.ubm_int_ok && c.rsu > 0.0)
-      collected = topk_fast_path<true>(c, n_songs, stride, k, need, s_key, s_song, s_hist, s_max, &s_count, s_ctl, &max_score, nullptr);
+      collected = topk_fast_path<true, kAllow>(c, n_songs, stride, k, need, s_key, s_song, s_hist, s_max, &s_count, s_ctl, &max_score, nullptr);
     else
-      collected = topk_fast_path<false>(c, n_songs, stride, k, need, s_key, s_song, s_hist, s_max, &s_count, s_ctl, &max_score, bp.rsd_up);
+      collected = topk_fast_path<false, kAllow>(c, n_songs, stride, k, need, s_key, s_song, s_hist, s_max, &s_count, s_ctl, &max_score, bp.rsd_up);
     __syncthreads();
   } else {
     // ---- short rows: exact maximum
     unsigned long long mx = 0;
-    scan_row(c, n_songs, [&](int, unsigned long long kb, bool ok) { if (ok && kb > mx) mx = kb; });
+    scan_row<kAllow>(c, n_songs, [&](int, unsigned long long kb, bool ok) { if (ok && kb > mx) mx = kb; });
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xffffffffu, mx, o); mx = other > mx ? other : mx; }
     if (lane == 0) s_max[warp] = mx;
@@ -569,7 +588,7 @@ topk_kernel(BlendParams bp, const long long* __restrict__ te_ptr, const long lon
     const int d = __double2int_rz(__dmul_rn(__longlong_as_double(static_cast<long long>(kb)), scale));
     return static_cast<uint32_t>(d > kTopkBins - 1 ? kTopkBins - 1 : d);
   };
-  auto scan = [&](auto&& f) { scan_row(c, n_songs, f); };
+  auto scan = [&](auto&& f) { scan_row<kAllow>(c, n_songs, f); };
   if (!collected) {
     if (tid == 0 && bp.stats) atomicAdd(bp.stats + (stride > 1 ? 0 : 1), 1u);   // rows the fast path handed back / short rows
     // ---- exact histogram over the whole row
@@ -612,8 +631,12 @@ int launch_topk(const BlendParams& bp, const long long* te_ptr, const long long*
                 int* out_song, double* out_score, int* out_len, cudaStream_t st) {
   if (n_users <= 0) return 0;
   if (k <= 0 || k > kTopkCap / 2) return -2;
-  topk_kernel<<<n_users, kTopkThreads, 0, st>>>(bp, te_ptr, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_songs, rsa, rsd, k,
-                                                out_song, out_score, out_len);
+  if (bp.allow)
+    topk_kernel<true><<<n_users, kTopkThreads, 0, st>>>(bp, te_ptr, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_songs, rsa, rsd, k,
+                                                      out_song, out_score, out_len);
+  else
+    topk_kernel<false><<<n_users, kTopkThreads, 0, st>>>(bp, te_ptr, sint_u, sint_i, spitch, sel, sel_pitch_words, u0, n_songs, rsa, rsd, k,
+                                                       out_song, out_score, out_len);
   return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 

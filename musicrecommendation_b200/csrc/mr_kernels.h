@@ -116,6 +116,7 @@ struct BlendParams {
   const long long* te_end;   // [U] end of each test row's scored columns: te_ptr + 1, or the in-window prefix ends (song window)
   int song_off;              // added to the ranked column ids: first song of the window (0 without one)
   unsigned int* stats;       // [3] or null: rows the fast path of the select handed to the exact path, short rows (exact path by design), degenerate rows (radix select)
+  const uint32_t* allow;     // filtered top-k, full-row path (DESIGN.md §4.11): bitmap of the allowed columns (bit c % 32 of word c / 32), or null
 };
 int launch_select_bits(const BlendParams& bp, const long long* te_ptr, const int* te_col, int u0, int n_users, int n_songs,
                        uint64_t* sel, long long sel_pitch_words, cudaStream_t st);
@@ -218,5 +219,11 @@ struct AudienceArgs {
   unsigned int* radix_rows;                          // columns that took the radix select, or null
 };
 int launch_audience(const AudienceArgs& a, int n_q, int u0, int nb, int k, cudaStream_t st);
+
+// ---- filtered top-k, candidate path (k10_filter.cu, DESIGN.md §4.11): per test user u0 + r the exact top-k of the masked panel rows r over
+// the ascending allowed columns cols[0 .. n_cols); ids are reported as column + bp.song_off; bp.stats[2] counts the rows through the radix select
+int launch_candidate_topk(const BlendParams& bp, const long long* sint_u, const long long* sint_i, long long spitch, const uint64_t* sel,
+                          long long sel_pitch_words, int u0, int n_users, const int* cols, int n_cols, const double* rsa, const double* rsd, int k,
+                          int* out_song, double* out_score, int* out_len, cudaStream_t st);
 
 }  // namespace mr

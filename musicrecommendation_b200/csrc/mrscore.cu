@@ -103,7 +103,7 @@ struct mr_handle {
   int U = 0; long long nnz_te = 0; bool have_test = false;
   // grow-only device buffers of the test shard, its results and the workspaces: steady-state mr_set_test_users / mr_topk calls do no cudaMalloc
   enum { SL_TE_PTR, SL_TE_COL, SL_TE_GROW, SL_RSA, SL_PAIR_BASE, SL_ROWS, SL_HU_PTR, SL_HU_ROW, SL_HU_SONG, SL_HU_Q, SL_TU_USER,
-         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_AUD_OUT, SL_AUD_Q, SL_N };
+         SL_TU_SONG, SL_TU_LPTR, SL_TU_PTR, SL_EX_PTR, SL_EX_SONG, SL_EX_G, SL_EX_GQ, SL_L_FLAG, SL_L_HEADPOS, SL_L_DEG, SL_L_LSUM, SL_L_TMP, SL_COPY_DESC, SL_SEG, SL_GRP_HDR, SL_GE_ROW, SL_GE_Q, SL_SPLIT_ROWS, SL_SINT_U, SL_SINT_I, SL_SEL, SL_GRAM_IDS, SL_DENSE, SL_OUT_PACK, SL_TE_END, SL_PRE_G, SL_PRE_GQ, SL_PRE_EXC, SL_EVAL_MM, SL_EVAL_COLMAP, SL_EVAL_CNT, SL_LAB_PTR, SL_LAB_COL, SL_AGG_SPLIT, SL_MULTI_OUT, SL_SIM_IDS, SL_SIM_EV, SL_SIM_Q, SL_SIM_OUT, SL_SIM_LIDS, SL_SIM_LOUT, SL_SIM_SQU, SL_GRAM_G, SL_GRAM_A, SL_HEAD_G16, SL_HEAD_GQ32, SL_AUD_OUT, SL_AUD_Q, SL_FLT_BITS, SL_FLT_COLS, SL_FLT_EX_PTR, SL_FLT_EX_COL, SL_N };
   void* slot_p[SL_N] = {}; size_t slot_cap[SL_N] = {};
   long long *d_te_ptr = nullptr, *d_pair_base = nullptr; int *d_te_col = nullptr, *d_te_grow = nullptr; double* d_rsa = nullptr;
   std::vector<long long> h_te_ptr; std::vector<int> h_te_col;
@@ -134,6 +134,12 @@ struct mr_handle {
   double *d_simu_sqt = nullptr, *d_simu_squ = nullptr; bool simu_squ_ok = false; long long simu_short_rows = 0, simu_long_rows = 0;
   long long explain_rows = 0;   // mr_explain: count rows built since mr_load
   long long audience_rows = 0;  // mr_song_audience: query rows answered since mr_load
+  // filtered top-k (mr_set_topk_filter, DESIGN.md §4.11): the in-window part of the current shard's filter, dropped by mr_set_test_users.
+  // flt_n_allow: allowed columns of the window (d_flt_cols, ascending; bitmap d_flt_bits), -1 = every column; flt_n_ex: in-window exclusion
+  // entries (rows d_flt_ex_ptr [U + 1] over columns d_flt_ex_col).  Rows answered by each path since mr_load.
+  bool flt_on = false; int flt_n_allow = -1; long long flt_n_ex = 0;
+  uint32_t* d_flt_bits = nullptr; int* d_flt_cols = nullptr; long long* d_flt_ex_ptr = nullptr; int* d_flt_ex_col = nullptr;
+  long long flt_full_rows = 0, flt_cand_rows = 0;
   // profiling
   cudaEvent_t ev[2] = {nullptr, nullptr}; double t_ms[MR_T_N] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 };
@@ -765,6 +771,10 @@ struct Run {
   bool reuse = false;                   // EVAL_COUNT: the panels hold this set's masked numerators (resident reuse): no scoring at all
   const int2* aud_q = nullptr;          // AUDIENCE: [aud_n] device (column, list row), ascending column; the running lists are set.out[0]
   int aud_n = 0;
+  // TOPK under a filter (DESIGN.md §4.11): the exclusion rows masked after the listened pairs (ex_ptr [U + 1], or null), and the candidate
+  // path over the allowed columns cand_cols [n_cand] instead of the full-row select (whose bitmap, if any, is in each entry's BlendParams)
+  const long long* ex_ptr = nullptr; const int* ex_col = nullptr;
+  bool candidate = false; const int* cand_cols = nullptr; int n_cand = 0;
   bool eval() const { return what == Consumer::EVAL_RANGE || what == Consumer::EVAL_COUNT; }
 };
 
@@ -783,6 +793,12 @@ int consume_slice(mr_handle* h, const Run& run, long long* su, long long* si, ui
       const BlendParams& bp = set.bp[e];
       const bool blend_sel = bp.model == MODEL_AGG || bp.model == MODEL_STOCH;
       if (blend_sel) MR_LAUNCH(h, launch_select_bits(bp, h->d_te_ptr, h->d_te_col, u0, n, h->n_cols, sel, h->sel_pitch, st));
+      if (run.candidate) {
+        MR_LAUNCH(h, launch_candidate_topk(bp, bp.model != MODEL_IBM ? su : nullptr, bp.model != MODEL_UBM ? si : nullptr, h->spitch,
+                                           blend_sel ? sel : nullptr, h->sel_pitch, u0, n, run.cand_cols, run.n_cand, h->d_rsa, h->d_rsd, run.k,
+                                           set.out[e].song, set.out[e].score, set.out[e].len, st));
+        continue;
+      }
       MR_LAUNCH(h, launch_topk(bp, h->d_te_ptr, bp.model != MODEL_IBM ? su : nullptr, bp.model != MODEL_UBM ? si : nullptr, h->spitch,
                                blend_sel ? sel : nullptr, h->sel_pitch, u0, n, h->n_cols, h->d_rsa, h->d_rsd, run.k, set.out[e].song,
                                set.out[e].score, set.out[e].len, st));
@@ -861,6 +877,7 @@ int item_slices(mr_handle* h, const Run& run, const Slicing& sl, int b0, int nb,
     long long* si = (sl.models & 2) ? pi + static_cast<long long>(s0) * h->spitch : nullptr;
     uint64_t* sel = sl.sel ? h->d_sel + static_cast<long long>(s0) * h->sel_pitch : nullptr;
     if (!run.reuse) MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, u0, sn, su, si, h->spitch, ts));
+    if (run.ex_ptr) MR_LAUNCH(h, launch_mask_listened(run.ex_ptr, run.ex_ptr + 1, run.ex_col, u0, sn, su, si, h->spitch, ts));
     if (const int rc = consume_slice(h, run, su, si, sel, u0, sn, ts)) return rc;
     if (run.topk_host) {
       MR_CUDA(h, cudaEventRecord(h->ev_slice, ts));
@@ -1012,6 +1029,7 @@ int run_batches(mr_handle* h, const Run& run) {
     {
       PhaseTimer t(h, run.eval() ? MR_T_OTHER : MR_T_TOPK);   // closed before audience_columns opens its own timer on the same events
       MR_LAUNCH(h, launch_mask_listened(h->d_te_ptr, h->d_te_end, h->d_te_col, b0, nb, su, si, h->spitch, h->stream));
+      if (run.ex_ptr) MR_LAUNCH(h, launch_mask_listened(run.ex_ptr, run.ex_ptr + 1, run.ex_col, b0, nb, su, si, h->spitch, h->stream));
       rc = run.what == Consumer::DENSE ? dense_out(h, run.set.bp[0].model, su ? su : si, *run.dense, b0, nb)
                                        : consume_slice(h, run, su, si, h->d_sel, b0, nb, h->stream);
       if (rc) return rc;
@@ -1335,7 +1353,7 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
   MR_CUDA(h, cudaSetDevice(h->device));
   MR_CUDA(h, cudaStreamSynchronize(h->stream));
   lap("check_csr + sync");
-  h->have_test = false; h->have_topk = false; h->out_k = 0; h->multi_n = 0; ++h->gen;
+  h->have_test = false; h->have_topk = false; h->out_k = 0; h->multi_n = 0; h->flt_on = false; ++h->gen;
   const int U = n_test; const long long nnz = te_rowptr[U];
   h->U = U; h->nnz_te = nnz;
   h->deg_test.assign(deg_test, deg_test + U); h->simu_squ_ok = false;
@@ -2485,12 +2503,32 @@ int mr_topk(mr_handle* h, int model, double param, uint64_t seed, int k, int32_t
   return topk_impl(h, model, param, seed, k, &ho);
 }
 
-int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k) {
+}  // extern "C"
+
+namespace {
+
+// Fraction of the window's columns below which a filtered top-k ranks the allowed columns (candidate path) instead of streaming the rows
+// with the allowed-column bitmap (full-row path): on the MSD shape the candidate path wins at 1 % and loses from 5 % on, for UBM, IBM and
+// AGG (DESIGN.md §4.11).  MRSCORE_FILTER_PATH=full|candidate forces a path (developer aid for timing both at one size).
+constexpr double kCandidateFrac = 0.03;
+
+// A model set's top-k lists into the SL_MULTI_OUT blocks (mr_topk_multi_device), optionally under the handle's filter.
+int topk_set(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k, bool filtered) {
   int rc = require_test(h);
   if (rc) return rc;
   if (k < 1 || k > 1024) return fail(h, MR_ERR_BAD_ARG, "k must be in [1,1024], got %d", k);
   Run run{ModelSet(), Consumer::TOPK, k};
   if ((rc = make_set(h, n_models, models, params, seeds, "getTopK", true, &run.set))) return rc;
+  if (filtered) {
+    if (!h->flt_on) return fail(h, MR_ERR_STATE, "no top-k filter is set on this shard (mr_set_topk_filter)");
+    if (h->flt_n_ex > 0) { run.ex_ptr = h->d_flt_ex_ptr; run.ex_col = h->d_flt_ex_col; }
+    const char* force = getenv("MRSCORE_FILTER_PATH");
+    run.candidate = h->flt_n_allow >= 0 && h->flt_n_allow < kCandidateFrac * h->n_cols;
+    if (force && h->flt_n_allow >= 0) run.candidate = strcmp(force, "candidate") == 0 || (run.candidate && strcmp(force, "full") != 0);
+    run.cand_cols = h->d_flt_cols; run.n_cand = std::max(h->flt_n_allow, 0);
+    if (!run.candidate && h->flt_n_allow >= 0)
+      for (int e = 0; e < run.set.n; ++e) run.set.bp[e].allow = h->d_flt_bits;
+  }
   // one block per entry in a grow-only slot of its own: the single-model result (mr_topk_fetch, mr_map_at_k) stays
   const TopkBlock blk(h->U, k);
   const size_t need = blk.bytes * static_cast<size_t>(n_models);
@@ -2510,7 +2548,34 @@ int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const do
   for (int e = 0; e < n_models; ++e) run.set.out[e] = blk.at(base + blk.bytes * e);
   if ((rc = run_batches(h, run))) return rc;
   h->multi_n = n_models; h->multi_k = k;
+  if (filtered) (run.candidate ? h->flt_cand_rows : h->flt_full_rows) += static_cast<long long>(h->U) * n_models;
   return MR_OK;
+}
+
+// The set's lists copied to the caller's host arrays (mr_topk_multi, mr_topk_filtered).
+int topk_set_host(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k, int32_t* const* out_song,
+                  double* const* out_score, int32_t* const* out_len, bool filtered) {
+  if (!h) return MR_ERR_STATE;
+  if (n_models < 1 || n_models > kMaxSet) return fail(h, MR_ERR_BAD_ARG, "getTopK: n_models = %d outside 1..%d", n_models, kMaxSet);
+  if (!out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null output");
+  for (int e = 0; e < n_models; ++e)
+    if (!out_song[e] || !out_score[e] || !out_len[e]) return fail(h, MR_ERR_BAD_ARG, "entry %d: null output", e);
+  int rc = topk_set(h, n_models, models, params, seeds, k, filtered);
+  if (rc) return rc;
+  const TopkBlock blk(h->U, k);
+  char* const base = static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]);
+  for (int e = 0; e < n_models; ++e)
+    if ((rc = copy_topk(h, TopkOut{out_song[e], out_score[e], out_len[e]}, blk.at(base + blk.bytes * e), k, 0, h->U, h->stream))) return rc;
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int mr_topk_multi_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k) {
+  return topk_set(h, n_models, models, params, seeds, k, false);
 }
 
 int mr_topk_multi_ptrs(mr_handle* h, int i, int k, void** song, void** score, void** len) {
@@ -2528,19 +2593,84 @@ int mr_topk_multi_ptrs(mr_handle* h, int i, int k, void** song, void** score, vo
 
 int mr_topk_multi(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k, int32_t* const* out_song,
                   double* const* out_score, int32_t* const* out_len) {
-  if (!h) return MR_ERR_STATE;
-  if (n_models < 1 || n_models > kMaxSet) return fail(h, MR_ERR_BAD_ARG, "getTopK: n_models = %d outside 1..%d", n_models, kMaxSet);
-  if (!out_song || !out_score || !out_len) return fail(h, MR_ERR_BAD_ARG, "null output");
-  for (int e = 0; e < n_models; ++e)
-    if (!out_song[e] || !out_score[e] || !out_len[e]) return fail(h, MR_ERR_BAD_ARG, "entry %d: null output", e);
-  int rc = mr_topk_multi_device(h, n_models, models, params, seeds, k);
+  return topk_set_host(h, n_models, models, params, seeds, k, out_song, out_score, out_len, false);
+}
+
+int mr_set_topk_filter(mr_handle* h, const int32_t* allow_songs, int n_allow, const int64_t* ex_rowptr, const int32_t* ex_col) {
+  int rc = require_test(h);
   if (rc) return rc;
-  const TopkBlock blk(h->U, k);
-  char* const base = static_cast<char*>(h->slot_p[mr_handle::SL_MULTI_OUT]);
-  for (int e = 0; e < n_models; ++e)
-    if ((rc = copy_topk(h, TopkOut{out_song[e], out_score[e], out_len[e]}, blk.at(base + blk.bytes * e), k, 0, h->U, h->stream))) return rc;
-  MR_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->flt_on = false;
+  if (!allow_songs && n_allow == -1 && !ex_rowptr) return MR_OK;   // cleared
+  if (n_allow < -1 || (n_allow > 0 && !allow_songs)) return fail(h, MR_ERR_BAD_ARG, "allowed songs: n_allow = %d with %s list", n_allow, allow_songs ? "a" : "a null");
+  for (int i = 0; i < n_allow; ++i)
+    if (allow_songs[i] < 0 || allow_songs[i] >= h->S) return fail(h, MR_ERR_BAD_ARG, "allowed song %d (entry %d) out of range [0,%d)", allow_songs[i], i, h->S);
+  if (ex_rowptr && (rc = check_csr(h, "exclusions", h->U, h->S, ex_rowptr, ex_col))) return rc;
+  // the in-window part, in columns: ids in [win_lo, win_hi) become id - win_lo (window order = id order); the others are dropped
+  const int lo = h->win_lo, hi = h->win_lo + h->n_cols, n_words = (h->n_cols + 31) / 32;
+  std::vector<uint32_t> bits;
+  std::vector<int> cols;
+  if (n_allow >= 0) {
+    bits.assign(static_cast<size_t>(n_words), 0u);
+    for (int i = 0; i < n_allow; ++i)
+      if (allow_songs[i] >= lo && allow_songs[i] < hi) bits[(allow_songs[i] - lo) >> 5] |= 1u << ((allow_songs[i] - lo) & 31);
+    for (int c = 0; c < h->n_cols; ++c)
+      if ((bits[c >> 5] >> (c & 31)) & 1u) cols.push_back(c);
+  }
+  std::vector<long long> ex_ptr;
+  std::vector<int> ex_c;
+  long long n_ex = 0;
+  if (ex_rowptr) {
+    const int U = h->U;
+    std::vector<long long> b(U), e(U);   // the in-window entries of a row are one ascending run
+    parallel_rows(U, [&](int u_lo, int u_hi) {
+      for (int u = u_lo; u < u_hi; ++u) {
+        const int32_t *rb = ex_col + ex_rowptr[u], *re = ex_col + ex_rowptr[u + 1];
+        b[u] = std::lower_bound(rb, re, lo) - ex_col; e[u] = std::lower_bound(rb, re, hi) - ex_col;
+      }
+    });
+    ex_ptr.assign(static_cast<size_t>(U) + 1, 0);
+    for (int u = 0; u < U; ++u) ex_ptr[u + 1] = ex_ptr[u] + (e[u] - b[u]);
+    n_ex = ex_ptr[U];
+    ex_c.resize(static_cast<size_t>(n_ex));
+    parallel_rows(U, [&](int u_lo, int u_hi) {
+      for (int u = u_lo; u < u_hi; ++u)
+        for (long long i = b[u], o = ex_ptr[u]; i < e[u]; ++i, ++o) ex_c[o] = ex_col[i] - lo;
+    });
+  }
+  // the device copies must fit inside the caller's reserve that the batch plan leaves free, and be free now; the plan is not changed for it
+  const int slots[4] = {mr_handle::SL_FLT_BITS, mr_handle::SL_FLT_COLS, mr_handle::SL_FLT_EX_PTR, mr_handle::SL_FLT_EX_COL};
+  const size_t bytes[4] = {bits.size() * 4, cols.size() * 4, n_ex > 0 ? ex_ptr.size() * 8 : 0, ex_c.size() * 4};
+  size_t need = 0, held = 0; bool grows = false;
+  for (int i = 0; i < 4; ++i) { need += bytes[i]; held += h->slot_cap[slots[i]]; grows = grows || h->slot_cap[slots[i]] < bytes[i]; }
+  size_t avail = kCallerReserve;
+  if (grows) {
+    size_t free_b = 0, total_b = 0;
+    MR_CUDA(h, cudaMemGetInfo(&free_b, &total_b));
+    avail = std::min(avail, free_b + held);
+  }
+  if (need > avail)
+    return fail(h, MR_ERR_OOM, "mr_set_topk_filter: the filter needs %zu bytes of device memory, more than the %zu bytes of the caller's reserve "
+                "that are free", need, avail);
+  if ((rc = slot_upload(h, mr_handle::SL_FLT_BITS, &h->d_flt_bits, bits.data(), bits.size())) ||
+      (rc = slot_upload(h, mr_handle::SL_FLT_COLS, &h->d_flt_cols, cols.data(), cols.size())))
+    return rc;
+  if (n_ex > 0 && ((rc = slot_upload(h, mr_handle::SL_FLT_EX_PTR, &h->d_flt_ex_ptr, ex_ptr.data(), ex_ptr.size())) ||
+                   (rc = slot_upload(h, mr_handle::SL_FLT_EX_COL, &h->d_flt_ex_col, ex_c.data(), ex_c.size()))))
+    return rc;
+  MR_CUDA(h, cudaStreamSynchronize(h->stream));   // the pageable host arrays must outlive their uploads
+  h->flt_n_allow = n_allow >= 0 ? static_cast<int>(cols.size()) : -1;
+  h->flt_n_ex = n_ex;
+  h->flt_on = true;
   return MR_OK;
+}
+
+int mr_topk_filtered_device(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k) {
+  return topk_set(h, n_models, models, params, seeds, k, true);
+}
+
+int mr_topk_filtered(mr_handle* h, int n_models, const int* models, const double* params, const uint64_t* seeds, int k, int32_t* const* out_song,
+                     double* const* out_score, int32_t* const* out_len) {
+  return topk_set_host(h, n_models, models, params, seeds, k, out_song, out_score, out_len, true);
 }
 
 int mr_song_audience(mr_handle* h, int model, double param, uint64_t seed, const int32_t* song_ids, int n, int k, int32_t* out_user,
@@ -2604,12 +2734,12 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[27] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[29] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
                          h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
                          h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows, h->explain_rows,
-                         h->audience_rows, st[3]};
-  for (int i = 0; i < n && i < 27; ++i) out[i] = v[i];
+                         h->audience_rows, st[3], h->flt_full_rows, h->flt_cand_rows};
+  for (int i = 0; i < n && i < 29; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

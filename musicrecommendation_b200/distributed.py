@@ -185,6 +185,47 @@ def song_audience(mr, model: int, k: int, param: float = 0.5, seed: int = 0, son
     return (ids[r0:r1],) + tuple(t.cpu().numpy() for t in out)
 
 
+def shard_exclusions(ex_ptr, ex_col, u0: int, u1: int):
+    """Rows [u0, u1) of an exclusion CSR over the whole test set, as the CSR of that test-user shard (rowptr from 0)."""
+    ex_ptr = np.asarray(ex_ptr, np.int64)
+    return ex_ptr[u0:u1 + 1] - ex_ptr[u0], np.asarray(ex_col, np.int32)[ex_ptr[u0]:ex_ptr[u1]]
+
+
+def topk_filtered(mr, specs, k: int, allowed=None, exclude=None, group=None):
+    """getTopKMultiFiltered of a job whose ranks each hold one part of the model (DESIGN.md §4.11).  Every rank passes the same global
+    filter: `allowed` song ids (None = every song) and `exclude`, a CSR (rowptr, col) over ALL test users (None = no exclusions).
+      song partitioning (the handle has a song window, and sees every test user): each rank ranks its window under the filter (the handle
+        keeps the in-window part), exchange_song_partitions hands rank r every window's lists of ITS users shard_range(U, rank, world), and
+        mr_topk_merge joins them on the GPU: exact, the windows are disjoint.
+      test-user sharding (mr.ds is the shard [u0, u1) of shard_test_users, set with its pair base): each rank filters with its rows of
+        `exclude` and ranks its shard.
+    Either way returns, per entry, (song, score, len) as numpy arrays of this rank's users, rows shard_range(U, rank, world)."""
+    import torch
+    import torch.distributed as dist
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    lo, hi = mr.song_window
+    windowed = (lo, hi) != (0, mr.ds.S)
+    if exclude is not None and not windowed:
+        u0, u1 = mr.ds.meta.get("shard", (0, mr.ds.U))
+        exclude = shard_exclusions(exclude[0], exclude[1], u0, u1)
+    mr.setTopKFilter(allowed, exclude)
+    lists = mr.getTopKMultiFiltered(specs, k)
+    if not windowed:
+        return lists
+    dev = _collective_device(group)
+    out = []
+    for song, score, ln in lists:
+        ps, pv, pl = exchange_song_partitions(torch.from_numpy(song).to(dev), torch.from_numpy(score).to(dev), torch.from_numpy(ln).to(dev),
+                                              mr.ds.U, world, rank, group)
+        ps, pv, pl = ps.cuda(), pv.cuda(), pl.cuda()
+        res = (torch.empty_like(ps[0]), torch.empty_like(pv[0]), torch.empty_like(pl[0]))
+        torch.cuda.synchronize()      # the parts are written on torch's streams, the join runs on the library stream
+        mr.mergeTopK(ps, pv, pl, *res)
+        mr.sync()
+        out.append(tuple(t.cpu().numpy() for t in res))
+    return out
+
+
 def _collective_device(group):
     import torch
     import torch.distributed as dist

@@ -401,6 +401,43 @@ class MusicRecommender:
         models, params, seeds = model_set_arrays(specs)
         self._check(self._lib.mr_topk_multi_device(self._h, len(models), _p(models), _p(params), _p(seeds), k))
 
+    def setTopKFilter(self, allowed=None, exclude=None):
+        """The filter of getTopKFiltered for the current shard (mr_set_topk_filter, DESIGN.md §4.11): `allowed` global song ids (any order,
+        duplicates ignored; None = every song), `exclude` a CSR (rowptr [U + 1], col) of songs not to recommend per test user of the shard,
+        ids ascending within a row (exclusions_from_topk turns a previous page into one).  set_test_users drops the filter."""
+        a = None if allowed is None else np.ascontiguousarray(allowed, np.int32).reshape(-1)
+        ep = ec = None
+        if exclude is not None:
+            ep = np.ascontiguousarray(exclude[0], np.int64).reshape(-1)
+            ec = np.ascontiguousarray(exclude[1], np.int32).reshape(-1)
+            if len(ep) != self.ds.U + 1:
+                raise ValueError(f"exclusion rowptr has {len(ep)} entries, the shard has {self.ds.U} test users")
+        self._check(self._lib.mr_set_topk_filter(self._h, None if a is None else _p(a), -1 if a is None else len(a),
+                                                 None if ep is None else _p(ep), None if ec is None else _p(ec)))
+
+    def clearTopKFilter(self):
+        self._check(self._lib.mr_set_topk_filter(self._h, None, -1, None, None))
+
+    def getTopKMultiFiltered(self, specs, k: int = 500):
+        """getTopKMulti under the filter of setTopKFilter (mr_topk_filtered): per entry each user's ranking without the songs the filter
+        removes, truncated to k, one (song [U,k] int32, score [U,k] f64, len [U]) per entry."""
+        models, params, seeds = model_set_arrays(specs)
+        U, n = self.ds.U, len(models)
+        kk = max(int(k), 0)                 # a k outside 1..1024 is refused by the library (MR_ERR_BAD_ARG), not by numpy
+        out = [(np.empty((U, kk), np.int32), np.empty((U, kk), np.float64), np.empty(U, np.int32)) for _ in range(n)]
+        tab = lambda j: (C.c_void_p * n)(*[o[j].ctypes.data for o in out])      # noqa: E731
+        self._check(self._lib.mr_topk_filtered(self._h, n, _p(models), _p(params), _p(seeds), k, tab(0), tab(1), tab(2)))
+        return out
+
+    def getTopKFiltered(self, model: int = _lib.MR_UBM, k: int = 500, param: float = 0.5, seed: int = 0):
+        """getTopK under the filter of setTopKFilter: (song [U,k] int32, score [U,k] f64, len [U])."""
+        return self.getTopKMultiFiltered([(model, param, seed)], k)[0]
+
+    def topk_filtered_device(self, specs, k: int = 500):
+        """mr_topk_filtered_device: the filtered lists stay in HBM as the last set result (topk_multi_device_tensors reads them)."""
+        models, params, seeds = model_set_arrays(specs)
+        self._check(self._lib.mr_topk_filtered_device(self._h, len(models), _p(models), _p(params), _p(seeds), k))
+
     def topk_multi_device_tensors(self, i: int, k: int):
         """torch views (no copy) of entry i of the last set top-k on the device: (song int32 [U,k], score f64 [U,k], len int32 [U])."""
         ps, pv, pl = C.c_void_p(), C.c_void_p(), C.c_void_p()
@@ -541,13 +578,13 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 27)()
-        self._lib.mr_get_info(self._h, v, 27)
+        v = (C.c_int64 * 29)()
+        self._lib.mr_get_info(self._h, v, 29)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
                          "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows",
                          "similar_user_short_rows", "similar_user_long_rows", "explain_rows", "audience_rows",
-                         "audience_radix_selects"], list(v)))
+                         "audience_radix_selects", "filter_full_rows", "filter_candidate_rows"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
@@ -871,6 +908,42 @@ def song_audience_host(scores: np.ndarray, songs, k: int):
         user[r, :ln[r]] = order[r, :ln[r]]
         score[r, :ln[r]] = cols[order[r, :ln[r]], r]
     return user, score, ln
+
+
+def exclusions_from_topk(song, ln):
+    """Exclusion rows (rowptr [U + 1] int64, col int32) holding each user's listed songs of a previous top-k (song [U, k], len [U]), for
+    setTopKFilter: the next page is the top-k with this page excluded."""
+    song = np.asarray(song)
+    ln = np.asarray(ln, np.int64).reshape(-1)
+    ptr = np.zeros(len(ln) + 1, np.int64)
+    np.cumsum(ln, out=ptr[1:])
+    keep = np.arange(song.shape[1])[None, :] < ln[:, None]
+    rows = np.sort(np.where(keep, song, np.iinfo(np.int32).max), axis=1)   # each row's listed songs first, ascending
+    return ptr, np.ascontiguousarray(rows[keep], np.int32)
+
+
+def topk_filtered_host(scores: np.ndarray, allowed, ex_ptr, ex_col, k: int):
+    """numpy mirror of mr_topk_filtered over a dense model [U, S] (NaN at listened pairs, as mr_score_dense and the oracle give it):
+    per user the non-NaN entries of the allowed songs (None = all) outside the user's exclusion row (ex_ptr None = none), ordered by
+    (-score, song), the first k.  Returns (song [U, k] int32, score [U, k] f64, len [U] int32), song -1 / score 0.0 past len."""
+    sc = np.array(scores, np.float64)
+    U, S = sc.shape
+    if allowed is not None:
+        keep = np.zeros(S, bool)
+        keep[np.asarray(allowed, np.int64)] = True
+        sc[:, ~keep] = np.nan
+    if ex_ptr is not None:
+        ex_ptr = np.asarray(ex_ptr, np.int64)
+        rows = np.repeat(np.arange(U), np.diff(ex_ptr))
+        sc[rows, np.asarray(ex_col, np.int64)[:ex_ptr[-1]]] = np.nan
+    order = np.argsort(-sc, axis=1, kind="stable")[:, :k]             # NaN sorts last; equal scores keep song order
+    ln = np.minimum(k, (~np.isnan(sc)).sum(axis=1)).astype(np.int32)
+    song = np.full((U, k), -1, np.int32)
+    score = np.zeros((U, k), np.float64)
+    for u in range(U):
+        song[u, :ln[u]] = order[u, :ln[u]]
+        score[u, :ln[u]] = sc[u, order[u, :ln[u]]]
+    return song, score, ln
 
 
 def explain_host(ds: Dataset, model: int, users, songs, m: int) -> Explanation:

@@ -403,7 +403,12 @@ int mr_get_info(mr_handle* h, int64_t* out, int n);          /* [engine, kernel 
                                                                  mr_similar_users rows since mr_load: answered by the short path, by the long path,
                                                                  mr_explain count rows built since mr_load,
                                                                  mr_song_audience since mr_load: query rows answered, column selects through the radix select,
-                                                                 mr_topk_filtered rows since mr_load: answered by the full-row path, by the candidate path] */
+                                                                 mr_topk_filtered rows since mr_load: answered by the full-row path, by the candidate path,
+                                                                 carry events of the u32 weighted-count panel in the last scoring call (sparse
+                                                                 user-space IBM; 0 after any other call), staged head rows (the rest are built
+                                                                 in place), whether the last head-row build used the packed 64-bit accumulator,
+                                                                 byte planes of the weights in the last tensor-engine head-row build (0 = none),
+                                                                 whether the top-k select may rank the UBM integers of the current shard] */
 void* mr_stream(mr_handle* h);                               /* cudaStream_t every call's work is ordered on: what a caller enqueues on it
                                                                  after a call returns runs behind that call's results (internally the
                                                                  batches of a top-k call also use a second stream, joined back before

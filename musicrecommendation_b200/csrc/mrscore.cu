@@ -95,6 +95,7 @@ struct mr_handle {
   int* d_head_song = nullptr; long long* d_head_lst_ptr = nullptr;
   uint16_t* d_g16 = nullptr; uint32_t* d_gq32 = nullptr;   // packed head rows, slots SL_HEAD_G16 / SL_HEAD_GQ32 (kept across mr_invalidate_prepared)
   int n_head_staged = 0;               // rows [0, n_head_staged) are built in a 64-bit staging area and packed; the rest directly in place
+  bool head_packed = false; int head_planes = 0;   // last head-row build: packed 64-bit accumulator; byte planes of the tensor engine (0 = scatter)
   long long opt_head_min_deg = 0;      // mr_set_option(MR_OPT_HEAD_MIN_DEG): 0 = default rule
   long long* d_ex_ptr = nullptr; int* d_ex_song = nullptr; uint32_t* d_ex_g = nullptr; unsigned long long* d_ex_gq = nullptr; long long n_ex = 0;
   long long *d_hu_ptr = nullptr; int *d_hu_row = nullptr, *d_hu_song = nullptr; uint32_t* d_hu_q = nullptr;
@@ -112,7 +113,9 @@ struct mr_handle {
   // workspaces
   uint8_t *d_Ate = nullptr, *d_Aj = nullptr; uint16_t* d_ct = nullptr; long long *d_sint_u = nullptr, *d_sint_i = nullptr;
   uint32_t* d_wi = nullptr;             // IBM user-space weighted counts u32[T][128] (sparse engine)
-  unsigned int* d_carry_count = nullptr; uint2* d_carry_events = nullptr; unsigned int carry_cap = 1u << 20; unsigned int* h_carry_seen = nullptr;
+  unsigned int* d_carry_count = nullptr; uint2* d_carry_events = nullptr; unsigned int carry_cap = 1u << 20;   // MRSCORE_CARRY_CAP
+  unsigned int* h_carry_seen = nullptr; int carry_seen_cap = 0;   // pinned, one event count per user batch of the current call
+  long long carry_events = 0;           // carry events of the last scoring call (sparse user-space IBM; 0 for any other call)
   uint64_t* d_sel = nullptr; long long sel_pitch = 0; int32_t* d_g = nullptr;   // d_g / d_Aj: the Gram workspace, slots SL_GRAM_G / SL_GRAM_A
   double* d_dense = nullptr;
   // results
@@ -425,6 +428,7 @@ int start_head_rows(mr_handle* h, cudaStream_t st) {
     chunk = std::max<long long>(4, std::min<long long>((64LL << 20) / (h->spitch * (packed ? 8 : 12)), 4096));
     if (const char* e = getenv("MRSCORE_PRECOMPUTE_CHUNK")) chunk = std::max(1LL, atoll(e));
   }
+  h->head_packed = packed; h->head_planes = tensor ? n_planes : 0;
   // The staging rows and the exception list live in grow-only slots of the handle: a rebuild (mr_invalidate_prepared + mr_prepare, i.e.
   // every step of a job that counts the model build) does no cudaMalloc / cudaFree — next to 100+ GB of live allocations those cost
   // tens to hundreds of milliseconds, more than the kernels of a song partition's precompute.  Only the tensor engine's dense operands
@@ -909,7 +913,7 @@ int user_panels(mr_handle* h, int b0, int nb, bool need_ubm, bool need_ibm) {
     MR_CUDA(h, cudaMemsetAsync(h->d_sint_i, 0, static_cast<size_t>(kUserBatch) * h->spitch * sizeof(long long), h->stream));
     MR_LAUNCH(h, launch_aggregate_w32(items, h->d_csc_idx, h->d_wi, h->T, h->d_sint_i, h->spitch, h->num_sms, h->stream));
     MR_LAUNCH(h, launch_carry_fixup(carry, h->d_tr_ptr, h->d_tr_col, h->d_sint_i, h->spitch, h->stream));
-    MR_CUDA(h, cudaMemcpyAsync(h->h_carry_seen + (b0 / kUserBatch) % 4096, h->d_carry_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
+    MR_CUDA(h, cudaMemcpyAsync(h->h_carry_seen + b0 / kUserBatch, h->d_carry_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, h->stream));
     return MR_OK;
   }
   const int bi = b0 / kUserBatch;
@@ -957,6 +961,21 @@ int run_batches(mr_handle* h, const Run& run) {
   if (!run.reuse) ++h->gen;
   if (item_space && (rc = ensure_head_rows(h))) return rc;
   const int batch = item_space ? h->batch_rows : kUserBatch;
+  // the sparse user-space IBM panel: each batch's carry-event count lands in its own zeroed slot of this call (user_panels), so the
+  // check below sees exactly the batches of this call.  The sync first: a call that failed mid-shard may have left copies in flight.
+  const bool carries = need_ibm && !item_space && h->engine == MR_ENGINE_SPARSE;
+  const int n_user_batches = (h->U + kUserBatch - 1) / kUserBatch;
+  h->carry_events = 0;
+  if (carries) {
+    MR_CUDA(h, cudaStreamSynchronize(h->stream));
+    if (h->carry_seen_cap < n_user_batches) {
+      if (h->h_carry_seen) cudaFreeHost(h->h_carry_seen);
+      h->h_carry_seen = nullptr; h->carry_seen_cap = 0;
+      MR_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&h->h_carry_seen), static_cast<size_t>(n_user_batches) * sizeof(unsigned int)));
+      h->carry_seen_cap = n_user_batches;
+    }
+    memset(h->h_carry_seen, 0, static_cast<size_t>(n_user_batches) * sizeof(unsigned int));
+  }
   // Batch pipeline (item-space top-k of a pure model over >= 2 batches; not under MR_PROFILE, whose phase timers serialise the
   // stream): the head pass of batch b + 1 is issued on the library stream while the tail scatter, mask and select of batch b run on
   // slice_stream.  A pure model leaves the other model's Sint panel idle, so consecutive batches alternate between the two panels: no
@@ -1037,13 +1056,14 @@ int run_batches(mr_handle* h, const Run& run) {
     if (run.what == Consumer::AUDIENCE && (rc = audience_columns(h, run, su, si, b0, nb, h->stream))) return rc;
   }
   join.armed = false;
-  if (need_ibm && !item_space && h->engine == MR_ENGINE_SPARSE) {
-    // the carry list of the u32 weighted-count panel must not have overflowed (it never does on real data: an event needs
-    // more than ~64 songs shared between one test user and one train user)
+  if (carries) {
+    // the carry list of the u32 weighted-count panel must not have overflowed in any batch (it never does on real data: an event
+    // needs more than ~64 songs shared between one test user and one train user)
     MR_CUDA(h, cudaStreamSynchronize(h->stream));
-    for (int i = 0; i < 4096; ++i)
-      if (h->h_carry_seen[i] > h->carry_cap)
-        return fail(h, MR_ERR_OOM, "IBM weighted-count carry list overflowed (%u events > capacity %u)", h->h_carry_seen[i], h->carry_cap);
+    unsigned int worst = 0;
+    for (int i = 0; i < n_user_batches; ++i) { h->carry_events += h->h_carry_seen[i]; worst = std::max(worst, h->h_carry_seen[i]); }
+    if (worst > h->carry_cap)
+      return fail(h, MR_ERR_OOM, "IBM weighted-count carry list overflowed (%u events > capacity %u)", worst, h->carry_cap);
   }
   return MR_OK;
 }
@@ -1280,10 +1300,10 @@ int mr_load(mr_handle* h, int n_train, int n_test, int n_songs, const int64_t* t
   if ((rc = dev_alloc(h, &h->d_ct, static_cast<size_t>(T) * kUserBatch, h->allocs))) return rc;
   if (h->engine == MR_ENGINE_SPARSE) {
     if ((rc = dev_alloc(h, &h->d_wi, static_cast<size_t>(T) * kUserBatch, h->allocs))) return rc;
+    // test aid: a small carry list lets a test reach its overflow error, which real data cannot (it needs ~10^6 wrapping pairs)
+    if (const char* e = getenv("MRSCORE_CARRY_CAP")) h->carry_cap = static_cast<unsigned int>(std::max(1LL, std::min<long long>(atoll(e), 1LL << 20)));
     if ((rc = dev_alloc(h, &h->d_carry_count, 1, h->allocs))) return rc;
     if ((rc = dev_alloc(h, &h->d_carry_events, h->carry_cap, h->allocs))) return rc;
-    MR_CUDA(h, cudaMallocHost(reinterpret_cast<void**>(&h->h_carry_seen), 4096 * sizeof(unsigned int)));
-    memset(h->h_carry_seen, 0, 4096 * sizeof(unsigned int));
   }
   if (const char* e = getenv("MRSCORE_ITEM_BATCH")) h->item_batch_cap = std::max(128, atoi(e));   // developer override of MR_OPT_ITEM_BATCH
   if (const char* e = getenv("MRSCORE_HEAD_WORDS_U")) { const int w = atoi(e); if (w == 1 || w == 2 || w == 4) h->head_words_u = w; }
@@ -1451,6 +1471,8 @@ int mr_set_test_users(mr_handle* h, int n_test, const int64_t* te_rowptr, const 
       }
       h->ubm_int_ok = worst < (1ULL << 52);
     }
+    // test aid: the fp64 UBM select, which data reaches only past ~2^28 train listens, on any shard (it must give the same lists)
+    if (getenv("MRSCORE_UBM_FP64_SELECT")) h->ubm_int_ok = false;
     MR_CUDA(h, cudaStreamSynchronize(h->stream));
     h->n_head_entries = hu_ptr[U]; h->n_tail_entries = h->h_tu_ptr[U];
     h->h_tu_lptr.resize(static_cast<size_t>(h->n_tail_entries) + 1);
@@ -2734,12 +2756,13 @@ int mr_get_info(mr_handle* h, int64_t* out, int n) {
   if (!h || !out) return MR_ERR_BAD_ARG;
   unsigned int st[4] = {0, 0, 0, 0};
   if (n > 16 && h->d_topk_stats && cudaMemcpy(st, h->d_topk_stats, sizeof st, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(h, MR_ERR_CUDA, "mr_get_info: reading the select counters failed");
-  const int64_t v[29] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
+  const int64_t v[34] = {h->engine, h->launches, static_cast<int64_t>(h->dense_bytes), h->n_items, h->num_sms, static_cast<int64_t>(h->dev_bytes), h->space, h->n_head,
                          h->n_head_entries, h->n_tail_entries, h->n_ex, h->batch_rows, h->n_groups,
                          h->h_split_ptr.empty() ? 0 : h->h_split_ptr.back(), h->n_cols, h->win_lo, st[0], st[1], st[2], h->passes,
                          h->sim_short_rows, h->sim_long_rows, h->simu_short_rows, h->simu_long_rows, h->explain_rows,
-                         h->audience_rows, st[3], h->flt_full_rows, h->flt_cand_rows};
-  for (int i = 0; i < n && i < 29; ++i) out[i] = v[i];
+                         h->audience_rows, st[3], h->flt_full_rows, h->flt_cand_rows,
+                         h->carry_events, h->n_head_staged, h->head_packed ? 1 : 0, h->head_planes, h->ubm_int_ok ? 1 : 0};
+  for (int i = 0; i < n && i < 34; ++i) out[i] = v[i];
   return MR_OK;
 }
 int mr_prepare_async(mr_handle* h) {

@@ -578,13 +578,14 @@ class MusicRecommender:
         return dict(zip(_lib.TIMING_NAMES, list(t)))
 
     def info(self) -> dict:
-        v = (C.c_int64 * 29)()
-        self._lib.mr_get_info(self._h, v, 29)
+        v = (C.c_int64 * 34)()
+        self._lib.mr_get_info(self._h, v, 34)
         return dict(zip(["engine", "launches", "dense_bytes", "n_items", "num_sms", "device_bytes", "space", "n_head", "head_entries",
                          "tail_entries", "head_exceptions", "batch_rows", "head_groups", "split_users", "n_cols", "win_lo", "topk_fast_rejects",
                          "topk_short_rows", "topk_degenerate_rows", "scoring_passes", "similar_short_rows", "similar_long_rows",
                          "similar_user_short_rows", "similar_user_long_rows", "explain_rows", "audience_rows",
-                         "audience_radix_selects", "filter_full_rows", "filter_candidate_rows"], list(v)))
+                         "audience_radix_selects", "filter_full_rows", "filter_candidate_rows", "carry_events", "head_staged_rows",
+                         "head_packed", "head_planes", "ubm_int_ok"], list(v)))
 
     # ------------------------------------------------------------------ model file I/O (MR:489-512)
     def writeModelOnFile(self, model: Model, outputFileName: str = "") -> int:
